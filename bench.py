@@ -2,6 +2,7 @@
 """bench.py -- throughput of the 2-FGNN siamese forward (BASELINE.json metric) on N B200s.
 
     python bench.py --gpus 1 --steps 5 --warmup 3            # this implementation
+    python bench.py --gpus 1 --steps 5 --warmup 3 --dump-outputs DIR   # ... and write the last step's outputs as .npy
     python bench.py --impl reference --steps 3 --warmup 1    # CPU reference arm (oracle port)
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
@@ -35,6 +36,27 @@ WORKLOADS = {
 }
 DEFAULT_WORKLOAD = "cfg3_regular_n500_c64_b64_fwd"
 METRIC = "graph-pairs/sec 2-FGNN siamese fwd at n=500"
+DUMP_LIMIT_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, arrays, seed=0):
+    """Write each array as out_dir/<name>.npy: float64 stays float64, everything else is stored as float32.  Arrays
+    are indexed by pair along their first axis (0-d arrays are scalars).  When all of them together exceed 64 MB,
+    every array keeps the same fixed, seeded sample of pairs, whose indices are written as pair_index.npy."""
+    import numpy as np
+    host = {k: v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else np.asarray(v) for k, v in arrays.items()}
+    host = {k: v if v.dtype == np.float64 else v.astype(np.float32) for k, v in host.items()}
+    budget = DUMP_LIMIT_BYTES - 4096 * (len(host) + 1)        # room for the .npy headers, pair_index.npy's included
+    if sum(v.nbytes for v in host.values()) > budget:
+        pairs = max(v.shape[0] for v in host.values() if v.ndim)
+        per_pair = sum(v.nbytes // v.shape[0] for v in host.values() if v.ndim) + 8      # + its float64 pair_index entry
+        scalars = sum(v.nbytes for v in host.values() if not v.ndim)
+        keep = np.sort(np.random.default_rng(seed).choice(pairs, (budget - scalars) // per_pair, replace=False))
+        host = {k: v[keep] if v.ndim else v for k, v in host.items()}
+        host["pair_index"] = keep.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 def load_peaks():
@@ -375,7 +397,15 @@ def main():
     ap.add_argument("--train", action="store_true",
                     help="time the data-parallel TRAINING step (fwd + bwd + flat all-reduce + Adam) in --precision "
                          "instead of the forward; secondary line for configs[1]/[4], not the headline")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed on rank 0 as DIR/<name>.npy "
+                         "(forward: per-pair CE sums, correct rows and both embedding batches; --train: loss, correct, "
+                         "rows); inputs and weights are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of this implementation's timed step (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     cfg = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
@@ -431,6 +461,8 @@ def main():
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
             dist.destroy_process_group()
+        if rank == 0 and args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"loss": float(loss), "correct": float(ok), "rows": float(rows)})
         if rank == 0:
             print(json.dumps({"metric": "graph-pairs/sec 2-FGNN siamese training step (fwd+bwd+allreduce+Adam)",
                               "value": pairs * world * args.steps / (ms / 1e3), "unit": "pairs/s", "n_gpus": world,
@@ -456,7 +488,9 @@ def main():
         return _ops.head_fused(e1, e2, None, args.precision)[:2]
 
     def step_resident():
-        return head(model.embed({"input": x1_d}), model.embed({"input": x2_d}))
+        e1 = model.embed({"input": x1_d})
+        e2 = model.embed({"input": x2_d})
+        return (*head(e1, e2), e1, e2)
 
     copy_stream = torch.cuda.Stream(device=dev)
     x2_ready = torch.cuda.Event()
@@ -506,11 +540,13 @@ def main():
         torch.cuda.synchronize(dev)
 
     def timed(fn, steps):
+        """(ms over `steps` calls of fn, what the last call returned); no step's result is held across the next step."""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(steps):
+        for _ in range(steps - 1):
             fn()
+        last = fn()
         e1.record()
         torch.cuda.synchronize(dev)
         ms = e0.elapsed_time(e1)
@@ -518,7 +554,7 @@ def main():
             t = torch.tensor([ms], device=dev, dtype=torch.float64)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms
+        return ms, last
 
     with torch.no_grad():
         for _ in range(args.warmup):
@@ -531,9 +567,13 @@ def main():
         lib.fgnn_profile_reset()
         lib.fgnn_profile_enable(1)
         lib.fgnn_reset_launch_count()
-        ms = timed(step_resident, args.steps)
+        ms, last = timed(step_resident, args.steps)
         launches = int(lib.fgnn_launch_count())
         lib.fgnn_profile_enable(0)
+        outputs = None
+        if args.dump_outputs:
+            outputs = {k: t.cpu() for k, t in zip(("ce_sum", "correct", "emb1", "emb2"), last)}
+        del last
         import ctypes as C
         kinds = {}
         for kind, name in ((0, "tc_mlp_kernel"), (1, "tc_matmul_kernel"), (2, "plane_stats16_kernel")):
@@ -545,7 +585,7 @@ def main():
             step_e2e()
         torch.cuda.synchronize(dev)
         pipe["primed"] = False                       # the timed run starts with an exposed copy of its own first input
-        ms_e2e = timed(step_e2e, args.steps)
+        ms_e2e, _ = timed(step_e2e, args.steps)
         if rank == 0:
             sampler.stop_flag.set()
             sampler.join(timeout=3)
@@ -573,14 +613,14 @@ def main():
                 res_h.copy_(torch.stack((loss, ok.float())), non_blocking=False)
 
             step_e2e_adj()
-            ms_adj = timed(step_e2e_adj, args.steps)
+            ms_adj, _ = timed(step_e2e_adj, args.steps)
             e2e_adj = {"value": pairs * world * args.steps / (ms_adj / 1e3), "unit": "pairs/s",
                        "h2d_bytes_per_step": int(a1_h.numel() * 2), "d2h_bytes_per_step": 8,
                        "what": "model.loss_and_accuracy_from_adjacency(adj1, adj2): uint8 adjacency from pinned host memory, "
                                "features built on the device (fgnn_embed_fwd_adjacency_u8); H2D copies not pipelined"}
         step_e2e_scores()
         k_sc = max(2, args.steps // 4)
-        ms_sc = timed(step_e2e_scores, k_sc)
+        ms_sc, _ = timed(step_e2e_scores, k_sc)
         e2e_scores = {"value": pairs * world * k_sc / (ms_sc / 1e3), "unit": "pairs/s", "steps": k_sc,
                       "d2h_bytes_per_step": int(scores_h.numel() * 4),
                       "what": "model.forward(x1, x2) with the (B,N,N) fp32 scores copied back to pinned host memory; "
@@ -597,6 +637,8 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
 
     from oracle import fgnn_oracle as O
     total_pairs = pairs * world * args.steps

@@ -231,16 +231,12 @@ def test_ragged_constant_n_vertices_default(prec):
                     in_features=c, out_features=c, depth_of_mlp=depth)          # flag left at its default (True)
     model = pkg.models.Siamese_Node_Exp(2, node_emb)
     model.load_state_dict(state_dict_of(z))
-    model = model.to(DEV).set_precision("fp32")
+    model = model.to(DEV).set_precision(prec)          # fp16: the width-16 fixture runs zero-padded to 32 channels
     graphs = [O.adjacency_to_features(torch.from_numpy(z[f"W1/{i}"].astype(np.float32))) for i in range(len(sizes))]
     x = mt.from_list(graphs, dims=(1, 2)).to(DEV)
     with torch.no_grad():
-        if prec == "fp32":
-            e = model.embed({"input": x}).tensor.rename(None).cpu()
-            tol = 1e-4
-        else:
-            # width 16 is below the tensor-core path's widths: check the flag through the conv-chain entry point
-            pytest.skip("width-16 fixture: the 16-bit constant-n case is covered by test_tc_mlp_constant_n")
+        e = model.embed({"input": x}).tensor.rename(None).cpu()
+    tol = 1e-4 if prec == "fp32" else EMB_TOL[prec]
     for i, n in enumerate(sizes):
         assert rel_fro(e[i, :, :n], z["masked_cstn_emb1"][i, :, :n]) < tol
         assert float(e[i, :, n:].abs().sum()) == 0
@@ -497,18 +493,18 @@ def test_tc_embedder_other_widths_run_zero_padded(widths):
     assert abs(loss_a - float(loss_b)) < 1e-4 * max(1.0, abs(loss_a)) and int(rows_b) == sum(sizes)
 
 
-def test_bench_line_carries_the_contract_keys():
+def test_bench_line_carries_the_contract_keys(tmp_path):
     """bench.py (our arm) on the smallest workload: ONE JSON line with the contract's keys -- roofline of the dominant kernel
     (measured live with CUDA events), clocks sampled during the timed region, e2e from pinned host buffers with its byte
-    counts, the count of our kernel launches."""
+    counts, the count of our kernel launches -- and, with --dump-outputs, the last timed step's outputs as .npy files."""
     import json
     import os
     import subprocess
     import sys as _sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     out = subprocess.run([_sys.executable, os.path.join(root, "bench.py"), "--steps", "3", "--warmup", "3", "--no-secondary",
-                          "--no-cpu-baseline", "--workload", "cfg1_er_n50_c32_b32_fwd"], capture_output=True, text=True,
-                         timeout=600, cwd=root)
+                          "--no-cpu-baseline", "--workload", "cfg1_er_n50_c32_b32_fwd", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600, cwd=root)
     assert out.returncode == 0, out.stderr[-2000:]
     lines = [l for l in out.stdout.splitlines() if l.startswith("{")]
     assert len(lines) == 1
@@ -522,3 +518,10 @@ def test_bench_line_carries_the_contract_keys():
     e = d["e2e"]
     assert e["value"] > 0 and e["h2d_bytes_per_step"] == 2 * 32 * 2 * 50 * 50 * 4 and e["d2h_bytes_per_step"] == 8
     assert "sm_mhz" in d["clocks"] and "reasons" in d["clocks"]
+    dumped = {k: np.load(tmp_path / f"{k}.npy") for k in ("ce_sum", "correct", "emb1", "emb2")}
+    assert sorted(os.listdir(tmp_path)) == sorted(f"{k}.npy" for k in dumped)
+    assert all(v.dtype == np.float32 and np.isfinite(v).all() for v in dumped.values())
+    assert dumped["ce_sum"].shape == dumped["correct"].shape == (32,) and dumped["emb1"].shape == dumped["emb2"].shape == (32, 32, 50)
+    # the per-pair loss and accuracy are those of the dumped embeddings (the head is deterministic)
+    ce, correct, _ = _ops.head_fused(torch.from_numpy(dumped["emb1"]).to(DEV), torch.from_numpy(dumped["emb2"]).to(DEV), None, "fp16")
+    assert rel_fro(ce.cpu(), dumped["ce_sum"]) < 1e-6 and np.array_equal(correct.cpu().numpy(), dumped["correct"])

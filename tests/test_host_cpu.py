@@ -168,6 +168,31 @@ def test_lightning_checkpoint_loads_through_get_siamese_model_test(tmp_path):
                        sd["node_embedder.ne_bm_block1_mlp1.convs.0.weight"])
 
 
+def test_bench_dump_outputs_samples_the_same_pairs_under_the_limit(tmp_path, monkeypatch):
+    """bench.dump_outputs: float64 stays float64, the rest is stored as float32; above the size limit every per-pair array
+    keeps the same seeded sample of pairs (identical from call to call), listed in pair_index.npy."""
+    import bench
+    gen = torch.Generator().manual_seed(1)
+    arrays = {"ce_sum": torch.rand(40, generator=gen), "correct": torch.arange(40, dtype=torch.int32),
+              "emb1": torch.rand((40, 8, 200), generator=gen), "loss": torch.tensor(0.5, dtype=torch.float64)}
+    bench.dump_outputs(str(tmp_path / "all"), arrays)
+    assert sorted(os.listdir(tmp_path / "all")) == ["ce_sum.npy", "correct.npy", "emb1.npy", "loss.npy"]
+    assert np.array_equal(np.load(tmp_path / "all" / "emb1.npy"), arrays["emb1"].numpy())
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 200_000)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == sorted(os.listdir(tmp_path / "b")) and "pair_index.npy" in names
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in names) <= 200_000
+    a = {f[:-4]: np.load(tmp_path / "a" / f) for f in names}
+    assert all(np.array_equal(v, np.load(tmp_path / "b" / f"{k}.npy")) for k, v in a.items())
+    idx = a["pair_index"].astype(np.int64)
+    assert 0 < len(idx) < 40 and np.all(np.diff(idx) > 0) and a["pair_index"].dtype == np.float64
+    assert a["correct"].dtype == np.float32 and np.array_equal(a["correct"], idx)
+    assert np.array_equal(a["emb1"], arrays["emb1"].numpy()[idx]) and np.array_equal(a["ce_sum"], arrays["ce_sum"].numpy()[idx])
+    assert a["loss"].dtype == np.float64 and float(a["loss"]) == 0.5
+
+
 def test_bench_reference_arm_prints_the_contract_line():
     """`bench.py --impl reference` (the CPU arm the driver runs beside ours) on the smallest workload: ONE JSON line with the
     contract's keys, `impl: reference`, an e2e object without copies, and a cpu_baseline that says which implementation was
