@@ -86,14 +86,13 @@ _SIGNATURES = {
     "fgnn_head_workspace_bytes": (_sz, [_i32, _i32]),
     "fgnn_head_fwd": (C.c_int, [_i32, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp, _sz, _vp]),
     "fgnn_embed_workspace_bytes": (_sz, [C.POINTER(EmbedParams), _i32, _i32, _i32]),
-    "fgnn_embed_fwd": (C.c_int, [C.POINTER(EmbedParams), _i32, _vp, _vp, _i32, _i32, _vp, _vp, _vp, _sz, _vp]),
+    "fgnn_embed_fwd": (C.c_int, [C.POINTER(EmbedParams), _i32, _vp, _vp, _i32, _i32, _vp, _vp, _sz, _vp]),
     "fgnn_embed_fwd_adjacency_u8": (C.c_int, [C.POINTER(EmbedParams), _i32, _vp, _vp, _i32, _i32, _vp, _vp, _sz, _vp]),
     "fgnn_embed_train_workspace_bytes": (_sz, [C.POINTER(EmbedParams), _i32, _i32, _i32]),
     "fgnn_embed_fwd_train": (C.c_int, [C.POINTER(EmbedParams), _i32, _vp, _vp, _i32, _i32, _vp, _vp, _sz, _vp]),
     "fgnn_embed_bwd": (C.c_int, [C.POINTER(EmbedParams), C.POINTER(EmbedGrads), _i32, _vp, _i32, _i32, _i32, _vp, _vp, _sz, _vp]),
     "fgnn_adam_step_f32": (C.c_int, [_vp, _vp, _vp, _vp, C.c_int64, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float,
                                      _i32, _vp, _vp, _vp]),
-    "fgnn_debug_dump_timing": (None, []),
     "fgnn_profile_enable": (None, [C.c_int]),
     "fgnn_profile_reset": (None, []),
     "fgnn_profile_read": (C.c_int, [_i32, C.POINTER(C.c_double), C.POINTER(C.c_int64)]),

@@ -6,7 +6,7 @@ stream.  Inputs must be CUDA float32 tensors; anything else raises (no CPU fallb
 from __future__ import annotations
 
 import ctypes as C
-from typing import List, Optional, Sequence, Tuple
+from typing import Optional, Sequence, Tuple
 
 import torch
 
@@ -342,7 +342,7 @@ def features_from_adjacency(adj: torch.Tensor, n_dev: Optional[torch.Tensor] = N
 
 
 def embed_fwd(params: L.EmbedParams, precision: int, x: torch.Tensor, c_out: int,
-              n_dev: Optional[torch.Tensor], n_host: Optional[List[int]]) -> torch.Tensor:
+              n_dev: Optional[torch.Tensor]) -> torch.Tensor:
     """Fused node_embedding forward: x (G,c_in,N,N) -> (G,C,N)."""
     lib = L.get_lib()
     x = L.require_cuda_f32(x, "input")
@@ -354,12 +354,8 @@ def embed_fwd(params: L.EmbedParams, precision: int, x: torch.Tensor, c_out: int
     if nbytes == 0:
         raise L.FgnnError("fgnn_embed_workspace_bytes returned 0: " + lib.fgnn_last_error().decode())
     ws = L.workspace(x.device, nbytes)
-    nh = None
-    if n_host is not None:
-        nh = (C.c_int32 * G)(*n_host)
-    L.check(lib.fgnn_embed_fwd(C.byref(params), precision, L.ptr(x), L.ptr(emb), G, N, _npg(n_dev),
-                               C.cast(nh, C.c_void_p) if nh is not None else None, L.ptr(ws), ws.numel(),
-                               L.stream_ptr(x.device)), "fgnn_embed_fwd")
+    L.check(lib.fgnn_embed_fwd(C.byref(params), precision, L.ptr(x), L.ptr(emb), G, N, _npg(n_dev), L.ptr(ws),
+                               ws.numel(), L.stream_ptr(x.device)), "fgnn_embed_fwd")
     return emb
 
 

@@ -260,19 +260,15 @@ size_t fgnn_embed_workspace_bytes(const fgnn_embed_params* p, int32_t precision,
 }
 
 int fgnn_embed_fwd(const fgnn_embed_params* p, int32_t precision, const float* x, float* emb,
-                   int32_t G, int32_t N, const int32_t* n_per_graph,
-                   const int32_t* n_per_graph_host, void* workspace, size_t workspace_bytes,
+                   int32_t G, int32_t N, const int32_t* n_per_graph, void* workspace, size_t workspace_bytes,
                    void* stream) {
   if (int e = check_embed(p, G, N)) return e;
   FGNN_CHECK_ARG(x && emb && workspace, "null pointer");
-  FGNN_CHECK_ARG((n_per_graph == nullptr) == (n_per_graph_host == nullptr),
-                 "n_per_graph and n_per_graph_host must both be given or both be NULL");
   cudaStream_t st = (cudaStream_t)stream;
   if (precision == FGNN_FP32)
     return f32_embed_fwd(*p, x, emb, G, N, n_per_graph, workspace, workspace_bytes, st);
   if (precision == FGNN_BF16 || precision == FGNN_FP16)
-    return tc::embed_fwd(*p, precision, x, emb, G, N, n_per_graph, n_per_graph_host, workspace,
-                         workspace_bytes, st);
+    return tc::embed_fwd(*p, precision, x, emb, G, N, n_per_graph, workspace, workspace_bytes, st);
   return fail(FGNN_ERR_INVALID, "unknown precision %d", precision);
 }
 
@@ -337,8 +333,6 @@ int fgnn_debug_tc_mlp(int32_t precision, const fgnn_mlp_params* p, const float* 
   FGNN_CHECK_ARG(p != nullptr, "null params");
   return tc::debug_mlp(precision, *p, x, y, G, N, n_per_graph, workspace, workspace_bytes, (cudaStream_t)stream);
 }
-
-void fgnn_debug_dump_timing(void) { tc::dump_timing(); }
 
 void fgnn_profile_enable(int on) {
   std::lock_guard<std::mutex> lk(prof::g_mu);

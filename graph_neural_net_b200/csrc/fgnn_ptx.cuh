@@ -25,10 +25,6 @@ __device__ __forceinline__ void fence_barrier_init() {
 __device__ __forceinline__ void fence_proxy_async_smem() {
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
 }
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes)
-               : "memory");
-}
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
@@ -45,35 +41,6 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
 }
 // Bounded wait: a protocol bug must surface as a CUDA error, never as a hung GPU box.  The slow path is
 // kept out of line so that every wait site costs a handful of instructions.
-#ifdef FGNN_DEBUG_WAIT
-// Bring-up aid: a wait that exceeds ~10 ms is RECORDED (block, thread, barrier address, parity) and abandoned, so
-// that the kernel runs to completion and the host can print who was stuck on what (fgnn_debug_dump_timing()).
-__device__ unsigned int g_wait_dbg[4 + 128 * 4];
-__device__ __noinline__ void mbar_wait_slow(uint32_t bar_addr, uint32_t parity) {
-  const long long t0 = clock64();
-  uint32_t ok = 0;
-  while (!ok) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(bar_addr), "r"(parity)
-        : "memory");
-    if (!ok && clock64() - t0 > 20000000LL) {
-      if (threadIdx.x % 32 != 0) return;
-      const unsigned int i = atomicAdd(&g_wait_dbg[0], 1u);
-      if (i < 128) {
-        g_wait_dbg[4 + 4 * i] = blockIdx.x;
-        g_wait_dbg[5 + 4 * i] = threadIdx.x;
-        g_wait_dbg[6 + 4 * i] = bar_addr;
-        g_wait_dbg[7 + 4 * i] = parity;
-      }
-      return;
-    }
-  }
-}
-#else
 __device__ __noinline__ void mbar_wait_slow(uint32_t bar_addr, uint32_t parity) {
   // The loop is three instructions: a quarter of all issue slots of the conv-chain kernel used to go to polling
   // (try_wait + clock read + compare per spin, ~10 waiting warps per SM, and the waiting control warps have the
@@ -101,7 +68,6 @@ __device__ __noinline__ void mbar_wait_slow(uint32_t bar_addr, uint32_t parity) 
     }
   }
 }
-#endif
 // (A suspend-time hint on try_wait -- NANOSLEEP.SYNCS instead of polling -- was measured 3-5% slower end to end,
 // for the control roles as well: every hand-off in the conv-chain kernel is latency-critical.)
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
@@ -111,13 +77,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
 // ---- TMA ------------------------------------------------------------------------------------
 __device__ __forceinline__ void prefetch_tensormap(const CUtensorMap* m) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(m) : "memory");
-}
-__device__ __forceinline__ void tma_load_3d(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0,
-                                            int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(smem_u32(smem_dst)), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
 }
 
 __device__ __forceinline__ void tma_store_3d(const CUtensorMap* map, const void* smem_src, int c0, int c1, int c2) {
@@ -147,10 +106,6 @@ __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence:
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-
-// register hand-over between warp groups (all four warps of an aligned group of four execute the same instruction)
-template <int N> __device__ __forceinline__ void setmaxnreg_inc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(N)); }
-template <int N> __device__ __forceinline__ void setmaxnreg_dec() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(N)); }
 
 // ---- tcgen05: descriptors ---------------------------------------------------------------------
 // Shared-memory matrix descriptor, 128-byte swizzle.  Fields (bits): start>>4 [0,14), LBO>>4 [16,30),
@@ -194,17 +149,8 @@ __device__ __forceinline__ void mma_ss(uint32_t d_tmem, uint64_t a_desc, uint64_
       ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
-// D[tmem] (+)= A[tmem] * B[smem desc]           (A: 128 lanes x K 16-bit values packed 2 per column)
-__device__ __forceinline__ void mma_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t idesc,
-                                       uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "r"(a_tmem), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// Same two MMAs with the 64-bit descriptors passed as (lo, hi) register pairs: the issuing thread is a
-// single lane running dependent scalar code, so descriptor updates are kept to one 32-bit add.
+// mma_ss with the 64-bit descriptors passed as (lo, hi) register pairs: the issuing thread is a single lane
+// running dependent scalar code, so descriptor updates are kept to one 32-bit add.
 __device__ __forceinline__ void mma_ss2(uint32_t d_tmem, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi,
                                         uint32_t idesc, uint32_t accumulate) {
   asm volatile(
@@ -214,6 +160,7 @@ __device__ __forceinline__ void mma_ss2(uint32_t d_tmem, uint32_t a_lo, uint32_t
       ::"r"(d_tmem), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// D[tmem] (+)= A[tmem] * B[smem desc]   (A: 128 lanes x K 16-bit values packed 2 per column; B descriptor as (lo, hi))
 __device__ __forceinline__ void mma_ts2(uint32_t d_tmem, uint32_t a_tmem, uint32_t b_lo, uint32_t b_hi, uint32_t idesc,
                                         uint32_t accumulate) {
   asm volatile(
@@ -253,33 +200,6 @@ __device__ __forceinline__ void tma_load_3d_e(void* smem_dst, const CUtensorMap*
       ::"r"(smem_u32(smem_dst)), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
       : "memory");
 }
-// ---- thread-block clusters ------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {   // every thread of every CTA of the cluster
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// TMA load delivered to the same shared-memory offset (and signalling the mbarrier at the same offset) of every CTA in
-// `cta_mask`
-__device__ __forceinline__ void tma_load_3d_mc_e(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2,
-                                                 uint16_t cta_mask) {
-  asm volatile(
-      "{\n\t.reg .pred P;\n\telect.sync _|P, 0xffffffff;\n\t"
-      "@P cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4, %5}], [%2], %6;\n\t}"
-      ::"r"(smem_u32(smem_dst)), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "h"(cta_mask)
-      : "memory");
-}
-// tcgen05.commit arriving on the mbarrier at the same offset in every CTA of `cta_mask`
-__device__ __forceinline__ void mma_commit_mc_e(uint64_t* bar, uint16_t cta_mask) {
-  asm volatile(
-      "{\n\t.reg .pred P;\n\telect.sync _|P, 0xffffffff;\n\t"
-      "@P tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;\n\t}"
-      ::"r"(smem_u32(bar)), "h"(cta_mask)
-      : "memory");
-}
 // 1-D bulk copy global -> shared (size a multiple of 16 bytes), completing on an mbarrier like a TMA load
 __device__ __forceinline__ void bulk_load_1d_e(void* smem_dst, const void* gsrc, uint32_t bytes, uint64_t* bar) {
   asm volatile(
@@ -296,16 +216,6 @@ __device__ __forceinline__ void mma_ss2_e(uint32_t d_tmem, uint32_t a_lo, uint32
       "elect.sync _|P, 0xffffffff;\n\t"
       "@P tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %5, p;\n\t}"
       ::"r"(d_tmem), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void mma_ts2_e(uint32_t d_tmem, uint32_t a_tmem, uint32_t b_lo, uint32_t b_hi,
-                                          uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p, P;\n\t.reg .b64 db;\n\tsetp.ne.b32 p, %5, 0;\n\t"
-      "mov.b64 db, {%2, %3};\n\t"
-      "elect.sync _|P, 0xffffffff;\n\t"
-      "@P tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], db, %4, p;\n\t}"
-      ::"r"(d_tmem), "r"(a_tmem), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
       : "memory");
 }
 __device__ __forceinline__ void mma_commit_e(uint64_t* bar) {
@@ -365,28 +275,8 @@ __device__ __forceinline__ void tmem_ld_16x256b_x4(uint32_t taddr, uint32_t (&r)
       : "r"(taddr)
       : "memory");
 }
-// 16 lanes x 128 bit per step (4 columns): thread t stores r[2k] to lane t/4 and r[2k+1] to lane t/4 + 8, column
-// 4k + t%4 -- the packed-pair image of the 16x256b load fragment (columns 8k + 2(t%4), +1 -> one 16-bit pair).
-__device__ __forceinline__ void tmem_st_16x128b_x8(uint32_t taddr, const uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.16x128b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};"
-      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]),
-        "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
-      : "memory");
-}
-__device__ __forceinline__ void tmem_st_16x128b_x4(uint32_t taddr, const uint32_t (&r)[8]) {
-  asm volatile("tcgen05.st.sync.aligned.16x128b.x4.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};"
-               ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7])
-               : "memory");
-}
-// four transposed 8x8 b16 matrices: matrix i takes register r_i; thread t holds elements (col t/4, rows 2(t%4), +1)
-// in the (low, high) halves of r_i; row r of matrix i (16 bytes) goes to the address supplied by thread 8i + r
-__device__ __forceinline__ void stmatrix_x4_trans(uint32_t saddr, uint32_t r0, uint32_t r1, uint32_t r2, uint32_t r3) {
-  asm volatile("stmatrix.sync.aligned.m8n8.x4.trans.shared.b16 [%0], {%1, %2, %3, %4};"
-               ::"r"(saddr), "r"(r0), "r"(r1), "r"(r2), "r"(r3)
-               : "memory");
-}
-// two transposed 8x8 b16 matrices: row r of matrix i goes to the address supplied by thread 8i + r (threads 0-15)
+// two transposed 8x8 b16 matrices: matrix i takes register r_i; thread t holds elements (col t/4, rows 2(t%4), +1)
+// in the (low, high) halves of r_i; row r of matrix i (16 bytes) goes to the address supplied by thread 8i + r (threads 0-15)
 __device__ __forceinline__ void stmatrix_x2_trans(uint32_t saddr, uint32_t r0, uint32_t r1) {
   asm volatile("stmatrix.sync.aligned.m8n8.x2.trans.shared.b16 [%0], {%1, %2};" ::"r"(saddr), "r"(r0), "r"(r1) : "memory");
 }
@@ -422,37 +312,17 @@ __device__ __forceinline__ uint32_t tmem_ld1(uint32_t taddr) {
   asm volatile("tcgen05.ld.sync.aligned.32x32b.x1.b32 {%0}, [%1];" : "=r"(r) : "r"(taddr) : "memory");
   return r;
 }
-__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
-      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};"
-      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]),
-        "r"(r[8]), "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
-      : "memory");
-}
 
 // ---- 16-bit element helpers ----------------------------------------------------------------------
-// 16-byte load from a SHARED-space address.  A `const float*` that may point to one of several shared arrays is a
+// 16-byte load from a SHARED-space address.  A pointer that may point to one of several shared arrays is a
 // generic pointer to the compiler, which then emits LD.E (generic) instead of LDS; volatile so that it is neither
 // hoisted over the barrier that publishes the data nor merged with another load.
-__device__ __forceinline__ float4 lds128(uint32_t saddr) {
-  float4 v;
-  asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(saddr));
-  return v;
-}
 __device__ __forceinline__ uint4 lds128u(uint32_t saddr) {
   uint4 v;
   asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(saddr));
   return v;
 }
 template <typename T> struct Elem;
-// packed fp32x2 add (Blackwell FADD2) and fused relu + round + pack to a 16-bit pair
-__device__ __forceinline__ void add2(float& a, float& b, float c, float d) {
-  asm("{\n\t.reg .b64 x, y;\n\tmov.b64 x, {%0, %1};\n\tmov.b64 y, {%2, %3};\n\t"
-      "add.rn.f32x2 x, x, y;\n\tmov.b64 {%0, %1}, x;\n\t}"
-      : "+f"(a), "+f"(b)
-      : "f"(c), "f"(d));
-}
 // (qa, qb) += (x * x, y * y) and (sa, sb) += (x, y) as packed fp32x2 operations
 __device__ __forceinline__ void sum_sq2(float& sa, float& sb, float& qa, float& qb, float x, float y) {
   asm("{\n\t.reg .b64 v, s, q;\n\tmov.b64 v, {%4, %5};\n\tmov.b64 s, {%0, %1};\n\tmov.b64 q, {%2, %3};\n\t"

@@ -387,17 +387,6 @@ constexpr int kWProd = 4 * kSlots, kWL1 = kWProd + 1;
 // kernel at the smallest setmaxnreg value -- every role spilled.)
 constexpr int kMlpThreads = (kWL1 + 1) * 32;
 
-// Optional cycle accounting of one epilogue warp and the first-layer issuer (compile with -DFGNN_TC_TIMING; bring-up only).
-#ifdef FGNN_TC_TIMING
-__device__ unsigned long long g_tc_timing[32];
-#define TIMING_DECL long long tm_t0 = clock64(), tm_acc[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0}
-#define TIMING_MARK(slot) do { long long tm_t1 = clock64(); tm_acc[slot] += tm_t1 - tm_t0; tm_t0 = tm_t1; } while (0)
-#define TIMING_FLUSH(base, cond) do { if (cond) for (int tm_i = 0; tm_i < 12; ++tm_i) atomicAdd(&g_tc_timing[(base) + tm_i], (unsigned long long)tm_acc[tm_i]); } while (0)
-#else
-#define TIMING_DECL
-#define TIMING_MARK(slot)
-#define TIMING_FLUSH(base, cond)
-#endif
 constexpr int kMaxInStages = 4;
 __host__ __device__ inline int mlp_in_stages(int K1) { return K1 >= 128 ? 3 : 4; }   // 32 KB stages at K1 = 128
 
@@ -597,25 +586,20 @@ tc_mlp_kernel(const __grid_constant__ CUtensorMap map_x0, const __grid_constant_
       int issue_gidx = 0;                      // graphs (relative to g_first) whose weight buffer has been released
       uint32_t ph_free = 0;                    // phase bits of acc_free[s]
       const int ntiles = t_end - t_begin;
-      TIMING_DECL;
       for (int seq = 0; seq < ntiles; ++seq) {
-        TIMING_MARK(0);
         const int st = (int)(seq % kInStages);
         walker_seek(wi, t_begin + seq);
         const int gidx = wi.g - g_first;
         for (; issue_gidx < gidx; ++issue_gidx) mma_commit_e(&w1_empty[issue_gidx & 1]);   // every MMA that read it was issued
         const int wbuf = gidx & 1;
         mbar_wait(&w1_full[wbuf], (uint32_t)(gidx >> 1) & 1u);
-        TIMING_MARK(1);
         mbar_wait(&in_full[st], (uint32_t)(seq / kInStages) & 1u);
-        TIMING_MARK(2);
         const int s0 = (int)((seq * NMLP) % kSlots);
 #pragma unroll
         for (int m = 0; m < NMLP; ++m) {
           if (seq * NMLP + m >= kSlots) { mbar_wait(&acc_free[s0 + m], (ph_free >> (s0 + m)) & 1u); ph_free ^= 1u << (s0 + m); }
         }
         tc_fence_after();
-        TIMING_MARK(3);
         const uint32_t a_lo0 = a_desc_lo0 + (uint32_t)st * (stage_bytes >> 4);
         const uint32_t b_lo0 = w1_desc_lo0 + (((uint32_t)wbuf * w1_buf_bytes) >> 4);
         if (elect_one_sync()) {
@@ -650,9 +634,7 @@ tc_mlp_kernel(const __grid_constant__ CUtensorMap map_x0, const __grid_constant_
           for (int m = 0; m < NMLP; ++m) mma_commit(&mma_done[s0 + m]);
         }
         __syncwarp();
-        TIMING_MARK(4);
       }
-      TIMING_FLUSH(16, lane == 0);
       Walker wl = wi;                          // the producer may still wait for the release of later graphs
       walker_seek(wl, t_end - 1);
       for (; issue_gidx < wl.g - g_first + 1; ++issue_gidx) mma_commit_e(&w1_empty[issue_gidx & 1]);
@@ -739,10 +721,8 @@ tc_mlp_kernel(const __grid_constant__ CUtensorMap map_x0, const __grid_constant_
       pool_mn = INFINITY;
     };
 
-    TIMING_DECL;
     int cur_g = -1, tp_i = 0, tp_j = 0;      // pixel (row, physical column) of the current tile's first pixel
     for (int v = s; v < V; v += kSlots) {
-      TIMING_MARK(10);
       const int seq = v / NMLP;
       walker_seek(w, t_begin + seq);
       const int g = w.g, n = w.n;
@@ -766,11 +746,9 @@ tc_mlp_kernel(const __grid_constant__ CUtensorMap map_x0, const __grid_constant_
 #pragma unroll 1
       for (int l = 0; l < depth - 1; ++l) {
         // ---------------- hidden pass: accumulator -> relu(acc + b) as the next layer's 16-bit A operand in TMEM ----------------
-        TIMING_MARK(0);
         mbar_wait(&mma_done[s], ph_mma);
         ph_mma ^= 1u;
         tc_fence_after();
-        TIMING_MARK(1);
         {
           // the bias is already in the accumulator (extra MMA step), so the pass is relu + round + pack; 32 columns per
           // round (the epilogue warps also carry the statistics accumulators: registers)
@@ -790,9 +768,7 @@ tc_mlp_kernel(const __grid_constant__ CUtensorMap map_x0, const __grid_constant_
         tc_fence_before();
         // the staging buffer must be free before the final pass: the store of this group's previous tile has read it
         if (l == depth - 2 && storer) bulk_wait_group_read0();
-        TIMING_MARK(2);
         named_bar_sync(bar_id, 128);           // all four quadrants of the operand are written (and fenced)
-        TIMING_MARK(3);
         if (quad == 0) {
           // this group issues its own next layer: A = packed activations in TMEM, B = the layer's weights in smem
           if (!wh_ready) { mbar_wait(wh_full, 0); wh_ready = true; }
@@ -813,7 +789,6 @@ tc_mlp_kernel(const __grid_constant__ CUtensorMap map_x0, const __grid_constant_
           }
           __syncwarp();
         }
-        TIMING_MARK(4);
       }
       // ---------------- final pass: raw accumulator -> staged 16-bit tile -> TMA store + statistics ----------------
       if (depth == 1) {                        // (with hidden layers the last hidden pass's barrier covers this)
@@ -823,7 +798,6 @@ tc_mlp_kernel(const __grid_constant__ CUtensorMap map_x0, const __grid_constant_
       mbar_wait(&mma_done[s], ph_mma);
       ph_mma ^= 1u;
       tc_fence_after();
-      TIMING_MARK(5);
       // pixel coordinates: at most two row wraps from the tile's first pixel
       int pi = tp_i;
       int pj = tp_j + et;
@@ -925,10 +899,8 @@ tc_mlp_kernel(const __grid_constant__ CUtensorMap map_x0, const __grid_constant_
             for (int cq = 0; cq < COUT / 32; ++cq) round(std::false_type{}, hr, cq);
         }
       }
-      TIMING_MARK(6);
       fence_proxy_async_smem();            // generic-proxy smem writes -> visible to the TMA (async proxy)
       named_bar_sync(bar_id, 128);         // the tile is staged
-      TIMING_MARK(7);
       if (storer) {
         // store it: one 64-pixel half per TMA (a half never straddles a row because NPC % 64 == 0)
         const CUtensorMap* mo = (m == 0) ? &map_o0 : &map_o1;
@@ -937,7 +909,6 @@ tc_mlp_kernel(const __grid_constant__ CUtensorMap map_x0, const __grid_constant_
         if (prw < geo.N) tma_store_3d(mo, tile + (size_t)(quad >> 1) * (COUT * 128), col, prow, g * COUT);
         bulk_commit_group();
       }
-      TIMING_MARK(8);
       // ones rows of Y1 (layout A): the last logical row of every 127-row matmul tile writes the row below it
       if (mode == kOutA && args.ones[m] && in_plane && pi < n) {
         const int mt = pi / kTM1;
@@ -947,7 +918,6 @@ tc_mlp_kernel(const __grid_constant__ CUtensorMap map_x0, const __grid_constant_
           for (int cc = 0; cc < COUT; ++cc) o1[(long)cc * geo.PSA] = ov;
         }
       }
-      TIMING_MARK(9);
       // ---------------- statistics of the staged tile: sum / sum of squares per channel (+ row max / min) ----------------
       if constexpr (!kRegStats) {
       if (g != acc_g) { flush(); acc_g = g; }
@@ -1036,7 +1006,6 @@ tc_mlp_kernel(const __grid_constant__ CUtensorMap map_x0, const __grid_constant_
       }
       }
     }
-    TIMING_FLUSH(0, threadIdx.x == 0);
     if (POOL && pool_row >= 0) pool_flush();
     if (storer) bulk_wait_group0();   // every store has landed before the CTA exits
     if constexpr (kRegStats) flush_reg(); else flush();
@@ -1077,23 +1046,20 @@ struct MatmulCfg {
       (size_t)kStages * kStageBytes + kStoreBytes + 2 * BN * sizeof(float) + (2 * kStages + 4) * 8 + 16;   // + barriers, TMEM slot
 };
 
-// Work items of the matmul: (plane, group of `cl` consecutive row tiles, column tile).  cl = 1: one item per CTA;
-// cl = 2: one item per 2-CTA cluster, CTA rank r takes row tile cl * m + r (a row tile beyond the graph is computed on
-// zero-filled operands and never stored).
+// Work items of the matmul: (plane, row tile, column tile), dealt to the CTAs round robin.
 struct TileWalker {
-  int g = 0, cl = 1;
+  int g = 0;
   long base = 0;
   int mt = 0, nt = 0;
   long tiles_g = 0;
   __device__ void set(const int32_t* npg, int N, int C, int TN1) {
     int n = graph_n(npg, g, N);
-    mt = ((n + kTM1 - 1) / kTM1 + cl - 1) / cl;
+    mt = (n + kTM1 - 1) / kTM1;
     nt = (n + TN1 - 1) / TN1;
     tiles_g = (long)mt * nt * C;
   }
-  __device__ void init(const int32_t* npg, int N, int C, int TN1, int cl_ = 1) {
+  __device__ void init(const int32_t* npg, int N, int C, int TN1) {
     g = 0;
-    cl = cl_;
     base = 0;
     set(npg, N, C, TN1);
   }
@@ -1115,7 +1081,7 @@ struct TileWalker {
   }
 };
 
-template <typename T, int BN, int CL>
+template <typename T, int BN>
 __global__ void __launch_bounds__(192, 1)
 tc_matmul_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
                  const __grid_constant__ CUtensorMap map_o32, const __grid_constant__ CUtensorMap map_o31,
@@ -1139,30 +1105,21 @@ tc_matmul_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
   const int warp = uniform_warp_idx(), lane = threadIdx.x % 32;
   const Geo geo = args.geo;
 
-  long total = 0;                              // work items: (plane, group of CL row tiles, column tile)
+  long total = 0;                              // work items: (plane, row tile, column tile)
   for (int g = 0; g < args.G; ++g) {
     int n = graph_n(args.n_per_graph, g, geo.N);
-    total += (long)(((n + kTM1 - 1) / kTM1 + CL - 1) / CL) * ((n + geo.TN1 - 1) / geo.TN1) * args.C;
+    total += (long)((n + kTM1 - 1) / kTM1) * ((n + geo.TN1 - 1) / geo.TN1) * args.C;
   }
-  // CL = 2: the two CTAs of a cluster work on row tiles 2m and 2m+1 of the same (plane, column tile).  They need the SAME
-  // B tile, so each loads half of it and multicasts that half into both CTAs' shared memory (same offsets, same barrier
-  // offsets): the B stream out of L2 -- two thirds of this kernel's operand traffic, which bounds it -- is halved.  A stage
-  // may only be overwritten once BOTH CTAs' MMAs have read it: every tcgen05.commit of a k tile arrives on the `empty`
-  // barrier of both CTAs (multicast commit), and `empty` counts CL arrivals.
-  const uint32_t cta_rank = CL > 1 ? cluster_ctarank() : 0u;
-  const long item0 = CL > 1 ? (long)(blockIdx.x / CL) : (long)blockIdx.x;
-  const long item_step = (long)(gridDim.x / CL);
-  constexpr uint16_t kClusterMask = (uint16_t)((1u << CL) - 1u);
+  const long item0 = blockIdx.x, item_step = gridDim.x;
 
   if (threadIdx.x == 0) {
-    for (int s = 0; s < kStages; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], CL); }
+    for (int s = 0; s < kStages; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
     for (int s = 0; s < 2; ++s) { mbar_init(&tmem_full[s], 1); mbar_init(&tmem_empty[s], 4); }
     fence_barrier_init();
   }
   if (warp == 0) tmem_alloc(tmem_slot, kTmemCols);
   tc_fence_before();
   __syncthreads();
-  if (CL > 1) cluster_sync_all();              // the peer's barriers are initialised before anything is sent to them
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
@@ -1174,13 +1131,12 @@ tc_matmul_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
         prefetch_tensormap(&map_b);
       }
       TileWalker tw;
-      tw.init(args.n_per_graph, geo.N, args.C, geo.TN1, CL);
+      tw.init(args.n_per_graph, geo.N, args.C, geo.TN1);
       int stage = 0;
       uint32_t phase = 0;
       for (long t = item0; t < total; t += item_step) {
         int q, m, nn, n;
         tw.locate(t, args.n_per_graph, geo.N, args.C, geo.TN1, q, m, nn, n);
-        m = m * CL + (int)cta_rank;
         const int kts = (phys_k_end(n, geo.TN1) + 63) / 64;     // K runs over PHYSICAL columns of Y1 / rows of Y2
         for (int kt = 0; kt < kts; ++kt) {
           mbar_wait(&empty[stage], phase ^ 1);
@@ -1188,14 +1144,8 @@ tc_matmul_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
           uint8_t* sb = sa + 128 * 128;
           mbar_arrive_expect_tx_e(&full[stage], (uint32_t)Cfg::kStageBytes);
           tma_load_3d_e(sa, &map_a, &full[stage], kt * 64, m * 128, q);     // rows beyond the plane are zero-filled
-          if constexpr (CL == 1) {
-            for (int u = 0; u < BN / 64; ++u)
-              tma_load_3d_e(sb + (size_t)u * 8192, &map_b, &full[stage], nn * BN + u * 64, kt * 64, q);
-          } else {
-            // this CTA's half of the 64-column chunks, delivered to both CTAs of the cluster
-            for (int u = (int)cta_rank * (BN / 128); u < ((int)cta_rank + 1) * (BN / 128); ++u)
-              tma_load_3d_mc_e(sb + (size_t)u * 8192, &map_b, &full[stage], nn * BN + u * 64, kt * 64, q, kClusterMask);
-          }
+          for (int u = 0; u < BN / 64; ++u)
+            tma_load_3d_e(sb + (size_t)u * 8192, &map_b, &full[stage], nn * BN + u * 64, kt * 64, q);
           if (++stage == kStages) { stage = 0; phase ^= 1; }
         }
       }
@@ -1209,7 +1159,7 @@ tc_matmul_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
       const uint32_t a_desc_lo0 = (uint32_t)a_d0, a_desc_hi = (uint32_t)(a_d0 >> 32);
       const uint32_t b_desc_lo0 = (uint32_t)b_d0, b_desc_hi = (uint32_t)(b_d0 >> 32);
       TileWalker tw;
-      tw.init(args.n_per_graph, geo.N, args.C, geo.TN1, CL);
+      tw.init(args.n_per_graph, geo.N, args.C, geo.TN1);
       int stage = 0;
       uint32_t phase = 0;
       int as = 0;
@@ -1230,8 +1180,7 @@ tc_matmul_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
           for (int k = 0; k < 4; ++k)
             mma_ss2_e(d_tmem, a_lo + (uint32_t)k * (32u >> 4), a_desc_hi, b_lo + (uint32_t)k * (2048u >> 4), b_desc_hi,
                       idesc, (kt > 0 || k > 0) ? 1u : 0u);
-          if constexpr (CL == 1) mma_commit_e(&empty[stage]);
-          else mma_commit_mc_e(&empty[stage], kClusterMask);      // frees the stage in BOTH CTAs (each multicasts into it)
+          mma_commit_e(&empty[stage]);
           if (++stage == kStages) { stage = 0; phase ^= 1; }
         }
         mma_commit_e(&tmem_full[as]);
@@ -1242,14 +1191,13 @@ tc_matmul_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
     // ================= epilogue (warps 2..5, TMEM lane quadrant = warp % 4) =================
     const int quad = warp % 4;
     TileWalker tw;
-    tw.init(args.n_per_graph, geo.N, args.C, geo.TN1, CL);
+    tw.init(args.n_per_graph, geo.N, args.C, geo.TN1);
     int as = 0;
     uint32_t aphase = 0;
     int sbuf = 0;                            // staging buffer of the next 64-column chunk
     for (long t = item0; t < total; t += item_step) {
       int q, m, nn, n;
       tw.locate(t, args.n_per_graph, geo.N, args.C, geo.TN1, q, m, nn, n);
-      m = m * CL + (int)cta_rank;
       float a1 = 1.f, s1 = 0.f, a2 = 1.f, s2 = 0.f;
       if (args.coef_a) { a1 = args.coef_a[2 * q]; s1 = args.coef_a[2 * q + 1]; }
       if (args.coef_b) { a2 = args.coef_b[2 * q]; s2 = args.coef_b[2 * q + 1]; }
@@ -1329,7 +1277,6 @@ tc_matmul_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
   }
   tc_fence_before();
   __syncthreads();
-  if (CL > 1) cluster_sync_all();            // the peer may still multicast into / arrive on this CTA's shared memory
   tc_fence_after();
   if (warp == 0) {
     __syncwarp();
@@ -1585,147 +1532,16 @@ int launch_matmul(const T* y1, const T* y2, T* out, const float* coef_a, const f
   if (int e = make_map3(&mo31, is_bf16, out, geo.NPC, geo.N, planes, geo.NPC, (uint64_t)geo.PSC, 64, 31)) return e;
   MatmulArgs<T> a{G, C, geo, out, coef_a, coef_b, npg};
   const int grid = num_sms();
-#define FGNN_MM_LAUNCH(BNV)                                                                              \
-  do {                                                                                                   \
-    /* per device and cheap: set on every call */                                                        \
-    FGNN_CUDA(cudaFuncSetAttribute(tc_matmul_kernel<T, BNV, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                   (int)MatmulCfg<BNV>::kSmemBytes));                                    \
-    tc_matmul_kernel<T, BNV, 1><<<grid, 192, MatmulCfg<BNV>::kSmemBytes, st>>>(ma, mb, mo32, mo31, a);                \
-  } while (0)
+  auto kernel = geo.BN == 64 ? tc_matmul_kernel<T, 64> : geo.BN == 128 ? tc_matmul_kernel<T, 128> : tc_matmul_kernel<T, 256>;
+  const size_t smem = geo.BN == 64 ? MatmulCfg<64>::kSmemBytes
+                                   : geo.BN == 128 ? MatmulCfg<128>::kSmemBytes : MatmulCfg<256>::kSmemBytes;
   prof::begin(prof::kMatmul, st);
-  if (geo.BN == 64) FGNN_MM_LAUNCH(64);
-  else if (geo.BN == 128) FGNN_MM_LAUNCH(128);
-  else if (geo.MT < 2 || env_int("FGNN_MM_CLUSTER", 0) == 0) FGNN_MM_LAUNCH(256);
-  else {
-    // FGNN_MM_CLUSTER=1 and N > 127 (at least two row tiles per plane): 2-CTA clusters sharing the B tile by TMA multicast.
-    // Parity-tested, measured NEUTRAL at the headline shape (75.5 vs 74.9 ms per 8 steps): the kernel is bound by HBM (83 %
-    // of the measured copy bandwidth with its 2:1 read/write mix), not by the L2 -> SM operand stream, so it is off by default.
-    FGNN_CUDA(cudaFuncSetAttribute(tc_matmul_kernel<T, 256, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                   (int)MatmulCfg<256>::kSmemBytes));
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)(grid / 2 * 2));
-    cfg.blockDim = dim3(192);
-    cfg.dynamicSmemBytes = MatmulCfg<256>::kSmemBytes;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    FGNN_CUDA(cudaLaunchKernelEx(&cfg, tc_matmul_kernel<T, 256, 2>, ma, mb, mo32, mo31, a));
-  }
-#undef FGNN_MM_LAUNCH
+  // per device and cheap: set on every call
+  FGNN_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kernel<<<grid, 192, smem, st>>>(ma, mb, mo32, mo31, a);
   prof::end(prof::kMatmul, st);
   FGNN_LAUNCHED();
   return FGNN_OK;
-}
-
-template <typename T>
-struct MlpLaunch {
-  const T* src[2];
-  int c_src[2];
-  int nsrc;
-  int nmlp;
-  const T* w1f;        // [G][nmlp][COUT][K1g]
-  const float* bias1;  // [G][nmlp][COUT]
-  const T* bias1_tile; // [G][nmlp COUT / 8][2][8][8] the folded bias as an MMA step (required when depth > 1)
-  const T* wh;         // [nmlp][depth-1][COUT][Kh]
-  const float* bias[2][FGNN_MAX_DEPTH];
-  int depth, c_out;
-  T* out[2];
-  int out_mode[2];
-  int ones[2];
-  double* stat_acc;    // [G][nmlp][COUT][2], zeroed here
-  unsigned int* rowenc[2];   // fused max pooling instead of the store (see MlpArgs), or null
-  int relu_out;              // depth-1 launches of the training path: out = relu(conv + bias) instead of the raw accumulator
-};
-
-template <typename T, int COUT, int NMLP>
-int launch_mlp_t(const MlpLaunch<T>& L, int G, const Geo& geo, const int32_t* npg, cudaStream_t st) {
-  constexpr int is_bf16 = Elem<T>::kFmt;
-  MlpArgs<T> a{};
-  a.G = G;
-  a.geo = geo;
-  a.nsrc = L.nsrc;
-  a.k_src[0] = round_up(L.c_src[0], 16);
-  a.k_src[1] = L.nsrc > 1 ? round_up(L.c_src[1], 16) : 0;
-  a.K1 = a.k_src[0] + a.k_src[1];
-  a.K1g = round_up(a.K1, 64);
-  a.depth = L.depth;
-  a.Kh = COUT < 64 ? 64 : COUT;
-  a.bias1 = L.bias1;
-  a.bias1_tile = L.bias1_tile;
-  FGNN_CHECK_ARG(L.depth == 1 || L.bias1_tile != nullptr, "conv chains with hidden layers need the folded bias tile");
-  for (int m = 0; m < NMLP; ++m) {
-    for (int l = 0; l < L.depth; ++l) a.bias[m][l] = L.bias[m][l];
-    a.out[m] = L.out[m];
-    a.out_mode[m] = L.out_mode[m];
-    a.ones[m] = L.ones[m];
-    a.rowenc[m] = L.rowenc[m];
-  }
-  a.stat_acc = L.stat_acc;
-  a.n_per_graph = npg;
-  FGNN_CHECK_ARG(a.K1 <= 256, "first-layer K=%d too wide for the tensor-core MLP kernel", a.K1);
-  CUtensorMap mx0, mx1, mw1, mwh, mo[2];
-  for (int m = 0; m < NMLP; ++m) {
-    const int rows = L.out_mode[m] == kOutA ? geo.PRA : (L.out_mode[m] == kOutB ? geo.PRB : geo.N);
-    if (int e = make_map3(&mo[m], is_bf16, L.out[m], geo.NPC, rows, (uint64_t)G * COUT, geo.NPC, (uint64_t)rows * geo.NPC,
-                          64, 1, COUT)) return e;
-  }
-  if (NMLP == 1) mo[1] = mo[0];
-  if (int e = make_map3(&mx0, is_bf16, L.src[0], geo.PSC, L.c_src[0], G, geo.PSC, (uint64_t)L.c_src[0] * geo.PSC, 64, a.k_src[0])) return e;
-  if (L.nsrc > 1) {
-    if (int e = make_map3(&mx1, is_bf16, L.src[1], geo.PSC, L.c_src[1], G, geo.PSC, (uint64_t)L.c_src[1] * geo.PSC, 64, a.k_src[1])) return e;
-  } else {
-    mx1 = mx0;
-  }
-  if (int e = make_map3(&mw1, is_bf16, L.w1f, a.K1g, COUT, (uint64_t)G * NMLP, a.K1g, (uint64_t)COUT * a.K1g, 64, COUT)) return e;
-  if (L.depth > 1) {
-    if (int e = make_map3(&mwh, is_bf16, L.wh, a.Kh, COUT, (uint64_t)NMLP * (L.depth - 1), a.Kh, (uint64_t)COUT * a.Kh, 64, COUT)) return e;
-  } else {
-    mwh = mw1;
-  }
-  const size_t smem = MlpSmem<COUT, NMLP>::bytes(a.K1, a.K1g, a.depth, a.Kh);
-  FGNN_CHECK_ARG(smem <= 227 * 1024, "MLP kernel needs %zu bytes of shared memory", smem);
-  const bool pool = a.rowenc[0] != nullptr;
-  FGNN_CHECK_ARG(!pool || NMLP == 1, "fused pooling is only built for single-MLP launches");
-  FGNN_CHECK_ARG(!L.relu_out || (L.depth == 1 && !pool), "relu_out is a depth-1, non-pooled launch");
-  {   // the opt-in is per device and cheap: set on every call
-    if (pool) {
-      if constexpr (NMLP == 1)
-        FGNN_CUDA(cudaFuncSetAttribute(tc_mlp_kernel<T, COUT, NMLP, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    } else if (L.relu_out) {
-      FGNN_CUDA(cudaFuncSetAttribute(tc_mlp_kernel<T, COUT, NMLP, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    } else {
-      FGNN_CUDA(cudaFuncSetAttribute(tc_mlp_kernel<T, COUT, NMLP, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    }
-  }
-  FGNN_CUDA(cudaMemsetAsync(L.stat_acc, 0, (size_t)G * NMLP * COUT * 2 * sizeof(double), st));
-  long total_tiles = (long)G * ((geo.PSC + kTileM - 1) / kTileM);
-  int grid = (int)std::min<long>((long)num_sms(), total_tiles);
-  if (grid < 1) grid = 1;
-  prof::begin(prof::kMlp, st);
-  if (pool) {
-    if constexpr (NMLP == 1) tc_mlp_kernel<T, COUT, NMLP, true, false><<<grid, kMlpThreads, smem, st>>>(mx0, mx1, mw1, mwh, mo[0], mo[1], a);
-  } else if (L.relu_out) {
-    tc_mlp_kernel<T, COUT, NMLP, false, true><<<grid, kMlpThreads, smem, st>>>(mx0, mx1, mw1, mwh, mo[0], mo[1], a);
-  } else {
-    tc_mlp_kernel<T, COUT, NMLP, false, false><<<grid, kMlpThreads, smem, st>>>(mx0, mx1, mw1, mwh, mo[0], mo[1], a);
-  }
-  prof::end(prof::kMlp, st);
-  FGNN_LAUNCHED();
-  return FGNN_OK;
-}
-
-template <typename T>
-int launch_mlp(const MlpLaunch<T>& L, int G, const Geo& geo, const int32_t* npg, cudaStream_t st) {
-  if (L.c_out == 32 && L.nmlp == 1) return launch_mlp_t<T, 32, 1>(L, G, geo, npg, st);
-  if (L.c_out == 32 && L.nmlp == 2) return launch_mlp_t<T, 32, 2>(L, G, geo, npg, st);
-  if (L.c_out == 64 && L.nmlp == 1) return launch_mlp_t<T, 64, 1>(L, G, geo, npg, st);
-  if (L.c_out == 64 && L.nmlp == 2) return launch_mlp_t<T, 64, 2>(L, G, geo, npg, st);
-  return fail(FGNN_ERR_UNSUPPORTED, "tensor-core path supports out_features 32 or 64 (got %d); use FGNN_FP32", L.c_out);
 }
 
 // fold + conv chain(s) + statistics finalisation for 1 or 2 MLPs sharing their input
@@ -1737,21 +1553,98 @@ struct MlpGroup {
   int c_src[2];
   const float* src_coef[2];
   int nsrc;
-  T* wf;
-  float* bf;
+  T* wf;             // [G][nmlp][C][K1g] folded first-layer weights
+  float* bf;         // [G][nmlp][C] folded first-layer bias
   T* bt;             // [G][nmlp][C][16] folded first-layer bias as an MMA step (may be null for depth-1 launches)
   const T* wh;       // [nmlp][depth-1][C][Kh]
   T* out[2];
   int out_mode[2];
   int ones[2];
   float* coef[2];
-  double* stat_acc;
-  unsigned int* rowenc[2];   // fused max pooling of this MLP's output instead of storing it (or null)
+  double* stat_acc;  // [G][nmlp][C][2], zeroed by the launch
+  unsigned int* rowenc[2];   // fused max pooling of this MLP's output instead of storing it (see MlpArgs), or null
   // training path (depth-1 launches, see fgnn_tc_train.cuh)
   int relu_out;              // out = relu(conv + bias) instead of the raw accumulator
   int no_coef;               // skip the GraphNorm coefficient finalisation (hidden layers, backward convs)
   float* gnstat[2];          // statistics kept for backward (or null)
 };
+
+template <typename T, int COUT, int NMLP>
+int launch_mlp_t(const MlpGroup<T>& M, int G, const Geo& geo, const int32_t* npg, cudaStream_t st) {
+  constexpr int is_bf16 = Elem<T>::kFmt;
+  MlpArgs<T> a{};
+  a.G = G;
+  a.geo = geo;
+  a.nsrc = M.nsrc;
+  a.k_src[0] = round_up(M.c_src[0], 16);
+  a.k_src[1] = M.nsrc > 1 ? round_up(M.c_src[1], 16) : 0;
+  a.K1 = a.k_src[0] + a.k_src[1];
+  a.K1g = round_up(a.K1, 64);
+  a.depth = M.mp[0]->depth;
+  a.Kh = COUT < 64 ? 64 : COUT;
+  a.bias1 = M.bf;
+  a.bias1_tile = M.bt;
+  FGNN_CHECK_ARG(a.depth == 1 || M.bt != nullptr, "conv chains with hidden layers need the folded bias tile");
+  for (int m = 0; m < NMLP; ++m) {
+    FGNN_CHECK_ARG(M.mp[m]->depth == a.depth, "MLPs fused in one launch must have the same depth");
+    for (int l = 0; l < a.depth; ++l) a.bias[m][l] = M.mp[m]->b[l];
+    a.out[m] = M.out[m];
+    a.out_mode[m] = M.out_mode[m];
+    a.ones[m] = M.ones[m];
+    a.rowenc[m] = M.rowenc[m];
+  }
+  a.stat_acc = M.stat_acc;
+  a.n_per_graph = npg;
+  FGNN_CHECK_ARG(a.K1 <= 256, "first-layer K=%d too wide for the tensor-core MLP kernel", a.K1);
+  CUtensorMap mx0, mx1, mw1, mwh, mo[2];
+  for (int m = 0; m < NMLP; ++m) {
+    const int rows = M.out_mode[m] == kOutA ? geo.PRA : (M.out_mode[m] == kOutB ? geo.PRB : geo.N);
+    if (int e = make_map3(&mo[m], is_bf16, M.out[m], geo.NPC, rows, (uint64_t)G * COUT, geo.NPC, (uint64_t)rows * geo.NPC,
+                          64, 1, COUT)) return e;
+  }
+  if (NMLP == 1) mo[1] = mo[0];
+  if (int e = make_map3(&mx0, is_bf16, M.src[0], geo.PSC, M.c_src[0], G, geo.PSC, (uint64_t)M.c_src[0] * geo.PSC, 64, a.k_src[0])) return e;
+  if (M.nsrc > 1) {
+    if (int e = make_map3(&mx1, is_bf16, M.src[1], geo.PSC, M.c_src[1], G, geo.PSC, (uint64_t)M.c_src[1] * geo.PSC, 64, a.k_src[1])) return e;
+  } else {
+    mx1 = mx0;
+  }
+  if (int e = make_map3(&mw1, is_bf16, M.wf, a.K1g, COUT, (uint64_t)G * NMLP, a.K1g, (uint64_t)COUT * a.K1g, 64, COUT)) return e;
+  if (a.depth > 1) {
+    if (int e = make_map3(&mwh, is_bf16, M.wh, a.Kh, COUT, (uint64_t)NMLP * (a.depth - 1), a.Kh, (uint64_t)COUT * a.Kh, 64, COUT)) return e;
+  } else {
+    mwh = mw1;
+  }
+  const size_t smem = MlpSmem<COUT, NMLP>::bytes(a.K1, a.K1g, a.depth, a.Kh);
+  FGNN_CHECK_ARG(smem <= 227 * 1024, "MLP kernel needs %zu bytes of shared memory", smem);
+  const bool pool = a.rowenc[0] != nullptr;
+  FGNN_CHECK_ARG(!pool || NMLP == 1, "fused pooling is only built for single-MLP launches");
+  FGNN_CHECK_ARG(!M.relu_out || (a.depth == 1 && !pool), "relu_out is a depth-1, non-pooled launch");
+  auto kernel = M.relu_out ? tc_mlp_kernel<T, COUT, NMLP, false, true> : tc_mlp_kernel<T, COUT, NMLP, false, false>;
+  if constexpr (NMLP == 1) {
+    if (pool) kernel = tc_mlp_kernel<T, COUT, NMLP, true, false>;
+  }
+  // the opt-in is per device and cheap: set on every call
+  FGNN_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  FGNN_CUDA(cudaMemsetAsync(M.stat_acc, 0, (size_t)G * NMLP * COUT * 2 * sizeof(double), st));
+  long total_tiles = (long)G * ((geo.PSC + kTileM - 1) / kTileM);
+  int grid = (int)std::min<long>((long)num_sms(), total_tiles);
+  if (grid < 1) grid = 1;
+  prof::begin(prof::kMlp, st);
+  kernel<<<grid, kMlpThreads, smem, st>>>(mx0, mx1, mw1, mwh, mo[0], mo[1], a);
+  prof::end(prof::kMlp, st);
+  FGNN_LAUNCHED();
+  return FGNN_OK;
+}
+
+template <typename T>
+int launch_mlp(const MlpGroup<T>& M, int C, int G, const Geo& geo, const int32_t* npg, cudaStream_t st) {
+  if (C == 32 && M.nmlp == 1) return launch_mlp_t<T, 32, 1>(M, G, geo, npg, st);
+  if (C == 32 && M.nmlp == 2) return launch_mlp_t<T, 32, 2>(M, G, geo, npg, st);
+  if (C == 64 && M.nmlp == 1) return launch_mlp_t<T, 64, 1>(M, G, geo, npg, st);
+  if (C == 64 && M.nmlp == 2) return launch_mlp_t<T, 64, 2>(M, G, geo, npg, st);
+  return fail(FGNN_ERR_UNSUPPORTED, "tensor-core path supports out_features 32 or 64 (got %d); use FGNN_FP32", C);
+}
 
 template <typename T>
 int run_mlp_group(const MlpGroup<T>& M, int C, int G, const Geo& geo, const int32_t* npg, cudaStream_t st) {
@@ -1770,27 +1663,7 @@ int run_mlp_group(const MlpGroup<T>& M, int C, int G, const Geo& geo, const int3
   FGNN_CHECK_ARG(fa.c[0] + fa.c[1] <= 512, "too many input channels for the fold kernel");
   fold_weights_kernel<T><<<dim3(G, M.nmlp, 8), 256, 0, st>>>(fa, M.wf, M.bf, M.bt);
   FGNN_LAUNCHED();
-  MlpLaunch<T> L{};
-  L.nmlp = M.nmlp;
-  L.nsrc = M.nsrc;
-  for (int s = 0; s < 2; ++s) { L.src[s] = M.src[s]; L.c_src[s] = M.c_src[s]; }
-  L.w1f = M.wf;
-  L.bias1 = M.bf;
-  L.bias1_tile = M.bt;
-  L.wh = M.wh;
-  L.depth = M.mp[0]->depth;
-  L.c_out = C;
-  for (int m = 0; m < M.nmlp; ++m) {
-    FGNN_CHECK_ARG(M.mp[m]->depth == L.depth, "MLPs fused in one launch must have the same depth");
-    for (int l = 0; l < L.depth; ++l) L.bias[m][l] = M.mp[m]->b[l];
-    L.out[m] = M.out[m];
-    L.out_mode[m] = M.out_mode[m];
-    L.ones[m] = M.ones[m];
-    L.rowenc[m] = M.rowenc[m];
-  }
-  L.stat_acc = M.stat_acc;
-  L.relu_out = M.relu_out;
-  if (int e = launch_mlp<T>(L, G, geo, npg, st)) return e;
+  if (int e = launch_mlp<T>(M, C, G, geo, npg, st)) return e;
   if (M.no_coef) return FGNN_OK;
   CoefArgs ca{};
   ca.acc = M.stat_acc;
@@ -2042,8 +1915,7 @@ size_t embed_workspace_bytes(const fgnn_embed_params& p, int G, int N) {
 }
 
 int embed_fwd(const fgnn_embed_params& p, int precision, const float* x, float* emb, int G, int N,
-              const int32_t* n_per_graph, const int32_t* /*n_per_graph_host*/, void* ws, size_t ws_bytes,
-              cudaStream_t st) {
+              const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
   if (!fgnn_device_supports_tcgen05())
     return fail(FGNN_ERR_UNSUPPORTED, "FGNN_BF16/FGNN_FP16 need an sm_100 device (tcgen05); there is no fallback");
   if (reinterpret_cast<uintptr_t>(ws) & 1023) return fail(FGNN_ERR_INVALID, "workspace must be 1024-byte aligned");
@@ -2195,43 +2067,6 @@ int debug_mlp(int precision, const fgnn_mlp_params& mp, const float* x, float* y
   if (precision == FGNN_BF16) return debug_mlp_t<__nv_bfloat16>(mp, x, y, G, N, n_per_graph, ws, ws_bytes, st);
   if (precision == FGNN_FP16) return debug_mlp_t<__half>(mp, x, y, G, N, n_per_graph, ws, ws_bytes, st);
   return fail(FGNN_ERR_INVALID, "precision must be FGNN_BF16 or FGNN_FP16");
-}
-
-void dump_timing() {
-#ifdef FGNN_TC_TIMING
-  {
-    unsigned long long h[32];
-    cudaDeviceSynchronize();
-    cudaMemcpyFromSymbol(h, g_tc_timing, sizeof(h));
-    const char* names[2][12] = {
-        {"index / walker / loop head", "hidden: wait mma_done", "hidden: ld + relu/pack + st", "hidden: named barrier", "hidden: MMA issue",
-         "final: wait mma_done", "final: ld + stats + cvt + stmatrix", "final: proxy fence + named barrier", "tail: TMA store issue",
-         "tail: ones rows", "tail: smem statistics (pooled launches) + loop", "-"},
-        {"loop", "wait w1_full", "wait in_full", "wait acc_free", "issue + commit", "-", "-", "-", "-", "-", "-", "-"}};
-    const char* role[2] = {"epilogue warp 0 (group 0)", "first-layer issuer"};
-    for (int r = 0; r < 2; ++r) {
-      unsigned long long tot = 0;
-      for (int i = 0; i < 12; ++i) tot += h[16 * r + i];
-      printf("%s (sum over CTAs, cycles):\n", role[r]);
-      for (int i = 0; i < 12; ++i)
-        if (h[16 * r + i]) printf("  %-62s %14llu %5.1f%%\n", names[r][i], h[16 * r + i], 100.0 * h[16 * r + i] / (tot ? tot : 1));
-    }
-    unsigned long long z[32] = {0};
-    cudaMemcpyToSymbol(g_tc_timing, z, sizeof(z));
-  }
-#endif
-#ifdef FGNN_DEBUG_WAIT
-  unsigned int h[4 + 128 * 4];
-  cudaError_t e = cudaDeviceSynchronize();
-  printf("sync: %s\n", cudaGetErrorString(e));
-  cudaMemcpyFromSymbol(h, ptx::g_wait_dbg, sizeof(h));
-  printf("abandoned waits: %u\n", h[0]);
-  for (unsigned i = 0; i < h[0] && i < 128; ++i)
-    printf("  block %3u thread %3u (warp %2u lane %2u) barrier smem+0x%x parity %u\n", h[4 + 4 * i], h[5 + 4 * i], h[5 + 4 * i] / 32,
-           h[5 + 4 * i] % 32, h[6 + 4 * i], h[7 + 4 * i]);
-  unsigned int z[4] = {0, 0, 0, 0};
-  cudaMemcpyToSymbol(ptx::g_wait_dbg, z, sizeof(z));
-#endif
 }
 
 }  // namespace tc

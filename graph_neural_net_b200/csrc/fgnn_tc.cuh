@@ -7,8 +7,7 @@ namespace tc {
 
 size_t embed_workspace_bytes(const fgnn_embed_params& p, int G, int N);
 int embed_fwd(const fgnn_embed_params& p, int precision, const float* x, float* emb, int G, int N,
-              const int32_t* n_per_graph, const int32_t* n_per_graph_host, void* ws, size_t ws_bytes,
-              cudaStream_t st);
+              const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st);
 
 int embed_fwd_adjacency(const fgnn_embed_params& p, int precision, const uint8_t* adj, float* emb, int G, int N,
                         const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st);
@@ -32,8 +31,6 @@ int debug_matmul(int precision, const float* a, const float* b, float* out, int 
 size_t debug_mlp_workspace_bytes(int G, int c_in, int c_out, int depth, int N);
 int debug_mlp(int precision, const fgnn_mlp_params& mp, const float* x, float* y, int G, int N,
               const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st);
-
-void dump_timing();
 
 }  // namespace tc
 

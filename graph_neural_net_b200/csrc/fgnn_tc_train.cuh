@@ -873,23 +873,13 @@ int launch_bmm_bwd(int mode, const T* a, const T* b, T* out, const float* coef, 
   if (int e = make_map3(&mo31, is_bf16, out, geo.NPC, geo.N, planes, geo.NPC, (uint64_t)geo.PSC, 64, 31)) return e;
   BmmBwdArgs<T> args{G, C, geo, coef, vec, npg};
   const int grid = num_sms();
-#define FGNN_BB_LAUNCH(BNV, MODEV)                                                                               \
-  do {                                                                                                           \
-    FGNN_CUDA(cudaFuncSetAttribute(tc_bmm_bwd_kernel<T, BNV, MODEV>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                   (int)MatmulCfg<BNV>::kSmemBytes));                                            \
-    tc_bmm_bwd_kernel<T, BNV, MODEV><<<grid, 192, MatmulCfg<BNV>::kSmemBytes, st>>>(ma, mb, mo32, mo31, args);   \
-  } while (0)
+  auto kernel = mode == 1 ? (geo.BN == 64 ? tc_bmm_bwd_kernel<T, 64, 1> : geo.BN == 128 ? tc_bmm_bwd_kernel<T, 128, 1> : tc_bmm_bwd_kernel<T, 256, 1>)
+                          : (geo.BN == 64 ? tc_bmm_bwd_kernel<T, 64, 2> : geo.BN == 128 ? tc_bmm_bwd_kernel<T, 128, 2> : tc_bmm_bwd_kernel<T, 256, 2>);
+  const size_t smem = geo.BN == 64 ? MatmulCfg<64>::kSmemBytes
+                                   : geo.BN == 128 ? MatmulCfg<128>::kSmemBytes : MatmulCfg<256>::kSmemBytes;
   prof::begin(prof::kMatmul, st);
-  if (mode == 1) {
-    if (geo.BN == 64) FGNN_BB_LAUNCH(64, 1);
-    else if (geo.BN == 128) FGNN_BB_LAUNCH(128, 1);
-    else FGNN_BB_LAUNCH(256, 1);
-  } else {
-    if (geo.BN == 64) FGNN_BB_LAUNCH(64, 2);
-    else if (geo.BN == 128) FGNN_BB_LAUNCH(128, 2);
-    else FGNN_BB_LAUNCH(256, 2);
-  }
-#undef FGNN_BB_LAUNCH
+  FGNN_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kernel<<<grid, 192, smem, st>>>(ma, mb, mo32, mo31, args);
   prof::end(prof::kMatmul, st);
   FGNN_LAUNCHED();
   return FGNN_OK;

@@ -255,12 +255,11 @@ class Network(nn.Module):
             raise L.FgnnError("this Network is not a node_embedding DAG; fused execution unavailable")
         prec = L.PRECISIONS[precision or self.precision]
         plain, n_dev, rewrap = _unwrap(x)
-        n_host = x.sizes_host() if isinstance(x, MaskedTensor) else None
         keep = []
         params = self._embed_params(keep)
         c_out = self._fused[2][-1][2].convs[-1].weight.shape[0]
         c_run = int(params.block[0].mlp1.c_out)               # the width the kernels run (zero-padded widths: see _padded_widths)
-        emb = _ops.embed_fwd(params, prec, plain, c_run, n_dev, n_host)
+        emb = _ops.embed_fwd(params, prec, plain, c_run, n_dev)
         if c_run != c_out:
             emb = emb[:, :c_out].contiguous()
         if isinstance(x, MaskedTensor):

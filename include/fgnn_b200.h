@@ -207,8 +207,7 @@ int fgnn_lap_fwd(const float* scores, int32_t* col_of_row, int32_t* correct, dou
  * workspace: fgnn_embed_workspace_bytes(...) bytes, 1024-byte aligned. */
 size_t fgnn_embed_workspace_bytes(const fgnn_embed_params* p, int32_t precision, int32_t G, int32_t N);
 int fgnn_embed_fwd(const fgnn_embed_params* p, int32_t precision, const float* x, float* emb,
-                   int32_t G, int32_t N, const int32_t* n_per_graph,
-                   const int32_t* n_per_graph_host, void* workspace, size_t workspace_bytes,
+                   int32_t G, int32_t N, const int32_t* n_per_graph, void* workspace, size_t workspace_bytes,
                    void* stream);
 
 /* Same embedder fed from a uint8 adjacency batch (G,N,N) instead of the fp32 (G,2,N,N) features: the two
@@ -259,10 +258,6 @@ void fgnn_reset_launch_count(void);
 void fgnn_profile_enable(int on);
 void fgnn_profile_reset(void);
 int fgnn_profile_read(int32_t kind, double* total_ms, int64_t* launches);
-
-/* Bring-up aid: prints the per-role cycle accounting of the conv-chain kernel when the library was
- * built with -DFGNN_TC_TIMING; a no-op otherwise. */
-void fgnn_debug_dump_timing(void);
 
 /* Diagnostics for the tensor-core building blocks (tests call these to check each kernel in
  * isolation against the fp32 operators): 16-bit planes are (G*C) planes of pitch_rows x pitch_cols. */
