@@ -9,7 +9,10 @@
 //   Regular:     the switch chain on simple d-regular graphs: start from a randomly relabelled circulant graph and apply
 //                kSwapsPerEdge * |E| double-edge-swap proposals (u,v),(s,t) -> (u,t),(s,v), rejected when they would
 //                create a loop or a parallel edge (its stationary distribution is uniform over simple d-regular graphs).
-//                One CTA per graph, adjacency bitmap in shared memory, the chain itself is sequential (one thread).
+//                One CTA per graph; the n x ceil(n/32)-word adjacency bitmap sits in shared memory up to N = 1264 and in the
+//                caller's workspace (L2-resident) above; the chain itself is sequential (one thread), so its time grows
+//                with |E| = n d / 2 (10 |E| proposals; not measured at large n).
+// N <= 4096 (vertex numbers are packed as 16-bit halves of an edge word, and the Regular workspace grows as G N^2).
 #include "fgnn_common.cuh"
 
 namespace fgnn {
@@ -17,6 +20,8 @@ namespace gen {
 namespace {
 
 constexpr int kSwapsPerEdge = 10;
+constexpr int kMaxN = 4096;
+constexpr size_t kSmemCap = 200 * 1024;   // dynamic shared memory the Regular kernel asks for at most
 
 __host__ __device__ inline uint64_t mix64(uint64_t x) {   // splitmix64 finaliser
   x += 0x9E3779B97F4A7C15ull;
@@ -64,7 +69,7 @@ struct Rng {   // sequential stream of the chain thread
 
 __global__ void __launch_bounds__(256, 1)
 regular_kernel(uint8_t* __restrict__ adj, int N, const int32_t* __restrict__ npg, float p, uint64_t seed,
-               uint32_t* __restrict__ edges_ws, long edges_per_graph, int edges_in_smem) {
+               uint32_t* __restrict__ edges_ws, long edges_per_graph, int edges_in_smem, uint32_t* __restrict__ bits_ws) {
   extern __shared__ uint32_t sm[];
   const int g = blockIdx.x;
   const int n = graph_n(npg, g, N);
@@ -72,8 +77,9 @@ regular_kernel(uint8_t* __restrict__ adj, int N, const int32_t* __restrict__ npg
   if ((n * d) & 1) d += 1;
   if (d > n - 1) d = n - 1 - (((n - 1) * n) & 1);   // cannot exceed the complete graph
   const int words = (n + 31) / 32;                   // bitmap row pitch
-  uint32_t* bits = sm;                               // [n][words]
-  uint16_t* perm = reinterpret_cast<uint16_t*>(bits + (size_t)n * words);   // [n]
+  // [n][words]: in shared memory, or this graph's slice of the workspace (bits_ws, row pitch ceil(N/32))
+  uint32_t* bits = bits_ws ? bits_ws + (size_t)g * N * ((N + 31) / 32) : sm;
+  uint16_t* perm = reinterpret_cast<uint16_t*>(bits_ws ? sm : bits + (size_t)n * words);   // [n]
   uint32_t* edges = edges_in_smem ? reinterpret_cast<uint32_t*>(perm + ((n + 1) & ~1)) : edges_ws + (size_t)g * edges_per_graph;
   for (int k = threadIdx.x; k < n * words; k += blockDim.x) bits[k] = 0u;
   if (threadIdx.x == 0) {
@@ -130,9 +136,12 @@ regular_kernel(uint8_t* __restrict__ adj, int N, const int32_t* __restrict__ npg
   }
 }
 
-size_t regular_smem(int n, bool with_edges, long E) {
-  const int words = (n + 31) / 32;
-  return (size_t)n * words * 4 + (size_t)((n + 1) & ~1) * 2 + (with_edges ? (size_t)E * 4 : 0) + 16;
+size_t regular_bitmap_bytes(int n) { return (size_t)n * ((n + 31) / 32) * 4; }
+bool regular_bitmap_in_smem(int n) { return regular_bitmap_bytes(n) + (size_t)((n + 1) & ~1) * 2 + 16 <= kSmemCap; }
+size_t regular_edges_per_graph(int n) { return (size_t)n * n / 2 + 16; }
+
+size_t regular_smem(int n, bool with_bitmap, bool with_edges, long E) {
+  return (with_bitmap ? regular_bitmap_bytes(n) : 0) + (size_t)((n + 1) & ~1) * 2 + (with_edges ? (size_t)E * 4 : 0) + 16;
 }
 
 }  // namespace
@@ -140,8 +149,11 @@ size_t regular_smem(int n, bool with_edges, long E) {
 }  // namespace fgnn
 
 extern "C" size_t fgnn_generate_workspace_bytes(int32_t G, int32_t N, int32_t generator) {
-  if (generator != 1) return 256;
-  return fgnn::align_up((size_t)G * ((size_t)N * N / 2 + 16) * sizeof(uint32_t), 256);   // edge lists when they do not fit on chip
+  using namespace fgnn::gen;
+  if (generator != 1 || N < 1) return 256;
+  // edge lists and, above N = 1264, adjacency bitmaps when they do not fit on chip
+  const size_t bitmaps = regular_bitmap_in_smem(N) ? 0 : (size_t)G * regular_bitmap_bytes(N);
+  return fgnn::align_up((size_t)G * regular_edges_per_graph(N) * sizeof(uint32_t) + bitmaps, 256);
 }
 
 extern "C" int fgnn_generate_pairs_u8(uint8_t* adj1, uint8_t* adj2, int32_t G, int32_t N, const int32_t* n_per_graph,
@@ -151,18 +163,23 @@ extern "C" int fgnn_generate_pairs_u8(uint8_t* adj1, uint8_t* adj2, int32_t G, i
   using namespace fgnn::gen;
   cudaStream_t st = (cudaStream_t)stream;
   FGNN_CHECK_ARG(adj1 && adj2, "null pointer");
-  FGNN_CHECK_ARG(G >= 1 && G <= 65535 && N >= 2 && N <= 1024, "G=%d N=%d out of range", G, N);
+  FGNN_CHECK_ARG(G >= 1 && G <= 65535 && N >= 2 && N <= kMaxN, "graph generator supports G <= 65535 and 2 <= N <= %d (got G=%d N=%d)",
+                 kMaxN, G, N);
   FGNN_CHECK_ARG(edge_density > 0.f && edge_density < 1.f && noise >= 0.f && noise <= 1.f, "edge_density %f / noise %f out of range",
                  (double)edge_density, (double)noise);
   FGNN_CHECK_ARG(generator == 0 || generator == 1, "generator must be 0 (ErdosRenyi) or 1 (Regular); BarabasiAlbert is not built");
   const float pe2 = edge_density * noise / (1.f - edge_density);
   if (generator == 1) {
     FGNN_CHECK_ARG(workspace && workspace_bytes >= fgnn_generate_workspace_bytes(G, N, 1), "generator workspace too small");
-    const long E = (long)N * N / 2 + 16;
-    const bool in_smem = regular_smem(N, true, (long)N * ((int)(edge_density * N) + 1) / 2 + 1) <= 200 * 1024;
-    const size_t smem = regular_smem(N, in_smem, (long)N * ((int)(edge_density * N) + 1) / 2 + 1);
+    const long E = (long)regular_edges_per_graph(N);
+    const long e_max = (long)N * ((int)(edge_density * N) + 1) / 2 + 1;
+    const bool bits_in_smem = regular_bitmap_in_smem(N);
+    const bool in_smem = regular_smem(N, bits_in_smem, true, e_max) <= kSmemCap;
+    const size_t smem = regular_smem(N, bits_in_smem, in_smem, e_max);
+    uint32_t* edges_ws = static_cast<uint32_t*>(workspace);
+    uint32_t* bits_ws = bits_in_smem ? nullptr : edges_ws + (size_t)G * E;
     FGNN_CUDA(cudaFuncSetAttribute(regular_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    regular_kernel<<<G, 256, smem, st>>>(adj1, N, n_per_graph, edge_density, seed, static_cast<uint32_t*>(workspace), E, in_smem ? 1 : 0);
+    regular_kernel<<<G, 256, smem, st>>>(adj1, N, n_per_graph, edge_density, seed, edges_ws, E, in_smem ? 1 : 0, bits_ws);
     FGNN_LAUNCHED();
   }
   dim3 grid((N + 127) / 128, N, G);

@@ -11,7 +11,10 @@
 // compacted by swap-with-last) and keeps, among the columns of lowest path cost, the LAST unassigned one of the
 // list, else the FIRST assigned one; the kernel keeps the same list in shared memory and reduces over list
 // POSITIONS with that preference.  One CTA per graph: the scan of every Dijkstra step is spread over the CTA's
-// threads and closed by a block-wide arg-min; duals, path and matching arrays live in shared memory.
+// threads and closed by a block-wide arg-min; duals, path and matching arrays live in shared memory: 53 bytes per
+// column (smem_bytes), so the padded size N is limited by the device's opt-in shared memory per block -- N <= 4380 with
+// the 227 KB of an sm_100 device, 217 104 bytes at N = 4096.  Indices into the (G,N,N) scores are 64-bit; the rest are
+// column / row numbers < N.
 #include "fgnn_common.cuh"
 
 #include <cfloat>
@@ -186,6 +189,16 @@ lap_kernel(const float* __restrict__ scores, int32_t* __restrict__ col_of_row, i
 
 inline size_t smem_bytes(int N) { return align_up((size_t)N * (3 * sizeof(double) + 5 * sizeof(int) + 1), 16) + (size_t)N * 2 * sizeof(float) + 16; }
 
+// largest N whose dynamic shared memory fits next to the kernel's static shared memory in `limit` bytes
+int max_n(size_t limit) {
+  int lo = 0, hi = 1 << 16;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) / 2;
+    if (smem_bytes(mid) <= limit) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
 }  // namespace
 
 int lap_fwd(const float* scores, int32_t* col_of_row, int32_t* correct, double* total_cost, int G, int N,
@@ -193,7 +206,15 @@ int lap_fwd(const float* scores, int32_t* col_of_row, int32_t* correct, double* 
   FGNN_CHECK_ARG(scores && correct, "null pointer");
   FGNN_CHECK_ARG(G >= 1 && N >= 1, "bad sizes G=%d N=%d", G, N);
   const size_t smem = smem_bytes(N);
-  if (smem > 200 * 1024) return fail(FGNN_ERR_UNSUPPORTED, "linear assignment supports N <= 3800 (got %d)", N);
+  int dev = 0, optin = 0;
+  FGNN_CUDA(cudaGetDevice(&dev));
+  FGNN_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+  cudaFuncAttributes fa;
+  FGNN_CUDA(cudaFuncGetAttributes(&fa, lap_kernel));
+  const size_t limit = (size_t)optin > fa.sharedSizeBytes ? (size_t)optin - fa.sharedSizeBytes : 0;
+  if (smem > limit)
+    return fail(FGNN_ERR_UNSUPPORTED, "linear assignment supports N <= %d on this device (%d bytes of shared memory per block; got %d)",
+                max_n(limit), optin, N);
   FGNN_CUDA(cudaFuncSetAttribute(lap_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   lap_kernel<<<G, kThreads, smem, st>>>(scores, col_of_row, correct, total_cost, N, n_per_graph);
   FGNN_LAUNCHED();

@@ -25,6 +25,7 @@
 #include "fgnn_ptx.cuh"
 
 #include <algorithm>
+#include <climits>
 #include <type_traits>
 #include <cstdlib>
 #include <cstring>
@@ -36,7 +37,10 @@ using namespace ptx;
 
 namespace {
 
-constexpr int kMaxN = 1024;
+// Largest padded graph size of the 16-bit inference path (embedder, fused head).  At N = 4096 a plane holds
+// 4096 x 4352 = 17.8 M pixels and one graph 139 264 conv-chain tiles: per-graph pixel and tile indices fit in int,
+// and make_plan checks the per-launch tile count (see there).  Training keeps its own, lower limit (kMaxTrainN).
+constexpr int kMaxN = 4096;
 constexpr int kTileM = 128;  // pixels per MLP tile / physical rows per matmul tile
 constexpr int kTM1 = 127;    // logical rows per matmul tile
 
@@ -84,7 +88,8 @@ __device__ __forceinline__ int rows_cover(const int32_t* n_per_graph, int g, con
   int r = (phys_k_end(n_per_graph[g], geo.TN1) + 63) / 64 * 64;
   return r < geo.N ? r : geo.N;
 }
-// (32-bit tile arithmetic: a plane has at most 1024 x 1280 physical pixels, a launch at most 65535 planes' worth of tiles)
+// (32-bit tile arithmetic: a plane has at most kMaxN x NPC(kMaxN) = 4096 x 4352 physical pixels; the tile total of a
+// launch is bounded by make_plan)
 __device__ __forceinline__ int mlp_tiles(const int32_t* n_per_graph, int g, const Geo& geo) {
   return (rows_cover(n_per_graph, g, geo) * geo.NPC + kTileM - 1) / kTileM;
 }
@@ -139,8 +144,9 @@ to_planes_c_kernel(const float* __restrict__ x, T* __restrict__ out, int C, Geo 
 
 // uint8 adjacency (G,N,N) -> the two layout-C input planes of block 1: channel 0 = W, channel 1 = diag(W.sum(1))
 // (loaders/data_generator.py:118-125 without materialising the fp32 (G,2,N,N) tensor).  One warp per plane row;
-// values are 0/1 and integer degrees <= N <= 1024 (exact in fp16; bf16 rounds degrees above 256 exactly as
-// to_planes_kernel does on the fp32 features).
+// values are 0/1 and integer degrees <= N - 1 < 4096.  The degree is counted exactly and rounded to 16 bits once, to
+// nearest even, as the fp32 features are on the features-fed path: fp16 is exact up to 2048 and rounds larger degrees
+// to even numbers, bf16 is exact up to 256; both paths produce the same planes.
 template <typename T>
 __global__ void __launch_bounds__(256)
 adjacency_to_planes_kernel(const uint8_t* __restrict__ adj, T* __restrict__ out, Geo geo, long rows,
@@ -167,7 +173,8 @@ adjacency_to_planes_kernel(const uint8_t* __restrict__ adj, T* __restrict__ out,
   if (lane == 0 && i < n) d[i + i / geo.TN1] = Elem<T>::from_float((float)deg);
 }
 
-// zero the hole rows of layout-B planes (the conv kernel never writes them; they must contribute 0 to K sums)
+// zero the hole rows of layout-B planes (the conv kernel never writes them; they must contribute 0 to K sums).
+// idx < (PRB / BN) * NPC: 16 x 4352 at N = 4096.
 template <typename T>
 __global__ void zero_hole_rows_kernel(T* __restrict__ y, Geo geo) {
   T* plane = y + (long)blockIdx.y * geo.PSB;
@@ -1720,6 +1727,7 @@ int make_plan(const fgnn_embed_params& p, int G, int N, Plan& pl) {
     return fail(FGNN_ERR_UNSUPPORTED, "tensor-core path supports in/out_features 32 or 64 (got %d); use FGNN_FP32", pl.C);
   if (pl.cin0 > 64) return fail(FGNN_ERR_UNSUPPORTED, "original_features_num %d > 64 unsupported", pl.cin0);
   const int chunk_env = env_int("FGNN_TC_CHUNK", 0);
+  // per_graph: 16-bit planes of one graph (input, two block outputs, mult, Y1, Y2): 11.6 GB at N = 4096, C = 64
   long per_graph = ((long)(3 * pl.C + pl.cin0) * pl.geo.PSC + (long)pl.C * (pl.geo.PSA + pl.geo.PSB)) * 2;
   // activation planes of one pass: at most FGNN_TC_WS_GB (default 16) GB of the caller's workspace; the batch is cut
   // into EQUAL passes (64 graphs at the headline shape need 9.8 GB: one pass)
@@ -1729,6 +1737,12 @@ int make_plan(const fgnn_embed_params& p, int G, int N, Plan& pl) {
   chunk = std::min<long>(G, chunk);
   const long passes = (G + chunk - 1) / chunk;
   pl.chunk = (int)((G + passes - 1) / passes);
+  // The conv-chain kernel numbers the (graph, 128-pixel tile) work of a launch, times two fused MLPs, in int, and the
+  // pixel offset of a tile inside its graph too.  Refuse a plan whose counts could overflow rather than widen them.
+  const long tiles_per_graph = (pl.geo.PSC + kTileM - 1) / kTileM;
+  if (pl.geo.PSC > INT_MAX || (long)pl.chunk * 2 * tiles_per_graph > INT_MAX)
+    return fail(FGNN_ERR_UNSUPPORTED, "tensor-core path: %d graphs of N=%d per pass exceed the kernels' 32-bit tile counts",
+                pl.chunk, N);
   return FGNN_OK;
 }
 
@@ -1961,7 +1975,8 @@ int head_fwd(int precision, const float* e1, const float* e2, float* scores, flo
   if (!fgnn_device_supports_tcgen05())
     return fail(FGNN_ERR_UNSUPPORTED, "the fused head needs an sm_100 device (tcgen05); there is no fallback");
   FGNN_CHECK_ARG(e1 && e2 && ce_sum && correct && ws, "null pointer");
-  FGNN_CHECK_ARG(G >= 1 && G <= 65535 && N >= 1 && N <= kMaxN, "G=%d N=%d out of range", G, N);
+  FGNN_CHECK_ARG(G >= 1 && G <= 65535 && N >= 1 && N <= kMaxN, "fused head supports G <= 65535 and N <= %d (got G=%d N=%d)",
+                 kMaxN, G, N);
   FGNN_CHECK_ARG(C >= 16 && C <= 128 && C % 16 == 0, "the fused head needs an embedding width that is a multiple of 16, at most 128 (got %d)", C);
   if (ws_bytes < head_workspace_bytes(G, N)) return fail(FGNN_ERR_WORKSPACE, "head workspace too small");
   if (precision == FGNN_BF16) return head_fwd_t<__nv_bfloat16>(e1, e2, scores, ce_sum, correct, G, C, N, n_per_graph, ws, ws_bytes, st);
@@ -2002,7 +2017,7 @@ int debug_matmul(int precision, const float* a, const float* b, float* out, int 
                  const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
   if (!fgnn_device_supports_tcgen05()) return fail(FGNN_ERR_UNSUPPORTED, "needs an sm_100 device");
   FGNN_CHECK_ARG(a && b && out && ws, "null pointer");
-  FGNN_CHECK_ARG(N <= kMaxN, "N too large");
+  FGNN_CHECK_ARG(N <= kMaxN, "tensor-core matmul supports N <= %d (got %d)", kMaxN, N);
   if (precision == FGNN_BF16) return debug_matmul_t<__nv_bfloat16>(a, b, out, G, C, N, n_per_graph, ws, ws_bytes, st);
   if (precision == FGNN_FP16) return debug_matmul_t<__half>(a, b, out, G, C, N, n_per_graph, ws, ws_bytes, st);
   return fail(FGNN_ERR_INVALID, "precision must be FGNN_BF16 or FGNN_FP16");
@@ -2062,7 +2077,7 @@ int debug_mlp(int precision, const fgnn_mlp_params& mp, const float* x, float* y
               const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
   if (!fgnn_device_supports_tcgen05()) return fail(FGNN_ERR_UNSUPPORTED, "needs an sm_100 device");
   FGNN_CHECK_ARG(x && y && ws, "null pointer");
-  FGNN_CHECK_ARG(N <= kMaxN, "N too large");
+  FGNN_CHECK_ARG(N <= kMaxN, "tensor-core MLP supports N <= %d (got %d)", kMaxN, N);
   if (mp.c_out != 32 && mp.c_out != 64) return fail(FGNN_ERR_UNSUPPORTED, "c_out must be 32 or 64");
   if (precision == FGNN_BF16) return debug_mlp_t<__nv_bfloat16>(mp, x, y, G, N, n_per_graph, ws, ws_bytes, st);
   if (precision == FGNN_FP16) return debug_mlp_t<__half>(mp, x, y, G, N, n_per_graph, ws, ws_bytes, st);

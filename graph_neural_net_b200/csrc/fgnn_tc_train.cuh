@@ -890,7 +890,15 @@ struct TrainPlan {
   int C, cin0, D, nb, G;
 };
 
+// 16-bit training keeps every activation of the batch in one workspace (carve_train: about 51 plane sets per graph at
+// depth 3, 4 blocks; some 15 GB per graph at N = 2048, C = 32), so it stops at the padded size the inference path had
+// before it was extended to kMaxN.
+constexpr int kMaxTrainN = 1024;
+
 int make_train_plan(const fgnn_embed_params& p, int G, int N, TrainPlan& tp) {
+  if (N > kMaxTrainN)
+    return fail(FGNN_ERR_UNSUPPORTED, "16-bit training supports N <= %d (got %d): its workspace holds every activation of the "
+                "batch; embed larger graphs with the inference path (N <= %d)", kMaxTrainN, N, kMaxN);
   Plan pl;
   if (int e = make_plan(p, G, N, pl)) return e;
   tp.geo = pl.geo;

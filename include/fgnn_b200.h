@@ -148,7 +148,9 @@ int fgnn_features_from_adjacency_u8(const uint8_t* adj, float* out, int32_t G, i
  * generator 0 = "ErdosRenyi" (:39-44), 1 = "Regular" (:58-68: d = int(edge_density n), +1 if n d is odd; sampled by the
  * switch chain from a relabelled circulant graph), and adj2[g] = noise_erdos_renyi(adj1[g]) = W (1 - N1) + (1 - W) N2,
  * N1 ~ ER(noise), N2 ~ ER(edge_density noise / (1 - edge_density)) (:79-87).  uint8 (G,N,N), zero outside n_g x n_g;
- * counter-based generator: the same seed gives the same graphs.  Parity with networkx is distributional. */
+ * counter-based generator: the same seed gives the same graphs.  Parity with networkx is distributional.
+ * 2 <= N <= 4096.  "Regular" runs its switch chain on one thread per graph (10 |E| proposals, time grows with |E|);
+ * its workspace holds the edge lists and, above N = 1264, the adjacency bitmaps (G N ceil(N/32) words). */
 size_t fgnn_generate_workspace_bytes(int32_t G, int32_t N, int32_t generator);
 int fgnn_generate_pairs_u8(uint8_t* adj1, uint8_t* adj2, int32_t G, int32_t N, const int32_t* n_per_graph,
                            int32_t generator, float edge_density, float noise, uint64_t seed, void* workspace,
@@ -180,7 +182,7 @@ int fgnn_ce_bwd_f32(const float* scores, const float* row_lse, const float* coef
  * (toolbox/metrics.py:125-134) in the epilogue of the tcgen05 GEMM, flash style: online row max / sum of exponentials
  * over 256-column tiles.  e1,e2 (G,C,N) fp32 are split into 16-bit (hi, lo) operand pairs in shared memory
  * (Ahi Bhi + Alo Bhi + Ahi Blo: fp32-level accuracy), C a multiple of 16, at most 128.  ce_sum[G], correct[G] as
- * fgnn_ce_argmax_fwd_f32; scores (G,N,N) is written only when non-NULL (zero outside the n_g x n_g block).
+ * fgnn_ce_argmax_fwd_f32; scores (G,N,N) is written only when non-NULL (zero outside the n_g x n_g block).  N <= 4096.
  * Forward only (training differentiates through fgnn_scores_* / fgnn_ce_*). */
 size_t fgnn_head_workspace_bytes(int32_t G, int32_t N);
 int fgnn_head_fwd(int32_t precision, const float* e1, const float* e2, float* scores, float* ce_sum, int32_t* correct,
@@ -192,7 +194,9 @@ int fgnn_head_fwd(int32_t precision, const float* e1, const float* e2, float* sc
  * cost = -log_softmax(scores, -1) (fp32 weights formed in the kernel), found on the device by shortest augmenting
  * paths in double precision with scipy's operation order and tie rule, one CTA per graph.  scores (G,N,N);
  * col_of_row (G,N) int32 (rows >= n_g get -1; may be NULL); correct[G] = #rows with col(i) == i;
- * total_cost[G] = sum_i cost[i, col(i)] (may be NULL). */
+ * total_cost[G] = sum_i cost[i, col(i)] (may be NULL).  The working arrays take 53 N bytes of shared memory, so N is
+ * limited by the device's opt-in shared memory per block: N <= 4380 on sm_100 (227 KB); beyond it the call fails
+ * with FGNN_ERR_UNSUPPORTED and states the limit. */
 int fgnn_lap_fwd(const float* scores, int32_t* col_of_row, int32_t* correct, double* total_cost, int32_t G,
                  int32_t N, const int32_t* n_per_graph, void* stream);
 
@@ -203,8 +207,10 @@ int fgnn_lap_fwd(const float* scores, int32_t* col_of_row, int32_t* correct, dou
  * (models/utils.py:63-69, models/blocks_emb.py:16-43, models/trainers.py:64-65).
  *   precision FGNN_FP32 : composition of the fp32 operators above.
  *   precision FGNN_BF16 / FGNN_FP16 : TMA + tcgen05/TMEM kernels; activations live in HBM as
- *     16-bit pre-normalisation planes, GraphNorm is folded into the consumers (DESIGN.md).
- * workspace: fgnn_embed_workspace_bytes(...) bytes, 1024-byte aligned. */
+ *     16-bit pre-normalisation planes, GraphNorm is folded into the consumers (DESIGN.md).  N <= 4096; the
+ *     batch is cut into passes of equal size, each within FGNN_TC_WS_GB (default 16) GB of planes when a graph
+ *     fits (one graph takes 11.6 GB at N = 4096, C = 64, a pass is never less than one graph).
+ * workspace: fgnn_embed_workspace_bytes(...) bytes, 1024-byte aligned (0 when the shape is unsupported). */
 size_t fgnn_embed_workspace_bytes(const fgnn_embed_params* p, int32_t precision, int32_t G, int32_t N);
 int fgnn_embed_fwd(const fgnn_embed_params* p, int32_t precision, const float* x, float* emb,
                    int32_t G, int32_t N, const int32_t* n_per_graph, void* workspace, size_t workspace_bytes,
@@ -228,7 +234,8 @@ int fgnn_embed_fwd_adjacency_u8(const fgnn_embed_params* p, int32_t precision, c
  * As with the reference's AMP GradScaler, fp16 gradient planes can overflow for a given scale: the parameter
  * gradients are then non-finite and the caller skips the step and lowers grad_scale_log2 (training.py does; 9 is
  * the default, -24 .. 15 accepted; bf16 never overflows).  The workspace must be the one the forward call filled
- * (same G, N, parameters), fgnn_embed_train_workspace_bytes(...) bytes, 1024-byte aligned. */
+ * (same G, N, parameters), fgnn_embed_train_workspace_bytes(...) bytes, 1024-byte aligned.  N <= 1024: the
+ * workspace keeps every activation of the batch. */
 size_t fgnn_embed_train_workspace_bytes(const fgnn_embed_params* p, int32_t precision, int32_t G, int32_t N);
 int fgnn_embed_fwd_train(const fgnn_embed_params* p, int32_t precision, const float* x, float* emb, int32_t G,
                          int32_t N, const int32_t* n_per_graph, void* workspace, size_t workspace_bytes,
