@@ -44,9 +44,16 @@ constexpr int kMaxN = 4096;
 constexpr int kTileM = 128;  // pixels per MLP tile / physical rows per matmul tile
 constexpr int kTM1 = 127;    // logical rows per matmul tile
 
+// The three plane layouts (see the top of this file).  Their row counts, plane strides and logical -> physical row maps
+// are Geo's rows(), stride() and phys_row(); nothing else works them out.
+enum Layout { kLayoutC, kLayoutA, kLayoutB };
+
 struct Geo {
   int N, BN, TN1, NT, NPC, MT, PRA, PRB, BNLOG;
   long PSC, PSA, PSB;
+  __host__ __device__ int rows(Layout l) const { return l == kLayoutA ? PRA : (l == kLayoutB ? PRB : N); }
+  __host__ __device__ long stride(Layout l) const { return l == kLayoutA ? PSA : (l == kLayoutB ? PSB : PSC); }
+  __host__ __device__ int phys_row(int i, Layout l) const { return l == kLayoutA ? i + i / kTM1 : (l == kLayoutB ? i + i / TN1 : i); }
 };
 
 inline int round_up(int v, int a) { return (v + a - 1) / a * a; }
@@ -98,28 +105,26 @@ __device__ __forceinline__ int mlp_tiles(const int32_t* n_per_graph, int g, cons
 // small CUDA-core kernels
 // =============================================================================================
 
-// fp32 (G,C,N,N) -> 16-bit planes in layout C (mode 0), A (mode 1) or B (mode 2).  Padding, holes and the
-// ones row/column are written as zero (only the debug entry points use layouts A / B).
+// fp32 (G,C,N,N) -> 16-bit planes in layout A or B (the operands of debug_matmul).  Padding, holes and the inserted
+// rows are written as zero.
 template <typename T>
-__global__ void to_planes_kernel(const float* __restrict__ x, T* __restrict__ out, int C, Geo geo, int mode,
+__global__ void to_planes_kernel(const float* __restrict__ x, T* __restrict__ out, int C, Geo geo, Layout l,
                                  const int32_t* __restrict__ n_per_graph) {
   const int gc = blockIdx.y;
   const int g = gc / C;
   const int n = graph_n(n_per_graph, g, geo.N);
-  const long PS = mode == 0 ? geo.PSC : (mode == 1 ? geo.PSA : geo.PSB);
+  const long PS = geo.stride(l);
+  const int period = l == kLayoutA ? kTileM : geo.BN;   // physical rows per inserted row
   for (long p = (long)blockIdx.x * blockDim.x + threadIdx.x; p < PS; p += (long)gridDim.x * blockDim.x) {
     const int pi = (int)(p / geo.NPC), pj = (int)(p % geo.NPC);
-    bool hole = (pj % geo.BN) == geo.BN - 1;
-    const int j = pj - pj / geo.BN;
-    int i = pi;
-    if (mode == 1) { hole = hole || (pi % 128) == 127; i = pi - pi / 128; }
-    if (mode == 2) { hole = hole || (pi % geo.BN) == geo.BN - 1; i = pi - pi / geo.BN; }
+    const bool hole = (pj % geo.BN) == geo.BN - 1 || (pi % period) == period - 1;
+    const int i = pi - pi / period, j = pj - pj / geo.BN;
     float v = (!hole && i < n && j < n) ? x[((long)gc * geo.N + i) * geo.N + j] : 0.f;
     out[(long)gc * PS + p] = Elem<T>::from_float(v);
   }
 }
 
-// the layout-C case of to_planes_kernel, row-wise: no per-element division (BN is a power of two), two pixels per 32-bit store
+// fp32 (G,C,N,N) -> 16-bit layout-C planes, row-wise: no per-element division (BN is a power of two), two pixels per 32-bit store
 template <typename T>
 __global__ void __launch_bounds__(256)
 to_planes_c_kernel(const float* __restrict__ x, T* __restrict__ out, int C, Geo geo, const int32_t* __restrict__ n_per_graph) {
@@ -173,15 +178,16 @@ adjacency_to_planes_kernel(const uint8_t* __restrict__ adj, T* __restrict__ out,
   if (lane == 0 && i < n) d[i + i / geo.TN1] = Elem<T>::from_float((float)deg);
 }
 
-// zero the hole rows of layout-B planes (the conv kernel never writes them; they must contribute 0 to K sums).
-// idx < (PRB / BN) * NPC: 16 x 4352 at N = 4096.
+// zero the inserted rows, which the conv kernel never stores: rows 127 mod 128 of layout A (ones rows; the backward GEMM
+// Y1^T dM runs its K index over them), rows BN-1 mod BN of layout B (hole rows, 0 in K sums).  idx < 33 x 4352 at N = 4096.
 template <typename T>
-__global__ void zero_hole_rows_kernel(T* __restrict__ y, Geo geo) {
-  T* plane = y + (long)blockIdx.y * geo.PSB;
-  const int nholes = geo.PRB / geo.BN;
-  for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < nholes * geo.NPC; idx += gridDim.x * blockDim.x) {
+__global__ void zero_inserted_rows_kernel(T* __restrict__ y, Geo geo, Layout l) {
+  T* plane = y + (long)blockIdx.y * geo.stride(l);
+  const int period = l == kLayoutA ? kTileM : geo.BN;
+  const int nrows = geo.rows(l) / period;
+  for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < nrows * geo.NPC; idx += gridDim.x * blockDim.x) {
     const int h = idx / geo.NPC, col = idx % geo.NPC;
-    plane[(long)(h * geo.BN + geo.BN - 1) * geo.NPC + col] = Elem<T>::from_float(0.f);
+    plane[(long)(h * period + period - 1) * geo.NPC + col] = Elem<T>::from_float(0.f);
   }
 }
 
@@ -202,16 +208,8 @@ __global__ void from_planes_kernel(const T* __restrict__ in, float* __restrict__
   }
 }
 
-// fp32 hidden-layer weights (co, ci) -> 16-bit [co][Kh] zero padded (Kh multiple of 64)
-template <typename T>
-__global__ void convert_weight_kernel(const float* __restrict__ w, T* __restrict__ out, int co, int ci, int Kh) {
-  int idx = blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= co * Kh) return;
-  int o = idx / Kh, k = idx % Kh;
-  out[idx] = Elem<T>::from_float(k < ci ? w[o * ci + k] : 0.f);
-}
-
-// the same for all hidden-layer matrices of one block in ONE launch (blockIdx.y = matrix)
+// fp32 hidden-layer weights (co, ci) -> 16-bit [co][Kh] zero padded (Kh multiple of 64), for up to all hidden-layer
+// matrices of one block in ONE launch (blockIdx.y = matrix)
 struct ConvertBatch {
   const float* src[3 * (FGNN_MAX_DEPTH - 1)];
   long dst_off[3 * (FGNN_MAX_DEPTH - 1)];   // element offset of the matrix in `out`
@@ -365,8 +363,6 @@ __global__ void finalize_coef_kernel(CoefArgs a, int total) {
 // TMEM: accumulator of slot s in columns [s COUT, +COUT), its packed hidden activations and the ones columns of the
 // hidden layers' bias step in [kSlots COUT + s (COUT/2 + 8), + COUT/2 + 8).
 // =============================================================================================
-enum OutMode { kOutC = 0, kOutA = 1, kOutB = 2 };   // output plane layout: rows i / i + i/127 / i + i/(BN-1)
-
 template <typename T>
 struct MlpArgs {
   int G;
@@ -377,8 +373,8 @@ struct MlpArgs {
   const T* bias1_tile;                       // [G][NMLP COUT / 8][2][8][8] the same as a K = 16 MMA step (depth > 1 launches)
   const float* bias[2][FGNN_MAX_DEPTH];      // per MLP, layer l >= 1 biases
   T* out[2];                                 // per MLP output planes (direct stores of the ones row only)
-  int out_mode[2];                           // kOutC / kOutA / kOutB
-  int ones[2];                               // kOutA: write the ones rows; kOutB: holes hold ones
+  Layout out_mode[2];                        // output plane layout
+  int ones[2];                               // kLayoutA: write the ones rows; kLayoutB: holes hold ones
   double* stat_acc;                          // [G][NMLP][COUT][2]
   // Fused column-max pooling (last block): when rowenc[m] is set, MLP m's tile is NOT stored; the statistics pass
   // folds the row-wise max and min of its valid pixels into rowenc[m][g][c][i][2] (order-preserving unsigned codes
@@ -814,9 +810,9 @@ tc_mlp_kernel(const __grid_constant__ CUtensorMap map_x0, const __grid_constant_
       const bool hole = (pj & (geo.BN - 1)) == geo.BN - 1;
       const int j = pj - (pj >> geo.BNLOG);
       const bool valid = in_plane && !hole && pi < n && j < n;
-      const int mode = args.out_mode[m];
+      const Layout mode = args.out_mode[m];
       // holes of Y2 (layout B) hold ones on valid rows: they are the matmul's ones column
-      const float marker = (hole && mode == kOutB && args.ones[m] && pi < n) ? 1.f : 0.f;
+      const float marker = (hole && mode == kLayoutB && args.ones[m] && pi < n) ? 1.f : 0.f;
       {
         // Transposing store: the 16x256b TMEM load hands every thread channel PAIRS of four pixels (the mma
         // C-fragment layout), one packed convert per pair, and stmatrix.trans writes 8 channels x 8 pixels as
@@ -911,18 +907,18 @@ tc_mlp_kernel(const __grid_constant__ CUtensorMap map_x0, const __grid_constant_
       if (storer) {
         // store it: one 64-pixel half per TMA (a half never straddles a row because NPC % 64 == 0)
         const CUtensorMap* mo = (m == 0) ? &map_o0 : &map_o1;
-        const int prw = pi, col = pj;
-        const int prow = (mode == kOutA) ? prw + prw / kTM1 : (mode == kOutB ? prw + prw / geo.TN1 : prw);
-        if (prw < geo.N) tma_store_3d(mo, tile + (size_t)(quad >> 1) * (COUT * 128), col, prow, g * COUT);
+        const int prow = geo.phys_row(pi, mode);
+        if (pi < geo.N) tma_store_3d(mo, tile + (size_t)(quad >> 1) * (COUT * 128), pj, prow, g * COUT);
         bulk_commit_group();
       }
       // ones rows of Y1 (layout A): the last logical row of every 127-row matmul tile writes the row below it
-      if (mode == kOutA && args.ones[m] && in_plane && pi < n) {
+      if (mode == kLayoutA && args.ones[m] && in_plane && pi < n) {
         const int mt = pi / kTM1;
         if (pi - mt * kTM1 == kTM1 - 1 || pi == n - 1) {
-          T* o1 = args.out[m] + (long)g * COUT * geo.PSA + (long)(mt * 128 + 127) * geo.NPC + pj;
+          const long ps = geo.stride(kLayoutA);
+          T* o1 = args.out[m] + (long)g * COUT * ps + (long)(mt * 128 + 127) * geo.NPC + pj;
           const T ov = Elem<T>::from_float((!hole && j < n) ? 1.f : 0.f);
-          for (int cc = 0; cc < COUT; ++cc) o1[(long)cc * geo.PSA] = ov;
+          for (int cc = 0; cc < COUT; ++cc) o1[(long)cc * ps] = ov;
         }
       }
       // ---------------- statistics of the staged tile: sum / sum of squares per channel (+ row max / min) ----------------
@@ -1506,6 +1502,27 @@ int make_map3(CUtensorMap* m, int fmt_is_bf16, const void* base, uint64_t d0, ui
   return FGNN_OK;
 }
 
+// [planes][rows][NPC] view of planes in layout l, boxes of 64 columns x box_rows rows x box_planes planes
+template <typename T>
+int plane_map(CUtensorMap* m, const T* base, Layout l, const Geo& geo, uint64_t planes, uint32_t box_rows, uint32_t box_planes = 1) {
+  return make_map3(m, Elem<T>::kFmt, base, geo.NPC, geo.rows(l), planes, geo.NPC, (uint64_t)geo.stride(l), 64, box_rows, box_planes);
+}
+
+// flat [G][channels][PSC] view of layout-C planes: each plane is one row of PSC pixels; boxes of 64 pixels x box_channels
+// channels of one graph (channels beyond `channels` are zero-filled)
+template <typename T>
+int pixel_map(CUtensorMap* m, const T* base, int channels, int G, const Geo& geo, uint32_t box_channels) {
+  return make_map3(m, Elem<T>::kFmt, base, geo.PSC, channels, G, geo.PSC, (uint64_t)channels * geo.PSC, 64, box_channels);
+}
+
+// f(std::integral_constant<int, BN>{}) for the geometry's BN: the 128 x BN tile kernels are instantiated per BN
+template <typename F>
+int with_bn(const Geo& geo, F&& f) {
+  if (geo.BN == 64) return f(std::integral_constant<int, 64>{});
+  if (geo.BN == 128) return f(std::integral_constant<int, 128>{});
+  return f(std::integral_constant<int, 256>{});
+}
+
 int num_sms() {   // of the CURRENT device (a process may drive several GPUs): not cached across devices
   static int cache[64] = {0};
   int dev = 0;
@@ -1527,28 +1544,28 @@ int env_int(const char* name, int dflt) {
 template <typename T>
 int launch_matmul(const T* y1, const T* y2, T* out, const float* coef_a, const float* coef_b, int G, int C,
                   const Geo& geo, const int32_t* npg, cudaStream_t st) {
-  constexpr int is_bf16 = Elem<T>::kFmt;
   CUtensorMap ma, mb;
   const uint64_t planes = (uint64_t)G * C;
   // K = physical column of Y1 (layout A) = physical row of Y2 (layout B); reads past either extent are zero filled
-  if (int e = make_map3(&ma, is_bf16, y1, geo.NPC, geo.PRA, planes, geo.NPC, (uint64_t)geo.PSA, 64, 128)) return e;
-  if (int e = make_map3(&mb, is_bf16, y2, geo.NPC, geo.PRB, planes, geo.NPC, (uint64_t)geo.PSB, 64, 64)) return e;
+  if (int e = plane_map(&ma, y1, kLayoutA, geo, planes, 128)) return e;
+  if (int e = plane_map(&mb, y2, kLayoutB, geo, planes, 64)) return e;
   // output (layout C) as 64-column x 32-row (31 for the quadrant that ends with the ones row) store boxes
   CUtensorMap mo32, mo31;
-  if (int e = make_map3(&mo32, is_bf16, out, geo.NPC, geo.N, planes, geo.NPC, (uint64_t)geo.PSC, 64, 32)) return e;
-  if (int e = make_map3(&mo31, is_bf16, out, geo.NPC, geo.N, planes, geo.NPC, (uint64_t)geo.PSC, 64, 31)) return e;
+  if (int e = plane_map(&mo32, out, kLayoutC, geo, planes, 32)) return e;
+  if (int e = plane_map(&mo31, out, kLayoutC, geo, planes, 31)) return e;
   MatmulArgs<T> a{G, C, geo, out, coef_a, coef_b, npg};
   const int grid = num_sms();
-  auto kernel = geo.BN == 64 ? tc_matmul_kernel<T, 64> : geo.BN == 128 ? tc_matmul_kernel<T, 128> : tc_matmul_kernel<T, 256>;
-  const size_t smem = geo.BN == 64 ? MatmulCfg<64>::kSmemBytes
-                                   : geo.BN == 128 ? MatmulCfg<128>::kSmemBytes : MatmulCfg<256>::kSmemBytes;
-  prof::begin(prof::kMatmul, st);
-  // per device and cheap: set on every call
-  FGNN_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  kernel<<<grid, 192, smem, st>>>(ma, mb, mo32, mo31, a);
-  prof::end(prof::kMatmul, st);
-  FGNN_LAUNCHED();
-  return FGNN_OK;
+  return with_bn(geo, [&](auto bn) -> int {
+    constexpr int BN = decltype(bn)::value;
+    const size_t smem = MatmulCfg<BN>::kSmemBytes;
+    prof::begin(prof::kMatmul, st);
+    // per device and cheap: set on every call
+    FGNN_CUDA(cudaFuncSetAttribute(tc_matmul_kernel<T, BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    tc_matmul_kernel<T, BN><<<grid, 192, smem, st>>>(ma, mb, mo32, mo31, a);
+    prof::end(prof::kMatmul, st);
+    FGNN_LAUNCHED();
+    return FGNN_OK;
+  });
 }
 
 // fold + conv chain(s) + statistics finalisation for 1 or 2 MLPs sharing their input
@@ -1565,7 +1582,7 @@ struct MlpGroup {
   T* bt;             // [G][nmlp][C][16] folded first-layer bias as an MMA step (may be null for depth-1 launches)
   const T* wh;       // [nmlp][depth-1][C][Kh]
   T* out[2];
-  int out_mode[2];
+  Layout out_mode[2];
   int ones[2];
   float* coef[2];
   double* stat_acc;  // [G][nmlp][C][2], zeroed by the launch
@@ -1578,7 +1595,6 @@ struct MlpGroup {
 
 template <typename T, int COUT, int NMLP>
 int launch_mlp_t(const MlpGroup<T>& M, int G, const Geo& geo, const int32_t* npg, cudaStream_t st) {
-  constexpr int is_bf16 = Elem<T>::kFmt;
   MlpArgs<T> a{};
   a.G = G;
   a.geo = geo;
@@ -1604,18 +1620,16 @@ int launch_mlp_t(const MlpGroup<T>& M, int G, const Geo& geo, const int32_t* npg
   a.n_per_graph = npg;
   FGNN_CHECK_ARG(a.K1 <= 256, "first-layer K=%d too wide for the tensor-core MLP kernel", a.K1);
   CUtensorMap mx0, mx1, mw1, mwh, mo[2];
-  for (int m = 0; m < NMLP; ++m) {
-    const int rows = M.out_mode[m] == kOutA ? geo.PRA : (M.out_mode[m] == kOutB ? geo.PRB : geo.N);
-    if (int e = make_map3(&mo[m], is_bf16, M.out[m], geo.NPC, rows, (uint64_t)G * COUT, geo.NPC, (uint64_t)rows * geo.NPC,
-                          64, 1, COUT)) return e;
-  }
+  for (int m = 0; m < NMLP; ++m)   // one 64-pixel row piece of all COUT channels per store
+    if (int e = plane_map(&mo[m], M.out[m], M.out_mode[m], geo, (uint64_t)G * COUT, 1, COUT)) return e;
   if (NMLP == 1) mo[1] = mo[0];
-  if (int e = make_map3(&mx0, is_bf16, M.src[0], geo.PSC, M.c_src[0], G, geo.PSC, (uint64_t)M.c_src[0] * geo.PSC, 64, a.k_src[0])) return e;
+  if (int e = pixel_map(&mx0, M.src[0], M.c_src[0], G, geo, a.k_src[0])) return e;
   if (M.nsrc > 1) {
-    if (int e = make_map3(&mx1, is_bf16, M.src[1], geo.PSC, M.c_src[1], G, geo.PSC, (uint64_t)M.c_src[1] * geo.PSC, 64, a.k_src[1])) return e;
+    if (int e = pixel_map(&mx1, M.src[1], M.c_src[1], G, geo, a.k_src[1])) return e;
   } else {
     mx1 = mx0;
   }
+  constexpr int is_bf16 = Elem<T>::kFmt;
   if (int e = make_map3(&mw1, is_bf16, M.wf, a.K1g, COUT, (uint64_t)G * NMLP, a.K1g, (uint64_t)COUT * a.K1g, 64, COUT)) return e;
   if (a.depth > 1) {
     if (int e = make_map3(&mwh, is_bf16, M.wh, a.Kh, COUT, (uint64_t)NMLP * (a.depth - 1), a.Kh, (uint64_t)COUT * a.Kh, 64, COUT)) return e;
@@ -1758,12 +1772,12 @@ struct Buffers {
 };
 
 size_t carve(const Plan& pl, int num_blocks, Arena& ar, Buffers& B) {
-  const size_t actC = (size_t)pl.chunk * pl.C * pl.geo.PSC;
-  B.xin = ar.take<uint16_t>((size_t)pl.chunk * pl.cin0 * pl.geo.PSC, 1024);
+  const size_t actC = (size_t)pl.chunk * pl.C * pl.geo.stride(kLayoutC);
+  B.xin = ar.take<uint16_t>((size_t)pl.chunk * pl.cin0 * pl.geo.stride(kLayoutC), 1024);
   B.xa = ar.take<uint16_t>(actC, 1024);
   B.xb = ar.take<uint16_t>(actC, 1024);
-  B.y1 = ar.take<uint16_t>((size_t)pl.chunk * pl.C * pl.geo.PSA, 1024);
-  B.y2 = ar.take<uint16_t>((size_t)pl.chunk * pl.C * pl.geo.PSB, 1024);
+  B.y1 = ar.take<uint16_t>((size_t)pl.chunk * pl.C * pl.geo.stride(kLayoutA), 1024);
+  B.y2 = ar.take<uint16_t>((size_t)pl.chunk * pl.C * pl.geo.stride(kLayoutB), 1024);
   B.mult = ar.take<uint16_t>(actC, 1024);
   const size_t nc = (size_t)pl.chunk * pl.C;
   B.coef1 = ar.take<float>(nc * 2);
@@ -1829,7 +1843,7 @@ int embed_fwd_t(const fgnn_embed_params& p, const float* x, const uint8_t* adj, 
     }
     {
       dim3 grid(4, gc * C);
-      zero_hole_rows_kernel<T><<<grid, 256, 0, st>>>(reinterpret_cast<T*>(B.y2), geo);
+      zero_inserted_rows_kernel<T><<<grid, 256, 0, st>>>(reinterpret_cast<T*>(B.y2), geo, kLayoutB);
       FGNN_LAUNCHED();
     }
     const T* cur = reinterpret_cast<const T*>(B.xin);
@@ -1850,8 +1864,8 @@ int embed_fwd_t(const fgnn_embed_params& p, const float* x, const uint8_t* adj, 
         M.src[0] = cur; M.c_src[0] = cur_c; M.src_coef[0] = cur_coef; M.nsrc = 1;
         M.wf = reinterpret_cast<T*>(B.wf12); M.bf = B.bf12; M.bt = reinterpret_cast<T*>(B.bt12);
         M.wh = whb;
-        M.out[0] = y1; M.out_mode[0] = kOutA; M.ones[0] = 1; M.coef[0] = B.coef1;
-        M.out[1] = y2; M.out_mode[1] = kOutB; M.ones[1] = 1; M.coef[1] = B.coef2;
+        M.out[0] = y1; M.out_mode[0] = kLayoutA; M.ones[0] = 1; M.coef[0] = B.coef1;
+        M.out[1] = y2; M.out_mode[1] = kLayoutB; M.ones[1] = 1; M.coef[1] = B.coef2;
         M.stat_acc = B.stat_acc;
         if (int e = run_mlp_group<T>(M, C, gc, geo, n_c, st)) return e;
       }
@@ -1864,7 +1878,7 @@ int embed_fwd_t(const fgnn_embed_params& p, const float* x, const uint8_t* adj, 
         M.src[1] = cur; M.c_src[1] = cur_c; M.src_coef[1] = cur_coef; M.nsrc = 2;
         M.wf = reinterpret_cast<T*>(B.wf3); M.bf = B.bf3; M.bt = reinterpret_cast<T*>(B.bt3);
         M.wh = whb + (size_t)2 * dm1 * C * Kh;
-        M.out[0] = nxt; M.out_mode[0] = kOutC; M.ones[0] = 0; M.coef[0] = nxt_coef;
+        M.out[0] = nxt; M.out_mode[0] = kLayoutC; M.ones[0] = 0; M.coef[0] = nxt_coef;
         M.stat_acc = B.stat_acc;
         if (b == p.num_blocks - 1) {
           // the last block's output is only ever max-pooled: keep its row max / min and never write the planes
@@ -1889,6 +1903,17 @@ int embed_fwd_t(const fgnn_embed_params& p, const float* x, const uint8_t* adj, 
 
 #include "fgnn_tc_train.cuh"
 
+// Guard of the 16-bit entry points: an sm_100 device, then f(T{}) with T the element type of `precision`; any other
+// precision is refused.
+template <typename F>
+int with_16bit(int precision, const char* what, F&& f) {
+  if (!fgnn_device_supports_tcgen05())
+    return fail(FGNN_ERR_UNSUPPORTED, "%s needs an sm_100 device (tcgen05); there is no fallback", what);
+  if (precision == FGNN_BF16) return f(__nv_bfloat16{});
+  if (precision == FGNN_FP16) return f(__half{});
+  return fail(FGNN_ERR_INVALID, "%s supports FGNN_BF16 / FGNN_FP16 only (got precision %d)", what, precision);
+}
+
 }  // namespace
 
 size_t embed_train_workspace_bytes(const fgnn_embed_params& p, int G, int N) {
@@ -1901,23 +1926,19 @@ size_t embed_train_workspace_bytes(const fgnn_embed_params& p, int G, int N) {
 
 int embed_fwd_train(const fgnn_embed_params& p, int precision, const float* x, float* emb, int G, int N,
                     const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
-  if (!fgnn_device_supports_tcgen05())
-    return fail(FGNN_ERR_UNSUPPORTED, "FGNN_BF16/FGNN_FP16 need an sm_100 device (tcgen05); there is no fallback");
-  if (reinterpret_cast<uintptr_t>(ws) & 1023) return fail(FGNN_ERR_INVALID, "workspace must be 1024-byte aligned");
-  if (precision == FGNN_BF16) return embed_fwd_train_t<__nv_bfloat16>(p, x, emb, G, N, n_per_graph, ws, ws_bytes, st);
-  if (precision == FGNN_FP16) return embed_fwd_train_t<__half>(p, x, emb, G, N, n_per_graph, ws, ws_bytes, st);
-  return fail(FGNN_ERR_INVALID, "fgnn_embed_fwd_train is the 16-bit training path (FGNN_BF16 / FGNN_FP16)");
+  return with_16bit(precision, "fgnn_embed_fwd_train", [&](auto t) -> int {
+    if (reinterpret_cast<uintptr_t>(ws) & 1023) return fail(FGNN_ERR_INVALID, "workspace must be 1024-byte aligned");
+    return embed_fwd_train_t<decltype(t)>(p, x, emb, G, N, n_per_graph, ws, ws_bytes, st);
+  });
 }
 
 int embed_bwd(const fgnn_embed_params& p, const fgnn_embed_grads& g, int precision, const float* demb, int grad_scale_log2,
               int G, int N, const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
-  if (!fgnn_device_supports_tcgen05())
-    return fail(FGNN_ERR_UNSUPPORTED, "FGNN_BF16/FGNN_FP16 need an sm_100 device (tcgen05); there is no fallback");
-  if (reinterpret_cast<uintptr_t>(ws) & 1023) return fail(FGNN_ERR_INVALID, "workspace must be 1024-byte aligned");
-  if (grad_scale_log2 < -24 || grad_scale_log2 > 15) return fail(FGNN_ERR_INVALID, "grad_scale_log2 %d outside [-24, 15]", grad_scale_log2);
-  if (precision == FGNN_BF16) return embed_bwd_t<__nv_bfloat16>(p, g, demb, grad_scale_log2, G, N, n_per_graph, ws, ws_bytes, st);
-  if (precision == FGNN_FP16) return embed_bwd_t<__half>(p, g, demb, grad_scale_log2, G, N, n_per_graph, ws, ws_bytes, st);
-  return fail(FGNN_ERR_INVALID, "fgnn_embed_bwd is the 16-bit training path (FGNN_BF16 / FGNN_FP16)");
+  return with_16bit(precision, "fgnn_embed_bwd", [&](auto t) -> int {
+    if (reinterpret_cast<uintptr_t>(ws) & 1023) return fail(FGNN_ERR_INVALID, "workspace must be 1024-byte aligned");
+    if (grad_scale_log2 < -24 || grad_scale_log2 > 15) return fail(FGNN_ERR_INVALID, "grad_scale_log2 %d outside [-24, 15]", grad_scale_log2);
+    return embed_bwd_t<decltype(t)>(p, g, demb, grad_scale_log2, G, N, n_per_graph, ws, ws_bytes, st);
+  });
 }
 
 size_t embed_workspace_bytes(const fgnn_embed_params& p, int G, int N) {
@@ -1930,23 +1951,20 @@ size_t embed_workspace_bytes(const fgnn_embed_params& p, int G, int N) {
 
 int embed_fwd(const fgnn_embed_params& p, int precision, const float* x, float* emb, int G, int N,
               const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
-  if (!fgnn_device_supports_tcgen05())
-    return fail(FGNN_ERR_UNSUPPORTED, "FGNN_BF16/FGNN_FP16 need an sm_100 device (tcgen05); there is no fallback");
-  if (reinterpret_cast<uintptr_t>(ws) & 1023) return fail(FGNN_ERR_INVALID, "workspace must be 1024-byte aligned");
-  if (precision == FGNN_BF16) return embed_fwd_t<__nv_bfloat16>(p, x, nullptr, emb, G, N, n_per_graph, ws, ws_bytes, st);
-  return embed_fwd_t<__half>(p, x, nullptr, emb, G, N, n_per_graph, ws, ws_bytes, st);
+  return with_16bit(precision, "fgnn_embed_fwd", [&](auto t) -> int {
+    if (reinterpret_cast<uintptr_t>(ws) & 1023) return fail(FGNN_ERR_INVALID, "workspace must be 1024-byte aligned");
+    return embed_fwd_t<decltype(t)>(p, x, nullptr, emb, G, N, n_per_graph, ws, ws_bytes, st);
+  });
 }
 
 int embed_fwd_adjacency(const fgnn_embed_params& p, int precision, const uint8_t* adj, float* emb, int G, int N,
                         const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
-  if (!fgnn_device_supports_tcgen05())
-    return fail(FGNN_ERR_UNSUPPORTED, "FGNN_BF16/FGNN_FP16 need an sm_100 device (tcgen05); there is no fallback");
-  if (reinterpret_cast<uintptr_t>(ws) & 1023) return fail(FGNN_ERR_INVALID, "workspace must be 1024-byte aligned");
-  FGNN_CHECK_ARG(p.num_blocks >= 1 && p.block[0].mlp1.c_in == 2,
-                 "the adjacency input builds exactly the reference's 2 features (W, diag(deg))");
-  if (precision == FGNN_BF16) return embed_fwd_t<__nv_bfloat16>(p, nullptr, adj, emb, G, N, n_per_graph, ws, ws_bytes, st);
-  if (precision == FGNN_FP16) return embed_fwd_t<__half>(p, nullptr, adj, emb, G, N, n_per_graph, ws, ws_bytes, st);
-  return fail(FGNN_ERR_INVALID, "fgnn_embed_fwd_adjacency_u8 supports FGNN_BF16 / FGNN_FP16 (for FGNN_FP32 build the features with fgnn_features_from_adjacency_u8)");
+  return with_16bit(precision, "fgnn_embed_fwd_adjacency_u8", [&](auto t) -> int {
+    if (reinterpret_cast<uintptr_t>(ws) & 1023) return fail(FGNN_ERR_INVALID, "workspace must be 1024-byte aligned");
+    FGNN_CHECK_ARG(p.num_blocks >= 1 && p.block[0].mlp1.c_in == 2,
+                   "the adjacency input builds exactly the reference's 2 features (W, diag(deg))");
+    return embed_fwd_t<decltype(t)>(p, nullptr, adj, emb, G, N, n_per_graph, ws, ws_bytes, st);
+  });
 }
 
 size_t head_workspace_bytes(int G, int N) { return align_up((size_t)G * ((N + 127) / 128) * 2 * sizeof(float), 256); }
@@ -1972,16 +1990,14 @@ int head_fwd_t(const float* e1, const float* e2, float* scores, float* ce_sum, i
 
 int head_fwd(int precision, const float* e1, const float* e2, float* scores, float* ce_sum, int32_t* correct, int G, int C,
              int N, const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
-  if (!fgnn_device_supports_tcgen05())
-    return fail(FGNN_ERR_UNSUPPORTED, "the fused head needs an sm_100 device (tcgen05); there is no fallback");
-  FGNN_CHECK_ARG(e1 && e2 && ce_sum && correct && ws, "null pointer");
-  FGNN_CHECK_ARG(G >= 1 && G <= 65535 && N >= 1 && N <= kMaxN, "fused head supports G <= 65535 and N <= %d (got G=%d N=%d)",
-                 kMaxN, G, N);
-  FGNN_CHECK_ARG(C >= 16 && C <= 128 && C % 16 == 0, "the fused head needs an embedding width that is a multiple of 16, at most 128 (got %d)", C);
-  if (ws_bytes < head_workspace_bytes(G, N)) return fail(FGNN_ERR_WORKSPACE, "head workspace too small");
-  if (precision == FGNN_BF16) return head_fwd_t<__nv_bfloat16>(e1, e2, scores, ce_sum, correct, G, C, N, n_per_graph, ws, ws_bytes, st);
-  if (precision == FGNN_FP16) return head_fwd_t<__half>(e1, e2, scores, ce_sum, correct, G, C, N, n_per_graph, ws, ws_bytes, st);
-  return fail(FGNN_ERR_INVALID, "fgnn_head_fwd is the tensor-core head (FGNN_BF16 / FGNN_FP16 operand splitting)");
+  return with_16bit(precision, "fgnn_head_fwd", [&](auto t) -> int {
+    FGNN_CHECK_ARG(e1 && e2 && ce_sum && correct && ws, "null pointer");
+    FGNN_CHECK_ARG(G >= 1 && G <= 65535 && N >= 1 && N <= kMaxN, "fused head supports G <= 65535 and N <= %d (got G=%d N=%d)",
+                   kMaxN, G, N);
+    FGNN_CHECK_ARG(C >= 16 && C <= 128 && C % 16 == 0, "the fused head needs an embedding width that is a multiple of 16, at most 128 (got %d)", C);
+    if (ws_bytes < head_workspace_bytes(G, N)) return fail(FGNN_ERR_WORKSPACE, "head workspace too small");
+    return head_fwd_t<decltype(t)>(e1, e2, scores, ce_sum, correct, G, C, N, n_per_graph, ws, ws_bytes, st);
+  });
 }
 
 // ---- debug: one tensor-core matmul on fp32 host-layout tensors ---------------------------------
@@ -1996,31 +2012,28 @@ int debug_matmul_t(const float* a, const float* b, float* out, int G, int C, int
   Geo geo = make_geo(N);
   if (ws_bytes < debug_matmul_workspace_bytes(G, C, N)) return fail(FGNN_ERR_WORKSPACE, "debug workspace too small");
   Arena ar(ws, ws_bytes);
-  T* y1 = ar.take<T>((size_t)G * C * geo.PSA, 1024);
-  T* y2 = ar.take<T>((size_t)G * C * geo.PSB, 1024);
-  T* mo = ar.take<T>((size_t)G * C * geo.PSC, 1024);
-  dim3 gridA((unsigned)std::min<long>(64, (geo.PSA + 255) / 256), G * C);
-  dim3 gridC((unsigned)std::min<long>(64, (geo.PSC + 255) / 256), G * C);
-  to_planes_kernel<T><<<gridA, 256, 0, st>>>(a, y1, C, geo, 1, npg);
+  T* y1 = ar.take<T>((size_t)G * C * geo.stride(kLayoutA), 1024);
+  T* y2 = ar.take<T>((size_t)G * C * geo.stride(kLayoutB), 1024);
+  T* mo = ar.take<T>((size_t)G * C * geo.stride(kLayoutC), 1024);
+  auto grid = [&](Layout l) { return dim3((unsigned)std::min<long>(64, (geo.stride(l) + 255) / 256), G * C); };
+  to_planes_kernel<T><<<grid(kLayoutA), 256, 0, st>>>(a, y1, C, geo, kLayoutA, npg);
   FGNN_LAUNCHED();
-  dim3 gridB((unsigned)std::min<long>(64, (geo.PSB + 255) / 256), G * C);
-  to_planes_kernel<T><<<gridB, 256, 0, st>>>(b, y2, C, geo, 2, npg);
+  to_planes_kernel<T><<<grid(kLayoutB), 256, 0, st>>>(b, y2, C, geo, kLayoutB, npg);
   FGNN_LAUNCHED();
   FGNN_CUDA(cudaMemsetAsync(mo, 0, (size_t)G * C * geo.PSC * sizeof(T), st));
   if (int e = launch_matmul<T>(y1, y2, mo, nullptr, nullptr, G, C, geo, npg, st)) return e;
-  from_planes_kernel<T><<<gridC, 256, 0, st>>>(mo, out, nullptr, C, geo, npg);
+  from_planes_kernel<T><<<grid(kLayoutC), 256, 0, st>>>(mo, out, nullptr, C, geo, npg);
   FGNN_LAUNCHED();
   return FGNN_OK;
 }
 
 int debug_matmul(int precision, const float* a, const float* b, float* out, int G, int C, int N,
                  const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
-  if (!fgnn_device_supports_tcgen05()) return fail(FGNN_ERR_UNSUPPORTED, "needs an sm_100 device");
-  FGNN_CHECK_ARG(a && b && out && ws, "null pointer");
-  FGNN_CHECK_ARG(N <= kMaxN, "tensor-core matmul supports N <= %d (got %d)", kMaxN, N);
-  if (precision == FGNN_BF16) return debug_matmul_t<__nv_bfloat16>(a, b, out, G, C, N, n_per_graph, ws, ws_bytes, st);
-  if (precision == FGNN_FP16) return debug_matmul_t<__half>(a, b, out, G, C, N, n_per_graph, ws, ws_bytes, st);
-  return fail(FGNN_ERR_INVALID, "precision must be FGNN_BF16 or FGNN_FP16");
+  return with_16bit(precision, "fgnn_debug_tc_matmul", [&](auto t) -> int {
+    FGNN_CHECK_ARG(a && b && out && ws, "null pointer");
+    FGNN_CHECK_ARG(N <= kMaxN, "tensor-core matmul supports N <= %d (got %d)", kMaxN, N);
+    return debug_matmul_t<decltype(t)>(a, b, out, G, C, N, n_per_graph, ws, ws_bytes, st);
+  });
 }
 
 // ---- debug: one tensor-core MlpBlock_Real (fold -> conv chain + statistics -> normalise) ----------
@@ -2042,21 +2055,20 @@ int debug_mlp_t(const fgnn_mlp_params& mp, const float* x, float* y, int G, int 
   if (ws_bytes < debug_mlp_workspace_bytes(G, mp.c_in, C, mp.depth, N)) return fail(FGNN_ERR_WORKSPACE, "debug workspace too small");
   FGNN_CHECK_ARG(mp.c_in <= 128, "c_in too large for the debug entry");
   Arena ar(ws, ws_bytes);
-  T* xin = ar.take<T>((size_t)G * mp.c_in * geo.PSC, 1024);
-  T* out = ar.take<T>((size_t)G * C * geo.PSC, 1024);
+  T* xin = ar.take<T>((size_t)G * mp.c_in * geo.stride(kLayoutC), 1024);
+  T* out = ar.take<T>((size_t)G * C * geo.stride(kLayoutC), 1024);
   T* wf = ar.take<T>((size_t)G * C * K1g, 1024);
   T* wh = ar.take<T>((size_t)std::max(mp.depth - 1, 1) * C * Kh, 1024);
   float* bf = ar.take<float>((size_t)G * C);
   T* bt = ar.take<T>((size_t)G * C * 16, 1024);
   float* coef = ar.take<float>((size_t)G * C * 2);
   double* acc = ar.take<double>((size_t)G * C * 2);
-  {
-    dim3 grid((unsigned)std::min<long>(64, (geo.PSC + 255) / 256), G * mp.c_in);
-    to_planes_kernel<T><<<grid, 256, 0, st>>>(x, xin, mp.c_in, geo, 0, npg);
-    FGNN_LAUNCHED();
-  }
-  for (int l = 1; l < mp.depth; ++l) {
-    convert_weight_kernel<T><<<ceil_div(C * Kh, 256), 256, 0, st>>>(mp.w[l], wh + (size_t)(l - 1) * C * Kh, C, C, Kh);
+  to_planes_c_kernel<T><<<dim3((unsigned)std::min(N, 256), G * mp.c_in), 256, 0, st>>>(x, xin, mp.c_in, geo, npg);
+  FGNN_LAUNCHED();
+  ConvertBatch cb{};
+  for (int l = 1; l < mp.depth; ++l) { cb.src[l - 1] = mp.w[l]; cb.dst_off[l - 1] = (long)(l - 1) * C * Kh; }
+  if (mp.depth > 1) {
+    convert_weights_batch_kernel<T><<<dim3(ceil_div(C * Kh, 256), mp.depth - 1), 256, 0, st>>>(cb, wh, C, C, Kh);
     FGNN_LAUNCHED();
   }
   MlpGroup<T> M{};
@@ -2064,7 +2076,7 @@ int debug_mlp_t(const fgnn_mlp_params& mp, const float* x, float* y, int G, int 
   M.mp[0] = &mp;
   M.src[0] = xin; M.c_src[0] = mp.c_in; M.src_coef[0] = nullptr; M.nsrc = 1;
   M.wf = wf; M.bf = bf; M.bt = bt; M.wh = wh;
-  M.out[0] = out; M.out_mode[0] = kOutC; M.ones[0] = 0; M.coef[0] = coef;
+  M.out[0] = out; M.out_mode[0] = kLayoutC; M.ones[0] = 0; M.coef[0] = coef;
   M.stat_acc = acc;
   if (int e = run_mlp_group<T>(M, C, G, geo, npg, st)) return e;
   dim3 grid((unsigned)std::min<long>(64, (geo.PSC + 255) / 256), G * C);
@@ -2075,13 +2087,12 @@ int debug_mlp_t(const fgnn_mlp_params& mp, const float* x, float* y, int G, int 
 
 int debug_mlp(int precision, const fgnn_mlp_params& mp, const float* x, float* y, int G, int N,
               const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
-  if (!fgnn_device_supports_tcgen05()) return fail(FGNN_ERR_UNSUPPORTED, "needs an sm_100 device");
-  FGNN_CHECK_ARG(x && y && ws, "null pointer");
-  FGNN_CHECK_ARG(N <= kMaxN, "tensor-core MLP supports N <= %d (got %d)", kMaxN, N);
-  if (mp.c_out != 32 && mp.c_out != 64) return fail(FGNN_ERR_UNSUPPORTED, "c_out must be 32 or 64");
-  if (precision == FGNN_BF16) return debug_mlp_t<__nv_bfloat16>(mp, x, y, G, N, n_per_graph, ws, ws_bytes, st);
-  if (precision == FGNN_FP16) return debug_mlp_t<__half>(mp, x, y, G, N, n_per_graph, ws, ws_bytes, st);
-  return fail(FGNN_ERR_INVALID, "precision must be FGNN_BF16 or FGNN_FP16");
+  return with_16bit(precision, "fgnn_debug_tc_mlp", [&](auto t) -> int {
+    FGNN_CHECK_ARG(x && y && ws, "null pointer");
+    FGNN_CHECK_ARG(N <= kMaxN, "tensor-core MLP supports N <= %d (got %d)", kMaxN, N);
+    if (mp.c_out != 32 && mp.c_out != 64) return fail(FGNN_ERR_UNSUPPORTED, "c_out must be 32 or 64");
+    return debug_mlp_t<decltype(t)>(mp, x, y, G, N, n_per_graph, ws, ws_bytes, st);
+  });
 }
 
 }  // namespace tc

@@ -21,13 +21,6 @@
 //   dW0 = sum_g ( P_g diag(a_g) + (sum_px g0) s_g^T ),  P_g = sum_px g0 u^T  (per-graph pixel GEMM),  db0 = sum g0,
 // and the data gradient W0^T g0 is the gradient with respect to y, i.e. the "dy" of the producing MLP.
 
-enum RowMode { kRowC = 0, kRowA = 1, kRowB = 2 };
-
-__device__ __forceinline__ int phys_row_of(int i, int mode, int TN1) {
-  return mode == kRowA ? i + i / kTM1 : (mode == kRowB ? i + i / TN1 : i);
-}
-inline long plane_stride_of(const Geo& geo, int mode) { return mode == kRowA ? geo.PSA : (mode == kRowB ? geo.PSB : geo.PSC); }
-
 template <typename T>
 __device__ __forceinline__ void unpack8(const uint4& v, float (&f)[8]) {
   const float2 a = Elem<T>::unpack2(v.x), b = Elem<T>::unpack2(v.y), c = Elem<T>::unpack2(v.z), d = Elem<T>::unpack2(v.w);
@@ -67,13 +60,13 @@ __device__ __forceinline__ float block_sum(float v, float* s_red) {
 // acc[gc] += (sum dy, sum dy z) over the valid n x n block; dy = dya (+ dyb), layout C; z in layout zmode
 template <typename T>
 __global__ void __launch_bounds__(256)
-gn_bwd_stats_kernel(const T* __restrict__ dya, const T* __restrict__ dyb, const T* __restrict__ z, int zmode,
+gn_bwd_stats_kernel(const T* __restrict__ dya, const T* __restrict__ dyb, const T* __restrict__ z, Layout zmode,
                     double* __restrict__ acc, int C, Geo geo, const int32_t* __restrict__ npg) {
   __shared__ float s_red[8];
   const int gc = blockIdx.y, g = gc / C;
   const int n = graph_n(npg, g, geo.N);
   const int ch = geo.NPC / 8;
-  const long PSz = zmode == kRowA ? geo.PSA : (zmode == kRowB ? geo.PSB : geo.PSC);
+  const long PSz = geo.stride(zmode);
   const int pj_end = phys_k_end(n, geo.TN1);
   float s1 = 0.f, s2 = 0.f;
   for (long idx = (long)blockIdx.x * blockDim.x + threadIdx.x; idx < (long)n * ch; idx += (long)gridDim.x * blockDim.x) {
@@ -89,7 +82,7 @@ gn_bwd_stats_kernel(const T* __restrict__ dya, const T* __restrict__ dyb, const 
 #pragma unroll
       for (int e = 0; e < 8; ++e) d[e] += d2[e];
     }
-    unpack8<T>(*reinterpret_cast<const uint4*>(z + (long)gc * PSz + (long)phys_row_of(i, zmode, geo.TN1) * geo.NPC + pj0), zz);
+    unpack8<T>(*reinterpret_cast<const uint4*>(z + (long)gc * PSz + (long)geo.phys_row(i, zmode) * geo.NPC + pj0), zz);
 #pragma unroll
     for (int e = 0; e < 8; ++e)
       if (vm & (1u << e)) { s1 += d[e]; s2 = fmaf(d[e], zz[e], s2); }
@@ -141,7 +134,7 @@ __global__ void gn_param_grad_kernel(const double* __restrict__ acc, const float
 // bsum[gc] += sum of the ROUNDED dz (the last conv's bias gradient: zero up to rounding, as in the reference)
 template <typename T>
 __global__ void __launch_bounds__(256)
-gn_bwd_apply_kernel(const T* __restrict__ dya, const T* __restrict__ dyb, const T* __restrict__ z, int zmode,
+gn_bwd_apply_kernel(const T* __restrict__ dya, const T* __restrict__ dyb, const T* __restrict__ z, Layout zmode,
                     const float* __restrict__ bc, T* __restrict__ out, float* __restrict__ bsum, int C, Geo geo,
                     const int32_t* __restrict__ npg) {
   __shared__ float s_red[8];
@@ -150,7 +143,7 @@ gn_bwd_apply_kernel(const T* __restrict__ dya, const T* __restrict__ dyb, const 
   const int n = graph_n(npg, g, geo.N);
   const int rows = rows_cover(npg, g, geo);
   const int ch = geo.NPC / 8;
-  const long PSz = zmode == kRowA ? geo.PSA : (zmode == kRowB ? geo.PSB : geo.PSC);
+  const long PSz = geo.stride(zmode);
   const float a = bc[4 * (long)gc], be = bc[4 * (long)gc + 1], ga = bc[4 * (long)gc + 2];
   for (long idx = (long)blockIdx.x * blockDim.x + threadIdx.x; idx < (long)rows * ch; idx += (long)gridDim.x * blockDim.x) {
     const int i = (int)(idx / ch), pj0 = (int)(idx % ch) * 8;
@@ -166,7 +159,7 @@ gn_bwd_apply_kernel(const T* __restrict__ dya, const T* __restrict__ dyb, const 
 #pragma unroll
         for (int e = 0; e < 8; ++e) d[e] += d2[e];
       }
-      unpack8<T>(*reinterpret_cast<const uint4*>(z + (long)gc * PSz + (long)phys_row_of(i, zmode, geo.TN1) * geo.NPC + pj0), zz);
+      unpack8<T>(*reinterpret_cast<const uint4*>(z + (long)gc * PSz + (long)geo.phys_row(i, zmode) * geo.NPC + pj0), zz);
 #pragma unroll
       for (int e = 0; e < 8; ++e)
         if (vm & (1u << e)) r[e] = fmaf(a, d[e], fmaf(be, zz[e], ga));
@@ -342,16 +335,6 @@ __global__ void pool_scatter_kernel(const float* __restrict__ demb, const int32_
   const long gc = idx / geo.N;
   const int i = (int)(idx % geo.N);
   dy[gc * geo.PSC + (long)i * geo.NPC + a] = Elem<T>::from_float(scale[0] * demb[idx]);
-}
-
-// zero the ones rows of layout-A planes (rows 127 mod 128): the backward GEMM Y1^T dM runs its K index over them
-template <typename T>
-__global__ void zero_ones_rows_kernel(T* __restrict__ y, Geo geo) {
-  T* plane = y + (long)blockIdx.y * geo.PSA;
-  for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < geo.MT * geo.NPC; idx += gridDim.x * blockDim.x) {
-    const int t = idx / geo.NPC, col = idx % geo.NPC;
-    plane[(long)(t * 128 + 127) * geo.NPC + col] = Elem<T>::from_float(0.f);
-  }
 }
 
 // wt[r][dst_col0 + c] = w[c][col0 + r]   (r < rows, c < co): transposed (slices of) conv weights for the data gradients
@@ -822,14 +805,13 @@ tc_bmm_bwd_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
 template <typename T>
 int launch_wgrad(const T* gplanes, int co, const T* src0, int c0, const T* src1, int c1, float* out, long out_stride_g,
                  int G, const Geo& geo, const int32_t* npg, cudaStream_t st) {
-  constexpr int is_bf16 = Elem<T>::kFmt;
   const int k0 = round_up(c0, 16), k1 = src1 ? round_up(c1, 16) : 0;
   FGNN_CHECK_ARG(co <= 128 && k0 + k1 <= 128, "weight-gradient GEMM supports <= 128 channels per side (got %d x %d)", co, k0 + k1);
   CUtensorMap ma, mb0, mb1;
-  if (int e = make_map3(&ma, is_bf16, gplanes, geo.PSC, co, G, geo.PSC, (uint64_t)co * geo.PSC, 64, (co + 7) & ~7)) return e;
-  if (int e = make_map3(&mb0, is_bf16, src0, geo.PSC, c0, G, geo.PSC, (uint64_t)c0 * geo.PSC, 64, k0)) return e;
+  if (int e = pixel_map(&ma, gplanes, co, G, geo, (co + 7) & ~7)) return e;
+  if (int e = pixel_map(&mb0, src0, c0, G, geo, k0)) return e;
   if (src1) {
-    if (int e = make_map3(&mb1, is_bf16, src1, geo.PSC, c1, G, geo.PSC, (uint64_t)c1 * geo.PSC, 64, k1)) return e;
+    if (int e = pixel_map(&mb1, src1, c1, G, geo, k1)) return e;
   } else {
     mb1 = mb0;
   }
@@ -859,30 +841,30 @@ int launch_wgrad(const T* gplanes, int co, const T* src0, int c0, const T* src1,
 template <typename T>
 int launch_bmm_bwd(int mode, const T* a, const T* b, T* out, const float* coef, const float* vec, int G, int C,
                    const Geo& geo, const int32_t* npg, cudaStream_t st) {
-  constexpr int is_bf16 = Elem<T>::kFmt;
   CUtensorMap ma, mb, mo32, mo31;
   const uint64_t planes = (uint64_t)G * C;
   if (mode == 1) {
-    if (int e = make_map3(&ma, is_bf16, a, geo.NPC, geo.N, planes, geo.NPC, (uint64_t)geo.PSC, 64, 128)) return e;
-    if (int e = make_map3(&mb, is_bf16, b, geo.NPC, geo.PRB, planes, geo.NPC, (uint64_t)geo.PSB, 64, geo.BN)) return e;
+    if (int e = plane_map(&ma, a, kLayoutC, geo, planes, 128)) return e;
+    if (int e = plane_map(&mb, b, kLayoutB, geo, planes, geo.BN)) return e;
   } else {
-    if (int e = make_map3(&ma, is_bf16, a, geo.NPC, geo.PRA, planes, geo.NPC, (uint64_t)geo.PSA, 64, 64)) return e;
-    if (int e = make_map3(&mb, is_bf16, b, geo.NPC, geo.N, planes, geo.NPC, (uint64_t)geo.PSC, 64, 64)) return e;
+    if (int e = plane_map(&ma, a, kLayoutA, geo, planes, 64)) return e;
+    if (int e = plane_map(&mb, b, kLayoutC, geo, planes, 64)) return e;
   }
-  if (int e = make_map3(&mo32, is_bf16, out, geo.NPC, geo.N, planes, geo.NPC, (uint64_t)geo.PSC, 64, 32)) return e;
-  if (int e = make_map3(&mo31, is_bf16, out, geo.NPC, geo.N, planes, geo.NPC, (uint64_t)geo.PSC, 64, 31)) return e;
+  if (int e = plane_map(&mo32, out, kLayoutC, geo, planes, 32)) return e;
+  if (int e = plane_map(&mo31, out, kLayoutC, geo, planes, 31)) return e;
   BmmBwdArgs<T> args{G, C, geo, coef, vec, npg};
   const int grid = num_sms();
-  auto kernel = mode == 1 ? (geo.BN == 64 ? tc_bmm_bwd_kernel<T, 64, 1> : geo.BN == 128 ? tc_bmm_bwd_kernel<T, 128, 1> : tc_bmm_bwd_kernel<T, 256, 1>)
-                          : (geo.BN == 64 ? tc_bmm_bwd_kernel<T, 64, 2> : geo.BN == 128 ? tc_bmm_bwd_kernel<T, 128, 2> : tc_bmm_bwd_kernel<T, 256, 2>);
-  const size_t smem = geo.BN == 64 ? MatmulCfg<64>::kSmemBytes
-                                   : geo.BN == 128 ? MatmulCfg<128>::kSmemBytes : MatmulCfg<256>::kSmemBytes;
-  prof::begin(prof::kMatmul, st);
-  FGNN_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  kernel<<<grid, 192, smem, st>>>(ma, mb, mo32, mo31, args);
-  prof::end(prof::kMatmul, st);
-  FGNN_LAUNCHED();
-  return FGNN_OK;
+  return with_bn(geo, [&](auto bn) -> int {
+    constexpr int BN = decltype(bn)::value;
+    auto kernel = mode == 1 ? tc_bmm_bwd_kernel<T, BN, 1> : tc_bmm_bwd_kernel<T, BN, 2>;
+    const size_t smem = MatmulCfg<BN>::kSmemBytes;
+    prof::begin(prof::kMatmul, st);
+    FGNN_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<grid, 192, smem, st>>>(ma, mb, mo32, mo31, args);
+    prof::end(prof::kMatmul, st);
+    FGNN_LAUNCHED();
+    return FGNN_OK;
+  });
 }
 
 struct TrainPlan {
@@ -943,14 +925,14 @@ struct TrainBuf {
 size_t carve_train(const TrainPlan& tp, Arena& ar, TrainBuf& B) {
   const Geo& geo = tp.geo;
   const size_t G = tp.G, C = tp.C;
-  const size_t actC = G * C * geo.PSC;
+  const size_t actC = G * C * geo.stride(kLayoutC);
   B.planes_begin = align_up(ar.off, 1024);
-  B.xin = ar.take<uint16_t>(G * tp.cin0 * geo.PSC, 1024);
+  B.xin = ar.take<uint16_t>(G * tp.cin0 * geo.stride(kLayoutC), 1024);
   for (int b = 0; b < tp.nb; ++b) {
     for (int m = 0; m < 3; ++m)
       for (int l = 0; l < tp.D - 1; ++l) B.H[b][m][l] = ar.take<uint16_t>(actC, 1024);
-    B.Y1[b] = ar.take<uint16_t>(G * C * geo.PSA, 1024);
-    B.Y2[b] = ar.take<uint16_t>(G * C * geo.PSB, 1024);
+    B.Y1[b] = ar.take<uint16_t>(G * C * geo.stride(kLayoutA), 1024);
+    B.Y2[b] = ar.take<uint16_t>(G * C * geo.stride(kLayoutB), 1024);
     B.MULT[b] = ar.take<uint16_t>(actC, 1024);
     B.Z3[b] = ar.take<uint16_t>(actC, 1024);
   }
@@ -994,7 +976,7 @@ struct ConvCall {
   const float* src_coef[2] = {nullptr, nullptr};
   int nsrc = 1;
   T* out[2] = {nullptr, nullptr};
-  int out_mode[2] = {kOutC, kOutC};
+  Layout out_mode[2] = {kLayoutC, kLayoutC};
   int ones[2] = {0, 0};
   int relu = 0;
   const fgnn_mlp_params* gn[2] = {nullptr, nullptr};   // GraphNorm of the output (last layer): coefficients + statistics
@@ -1076,7 +1058,7 @@ int embed_fwd_train_t(const fgnn_embed_params& p, const float* x, float* emb, in
     const fgnn_block_params& bp = p.block[b];
     const fgnn_mlp_params* mlps[3] = {&bp.mlp1, &bp.mlp2, &bp.mlp3};
     T* y12[2] = {reinterpret_cast<T*>(B.Y1[b]), reinterpret_cast<T*>(B.Y2[b])};
-    const int mode12[2] = {kOutA, kOutB};
+    const Layout mode12[2] = {kLayoutA, kLayoutB};
     for (int l = 0; l < D; ++l) {
       const bool last = l == D - 1;
       if (l == 0) {   // mlp1 and mlp2 share the block input: one launch
@@ -1086,7 +1068,7 @@ int embed_fwd_train_t(const fgnn_embed_params& p, const float* x, float* emb, in
         for (int m = 0; m < 2; ++m) {
           cc.w[m] = mlps[m]->w[0]; cc.b[m] = mlps[m]->b[0];
           cc.out[m] = last ? y12[m] : reinterpret_cast<T*>(B.H[b][m][0]);
-          cc.out_mode[m] = last ? mode12[m] : kOutC;
+          cc.out_mode[m] = last ? mode12[m] : kLayoutC;
           cc.ones[m] = last ? 1 : 0;
           if (last) { cc.gn[m] = mlps[m]; cc.coef[m] = B.coef[b][m]; cc.gnstat[m] = B.gnstat[b][m]; }
         }
@@ -1098,7 +1080,7 @@ int embed_fwd_train_t(const fgnn_embed_params& p, const float* x, float* emb, in
           cc.src[0] = reinterpret_cast<const T*>(B.H[b][m][l - 1]); cc.c_src[0] = C;
           cc.w[0] = mlps[m]->w[l]; cc.b[0] = mlps[m]->b[l];
           cc.out[0] = last ? y12[m] : reinterpret_cast<T*>(B.H[b][m][l]);
-          cc.out_mode[0] = last ? mode12[m] : kOutC;
+          cc.out_mode[0] = last ? mode12[m] : kLayoutC;
           cc.ones[0] = last ? 1 : 0;
           if (last) { cc.gn[0] = mlps[m]; cc.coef[0] = B.coef[b][m]; cc.gnstat[0] = B.gnstat[b][m]; }
           cc.relu = last ? 0 : 1;
@@ -1145,7 +1127,7 @@ struct MlpBwd {
   const T* dya;
   const T* dyb;
   const T* z;
-  int zmode;
+  Layout zmode;
   const float* coef;
   const float* gnstat;
   void* const* H;               // hidden activations h_0 .. h_{D-2} (layout C)
@@ -1272,7 +1254,7 @@ int embed_bwd_t(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const fl
       MlpBwd<T> a{};
       a.mp = &bp.mlp3; a.gr = &bg.mlp3;
       a.dya = dOutA; a.dyb = dOutB;
-      a.z = reinterpret_cast<const T*>(B.Z3[b]); a.zmode = kRowC;
+      a.z = reinterpret_cast<const T*>(B.Z3[b]); a.zmode = kLayoutC;
       a.coef = B.coef[b][2]; a.gnstat = B.gnstat[b][2];
       a.H = B.H[b][2];
       a.src[0] = reinterpret_cast<const T*>(B.MULT[b]); a.c_src[0] = C; a.src_coef[0] = nullptr;
@@ -1303,7 +1285,7 @@ int embed_bwd_t(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const fl
       FGNN_LAUNCHED();
       plane_colsum_kernel<T><<<dim3((unsigned)((geo.NPC + 255) / 256), GC), 256, 0, st>>>(DM, B.colsum, C, geo, npg);
       FGNN_LAUNCHED();
-      zero_ones_rows_kernel<T><<<dim3(4, GC), 256, 0, st>>>(reinterpret_cast<T*>(B.Y1[b]), geo);
+      zero_inserted_rows_kernel<T><<<dim3(4, GC), 256, 0, st>>>(reinterpret_cast<T*>(B.Y1[b]), geo, kLayoutA);
       FGNN_LAUNCHED();
       prof::end(prof::kStats, st);
       if (int e = launch_bmm_bwd<T>(1, DM, reinterpret_cast<const T*>(B.Y2[b]), reinterpret_cast<T*>(B.DY1), B.coef[b][1], B.rowsum,
@@ -1318,7 +1300,7 @@ int embed_bwd_t(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const fl
       a.mp = m == 0 ? &bp.mlp1 : &bp.mlp2;
       a.gr = m == 0 ? &bg.mlp1 : &bg.mlp2;
       a.dya = reinterpret_cast<const T*>(m == 0 ? B.DY1 : B.DY2); a.dyb = nullptr;
-      a.z = reinterpret_cast<const T*>(m == 0 ? B.Y1[b] : B.Y2[b]); a.zmode = m == 0 ? kRowA : kRowB;
+      a.z = reinterpret_cast<const T*>(m == 0 ? B.Y1[b] : B.Y2[b]); a.zmode = m == 0 ? kLayoutA : kLayoutB;
       a.coef = B.coef[b][m]; a.gnstat = B.gnstat[b][m];
       a.H = B.H[b][m];
       a.src[0] = cur; a.c_src[0] = cur_c; a.src_coef[0] = cur_coef; a.nsrc = 1;
