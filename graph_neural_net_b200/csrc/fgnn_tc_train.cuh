@@ -867,41 +867,35 @@ int launch_bmm_bwd(int mode, const T* a, const T* b, T* out, const float* coef, 
   });
 }
 
+// Two plans for the 16-bit training entry points.
+//   KEEP-ALL   one pass over the whole batch: the forward leaves every activation in the workspace until the backward
+//              (carve_train: about 51 plane sets per graph at depth 3, 4 blocks; 107 GB for 64 graphs at N = 500, C = 64).
+//   RECOMPUTE  chosen only when the keep-all workspace exceeds T.  The workspace holds the 16-bit input planes of the
+//              whole batch and one keep-all carve of `chunk` graphs.  The forward runs pass by pass and keeps only emb;
+//              the backward computes the loss scale once over the whole d emb, then per pass re-runs that pass's
+//              forward from the input planes and runs the block-stack backward on it (about one extra training forward
+//              per step).  Parameter gradients accumulate across passes as they do across calls.
+// T = FGNN_TC_TRAIN_WS_GB GiB when set; otherwise half the current device's memory, because a siamese step holds two
+// embedder workspaces (x1, x2) until backward; unlimited when no device can be queried (host-only workspace queries).
+// chunk = FGNN_TC_CHUNK when set (as for inference), else the largest pass whose carve fits FGNN_TC_WS_GB (default 16)
+// GiB, never less than one graph; the passes are equal, the last one may be shorter.
+// The plan is a pure function of (parameter shapes, G, N, T, FGNN_TC_WS_GB, FGNN_TC_CHUNK).  fgnn_embed_bwd derives it
+// again from the same arguments and must reach the forward call's answer: neither the variables nor the device may
+// change between the two calls.
 struct TrainPlan {
   Geo geo;
-  int C, cin0, D, nb, G;
+  int C, cin0, D, nb;
+  int G;            // graphs of one pass: the whole batch on keep-all, `chunk` on recompute (pass_plan lowers it for a short last pass)
+  int batch;        // graphs of the call
+  bool recompute;
 };
 
-// 16-bit training keeps every activation of the batch in one workspace (carve_train: about 51 plane sets per graph at
-// depth 3, 4 blocks; some 15 GB per graph at N = 2048, C = 32), so it stops at the padded size the inference path had
-// before it was extended to kMaxN.
+// 16-bit training keeps every activation of a pass in its workspace, and a pass holds at least one graph (some 15 GB
+// at N = 2048, C = 32), so it stops at the padded size the inference path had before it was extended to kMaxN.
 constexpr int kMaxTrainN = 1024;
 
-int make_train_plan(const fgnn_embed_params& p, int G, int N, TrainPlan& tp) {
-  if (N > kMaxTrainN)
-    return fail(FGNN_ERR_UNSUPPORTED, "16-bit training supports N <= %d (got %d): its workspace holds every activation of the "
-                "batch; embed larger graphs with the inference path (N <= %d)", kMaxTrainN, N, kMaxN);
-  Plan pl;
-  if (int e = make_plan(p, G, N, pl)) return e;
-  tp.geo = pl.geo;
-  tp.C = pl.C;
-  tp.cin0 = pl.cin0;
-  tp.nb = p.num_blocks;
-  tp.G = G;
-  tp.D = p.block[0].mlp1.depth;
-  for (int b = 0; b < p.num_blocks; ++b) {
-    const fgnn_block_params& bp = p.block[b];
-    if (bp.mlp1.depth != tp.D || bp.mlp2.depth != tp.D || bp.mlp3.depth != tp.D)
-      return fail(FGNN_ERR_UNSUPPORTED, "16-bit training needs the same depth_of_mlp in every MLP");
-  }
-  if (tp.D < 1 || tp.D > FGNN_MAX_DEPTH) return fail(FGNN_ERR_INVALID, "bad depth %d", tp.D);
-  if (tp.cin0 > 64) return fail(FGNN_ERR_UNSUPPORTED, "original_features_num %d > 64 unsupported", tp.cin0);
-  if ((long)G * tp.C > 65535) return fail(FGNN_ERR_UNSUPPORTED, "16-bit training: G * C = %ld planes exceed one call's grid (split the batch)", (long)G * tp.C);
-  return FGNN_OK;
-}
-
 struct TrainBuf {
-  // kept from forward to backward
+  // kept from forward to backward (recompute: xin for the whole call, the rest for the current pass)
   void* xin;
   void* H[FGNN_MAX_BLOCKS][3][FGNN_MAX_DEPTH];
   void *Y1[FGNN_MAX_BLOCKS], *Y2[FGNN_MAX_BLOCKS], *MULT[FGNN_MAX_BLOCKS], *Z3[FGNN_MAX_BLOCKS];
@@ -926,8 +920,10 @@ size_t carve_train(const TrainPlan& tp, Arena& ar, TrainBuf& B) {
   const Geo& geo = tp.geo;
   const size_t G = tp.G, C = tp.C;
   const size_t actC = G * C * geo.stride(kLayoutC);
+  // recompute: the batch's input planes come first, outside the plane range that every pass zeroes
+  if (tp.recompute) B.xin = ar.take<uint16_t>((size_t)tp.batch * tp.cin0 * geo.stride(kLayoutC), 1024);
   B.planes_begin = align_up(ar.off, 1024);
-  B.xin = ar.take<uint16_t>(G * tp.cin0 * geo.stride(kLayoutC), 1024);
+  if (!tp.recompute) B.xin = ar.take<uint16_t>(G * tp.cin0 * geo.stride(kLayoutC), 1024);
   for (int b = 0; b < tp.nb; ++b) {
     for (int m = 0; m < 3; ++m)
       for (int l = 0; l < tp.D - 1; ++l) B.H[b][m][l] = ar.take<uint16_t>(actC, 1024);
@@ -963,6 +959,104 @@ size_t carve_train(const TrainPlan& tp, Arena& ar, TrainBuf& B) {
   B.Pglob = ar.take<float>(128 * 128);
   B.scale = ar.take<float>(4);
   return align_up(ar.off, 1024);
+}
+
+size_t train_workspace_bytes(const TrainPlan& tp) {
+  Arena ar(nullptr, 0);
+  TrainBuf B;
+  return carve_train(tp, ar, B);
+}
+
+// T of the plan selection, in bytes (see TrainPlan)
+size_t keep_all_limit() {
+  if (const char* v = getenv("FGNN_TC_TRAIN_WS_GB")) return (size_t)(std::min(std::max(atof(v), 0.0), 1e9) * (double)(1ull << 30));
+  static size_t cache[64] = {0};   // per device: the query is not free and runs three times per embedder call
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess) {
+    cudaGetLastError();            // no device: leave no error behind for a later launch check
+    return SIZE_MAX;
+  }
+  if (dev >= 0 && dev < 64 && cache[dev]) return cache[dev];
+  cudaDeviceProp prop;
+  if (cudaGetDeviceProperties(&prop, dev) != cudaSuccess) {
+    cudaGetLastError();
+    return SIZE_MAX;
+  }
+  const size_t t = prop.totalGlobalMem / 2;
+  if (dev >= 0 && dev < 64) cache[dev] = t;
+  return t;
+}
+
+int make_train_plan(const fgnn_embed_params& p, int G, int N, TrainPlan& tp) {
+  if (N > kMaxTrainN)
+    return fail(FGNN_ERR_UNSUPPORTED, "16-bit training supports N <= %d (got %d): its workspace holds every activation of at "
+                "least one graph; embed larger graphs with the inference path (N <= %d)", kMaxTrainN, N, kMaxN);
+  Plan pl;
+  if (int e = make_plan(p, G, N, pl)) return e;
+  tp.geo = pl.geo;
+  tp.C = pl.C;
+  tp.cin0 = pl.cin0;
+  tp.nb = p.num_blocks;
+  tp.G = G;
+  tp.batch = G;
+  tp.recompute = false;
+  tp.D = p.block[0].mlp1.depth;
+  for (int b = 0; b < p.num_blocks; ++b) {
+    const fgnn_block_params& bp = p.block[b];
+    if (bp.mlp1.depth != tp.D || bp.mlp2.depth != tp.D || bp.mlp3.depth != tp.D)
+      return fail(FGNN_ERR_UNSUPPORTED, "16-bit training needs the same depth_of_mlp in every MLP");
+  }
+  if (tp.D < 1 || tp.D > FGNN_MAX_DEPTH) return fail(FGNN_ERR_INVALID, "bad depth %d", tp.D);
+  if (tp.cin0 > 64) return fail(FGNN_ERR_UNSUPPORTED, "original_features_num %d > 64 unsupported", tp.cin0);
+  if ((long)G * tp.C > 65535) return fail(FGNN_ERR_UNSUPPORTED, "16-bit training: G * C = %ld planes exceed one call's grid (split the batch)", (long)G * tp.C);
+  if (train_workspace_bytes(tp) <= keep_all_limit()) return FGNN_OK;
+  tp.recompute = true;
+  int chunk = env_int("FGNN_TC_CHUNK", 0);
+  if (chunk <= 0) {   // the largest pass whose own carve (batch = 0: without the input planes) fits the budget, or 1
+    const size_t budget = (size_t)std::max(1, env_int("FGNN_TC_WS_GB", 16)) << 30;
+    TrainPlan q = tp;
+    q.batch = 0;
+    int lo = 1, hi = G;
+    while (lo < hi) {
+      q.G = lo + (hi - lo + 1) / 2;
+      if (train_workspace_bytes(q) <= budget) lo = q.G; else hi = q.G - 1;
+    }
+    chunk = lo;
+  }
+  chunk = std::min(chunk, G);
+  const int passes = (G + chunk - 1) / chunk;
+  tp.G = (G + passes - 1) / passes;
+  return FGNN_OK;
+}
+
+// the plan of the pass that starts at graph g0: the same carve, launches over the pass's graphs only
+TrainPlan pass_plan(const TrainPlan& tp, int g0) {
+  TrainPlan pp = tp;
+  pp.G = std::min(tp.G, tp.batch - g0);
+  return pp;
+}
+
+// Zero what a pass's producers never write but later reads cover, before every pass's forward.  Ragged batch: all the
+// kept planes and the backward scratch (rows beyond a graph's covered range are never written, the GEMM K loops read
+// them, and an earlier pass's larger graph leaves data there).  Otherwise: the physical rows / column chunks the
+// producers skip.  The recompute plan's input planes lie before planes_begin and are not touched.
+int zero_pass(const TrainPlan& tp, const TrainBuf& B, void* ws, bool ragged, cudaStream_t st) {
+  const Geo& geo = tp.geo;
+  const size_t GC = (size_t)tp.G * tp.C;
+  char* base = static_cast<char*>(ws);
+  if (ragged) {
+    FGNN_CUDA(cudaMemsetAsync(base + B.planes_begin, 0, B.planes_end - B.planes_begin, st));
+    FGNN_CUDA(cudaMemsetAsync(base + B.bwd_begin, 0, B.bwd_end - B.bwd_begin, st));
+  } else {
+    for (int b = 0; b < tp.nb; ++b) {
+      FGNN_CUDA(cudaMemsetAsync(B.Y1[b], 0, GC * geo.PSA * 2, st));
+      FGNN_CUDA(cudaMemsetAsync(B.Y2[b], 0, GC * geo.PSB * 2, st));
+      FGNN_CUDA(cudaMemsetAsync(B.MULT[b], 0, GC * geo.PSC * 2, st));
+    }
+    FGNN_CUDA(cudaMemsetAsync(B.DY1, 0, GC * geo.PSC * 2, st));
+    FGNN_CUDA(cudaMemsetAsync(B.DY2, 0, GC * geo.PSC * 2, st));
+  }
+  return FGNN_OK;
 }
 
 // one 1x1-conv layer (or two sharing their input) as a depth-1 launch of the conv-chain kernel
@@ -1020,38 +1114,14 @@ int run_conv(const ConvCall<T>& cc, const TrainPlan& tp, const TrainBuf& B, cons
   return run_mlp_group<T>(M, tp.C, tp.G, tp.geo, npg, st);
 }
 
+// training forward of one pass (tp.G graphs): their input planes xin -> emb (tp.G, C, N), and in B everything the
+// backward reads
 template <typename T>
-int embed_fwd_train_t(const fgnn_embed_params& p, const float* x, float* emb, int G, int N, const int32_t* npg, void* ws,
-                      size_t ws_bytes, cudaStream_t st) {
-  TrainPlan tp;
-  if (int e = make_train_plan(p, G, N, tp)) return e;
-  Arena ar(ws, ws_bytes);
-  TrainBuf B;
-  const size_t need = carve_train(tp, ar, B);
-  if (need > ws_bytes) return fail(FGNN_ERR_WORKSPACE, "training workspace too small: %zu < %zu", ws_bytes, need);
+int train_fwd_pass(const fgnn_embed_params& p, const TrainPlan& tp, const TrainBuf& B, const T* xin, float* emb,
+                   const int32_t* npg, cudaStream_t st) {
   const Geo& geo = tp.geo;
-  const int C = tp.C, D = tp.D;
-  char* base = static_cast<char*>(ws);
-  FGNN_CUDA(cudaMemsetAsync(B.zeros, 0, 512 * sizeof(float), st));
-  if (npg) {
-    // ragged batch: rows beyond a graph's covered range are never written; GEMM K loops may read them
-    FGNN_CUDA(cudaMemsetAsync(base + B.planes_begin, 0, B.planes_end - B.planes_begin, st));
-    FGNN_CUDA(cudaMemsetAsync(base + B.bwd_begin, 0, B.bwd_end - B.bwd_begin, st));
-  } else {
-    for (int b = 0; b < tp.nb; ++b) {   // physical rows / column chunks the producers skip
-      FGNN_CUDA(cudaMemsetAsync(B.Y1[b], 0, (size_t)G * C * geo.PSA * 2, st));
-      FGNN_CUDA(cudaMemsetAsync(B.Y2[b], 0, (size_t)G * C * geo.PSB * 2, st));
-      FGNN_CUDA(cudaMemsetAsync(B.MULT[b], 0, (size_t)G * C * geo.PSC * 2, st));
-    }
-    FGNN_CUDA(cudaMemsetAsync(B.DY1, 0, (size_t)G * C * geo.PSC * 2, st));
-    FGNN_CUDA(cudaMemsetAsync(B.DY2, 0, (size_t)G * C * geo.PSC * 2, st));
-  }
-  {
-    dim3 grid((unsigned)std::min(N, 256), G * tp.cin0);
-    to_planes_c_kernel<T><<<grid, 256, 0, st>>>(x, reinterpret_cast<T*>(B.xin), tp.cin0, geo, npg);
-    FGNN_LAUNCHED();
-  }
-  const T* cur = reinterpret_cast<const T*>(B.xin);
+  const int G = tp.G, N = geo.N, C = tp.C, D = tp.D;
+  const T* cur = xin;
   int cur_c = tp.cin0;
   const float* cur_coef = nullptr;
   for (int b = 0; b < tp.nb; ++b) {
@@ -1113,6 +1183,32 @@ int embed_fwd_train_t(const fgnn_embed_params& p, const float* x, float* emb, in
     dim3 grid((unsigned)((N + 7) / 8), G * C);
     colmax16_kernel<T><<<grid, 256, 0, st>>>(cur, cur_coef, emb, B.arg, C, geo, npg);
     FGNN_LAUNCHED();
+  }
+  return FGNN_OK;
+}
+
+template <typename T>
+int embed_fwd_train_t(const fgnn_embed_params& p, const float* x, float* emb, int G, int N, const int32_t* npg, void* ws,
+                      size_t ws_bytes, cudaStream_t st) {
+  TrainPlan tp;
+  if (int e = make_train_plan(p, G, N, tp)) return e;
+  Arena ar(ws, ws_bytes);
+  TrainBuf B;
+  const size_t need = carve_train(tp, ar, B);
+  if (need > ws_bytes) return fail(FGNN_ERR_WORKSPACE, "training workspace too small: %zu < %zu", ws_bytes, need);
+  const Geo& geo = tp.geo;
+  T* xin = reinterpret_cast<T*>(B.xin);
+  FGNN_CUDA(cudaMemsetAsync(B.zeros, 0, 512 * sizeof(float), st));
+  for (int g0 = 0; g0 < G; g0 += tp.G) {
+    const TrainPlan pp = pass_plan(tp, g0);
+    if (int e = zero_pass(pp, B, ws, npg != nullptr, st)) return e;
+    if (g0 == 0) {   // the whole batch, after the first zeroing: on keep-all the zeroed range holds xin
+      dim3 grid((unsigned)std::min(N, 256), G * tp.cin0);
+      to_planes_c_kernel<T><<<grid, 256, 0, st>>>(x, xin, tp.cin0, geo, npg);
+      FGNN_LAUNCHED();
+    }
+    if (int e = train_fwd_pass<T>(p, pp, B, xin + (size_t)g0 * tp.cin0 * geo.PSC, emb + (size_t)g0 * tp.C * N,
+                                  npg ? npg + g0 : nullptr, st)) return e;
   }
   return FGNN_OK;
 }
@@ -1214,20 +1310,13 @@ int mlp_bwd(const MlpBwd<T>& a, const TrainPlan& tp, const TrainBuf& B, const in
   return FGNN_OK;
 }
 
+// block-stack backward of one pass (tp.G graphs) whose forward state is in B: demb (tp.G, C, N), scaled by *B.scale
 template <typename T>
-int embed_bwd_t(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const float* demb, int grad_scale_log2, int G, int N,
-                const int32_t* npg, void* ws, size_t ws_bytes, cudaStream_t st) {
-  TrainPlan tp;
-  if (int e = make_train_plan(p, G, N, tp)) return e;
-  Arena ar(ws, ws_bytes);
-  TrainBuf B;
-  const size_t need = carve_train(tp, ar, B);
-  if (need > ws_bytes) return fail(FGNN_ERR_WORKSPACE, "training workspace too small: %zu < %zu", ws_bytes, need);
+int train_bwd_pass(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const TrainPlan& tp, const TrainBuf& B,
+                   const T* xin, const float* demb, const int32_t* npg, cudaStream_t st) {
   const Geo& geo = tp.geo;
-  const int C = tp.C, D = tp.D, GC = G * C;
+  const int G = tp.G, N = geo.N, C = tp.C, GC = G * C;
   const size_t plane_bytes = (size_t)GC * geo.PSC * sizeof(T);
-  grad_scale_kernel<<<1, 1024, 0, st>>>(demb, (long)GC * N, B.scale, grad_scale_log2);
-  FGNN_LAUNCHED();
   // gradient of the last block's normalised output: zero planes + the pooling scatter
   T* dOutA = reinterpret_cast<T*>(B.DX3[tp.nb & 1]);
   const T* dOutB = nullptr;
@@ -1240,7 +1329,7 @@ int embed_bwd_t(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const fl
   for (int b = tp.nb - 1; b >= 0; --b) {
     const fgnn_block_params& bp = p.block[b];
     const fgnn_block_grads& bg = gr.block[b];
-    const T* cur = b > 0 ? reinterpret_cast<const T*>(B.Z3[b - 1]) : reinterpret_cast<const T*>(B.xin);
+    const T* cur = b > 0 ? reinterpret_cast<const T*>(B.Z3[b - 1]) : xin;
     const int cur_c = b > 0 ? C : tp.cin0;
     const float* cur_coef = b > 0 ? B.coef[b - 1][2] : nullptr;
     T* A[2] = {reinterpret_cast<T*>(B.A0), reinterpret_cast<T*>(B.A1)};
@@ -1325,6 +1414,33 @@ int embed_bwd_t(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const fl
       dOutB = dx12;
     }
   }
-  (void)D;
+  return FGNN_OK;
+}
+
+template <typename T>
+int embed_bwd_t(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const float* demb, int grad_scale_log2, int G, int N,
+                const int32_t* npg, void* ws, size_t ws_bytes, cudaStream_t st) {
+  TrainPlan tp;
+  if (int e = make_train_plan(p, G, N, tp)) return e;
+  Arena ar(ws, ws_bytes);
+  TrainBuf B;
+  const size_t need = carve_train(tp, ar, B);
+  if (need > ws_bytes) return fail(FGNN_ERR_WORKSPACE, "training workspace too small: %zu < %zu", ws_bytes, need);
+  const Geo& geo = tp.geo;
+  // one loss scale for the whole batch, whatever the passes
+  grad_scale_kernel<<<1, 1024, 0, st>>>(demb, (long)G * tp.C * N, B.scale, grad_scale_log2);
+  FGNN_LAUNCHED();
+  const T* xin = reinterpret_cast<const T*>(B.xin);
+  for (int g0 = 0; g0 < G; g0 += tp.G) {
+    const TrainPlan pp = pass_plan(tp, g0);
+    const T* xin_p = xin + (size_t)g0 * tp.cin0 * geo.PSC;
+    const int32_t* npg_p = npg ? npg + g0 : nullptr;
+    if (tp.recompute) {
+      // re-derive the pass's activations; its embeddings land in rowsum, which the backward rewrites before reading it
+      if (int e = zero_pass(pp, B, ws, npg != nullptr, st)) return e;
+      if (int e = train_fwd_pass<T>(p, pp, B, xin_p, B.rowsum, npg_p, st)) return e;
+    }
+    if (int e = train_bwd_pass<T>(p, gr, pp, B, xin_p, demb + (size_t)g0 * tp.C * N, npg_p, st)) return e;
+  }
   return FGNN_OK;
 }

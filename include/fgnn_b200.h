@@ -234,8 +234,19 @@ int fgnn_embed_fwd_adjacency_u8(const fgnn_embed_params* p, int32_t precision, c
  * As with the reference's AMP GradScaler, fp16 gradient planes can overflow for a given scale: the parameter
  * gradients are then non-finite and the caller skips the step and lowers grad_scale_log2 (training.py does; 9 is
  * the default, -24 .. 15 accepted; bf16 never overflows).  The workspace must be the one the forward call filled
- * (same G, N, parameters), fgnn_embed_train_workspace_bytes(...) bytes, 1024-byte aligned.  N <= 1024: the
- * workspace keeps every activation of the batch. */
+ * (same G, N, parameters), fgnn_embed_train_workspace_bytes(...) bytes, 1024-byte aligned.  N <= 1024.
+ * Two plans, picked from the shapes by all three calls alike:
+ *   keep-all   the workspace keeps every activation of the batch from forward to backward (about 51 plane sets per
+ *              graph at depth 3, 4 blocks: 107 GB for 64 graphs of N = 500, C = 64).  Used while that size is <= T.
+ *   recompute  the workspace keeps the 16-bit input planes of the batch plus the activations of one pass of graphs;
+ *              the forward runs pass by pass and keeps only emb, the backward re-runs each pass's forward before its
+ *              backward (about one more forward per step; the loss scale is still chosen once over all of d emb).
+ *              Passes are equal and as large as fit FGNN_TC_WS_GB (default 16) GiB, never less than one graph
+ *              (FGNN_TC_CHUNK graphs when set, as for fgnn_embed_fwd).
+ * T is FGNN_TC_TRAIN_WS_GB GiB when set (0 always picks recompute); otherwise half the current device's memory, because
+ * a siamese step holds two workspaces (x1 and x2) until backward; unlimited when no device can be queried.  The plan
+ * must not change between fgnn_embed_fwd_train and fgnn_embed_bwd: keep these variables and the current device as
+ * they were for the workspace query. */
 size_t fgnn_embed_train_workspace_bytes(const fgnn_embed_params* p, int32_t precision, int32_t G, int32_t N);
 int fgnn_embed_fwd_train(const fgnn_embed_params* p, int32_t precision, const float* x, float* emb, int32_t G,
                          int32_t N, const int32_t* n_per_graph, void* workspace, size_t workspace_bytes,
