@@ -85,6 +85,8 @@ _SIGNATURES = {
     "fgnn_generate_pairs_u8": (C.c_int, [_vp, _vp, _i32, _i32, _vp, _i32, C.c_float, C.c_float, C.c_uint64, _vp, _sz, _vp]),
     "fgnn_head_workspace_bytes": (_sz, [_i32, _i32]),
     "fgnn_head_fwd": (C.c_int, [_i32, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp, _sz, _vp]),
+    "fgnn_head_fwd_train": (C.c_int, [_i32, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp, _sz, _vp]),
+    "fgnn_head_bwd": (C.c_int, [_i32, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp, _sz, _vp]),
     "fgnn_embed_workspace_bytes": (_sz, [C.POINTER(EmbedParams), _i32, _i32, _i32]),
     "fgnn_embed_fwd": (C.c_int, [C.POINTER(EmbedParams), _i32, _vp, _vp, _i32, _i32, _vp, _vp, _sz, _vp]),
     "fgnn_embed_fwd_adjacency_u8": (C.c_int, [C.POINTER(EmbedParams), _i32, _vp, _vp, _i32, _i32, _vp, _vp, _sz, _vp]),

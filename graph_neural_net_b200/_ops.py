@@ -277,24 +277,32 @@ def generate_pairs(generator: int, G: int, N: int, edge_density: float, noise: f
     return adj1, adj2
 
 
-def head_fused(e1: torch.Tensor, e2: torch.Tensor, n_dev, precision: str = "fp16", want_scores: bool = False):
-    """Fused siamese head on tensor cores (fgnn_head_fwd): e1, e2 (G,C,N) -> (ce_sum[G], correct[G], scores or None).
-    scores = e1^T e2 (reference models/trainers.py:67), ce_sum / correct as CrossEntropyIdentityFunction
-    (toolbox/losses.py:27-33, toolbox/metrics.py:125-134); the (G,N,N) scores are only materialised on request.
-    Forward only: under autograd use ScoresFunction + CrossEntropyIdentityFunction."""
-    lib = L.get_lib()
+def _head_operands(e1: torch.Tensor, e2: torch.Tensor, precision: str, what: str):
+    """Checked (G,C,N) fp32 operands of the tensor-core head, C zero-padded to a multiple of 16 (K of the MMA; zero
+    channels add nothing to e1^T e2) -> (e1, e2, padded C)."""
     e1 = L.require_cuda_f32(e1, "e1")
     e2 = L.require_cuda_f32(e2, "e2")
     if e1.shape != e2.shape or e1.dim() != 3:
-        raise L.FgnnError(f"head_fused: embeddings must both be (G,C,N), got {tuple(e1.shape)} and {tuple(e2.shape)}")
+        raise L.FgnnError(f"{what}: embeddings must both be (G,C,N), got {tuple(e1.shape)} and {tuple(e2.shape)}")
     if precision not in ("bf16", "fp16"):
-        raise L.FgnnError("head_fused is the tensor-core head (bf16 / fp16 operand splitting); fp32 uses the CUDA-core operators")
-    G, Cc, N = e1.shape
-    if Cc % 16:                                            # K of the MMA is a multiple of 16: zero channels add nothing to e1^T e2
+        raise L.FgnnError(f"{what} is the tensor-core head (bf16 / fp16 operand splitting); fp32 uses the CUDA-core operators")
+    Cc = e1.shape[1]
+    if Cc % 16:
         pad = 16 - Cc % 16
         e1 = torch.nn.functional.pad(e1, (0, 0, 0, pad)).contiguous()
         e2 = torch.nn.functional.pad(e2, (0, 0, 0, pad)).contiguous()
         Cc += pad
+    return e1, e2, Cc
+
+
+def head_fused(e1: torch.Tensor, e2: torch.Tensor, n_dev, precision: str = "fp16", want_scores: bool = False):
+    """Fused siamese head on tensor cores (fgnn_head_fwd): e1, e2 (G,C,N) -> (ce_sum[G], correct[G], scores or None).
+    scores = e1^T e2 (reference models/trainers.py:67), ce_sum / correct as CrossEntropyIdentityFunction
+    (toolbox/losses.py:27-33, toolbox/metrics.py:125-134); the (G,N,N) scores are only materialised on request.
+    Forward only: under autograd use HeadFunction (or ScoresFunction + CrossEntropyIdentityFunction)."""
+    lib = L.get_lib()
+    e1, e2, Cc = _head_operands(e1, e2, precision, "head_fused")
+    G, _, N = e1.shape
     ce = torch.empty(G, device=e1.device, dtype=torch.float32)
     correct = torch.empty(G, device=e1.device, dtype=torch.int32)
     scores = torch.empty((G, N, N), device=e1.device, dtype=torch.float32) if want_scores else None
@@ -303,6 +311,45 @@ def head_fused(e1: torch.Tensor, e2: torch.Tensor, n_dev, precision: str = "fp16
                               L.ptr(ce), L.ptr(correct), G, Cc, N, _npg(n_dev, G), L.ptr(ws), ws.numel(),
                               L.stream_ptr(e1.device)), "fgnn_head_fwd")
     return ce, correct, scores
+
+
+class HeadFunction(torch.autograd.Function):
+    """Differentiable fused head (fgnn_head_fwd_train / fgnn_head_bwd): e1, e2 (G,C,N) -> (ce_sum[G], correct[G]),
+    what ScoresFunction + CrossEntropyIdentityFunction compute (models/trainers.py:67, toolbox/losses.py:27-31,
+    toolbox/metrics.py:125-134) without the (G,N,N) scores or their gradient.  16-bit precisions only; correct is
+    not differentiable."""
+
+    @staticmethod
+    def forward(ctx, e1, e2, n_dev, precision):
+        lib = L.get_lib()
+        c_in = e1.shape[1] if e1.dim() == 3 else None
+        e1, e2, Cc = _head_operands(e1, e2, precision, "HeadFunction")
+        G, _, N = e1.shape
+        ce = torch.empty(G, device=e1.device, dtype=torch.float32)
+        correct = torch.empty(G, device=e1.device, dtype=torch.int32)
+        lse = torch.empty((G, N), device=e1.device, dtype=torch.float32)
+        ws = L.workspace(e1.device, lib.fgnn_head_workspace_bytes(G, N))
+        L.check(lib.fgnn_head_fwd_train(L.PRECISIONS[precision], L.ptr(e1), L.ptr(e2), L.ptr(ce), L.ptr(correct), L.ptr(lse),
+                                        G, Cc, N, _npg(n_dev, G), L.ptr(ws), ws.numel(), L.stream_ptr(e1.device)),
+                "fgnn_head_fwd_train")
+        ctx.save_for_backward(e1, e2, lse, n_dev if n_dev is not None else torch.empty(0))
+        ctx.has_n, ctx.precision, ctx.c_in = n_dev is not None, precision, c_in
+        ctx.mark_non_differentiable(correct)
+        return ce, correct
+
+    @staticmethod
+    def backward(ctx, dce, _dcorrect):
+        lib = L.get_lib()
+        e1, e2, lse, n_dev = ctx.saved_tensors
+        n_dev = n_dev if ctx.has_n else None
+        G, Cc, N = e1.shape
+        coef = L.require_cuda_f32(dce, "dce")
+        de1, de2 = torch.empty_like(e1), torch.empty_like(e2)
+        L.check(lib.fgnn_head_bwd(L.PRECISIONS[ctx.precision], L.ptr(e1), L.ptr(e2), L.ptr(lse), L.ptr(coef), L.ptr(de1),
+                                  L.ptr(de2), G, Cc, N, _npg(n_dev, G), None, 0, L.stream_ptr(e1.device)), "fgnn_head_bwd")
+        if Cc != ctx.c_in:
+            de1, de2 = de1[:, :ctx.c_in], de2[:, :ctx.c_in]
+        return de1, de2, None, None
 
 
 def graphnorm_fwd(x: torch.Tensor, n_dev, gn_w, gn_b, eps: float, constant_n: bool = True) -> torch.Tensor:

@@ -206,6 +206,21 @@ int fgnn_head_fwd(int32_t precision, const float* e1, const float* e2, float* sc
                       (cudaStream_t)stream);
 }
 
+int fgnn_head_fwd_train(int32_t precision, const float* e1, const float* e2, float* ce_sum, int32_t* correct, float* row_lse,
+                        int32_t G, int32_t C, int32_t N, const int32_t* n_per_graph, void* workspace, size_t workspace_bytes,
+                        void* stream) {
+  return tc::head_fwd_train(precision, e1, e2, ce_sum, correct, row_lse, G, C, N, n_per_graph, workspace, workspace_bytes,
+                            (cudaStream_t)stream);
+}
+
+int fgnn_head_bwd(int32_t precision, const float* e1, const float* e2, const float* row_lse, const float* coef, float* de1,
+                  float* de2, int32_t G, int32_t C, int32_t N, const int32_t* n_per_graph, void* workspace,
+                  size_t workspace_bytes, void* stream) {
+  (void)workspace;
+  (void)workspace_bytes;
+  return tc::head_bwd(precision, e1, e2, row_lse, coef, de1, de2, G, C, N, n_per_graph, (cudaStream_t)stream);
+}
+
 int fgnn_lap_fwd(const float* scores, int32_t* col_of_row, int32_t* correct, double* total_cost, int32_t G,
                  int32_t N, const int32_t* n_per_graph, void* stream) {
   return lap::lap_fwd(scores, col_of_row, correct, total_cost, G, N, n_per_graph, (cudaStream_t)stream);

@@ -1296,7 +1296,13 @@ tc_matmul_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
 //   from the fp32 embeddings as 16-bit (hi, lo) pairs: D = Ahi Bhi + Alo Bhi + Ahi Blo recovers fp32-level accuracy
 //   (the dropped lo x lo term is 2^-22 relative) at 3 x the (tiny, K = C) MMA work.
 // One CTA per (pair, 128-row tile); warps 0-3 = epilogue rows (TMEM quadrant = warp), warp 4 = MMA issuer; everybody
-// converts operands.
+// converts operands.  kRowLse (training forward) also stores every row's log-sum-exp for the backward below; it is a
+// template parameter, not a run-time flag, so that the inference instance is the kernel it was without it.
+// The backward (tc_head_bwd_kernel) needs no (G,N,N) buffer either: it recomputes S tile by tile from the same (hi, lo)
+// operands, forms dS = P - I in the epilogue from the saved lse, and accumulates dS E2^T (or dS^T E1^T) on tcgen05 as
+// three (hi, lo) MMAs per product; coef[g] = d loss / d ce_sum[g] scales the fp32 accumulator, not the 16-bit operand
+// (coef p falls below fp16's normal range at coef = 1 / #rows).  One CTA per (pair, 128-row tile) walks the column
+// tiles for d E1, one per (pair, 128-column tile) walks the row tiles for d E2: every output is written once.
 // =============================================================================================
 struct HeadArgs {
   const float* e1;       // (G,C,N)
@@ -1305,9 +1311,10 @@ struct HeadArgs {
   float* partial;        // [G][MT][2] = (sum CE, #correct) of the row tile
   int G, C, N, MT;
   const int32_t* n_per_graph;
+  float* row_lse;        // (G,N), kRowLse only: log sum_j exp(s_ij) of valid rows, 0 elsewhere
 };
 
-template <typename T>
+template <typename T, bool kRowLse>
 __global__ void __launch_bounds__(160, 1) tc_head_kernel(const HeadArgs a) {
   extern __shared__ uint8_t smem_head[];
   uint8_t* smem = smem_head + ((1024u - (smem_u32(smem_head) & 1023u)) & 1023u);
@@ -1329,6 +1336,8 @@ __global__ void __launch_bounds__(160, 1) tc_head_kernel(const HeadArgs a) {
   const bool want_scores = a.scores != nullptr;
   if (i0 >= n && !want_scores) {                            // nothing valid in this row tile
     if (threadIdx.x == 0) { a.partial[((size_t)b * a.MT + mt) * 2] = 0.f; a.partial[((size_t)b * a.MT + mt) * 2 + 1] = 0.f; }
+    if constexpr (kRowLse)
+      if (threadIdx.x < 128 && i0 + (int)threadIdx.x < N) a.row_lse[(size_t)b * N + i0 + threadIdx.x] = 0.f;
     return;
   }
   if (threadIdx.x == 0) { mbar_init(bar, 1); fence_barrier_init(); }
@@ -1431,6 +1440,8 @@ __global__ void __launch_bounds__(160, 1) tc_head_kernel(const HeadArgs a) {
     __syncthreads();                                        // accumulator and B tiles are free again
   }
   if (warp < 4) {
+    if constexpr (kRowLse)
+      if (i < N) a.row_lse[(size_t)b * N + i] = row_ok ? run_m + logf(run_l) : 0.f;
     float ce = row_ok ? (run_m + logf(run_l) - diag) : 0.f;
     float ok = (row_ok && best_j == i) ? 1.f : 0.f;
 #pragma unroll
@@ -1459,6 +1470,186 @@ __global__ void head_finalize_kernel(const float* __restrict__ partial, float* _
   for (int m = 0; m < MT; ++m) { ce += partial[((size_t)b * MT + m) * 2]; ok += partial[((size_t)b * MT + m) * 2 + 1]; }
   ce_sum[b] = ce;
   correct[b] = (int32_t)(ok + 0.5f);
+}
+
+// K_H backward (see above).  kRows: the CTA owns 128 rows i of S (x = E1, y = E2, dx = d E1) and its rows' lse;
+// otherwise 128 columns j (x = E2, y = E1, dx = d E2) and the walked tiles are rows of S, whose lse is staged in shared
+// memory.  Per walked 128-wide tile t of y:
+//   T = X^T Y_t (tcgen05, TMEM cols [0,128); = S or S^T)  ->  P = exp(s - lse_row) - [i == j], zero outside n x n,
+//   as 16-bit (hi, lo) K-major tiles  ->  D (TMEM cols [128, 128 + C)) += P Y_t^T.
+// The y tile is stored MN-major (K = channel) for the first product; the same bytes are the K-major B operand
+// (K = position, N = channel) of the second.  The steps of one tile are serialised (commit / wait): the kernel is
+// bound by the exponentials of the epilogue, not by the MMAs.
+struct HeadBwdArgs {
+  const float* x;        // (G,C,N): the side whose gradient this launch writes
+  const float* y;        // (G,C,N): the other side
+  const float* row_lse;  // (G,N)
+  const float* coef;     // [G]
+  float* dx;             // (G,C,N)
+  int C, N;
+  const int32_t* n_per_graph;
+};
+
+template <typename T, bool kRows>
+__global__ void __launch_bounds__(160, 1) tc_head_bwd_kernel(const HeadBwdArgs a) {
+  extern __shared__ uint8_t smem_head_bwd[];
+  uint8_t* smem = smem_head_bwd + ((1024u - (smem_u32(smem_head_bwd) & 1023u)) & 1023u);
+  const int C = a.C, N = a.N;
+  const uint32_t xy_bytes = (uint32_t)C * 256u;             // 128 positions x C x 2 bytes
+  uint8_t* sXhi = smem;
+  uint8_t* sXlo = sXhi + xy_bytes;
+  uint8_t* sYhi = sXlo + xy_bytes;
+  uint8_t* sYlo = sYhi + xy_bytes;
+  uint8_t* sPhi = sYlo + xy_bytes;                          // [2 K chunks][128 rows][128 B], 16-byte units XOR (row & 7)
+  uint8_t* sPlo = sPhi + 32768;
+  uint64_t* bar = reinterpret_cast<uint64_t*>(sPlo + 32768);   // [0] T ready, [1] P Y^T done
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bar + 2);
+  float* s_lse = reinterpret_cast<float*>(tmem_slot + 2);   // [128] lse of the walked rows (!kRows)
+  const int warp = uniform_warp_idx(), lane = threadIdx.x % 32;
+  const int t0 = blockIdx.x * 128, b = blockIdx.y;
+  const int n = graph_n(a.n_per_graph, b, N);
+  const float* xg = a.x + (size_t)b * C * N;
+  const float* yg = a.y + (size_t)b * C * N;
+  float* dxg = a.dx + (size_t)b * C * N;
+  if (t0 >= n) {                                            // no valid position: exact zeros
+    for (int idx = threadIdx.x; idx < C * 128; idx += blockDim.x) {
+      const int c = idx / 128, p = t0 + idx % 128;
+      if (p < N) dxg[(size_t)c * N + p] = 0.f;
+    }
+    return;
+  }
+  if (threadIdx.x == 0) { mbar_init(&bar[0], 1); mbar_init(&bar[1], 1); fence_barrier_init(); }
+  if (warp == 4) tmem_alloc(tmem_slot, 256);
+  auto put8 = [&](const float* src_row, int first, uint8_t* hi_tile, uint8_t* lo_tile, int c, int pos) {
+    uint32_t hw[4], lw[4];
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const int x0 = first + 2 * u, x1 = x0 + 1;
+      const float v0 = x0 < n ? src_row[x0] : 0.f, v1 = x1 < n ? src_row[x1] : 0.f;
+      const float h0 = Elem<T>::to_float(Elem<T>::from_float(v0)), h1 = Elem<T>::to_float(Elem<T>::from_float(v1));
+      hw[u] = Elem<T>::pack(v0, v1);
+      lw[u] = Elem<T>::pack(v0 - h0, v1 - h1);
+    }
+    const uint32_t off = (uint32_t)(pos >> 6) * (uint32_t)(C * 128) + (uint32_t)c * 128u + (uint32_t)((((pos & 63) >> 3) ^ (c & 7)) << 4);
+    *reinterpret_cast<uint4*>(hi_tile + off) = make_uint4(hw[0], hw[1], hw[2], hw[3]);
+    *reinterpret_cast<uint4*>(lo_tile + off) = make_uint4(lw[0], lw[1], lw[2], lw[3]);
+  };
+  for (int idx = threadIdx.x; idx < C * 16; idx += blockDim.x) {
+    const int c = idx / 16, q = idx % 16;
+    put8(xg + (size_t)c * N, t0 + q * 8, sXhi, sXlo, c, q * 8);
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_slot;
+  const int r = warp * 32 + lane;                           // row of the CTA's tile (epilogue warps)
+  const int p_own = t0 + r;                                 // its position: i (kRows) or j
+  const bool own_ok = warp < 4 && p_own < n;
+  const float lse_own = (kRows && own_ok) ? a.row_lse[(size_t)b * N + p_own] : 0.f;
+  uint32_t phase = 0;
+  for (int w0 = 0; w0 < n; w0 += 128) {
+    if (w0 > 0) { mbar_wait(&bar[1], phase ^ 1u); tc_fence_after(); }   // previous P Y^T has read sY and sP
+    for (int idx = threadIdx.x; idx < C * 16; idx += blockDim.x) {
+      const int c = idx / 16, q = idx % 16;
+      put8(yg + (size_t)c * N, w0 + q * 8, sYhi, sYlo, c, q * 8);
+    }
+    if (!kRows && threadIdx.x < 128) s_lse[threadIdx.x] = w0 + (int)threadIdx.x < n ? a.row_lse[(size_t)b * N + w0 + threadIdx.x] : 0.f;
+    fence_proxy_async_smem();
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 4) {
+      tc_fence_after();
+      const uint32_t idesc = make_idesc(Elem<T>::kFmt, 1, 1, 128, 128);
+      const uint64_t dxh = smem_desc_sw128(smem_u32(sXhi), (uint32_t)C * 128u, 1024u), dxl = smem_desc_sw128(smem_u32(sXlo), (uint32_t)C * 128u, 1024u);
+      const uint64_t dyh = smem_desc_sw128(smem_u32(sYhi), (uint32_t)C * 128u, 1024u), dyl = smem_desc_sw128(smem_u32(sYlo), (uint32_t)C * 128u, 1024u);
+      if (elect_one_sync()) {
+        for (int k = 0; k < C / 16; ++k) {
+          const uint64_t adv = (uint64_t)((uint32_t)k * 2048u >> 4);
+          mma_ss(tmem_base, dxh + adv, dyh + adv, idesc, k > 0 ? 1u : 0u);
+          mma_ss(tmem_base, dxl + adv, dyh + adv, idesc, 1u);
+          mma_ss(tmem_base, dxh + adv, dyl + adv, idesc, 1u);
+        }
+        mma_commit(&bar[0]);
+      }
+      __syncwarp();
+    }
+    if (warp < 4) {
+      mbar_wait(&bar[0], phase);
+      tc_fence_after();
+      const uint32_t taddr = tmem_base + ((uint32_t)(warp * 32) << 16);
+#pragma unroll 1
+      for (int c0 = 0; c0 < 128; c0 += 32) {
+        uint32_t v[32];
+        tmem_ld32(taddr + (uint32_t)c0, v);
+        tmem_wait_ld();
+        float pv[32];
+#pragma unroll
+        for (int u = 0; u < 32; ++u) {
+          const int q = w0 + c0 + u;                        // the walked position: j (kRows) or i
+          const float lse = kRows ? lse_own : s_lse[c0 + u];
+          pv[u] = (own_ok && q < n) ? __expf(__uint_as_float(v[u]) - lse) - (q == p_own ? 1.f : 0.f) : 0.f;
+        }
+#pragma unroll
+        for (int s8 = 0; s8 < 4; ++s8) {
+          uint32_t hw[4], lw[4];
+#pragma unroll
+          for (int e = 0; e < 4; ++e) {
+            const float v0 = pv[s8 * 8 + 2 * e], v1 = pv[s8 * 8 + 2 * e + 1];
+            const float h0 = Elem<T>::to_float(Elem<T>::from_float(v0)), h1 = Elem<T>::to_float(Elem<T>::from_float(v1));
+            hw[e] = Elem<T>::pack(v0, v1);
+            lw[e] = Elem<T>::pack(v0 - h0, v1 - h1);
+          }
+          const int k = c0 + s8 * 8;                        // K position of the 8 values
+          const uint32_t off = (uint32_t)(k >> 6) * 16384u + (uint32_t)r * 128u + (uint32_t)((((k & 63) >> 3) ^ (r & 7)) << 4);
+          *reinterpret_cast<uint4*>(sPhi + off) = make_uint4(hw[0], hw[1], hw[2], hw[3]);
+          *reinterpret_cast<uint4*>(sPlo + off) = make_uint4(lw[0], lw[1], lw[2], lw[3]);
+        }
+      }
+    }
+    fence_proxy_async_smem();
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 4) {
+      tc_fence_after();
+      const uint32_t idesc = make_idesc(Elem<T>::kFmt, 0, 0, 128, C);
+      const uint64_t dph = smem_desc_sw128(smem_u32(sPhi), 16u, 1024u), dpl = smem_desc_sw128(smem_u32(sPlo), 16u, 1024u);
+      const uint64_t dyh = smem_desc_sw128(smem_u32(sYhi), 16u, 1024u), dyl = smem_desc_sw128(smem_u32(sYlo), 16u, 1024u);
+      if (elect_one_sync()) {
+        for (int k = 0; k < 8; ++k) {                       // K = 128 walked positions, 16 per MMA
+          const uint64_t pa = (uint64_t)(((uint32_t)(k >> 2) * 16384u + (uint32_t)(k & 3) * 32u) >> 4);
+          const uint64_t ya = (uint64_t)(((uint32_t)(k >> 2) * (uint32_t)(C * 128) + (uint32_t)(k & 3) * 32u) >> 4);
+          mma_ss(tmem_base + 128u, dph + pa, dyh + ya, idesc, (w0 > 0 || k > 0) ? 1u : 0u);
+          mma_ss(tmem_base + 128u, dpl + pa, dyh + ya, idesc, 1u);
+          mma_ss(tmem_base + 128u, dph + pa, dyl + ya, idesc, 1u);
+        }
+        mma_commit(&bar[1]);
+      }
+      __syncwarp();
+    }
+    phase ^= 1u;
+  }
+  if (warp < 4) {
+    mbar_wait(&bar[1], phase ^ 1u);
+    tc_fence_after();
+    const uint32_t taddr = tmem_base + ((uint32_t)(warp * 32) << 16) + 128u;
+    const float cf = a.coef[b];
+#pragma unroll 1
+    for (int c0 = 0; c0 < C; c0 += 16) {
+      uint32_t v[16];
+      tmem_ld16(taddr + (uint32_t)c0, v);
+      tmem_wait_ld();
+      if (p_own < N) {
+#pragma unroll
+        for (int u = 0; u < 16; ++u) dxg[(size_t)(c0 + u) * N + p_own] = own_ok ? cf * __uint_as_float(v[u]) : 0.f;
+      }
+    }
+    tc_fence_before();
+  }
+  __syncthreads();
+  if (warp == 4) {
+    __syncwarp();
+    tmem_dealloc(tmem_base, 256);
+  }
 }
 
 // =============================================================================================
@@ -1969,18 +2160,19 @@ int embed_fwd_adjacency(const fgnn_embed_params& p, int precision, const uint8_t
 
 size_t head_workspace_bytes(int G, int N) { return align_up((size_t)G * ((N + 127) / 128) * 2 * sizeof(float), 256); }
 
-template <typename T>
-int head_fwd_t(const float* e1, const float* e2, float* scores, float* ce_sum, int32_t* correct, int G, int C, int N,
-               const int32_t* npg, void* ws, size_t ws_bytes, cudaStream_t st) {
+template <typename T, bool kRowLse>
+int head_fwd_t(const float* e1, const float* e2, float* scores, float* ce_sum, int32_t* correct, float* row_lse, int G, int C,
+               int N, const int32_t* npg, void* ws, cudaStream_t st) {
   HeadArgs a{};
   a.e1 = e1; a.e2 = e2; a.scores = scores;
   a.partial = static_cast<float*>(ws);
   a.G = G; a.C = C; a.N = N; a.MT = (N + 127) / 128;
   a.n_per_graph = npg;
+  a.row_lse = row_lse;
   const size_t smem = 1024 + (size_t)C * 256 * 2 + (size_t)C * 512 * 2 + 128;
-  FGNN_CUDA(cudaFuncSetAttribute(tc_head_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  FGNN_CUDA(cudaFuncSetAttribute(tc_head_kernel<T, kRowLse>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   prof::begin(prof::kGlue, st);
-  tc_head_kernel<T><<<dim3(a.MT, G), 160, smem, st>>>(a);
+  tc_head_kernel<T, kRowLse><<<dim3(a.MT, G), 160, smem, st>>>(a);
   FGNN_LAUNCHED();
   head_finalize_kernel<<<ceil_div(G, 128), 128, 0, st>>>(a.partial, ce_sum, correct, G, a.MT);
   prof::end(prof::kGlue, st);
@@ -1988,15 +2180,51 @@ int head_fwd_t(const float* e1, const float* e2, float* scores, float* ce_sum, i
   return FGNN_OK;
 }
 
+// the shapes every fused-head entry point accepts
+int check_head_shape(int G, int C, int N) {
+  FGNN_CHECK_ARG(G >= 1 && G <= 65535 && N >= 1 && N <= kMaxN, "fused head supports G <= 65535 and N <= %d (got G=%d N=%d)",
+                 kMaxN, G, N);
+  FGNN_CHECK_ARG(C >= 16 && C <= 128 && C % 16 == 0, "the fused head needs an embedding width that is a multiple of 16, at most 128 (got %d)", C);
+  return FGNN_OK;
+}
+
 int head_fwd(int precision, const float* e1, const float* e2, float* scores, float* ce_sum, int32_t* correct, int G, int C,
              int N, const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
   return with_16bit(precision, "fgnn_head_fwd", [&](auto t) -> int {
     FGNN_CHECK_ARG(e1 && e2 && ce_sum && correct && ws, "null pointer");
-    FGNN_CHECK_ARG(G >= 1 && G <= 65535 && N >= 1 && N <= kMaxN, "fused head supports G <= 65535 and N <= %d (got G=%d N=%d)",
-                   kMaxN, G, N);
-    FGNN_CHECK_ARG(C >= 16 && C <= 128 && C % 16 == 0, "the fused head needs an embedding width that is a multiple of 16, at most 128 (got %d)", C);
+    if (int e = check_head_shape(G, C, N)) return e;
     if (ws_bytes < head_workspace_bytes(G, N)) return fail(FGNN_ERR_WORKSPACE, "head workspace too small");
-    return head_fwd_t<decltype(t)>(e1, e2, scores, ce_sum, correct, G, C, N, n_per_graph, ws, ws_bytes, st);
+    return head_fwd_t<decltype(t), false>(e1, e2, scores, ce_sum, correct, nullptr, G, C, N, n_per_graph, ws, st);
+  });
+}
+
+int head_fwd_train(int precision, const float* e1, const float* e2, float* ce_sum, int32_t* correct, float* row_lse, int G,
+                   int C, int N, const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
+  return with_16bit(precision, "fgnn_head_fwd_train", [&](auto t) -> int {
+    FGNN_CHECK_ARG(e1 && e2 && ce_sum && correct && row_lse && ws, "null pointer");
+    if (int e = check_head_shape(G, C, N)) return e;
+    if (ws_bytes < head_workspace_bytes(G, N)) return fail(FGNN_ERR_WORKSPACE, "head workspace too small");
+    return head_fwd_t<decltype(t), true>(e1, e2, nullptr, ce_sum, correct, row_lse, G, C, N, n_per_graph, ws, st);
+  });
+}
+
+int head_bwd(int precision, const float* e1, const float* e2, const float* row_lse, const float* coef, float* de1, float* de2,
+             int G, int C, int N, const int32_t* n_per_graph, cudaStream_t st) {
+  return with_16bit(precision, "fgnn_head_bwd", [&](auto t) -> int {
+    using T = decltype(t);
+    FGNN_CHECK_ARG(e1 && e2 && row_lse && coef && de1 && de2, "null pointer");
+    if (int e = check_head_shape(G, C, N)) return e;
+    const size_t smem = 1024 + (size_t)C * 256 * 4 + 2 * 32768 + 16 + 8 + 128 * sizeof(float);
+    const dim3 grid((N + 127) / 128, G);
+    prof::begin(prof::kGlue, st);
+    FGNN_CUDA(cudaFuncSetAttribute(tc_head_bwd_kernel<T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    tc_head_bwd_kernel<T, true><<<grid, 160, smem, st>>>(HeadBwdArgs{e1, e2, row_lse, coef, de1, C, N, n_per_graph});
+    FGNN_LAUNCHED();
+    FGNN_CUDA(cudaFuncSetAttribute(tc_head_bwd_kernel<T, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    tc_head_bwd_kernel<T, false><<<grid, 160, smem, st>>>(HeadBwdArgs{e2, e1, row_lse, coef, de2, C, N, n_per_graph});
+    prof::end(prof::kGlue, st);
+    FGNN_LAUNCHED();
+    return FGNN_OK;
   });
 }
 

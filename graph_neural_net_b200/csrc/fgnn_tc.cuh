@@ -23,6 +23,11 @@ int embed_bwd(const fgnn_embed_params& p, const fgnn_embed_grads& g, int precisi
 size_t head_workspace_bytes(int G, int N);
 int head_fwd(int precision, const float* e1, const float* e2, float* scores, float* ce_sum, int32_t* correct, int G, int C,
              int N, const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st);
+// training: the same forward keeping each row's log-sum-exp, and its backward (d E1, d E2 without the (G,N,N) scores)
+int head_fwd_train(int precision, const float* e1, const float* e2, float* ce_sum, int32_t* correct, float* row_lse, int G,
+                   int C, int N, const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st);
+int head_bwd(int precision, const float* e1, const float* e2, const float* row_lse, const float* coef, float* de1, float* de2,
+             int G, int C, int N, const int32_t* n_per_graph, cudaStream_t st);
 
 size_t debug_matmul_workspace_bytes(int G, int C, int N);
 int debug_matmul(int precision, const float* a, const float* b, float* out, int G, int C, int N,

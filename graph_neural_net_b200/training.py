@@ -113,18 +113,40 @@ class FlatAdam(torch.optim.Optimizer):
                                                L.stream_ptr(self.flat_p.device)), "fgnn_adam_step_f32")
 
 
-def train_step_flat(model, opt: "FlatAdam", x1, x2, group: Optional[dist.ProcessGroup] = None):
+def train_step_flat(model, opt: "FlatAdam", x1, x2, group: Optional[dist.ProcessGroup] = None, fused_head: bool = False):
     """train_step with the flat trainer: same arithmetic, three framework launches instead of several per parameter
-    around the forward / backward (memset, all-reduce, fused Adam).  Returns (global loss, #correct, #rows)."""
+    around the forward / backward (memset, all-reduce, fused Adam).  Returns (global loss, #correct, #rows).
+    fused_head (16-bit precisions): the head and its backward run as the fused tensor-core kernels (_ops.HeadFunction)
+    instead of the scores, the cross-entropy and their gradients as (B,N,N) tensors; the same loss and gradients."""
     from . import _ops
+    from .maskedtensors.maskedtensor import MaskedTensor
     from .toolbox.losses import _as_batch
 
+    if fused_head and getattr(model, "precision", "fp32") == "fp32":
+        raise _ops.L.FgnnError("fused_head is the tensor-core head of the 16-bit precisions; fp32 trains through the "
+                               "CUDA-core scores and cross-entropy")
     opt.begin_step()
-    scores = model(x1, x2)
-    plain, n_dev, sizes = _as_batch(scores)
-    ce, correct = _ops.CrossEntropyIdentityFunction.apply(plain, n_dev)
-    local_sum = ce.sum()
-    local_sum.backward()                                   # gradients land in opt.flat_g (in place)
+    try:
+        if fused_head:
+            e1, e2 = model.embed(x1), model.embed(x2)
+            if isinstance(e1, MaskedTensor):
+                n_dev = e1.sizes_i32()
+                sizes = n_dev.to(torch.float32)
+                e1, e2 = e1.tensor.rename(None), e2.tensor.rename(None)
+            else:
+                n_dev = None
+                sizes = torch.full((e1.shape[0],), float(e1.shape[-1]), device=e1.device)
+            ce, correct = _ops.HeadFunction.apply(e1, e2, n_dev, model.precision)
+        else:
+            scores = model(x1, x2)
+            plain, n_dev, sizes = _as_batch(scores)
+            ce, correct = _ops.CrossEntropyIdentityFunction.apply(plain, n_dev)
+        local_sum = ce.sum()
+        local_sum.backward()                                   # gradients land in opt.flat_g (in place)
+    finally:
+        # the sink maps parameter addresses of THIS model to its flat buffer: left behind, it would capture the
+        # gradients of whatever later reuses those addresses (another model's parameters) and return none to autograd
+        _ops.GRAD_SINK.clear()
     grads = opt.flat_g[:opt.n]
     ex = opt.extras
     ex[0] = local_sum.detach()

@@ -182,12 +182,29 @@ int fgnn_ce_bwd_f32(const float* scores, const float* row_lse, const float* coef
  * (toolbox/metrics.py:125-134) in the epilogue of the tcgen05 GEMM, flash style: online row max / sum of exponentials
  * over 256-column tiles.  e1,e2 (G,C,N) fp32 are split into 16-bit (hi, lo) operand pairs in shared memory
  * (Ahi Bhi + Alo Bhi + Ahi Blo: fp32-level accuracy), C a multiple of 16, at most 128.  ce_sum[G], correct[G] as
- * fgnn_ce_argmax_fwd_f32; scores (G,N,N) is written only when non-NULL (zero outside the n_g x n_g block).  N <= 4096.
- * Forward only (training differentiates through fgnn_scores_* / fgnn_ce_*). */
+ * fgnn_ce_argmax_fwd_f32; scores (G,N,N) is written only when non-NULL (zero outside the n_g x n_g block).  N <= 4096,
+ * G <= 65535.  Training goes through fgnn_head_fwd_train / fgnn_head_bwd below. */
 size_t fgnn_head_workspace_bytes(int32_t G, int32_t N);
 int fgnn_head_fwd(int32_t precision, const float* e1, const float* e2, float* scores, float* ce_sum, int32_t* correct,
                   int32_t G, int32_t C, int32_t N, const int32_t* n_per_graph, void* workspace, size_t workspace_bytes,
                   void* stream);
+/* Training form of the fused head: the scores (models/trainers.py:67) and the summed cross-entropy against the identity
+ * matching (toolbox/losses.py:27-34) with autograd's backward through both, without ever forming the (G,N,N) scores
+ * or their gradient (fgnn_scores_* + fgnn_ce_* keep two such tensors per step).
+ * fgnn_head_fwd_train: ce_sum, correct bit-identical to fgnn_head_fwd, plus row_lse (G,N) fp32 = log sum_j exp(s_ij)
+ * of every valid row (0 for i >= n_g), kept for the backward; workspace as fgnn_head_workspace_bytes.
+ * fgnn_head_bwd: coef[G] = d loss / d ce_sum[g] (device);  with dS_ij = coef[g] (softmax(s_i)_j - [i == j]) it
+ * OVERWRITES de1[g,:,i] = sum_j dS_ij e2[g,:,j] and de2[g,:,j] = sum_i dS_ij e1[g,:,i] (G,C,N), zero at positions
+ * >= n_g -- what fgnn_ce_bwd_f32 followed by fgnn_scores_bwd_f32 compute.  S is recomputed from the (hi, lo) operands
+ * and dS is split into (hi, lo) operands too (fp32-level gradients); coef scales the fp32 accumulator.  Deterministic
+ * (every output written once, no atomics).  The backward needs no workspace (NULL, 0 are accepted).  Both calls take
+ * FGNN_BF16 / FGNN_FP16, C a multiple of 16 at most 128, N <= 4096, G <= 65535. */
+int fgnn_head_fwd_train(int32_t precision, const float* e1, const float* e2, float* ce_sum, int32_t* correct, float* row_lse,
+                        int32_t G, int32_t C, int32_t N, const int32_t* n_per_graph, void* workspace, size_t workspace_bytes,
+                        void* stream);
+int fgnn_head_bwd(int32_t precision, const float* e1, const float* e2, const float* row_lse, const float* coef, float* de1,
+                  float* de2, int32_t G, int32_t C, int32_t N, const int32_t* n_per_graph, void* workspace,
+                  size_t workspace_bytes, void* stream);
 
 /* accuracy_linear_assignment (toolbox/metrics.py:92-116), the metric training_step / validation_step call
  * (models/trainers.py:53,74): per graph the assignment scipy.optimize.linear_sum_assignment returns on

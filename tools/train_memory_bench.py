@@ -132,7 +132,6 @@ def main():
     res["cfg2_recompute_overhead"] = {"keep_all_ms_median": k, "recompute_ms_median": rc, "ratio": rc / k}
     print(json.dumps(res["cfg2_recompute_overhead"]), flush=True)
     del model, opt, b1, b2
-    _ops.GRAD_SINK.clear()
     torch.cuda.empty_cache()
 
     # shapes whose keep-all step does not fit one device: the default threshold picks the recompute plan
@@ -140,7 +139,6 @@ def main():
         model, opt, b1, b2 = setup(n, c, pairs)
         measure(f"n{n} c{c} {pairs} pairs", n, c, pairs, model, opt, b1, b2)
         del model, opt, b1, b2
-        _ops.GRAD_SINK.clear()
         torch.cuda.empty_cache()
 
     res["card_after"] = card()
