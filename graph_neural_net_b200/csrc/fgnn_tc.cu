@@ -208,41 +208,57 @@ __global__ void from_planes_kernel(const T* __restrict__ in, float* __restrict__
   }
 }
 
-// fp32 hidden-layer weights (co, ci) -> 16-bit [co][Kh] zero padded (Kh multiple of 64), for up to all hidden-layer
-// matrices of one block in ONE launch (blockIdx.y = matrix)
+// fp32 hidden-layer weights (rows, cols) -> 16-bit [co][Kh] zero padded (rows <= co, Kh multiple of 64), for up to all
+// hidden-layer matrices of one block in ONE launch (blockIdx.y = matrix)
 struct ConvertBatch {
   const float* src[3 * (FGNN_MAX_DEPTH - 1)];
   long dst_off[3 * (FGNN_MAX_DEPTH - 1)];   // element offset of the matrix in `out`
+  int rows, cols;                            // real shape of every source matrix
 };
 template <typename T>
-__global__ void convert_weights_batch_kernel(ConvertBatch cb, T* __restrict__ out, int co, int ci, int Kh) {
+__global__ void convert_weights_batch_kernel(ConvertBatch cb, T* __restrict__ out, int co, int Kh) {
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= co * Kh) return;
   const int o = idx / Kh, k = idx % Kh;
-  out[cb.dst_off[blockIdx.y] + idx] = Elem<T>::from_float(k < ci ? cb.src[blockIdx.y][o * ci + k] : 0.f);
+  out[cb.dst_off[blockIdx.y] + idx] = Elem<T>::from_float(o < cb.rows && k < cb.cols ? cb.src[blockIdx.y][o * cb.cols + k] : 0.f);
+}
+
+// up to 2 (FGNN_MAX_DEPTH - 2) fp32 vectors of `real` entries -> [blockIdx.y][C] zero padded (hidden-layer biases)
+struct PadBatch {
+  const float* src[2 * (FGNN_MAX_DEPTH - 2)];
+};
+__global__ void pad_vectors_kernel(PadBatch pb, float* __restrict__ out, int C, int real) {
+  const int c = threadIdx.x;
+  if (c < C) out[blockIdx.y * C + c] = c < real ? pb.src[blockIdx.y][c] : 0.f;
 }
 
 // Per-graph folded first-layer weights for up to two MLPs that share their input (mlp1/mlp2).
 //   Wf[g][m][co][koff_s + ch] = W_m[co][col_s + ch] * a_s[g][ch]
 //   bf[g][m][co]              = b_m[co] + sum_s sum_ch W_m[co][col_s + ch] * s_s[g][ch]
+// W_m and b_m have their real shapes; the source planes and the outputs are stored with c_s >= cr_s and c_out >= co_real
+// channels, and the padded rows and columns fold to zero (see make_plan).  Real column col_s + ch is stored column
+// (s ? c_0 : 0) + ch, so the bias sums visit the real terms in the order a zero-padded copy of W_m would.
 struct FoldArgs {
-  const float* w[2];     // per MLP: (c_out, c0 + c1)
-  const float* b[2];     // per MLP: (c_out)
+  const float* w[2];     // per MLP: (co_real, cr0 + cr1)
+  const float* b[2];     // per MLP: (co_real)
   const float* coef[2];  // per source: [G][c_s][2] or null (identity)
-  int c[2], koff[2], nsrc, nmlp;
-  int c_out, K1g;
+  int c[2], cr[2], koff[2], nsrc, nmlp;
+  int c_out, co_real, K1g;
 };
 template <typename T>
 __global__ void __launch_bounds__(256)
 fold_weights_kernel(FoldArgs a, T* __restrict__ wf, float* __restrict__ bf, T* __restrict__ bt) {
   const int g = blockIdx.x, m = blockIdx.y;
   const int cin = a.c[0] + (a.nsrc > 1 ? a.c[1] : 0);
-  __shared__ float s_a[512], s_s[512];          // per input column: scale and shift of its source channel
+  const int cin_real = a.cr[0] + (a.nsrc > 1 ? a.cr[1] : 0);
+  __shared__ float s_a[512], s_s[512];          // per stored input column: scale and shift of its source channel
+  __shared__ int s_col[512];                    // per stored input column: its column of W_m, or -1 (padding)
   for (int col = threadIdx.x; col < cin; col += blockDim.x) {
     const int s = (col < a.c[0]) ? 0 : 1;
     const int ch = col - (s ? a.c[0] : 0);
     s_a[col] = a.coef[s] ? a.coef[s][((long)g * a.c[s] + ch) * 2] : 1.f;
     s_s[col] = a.coef[s] ? a.coef[s][((long)g * a.c[s] + ch) * 2 + 1] : 0.f;
+    s_col[col] = ch < a.cr[s] ? (s ? a.cr[0] : 0) + ch : -1;
   }
   __syncthreads();
   T* wg = wf + ((long)g * a.nmlp + m) * a.c_out * a.K1g;
@@ -256,17 +272,19 @@ fold_weights_kernel(FoldArgs a, T* __restrict__ wf, float* __restrict__ bf, T* _
     int col = -1;
     if (k < a.koff[1] || a.nsrc == 1) { if (k < a.c[0]) col = k; }
     else if (k - a.koff[1] < a.c[1]) col = a.c[0] + (k - a.koff[1]);
-    if (col >= 0) v = w[co * cin + col] * s_a[col];
+    if (col >= 0 && co < a.co_real && s_col[col] >= 0) v = w[co * cin_real + s_col[col]] * s_a[col];
     wg[idx] = Elem<T>::from_float(v);
   }
   // folded bias: one warp per output channel
   const int warp = threadIdx.x / 32, lane = threadIdx.x % 32;
   for (int co = co_begin + warp; co < co_end; co += blockDim.x / 32) {
     float acc = 0.f;
-    for (int col = lane; col < cin; col += 32) acc = fmaf(w[co * cin + col], s_s[col], acc);
+    if (co < a.co_real)
+      for (int col = lane; col < cin; col += 32)
+        acc = fmaf(s_col[col] >= 0 ? w[co * cin_real + s_col[col]] : 0.f, s_s[col], acc);
     for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
     if (lane == 0) {
-      const float bias = a.b[m][co] + acc;
+      const float bias = co < a.co_real ? a.b[m][co] + acc : 0.f;
       bf[((long)g * a.nmlp + m) * a.c_out + co] = bias;
       if (bt) {
         // the same bias as one K = 16 step of the first-layer MMA (conv-chain kernel): row n = m c_out + co of a
@@ -284,14 +302,17 @@ fold_weights_kernel(FoldArgs a, T* __restrict__ wf, float* __restrict__ bf, T* _
   }
 }
 
-// emb[g][c][i] = max_j (a y[i][j] + s) from the row-wise max / min codes the conv chain left in rowenc (rows >= n -> 0)
+// emb[g][c][i] = max_j (a y[i][j] + s) from the row-wise max / min codes the conv chain left in rowenc (rows >= n -> 0);
+// emb is (G, co_real, N): the padded channels c >= co_real are not written
 __global__ void pool_finalize_kernel(const unsigned int* __restrict__ rowenc, const float* __restrict__ coef,
-                                     float* __restrict__ emb, int C, int N, long total, const int32_t* __restrict__ n_per_graph) {
+                                     float* __restrict__ emb, int C, int co_real, int N, long total,
+                                     const int32_t* __restrict__ n_per_graph) {
   const long idx = (long)blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= total) return;
   const int i = (int)(idx % N);
   const long gc = idx / N;
-  const int g = (int)(gc / C);
+  const int g = (int)(gc / C), c = (int)(gc % C);
+  if (c >= co_real) return;
   const int n = graph_n(n_per_graph, g, N);
   float out = 0.f;
   if (i < n) {
@@ -299,11 +320,12 @@ __global__ void pool_finalize_kernel(const unsigned int* __restrict__ rowenc, co
     const float mx = dec_ordered(rowenc[2 * idx]), mn = -dec_ordered(rowenc[2 * idx + 1]);
     out = fmaf(a, a >= 0.f ? mx : mn, sft);
   }
-  emb[idx] = out;
+  emb[((long)g * co_real + c) * N + i] = out;
 }
 
 // (sum, sum of squares) accumulated by the conv-chain epilogue -> GraphNorm scale / shift.
 //   acc[g][m][c][2] (double)  ->  coef_m[g][c] = {a, s}
+// gw / gb have co_real[m] entries (null gw: weight 1, bias 0); the padded channels get a zero affine, so a = s = 0.
 struct CoefArgs {
   const double* acc;
   float* coef[2];
@@ -311,6 +333,7 @@ struct CoefArgs {
   const float* gb[2];
   float eps[2];
   int constant_n[2];
+  int co_real[2];
   int nmlp, C, N;
   const int32_t* n_per_graph;
   float* gnstat[2];   // training: [G][C][4] = {mean, 1 / (var + eps), 1 / (2 sqrt(n (var + eps))), 0} kept for backward (or null)
@@ -327,9 +350,11 @@ __global__ void finalize_coef_kernel(CoefArgs a, int total) {
   const double mean = S / cnt;
   double var = SS / cnt - mean * mean;
   if (var < 0) var = 0;
-  const double sc = (double)(a.gw[m] ? a.gw[m][c] : 1.f) / (2.0 * sqrt((double)(a.constant_n[m] ? a.N : n) * (var + (double)a.eps[m])));
+  const bool real = c < a.co_real[m];
+  const float gw = real ? (a.gw[m] ? a.gw[m][c] : 1.f) : 0.f, gb = real && a.gb[m] ? a.gb[m][c] : 0.f;
+  const double sc = (double)gw / (2.0 * sqrt((double)(a.constant_n[m] ? a.N : n) * (var + (double)a.eps[m])));
   a.coef[m][((long)g * a.C + c) * 2] = (float)sc;
-  a.coef[m][((long)g * a.C + c) * 2 + 1] = (float)((double)(a.gb[m] ? a.gb[m][c] : 0.f) - sc * mean);
+  a.coef[m][((long)g * a.C + c) * 2 + 1] = (float)((double)gb - sc * mean);
   if (a.gnstat[m]) {
     float* gs = a.gnstat[m] + ((long)g * a.C + c) * 4;
     gs[0] = (float)mean;
@@ -1759,19 +1784,22 @@ int launch_matmul(const T* y1, const T* y2, T* out, const float* coef_a, const f
   });
 }
 
-// fold + conv chain(s) + statistics finalisation for 1 or 2 MLPs sharing their input
+// fold + conv chain(s) + statistics finalisation for 1 or 2 MLPs sharing their input.  The MLPs' parameters have their
+// real shapes (mp[m]->c_out <= C output channels, cr_src[s] <= c_src[s] channels read from source s); see make_plan.
 template <typename T>
 struct MlpGroup {
   int nmlp;
   const fgnn_mlp_params* mp[2];
   const T* src[2];
-  int c_src[2];
+  int c_src[2];              // channels of the source planes as stored
+  int cr_src[2];             // of which real
   const float* src_coef[2];
   int nsrc;
   T* wf;             // [G][nmlp][C][K1g] folded first-layer weights
   float* bf;         // [G][nmlp][C] folded first-layer bias
   T* bt;             // [G][nmlp][C][16] folded first-layer bias as an MMA step (may be null for depth-1 launches)
   const T* wh;       // [nmlp][depth-1][C][Kh]
+  float* bias_pad;   // room for [nmlp][depth-2][C] floats: the hidden biases zero-padded to C when c_out < C
   T* out[2];
   Layout out_mode[2];
   int ones[2];
@@ -1860,22 +1888,45 @@ int launch_mlp(const MlpGroup<T>& M, int C, int G, const Geo& geo, const int32_t
 
 template <typename T>
 int run_mlp_group(const MlpGroup<T>& M, int C, int G, const Geo& geo, const int32_t* npg, cudaStream_t st) {
+  const int co_real = M.mp[0]->c_out;
   FoldArgs fa{};
   fa.nmlp = M.nmlp;
   fa.nsrc = M.nsrc;
   for (int m = 0; m < M.nmlp; ++m) { fa.w[m] = M.mp[m]->w[0]; fa.b[m] = M.mp[m]->b[0]; }
   fa.c[0] = M.c_src[0];
   fa.c[1] = M.nsrc > 1 ? M.c_src[1] : 0;
+  fa.cr[0] = M.cr_src[0];
+  fa.cr[1] = M.nsrc > 1 ? M.cr_src[1] : 0;
   fa.coef[0] = M.src_coef[0];
   fa.coef[1] = M.nsrc > 1 ? M.src_coef[1] : nullptr;
   fa.koff[0] = 0;
   fa.koff[1] = round_up(M.c_src[0], 16);
   fa.c_out = C;
+  fa.co_real = co_real;
   fa.K1g = round_up(round_up(M.c_src[0], 16) + (M.nsrc > 1 ? round_up(M.c_src[1], 16) : 0), 64);
   FGNN_CHECK_ARG(fa.c[0] + fa.c[1] <= 512, "too many input channels for the fold kernel");
   fold_weights_kernel<T><<<dim3(G, M.nmlp, 8), 256, 0, st>>>(fa, M.wf, M.bf, M.bt);
   FGNN_LAUNCHED();
-  if (int e = launch_mlp<T>(M, C, G, geo, npg, st)) return e;
+  // the conv-chain kernel reads C entries of every hidden bias that feeds a ReLU: give it zero-padded copies
+  const int depth = M.mp[0]->depth;
+  MlpGroup<T> P = M;
+  fgnn_mlp_params padded[2];
+  if (co_real < C && depth > 2) {
+    FGNN_CHECK_ARG(M.bias_pad != nullptr, "zero-padded hidden layers need room for their biases");
+    PadBatch pb{};
+    for (int m = 0; m < M.nmlp; ++m) {
+      padded[m] = *M.mp[m];
+      for (int l = 1; l < depth - 1; ++l) {
+        const int v = m * (depth - 2) + l - 1;
+        pb.src[v] = M.mp[m]->b[l];
+        padded[m].b[l] = M.bias_pad + (size_t)v * C;
+      }
+      P.mp[m] = &padded[m];
+    }
+    pad_vectors_kernel<<<dim3(1, M.nmlp * (depth - 2)), 64, 0, st>>>(pb, M.bias_pad, C, co_real);
+    FGNN_LAUNCHED();
+  }
+  if (int e = launch_mlp<T>(P, C, G, geo, npg, st)) return e;
   if (M.no_coef) return FGNN_OK;
   CoefArgs ca{};
   ca.acc = M.stat_acc;
@@ -1889,6 +1940,7 @@ int run_mlp_group(const MlpGroup<T>& M, int C, int G, const Geo& geo, const int3
     ca.gb[m] = M.mp[m]->gn_b;
     ca.eps[m] = M.mp[m]->eps;
     ca.constant_n[m] = M.mp[m]->constant_n;
+    ca.co_real[m] = M.mp[m]->c_out;
     ca.gnstat[m] = M.gnstat[m];
   }
   const int total = G * M.nmlp * C;
@@ -1906,30 +1958,44 @@ struct Plan {
   int K1g12_max, K1g3_max;
 };
 
+// Widths.  The kernels run one width C in {32, 64} through every block: 32 when the widest MLP output is at most 32, else
+// 64.  Each block has one real output width co <= C (its three MLPs'), and its output planes hold C channels, of which
+// the first co are real; the input planes hold cin0 channels.  Parameters keep their real shapes, and every kernel that
+// reads one maps real indices to stored ones; mlp3's first layer reads cat[mult, block input], real columns [0, co) at
+// stored [0, C) and real [co, co + cin) at stored [C, C + cin).  Padded rows, columns, biases and GraphNorm affines are
+// zero, so the padded channels are exactly zero everywhere (a = s = 0) and the embeddings are (G, co_last, N).
 int make_plan(const fgnn_embed_params& p, int G, int N, Plan& pl) {
   if (N > kMaxN) return fail(FGNN_ERR_UNSUPPORTED, "tensor-core path supports N <= %d (got %d)", kMaxN, N);
   pl.geo = make_geo(N);
-  pl.C = p.block[0].mlp1.c_out;
   pl.cin0 = p.block[0].mlp1.c_in;
   pl.depth_max = 1;
   pl.K1g12_max = 64;
   pl.K1g3_max = 64;
-  int cur = pl.cin0;
+  int cmax = 0;
   for (int b = 0; b < p.num_blocks; ++b) {
     const fgnn_block_params& bp = p.block[b];
-    if (bp.mlp1.c_out != pl.C || bp.mlp2.c_out != pl.C || bp.mlp3.c_out != pl.C)
-      return fail(FGNN_ERR_UNSUPPORTED, "tensor-core path needs in_features == out_features for every block");
-    if (bp.mlp1.c_in != cur || bp.mlp2.c_in != cur || bp.mlp3.c_in != cur + pl.C)
+    const int co = bp.mlp1.c_out;
+    if (co < 1 || bp.mlp2.c_out != co || bp.mlp3.c_out != co)
+      return fail(FGNN_ERR_INVALID, "block %d: mlp1, mlp2 and mlp3 must have the same c_out >= 1", b);
+    if (co > 64)
+      return fail(FGNN_ERR_UNSUPPORTED, "tensor-core path supports in/out_features up to 64 (got %d); use FGNN_FP32", co);
+    cmax = std::max(cmax, co);
+  }
+  pl.C = cmax <= 32 ? 32 : 64;
+  int cur = pl.cin0, cur_store = pl.cin0;
+  for (int b = 0; b < p.num_blocks; ++b) {
+    const fgnn_block_params& bp = p.block[b];
+    const int co = bp.mlp1.c_out;
+    if (bp.mlp1.c_in != cur || bp.mlp2.c_in != cur || bp.mlp3.c_in != cur + co)
       return fail(FGNN_ERR_INVALID, "block %d: channel counts do not chain", b);
     if (bp.mlp1.depth != bp.mlp2.depth)
       return fail(FGNN_ERR_UNSUPPORTED, "block %d: mlp1 and mlp2 must have the same depth", b);
     pl.depth_max = std::max(pl.depth_max, std::max(bp.mlp1.depth, std::max(bp.mlp2.depth, bp.mlp3.depth)));
-    pl.K1g12_max = std::max(pl.K1g12_max, round_up(round_up(cur, 16), 64));
-    pl.K1g3_max = std::max(pl.K1g3_max, round_up(pl.C + round_up(cur, 16), 64));
-    cur = pl.C;
+    pl.K1g12_max = std::max(pl.K1g12_max, round_up(round_up(cur_store, 16), 64));
+    pl.K1g3_max = std::max(pl.K1g3_max, round_up(pl.C + round_up(cur_store, 16), 64));
+    cur = co;
+    cur_store = pl.C;
   }
-  if (pl.C != 32 && pl.C != 64)
-    return fail(FGNN_ERR_UNSUPPORTED, "tensor-core path supports in/out_features 32 or 64 (got %d); use FGNN_FP32", pl.C);
   if (pl.cin0 > 64) return fail(FGNN_ERR_UNSUPPORTED, "original_features_num %d > 64 unsupported", pl.cin0);
   const int chunk_env = env_int("FGNN_TC_CHUNK", 0);
   // per_graph: 16-bit planes of one graph (input, two block outputs, mult, Y1, Y2): 11.6 GB at N = 4096, C = 64
@@ -2006,6 +2072,7 @@ int embed_fwd_t(const fgnn_embed_params& p, const float* x, const uint8_t* adj, 
   for (int b = 0; b < p.num_blocks; ++b) {
     const fgnn_mlp_params* mlps[3] = {&p.block[b].mlp1, &p.block[b].mlp2, &p.block[b].mlp3};
     ConvertBatch cb{};
+    cb.rows = cb.cols = p.block[b].mlp1.c_out;
     int nmat = 0;
     for (int j = 0; j < 3; ++j)
       for (int l = 1; l < mlps[j]->depth; ++l) {
@@ -2015,7 +2082,7 @@ int embed_fwd_t(const fgnn_embed_params& p, const float* x, const uint8_t* adj, 
         ++nmat;
       }
     if (nmat > 0) {
-      convert_weights_batch_kernel<T><<<dim3(ceil_div(C * Kh, 256), nmat), 256, 0, st>>>(cb, reinterpret_cast<T*>(B.wh), C, C, Kh);
+      convert_weights_batch_kernel<T><<<dim3(ceil_div(C * Kh, 256), nmat), 256, 0, st>>>(cb, reinterpret_cast<T*>(B.wh), C, Kh);
       FGNN_LAUNCHED();
     }
   }
@@ -2038,7 +2105,7 @@ int embed_fwd_t(const fgnn_embed_params& p, const float* x, const uint8_t* adj, 
       FGNN_LAUNCHED();
     }
     const T* cur = reinterpret_cast<const T*>(B.xin);
-    int cur_c = pl.cin0;
+    int cur_c = pl.cin0, cur_real = pl.cin0;
     const float* cur_coef = nullptr;
     T* nxt = reinterpret_cast<T*>(B.xa);
     float* nxt_coef = B.coef3a;
@@ -2047,14 +2114,18 @@ int embed_fwd_t(const fgnn_embed_params& p, const float* x, const uint8_t* adj, 
     T* mult = reinterpret_cast<T*>(B.mult);
     for (int b = 0; b < p.num_blocks; ++b) {
       const fgnn_block_params& bp = p.block[b];
+      const int co = bp.mlp1.c_out;
       const T* whb = reinterpret_cast<const T*>(B.wh) + (size_t)b * 3 * dm1 * C * Kh;
+      // zero-padded hidden biases live in the other group's folded-weight buffer, which is free while a group runs
+      // (wf3 holds at least C * 64 and wf12 2 C * 64 16-bit values: room for 2 (FGNN_MAX_DEPTH - 2) C floats)
       {
         MlpGroup<T> M{};
         M.nmlp = 2;
         M.mp[0] = &bp.mlp1; M.mp[1] = &bp.mlp2;
-        M.src[0] = cur; M.c_src[0] = cur_c; M.src_coef[0] = cur_coef; M.nsrc = 1;
+        M.src[0] = cur; M.c_src[0] = cur_c; M.cr_src[0] = cur_real; M.src_coef[0] = cur_coef; M.nsrc = 1;
         M.wf = reinterpret_cast<T*>(B.wf12); M.bf = B.bf12; M.bt = reinterpret_cast<T*>(B.bt12);
         M.wh = whb;
+        M.bias_pad = static_cast<float*>(B.wf3);
         M.out[0] = y1; M.out_mode[0] = kLayoutA; M.ones[0] = 1; M.coef[0] = B.coef1;
         M.out[1] = y2; M.out_mode[1] = kLayoutB; M.ones[1] = 1; M.coef[1] = B.coef2;
         M.stat_acc = B.stat_acc;
@@ -2065,10 +2136,11 @@ int embed_fwd_t(const fgnn_embed_params& p, const float* x, const uint8_t* adj, 
         MlpGroup<T> M{};
         M.nmlp = 1;
         M.mp[0] = &bp.mlp3;
-        M.src[0] = mult; M.c_src[0] = C; M.src_coef[0] = nullptr;
-        M.src[1] = cur; M.c_src[1] = cur_c; M.src_coef[1] = cur_coef; M.nsrc = 2;
+        M.src[0] = mult; M.c_src[0] = C; M.cr_src[0] = co; M.src_coef[0] = nullptr;
+        M.src[1] = cur; M.c_src[1] = cur_c; M.cr_src[1] = cur_real; M.src_coef[1] = cur_coef; M.nsrc = 2;
         M.wf = reinterpret_cast<T*>(B.wf3); M.bf = B.bf3; M.bt = reinterpret_cast<T*>(B.bt3);
         M.wh = whb + (size_t)2 * dm1 * C * Kh;
+        M.bias_pad = static_cast<float*>(B.wf12);
         M.out[0] = nxt; M.out_mode[0] = kLayoutC; M.ones[0] = 0; M.coef[0] = nxt_coef;
         M.stat_acc = B.stat_acc;
         if (b == p.num_blocks - 1) {
@@ -2080,13 +2152,14 @@ int embed_fwd_t(const fgnn_embed_params& p, const float* x, const uint8_t* adj, 
       }
       cur = nxt;
       cur_c = C;
+      cur_real = co;
       cur_coef = nxt_coef;
       nxt = (nxt == reinterpret_cast<T*>(B.xa)) ? reinterpret_cast<T*>(B.xb) : reinterpret_cast<T*>(B.xa);
       nxt_coef = (nxt_coef == B.coef3a) ? B.coef3b : B.coef3a;
     }
     const long rows = (long)gc * C * N;
-    pool_finalize_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(B.rowenc, cur_coef, emb + (size_t)g0 * C * N, C, N,
-                                                                       rows, n_c);
+    pool_finalize_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(B.rowenc, cur_coef, emb + (size_t)g0 * cur_real * N, C,
+                                                                       cur_real, N, rows, n_c);
     FGNN_LAUNCHED();
   }
   return FGNN_OK;
@@ -2294,15 +2367,16 @@ int debug_mlp_t(const fgnn_mlp_params& mp, const float* x, float* y, int G, int 
   to_planes_c_kernel<T><<<dim3((unsigned)std::min(N, 256), G * mp.c_in), 256, 0, st>>>(x, xin, mp.c_in, geo, npg);
   FGNN_LAUNCHED();
   ConvertBatch cb{};
+  cb.rows = cb.cols = C;
   for (int l = 1; l < mp.depth; ++l) { cb.src[l - 1] = mp.w[l]; cb.dst_off[l - 1] = (long)(l - 1) * C * Kh; }
   if (mp.depth > 1) {
-    convert_weights_batch_kernel<T><<<dim3(ceil_div(C * Kh, 256), mp.depth - 1), 256, 0, st>>>(cb, wh, C, C, Kh);
+    convert_weights_batch_kernel<T><<<dim3(ceil_div(C * Kh, 256), mp.depth - 1), 256, 0, st>>>(cb, wh, C, Kh);
     FGNN_LAUNCHED();
   }
   MlpGroup<T> M{};
   M.nmlp = 1;
   M.mp[0] = &mp;
-  M.src[0] = xin; M.c_src[0] = mp.c_in; M.src_coef[0] = nullptr; M.nsrc = 1;
+  M.src[0] = xin; M.c_src[0] = M.cr_src[0] = mp.c_in; M.src_coef[0] = nullptr; M.nsrc = 1;
   M.wf = wf; M.bf = bf; M.bt = bt; M.wh = wh;
   M.out[0] = out; M.out_mode[0] = kLayoutC; M.ones[0] = 0; M.coef[0] = coef;
   M.stat_acc = acc;

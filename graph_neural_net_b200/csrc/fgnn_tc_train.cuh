@@ -113,11 +113,11 @@ __global__ void gn_bwd_coef_kernel(const double* __restrict__ acc, const float* 
   bc[4 * (long)gc + 3] = 0.f;
 }
 
-// d gn.weight[c] += inv * sum_g s0 (S2 - mu S1),  d gn.bias[c] += inv * sum_g S1     (layers.py:68-69)
+// d gn.weight[c] += inv * sum_g s0 (S2 - mu S1),  d gn.bias[c] += inv * sum_g S1     (layers.py:68-69), c < co_real
 __global__ void gn_param_grad_kernel(const double* __restrict__ acc, const float* __restrict__ gnstat, float* dgw, float* dgb,
-                                     const float* __restrict__ scale, int G, int C) {
+                                     const float* __restrict__ scale, int G, int C, int co_real) {
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
-  if (c >= C) return;
+  if (c >= co_real) return;
   double sw = 0.0, sb = 0.0;
   for (int g = 0; g < G; ++g) {
     const long gc = (long)g * C + c;
@@ -263,13 +263,13 @@ plane_colsum_kernel(const T* __restrict__ x, float* __restrict__ colsum, int C, 
   colsum[(long)gc * geo.NPC + pj] = s;
 }
 
-// ColumnMaxPooling of the training path: emb[gc][i] = max_j (a z[i][j] + s), arg = physical column of the maximum
-// (smallest column on ties); rows >= n -> 0 / -1.  One warp per row.
+// ColumnMaxPooling of the training path: emb[g][c][i] = max_j (a z[i][j] + s), arg = physical column of the maximum
+// (smallest column on ties); rows >= n -> 0 / -1.  One warp per row.  emb is (G, co_real, N), arg (G, C, N).
 template <typename T>
 __global__ void __launch_bounds__(256)
 colmax16_kernel(const T* __restrict__ z, const float* __restrict__ coef, float* __restrict__ emb, int32_t* __restrict__ arg,
-                int C, Geo geo, const int32_t* __restrict__ npg) {
-  const int gc = blockIdx.y, g = gc / C;
+                int C, int co_real, Geo geo, const int32_t* __restrict__ npg) {
+  const int gc = blockIdx.y, g = gc / C, c = gc % C;
   const int n = graph_n(npg, g, geo.N);
   const int i = blockIdx.x * 8 + threadIdx.x / 32, lane = threadIdx.x % 32;
   if (i >= geo.N) return;
@@ -296,7 +296,7 @@ colmax16_kernel(const T* __restrict__ z, const float* __restrict__ coef, float* 
     }
   }
   if (lane == 0) {
-    emb[(long)gc * geo.N + i] = i < n ? fmaf(a, sgn * best, sft) : 0.f;
+    if (c < co_real) emb[((long)g * co_real + c) * geo.N + i] = i < n ? fmaf(a, sgn * best, sft) : 0.f;
     arg[(long)gc * geo.N + i] = (i < n && bj != 0x7fffffff) ? bj : -1;   // a row of NaNs has no arg-max: no gradient
   }
 }
@@ -324,61 +324,67 @@ grad_scale_kernel(const float* __restrict__ demb, long total, float* __restrict_
   }
 }
 
-// dy of the last block's output: zero planes (memset by the caller) + scale * d emb at the pooling arg-max
+// dy of the last block's output: zero planes (memset by the caller) + scale * d emb at the pooling arg-max; demb is
+// (G, co_real, N), the padded channels get no gradient
 template <typename T>
 __global__ void pool_scatter_kernel(const float* __restrict__ demb, const int32_t* __restrict__ arg, const float* __restrict__ scale,
-                                    T* __restrict__ dy, Geo geo, long total) {
+                                    T* __restrict__ dy, int C, int co_real, Geo geo, long total) {
   const long idx = (long)blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= total) return;
   const int a = arg[idx];
   if (a < 0) return;
   const long gc = idx / geo.N;
   const int i = (int)(idx % geo.N);
-  dy[gc * geo.PSC + (long)i * geo.NPC + a] = Elem<T>::from_float(scale[0] * demb[idx]);
+  const int c = (int)(gc % C);
+  if (c >= co_real) return;
+  dy[gc * geo.PSC + (long)i * geo.NPC + a] = Elem<T>::from_float(scale[0] * demb[((gc / C) * co_real + c) * geo.N + i]);
 }
 
-// wt[r][dst_col0 + c] = w[c][col0 + r]   (r < rows, c < co): transposed (slices of) conv weights for the data gradients
-__global__ void transpose_slice_kernel(const float* __restrict__ w, float* __restrict__ wt, int co, int cin_total, int col0,
-                                       int rows, int dst_pitch, int dst_col0) {
+// wt[r][dst_col0 + c] = w[c][col0 + r]   (r < rows, c < co): transposed (slices of) conv weights for the data gradients.
+// w has its real shape (co_real, cin_total); the stored slice is zero beyond co_real columns and rows_real rows.
+__global__ void transpose_slice_kernel(const float* __restrict__ w, float* __restrict__ wt, int co, int co_real, int cin_total,
+                                       int col0, int rows, int rows_real, int dst_pitch, int dst_col0) {
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= rows * co) return;
   const int r = idx / co, c = idx % co;
-  wt[r * dst_pitch + dst_col0 + c] = w[c * cin_total + col0 + r];
+  wt[r * dst_pitch + dst_col0 + c] = c < co_real && r < rows_real ? w[c * cin_total + col0 + r] : 0.f;
 }
 
-// hidden-layer parameter gradients: dW[co][ci] += inv * P[co][ldp], db[co] += inv * sum_g bsum[g][co]
+// hidden-layer parameter gradients: dW[co][ci] += inv * P[co][ldp], db[co] += inv * sum_g bsum[g][co]; real (co, ci) out of
+// the stored C channels of bsum
 __global__ void wgrad_combine_hidden_kernel(const float* __restrict__ P, int ldp, const float* __restrict__ bsum, float* dW, float* db,
-                                            const float* __restrict__ scale, int G, int co, int ci) {
+                                            const float* __restrict__ scale, int G, int C, int co, int ci) {
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
   const float inv = 1.f / scale[0];
   if (idx < co * ci) dW[idx] += inv * P[(idx / ci) * ldp + idx % ci];
   if (idx < co && db) {
     float s = 0.f;
-    for (int g = 0; g < G; ++g) s += bsum[(long)g * co + idx];
+    for (int g = 0; g < G; ++g) s += bsum[(long)g * C + idx];
     db[idx] += inv * s;
   }
 }
 
 // first-layer parameter gradients through the per-graph GraphNorm fold (see the header of this file):
 //   dW[co][ci] += inv * sum_g ( P_g[co][k(ci)] a_src[g][ci] + bsum[g][co] s_src[g][ci] ),  db[co] += inv * sum_g bsum[g][co]
+// for the real entries only: real column (s ? cr_0 : 0) + ch of dW is channel ch of source s, stored at k = koff_s + ch
 struct CombineFirstArgs {
   const float* P;          // [G][co][ldp]
   const float* bsum;       // [G][co]
   const float* coef[2];    // per source [G][c_s][2] or null
-  int c[2], koff[2], nsrc;
-  int G, co, ldp;
-  float* dW;               // (co, c0 + c1)
+  int c[2], cr[2], koff[2], nsrc;
+  int G, co, co_real, ldp;
+  float* dW;               // (co_real, cr0 + cr1)
   float* db;
   const float* scale;
 };
 __global__ void wgrad_combine_first_kernel(CombineFirstArgs a) {
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-  const int cin = a.c[0] + (a.nsrc > 1 ? a.c[1] : 0);
+  const int cin = a.cr[0] + (a.nsrc > 1 ? a.cr[1] : 0);
   const float inv = 1.f / a.scale[0];
-  if (idx < a.co * cin) {
+  if (idx < a.co_real * cin) {
     const int co = idx / cin, col = idx % cin;
-    const int s = col < a.c[0] ? 0 : 1;
-    const int chn = col - (s ? a.c[0] : 0);
+    const int s = col < a.cr[0] ? 0 : 1;
+    const int chn = col - (s ? a.cr[0] : 0);
     const int k = a.koff[s] + chn;
     float acc = 0.f;
     for (int g = 0; g < a.G; ++g) {
@@ -389,7 +395,7 @@ __global__ void wgrad_combine_first_kernel(CombineFirstArgs a) {
     }
     a.dW[idx] += inv * acc;
   }
-  if (idx < a.co && a.db) {
+  if (idx < a.co_real && a.db) {
     float s = 0.f;
     for (int g = 0; g < a.G; ++g) s += a.bsum[(long)g * a.co + idx];
     a.db[idx] += inv * s;
@@ -885,6 +891,7 @@ int launch_bmm_bwd(int mode, const T* a, const T* b, T* out, const float* coef, 
 struct TrainPlan {
   Geo geo;
   int C, cin0, D, nb;
+  int c_emb;        // real channels of the embeddings (the last block's c_out)
   int G;            // graphs of one pass: the whole batch on keep-all, `chunk` on recompute (pass_plan lowers it for a short last pass)
   int batch;        // graphs of the call
   bool recompute;
@@ -997,6 +1004,7 @@ int make_train_plan(const fgnn_embed_params& p, int G, int N, TrainPlan& tp) {
   tp.C = pl.C;
   tp.cin0 = pl.cin0;
   tp.nb = p.num_blocks;
+  tp.c_emb = p.block[p.num_blocks - 1].mlp3.c_out;
   tp.G = G;
   tp.batch = G;
   tp.recompute = false;
@@ -1059,14 +1067,17 @@ int zero_pass(const TrainPlan& tp, const TrainBuf& B, void* ws, bool ragged, cud
   return FGNN_OK;
 }
 
-// one 1x1-conv layer (or two sharing their input) as a depth-1 launch of the conv-chain kernel
+// one 1x1-conv layer (or two sharing their input) as a depth-1 launch of the conv-chain kernel.  The weights have their
+// real shape (co_real, cr_src0 + cr_src1); co_real = 0 and cr_src = 0 mean the stored C and c_src (weights padded here).
 template <typename T>
 struct ConvCall {
   int nmlp = 1;
-  const float* w[2] = {nullptr, nullptr};     // (c_out, c_src0 + c_src1) fp32
-  const float* b[2] = {nullptr, nullptr};     // (c_out) or null
+  const float* w[2] = {nullptr, nullptr};     // (co_real, cr_src0 + cr_src1) fp32
+  const float* b[2] = {nullptr, nullptr};     // (co_real) or null
   const T* src[2] = {nullptr, nullptr};
   int c_src[2] = {0, 0};
+  int cr_src[2] = {0, 0};
+  int co_real = 0;
   const float* src_coef[2] = {nullptr, nullptr};
   int nsrc = 1;
   T* out[2] = {nullptr, nullptr};
@@ -1084,11 +1095,16 @@ int run_conv(const ConvCall<T>& cc, const TrainPlan& tp, const TrainBuf& B, cons
   MlpGroup<T> M{};
   M.nmlp = cc.nmlp;
   M.nsrc = cc.nsrc;
-  for (int s = 0; s < 2; ++s) { M.src[s] = cc.src[s]; M.c_src[s] = cc.c_src[s]; M.src_coef[s] = cc.src_coef[s]; }
+  for (int s = 0; s < 2; ++s) {
+    M.src[s] = cc.src[s];
+    M.c_src[s] = cc.c_src[s];
+    M.cr_src[s] = cc.cr_src[s] ? cc.cr_src[s] : cc.c_src[s];
+    M.src_coef[s] = cc.src_coef[s];
+  }
   for (int m = 0; m < cc.nmlp; ++m) {
     memset(&tmp[m], 0, sizeof(tmp[m]));
-    tmp[m].c_in = cc.c_src[0] + (cc.nsrc > 1 ? cc.c_src[1] : 0);
-    tmp[m].c_out = tp.C;
+    tmp[m].c_in = M.cr_src[0] + (cc.nsrc > 1 ? M.cr_src[1] : 0);
+    tmp[m].c_out = cc.co_real ? cc.co_real : tp.C;
     tmp[m].depth = 1;
     tmp[m].w[0] = cc.w[m];
     tmp[m].b[0] = cc.b[m] ? cc.b[m] : B.zeros;
@@ -1122,10 +1138,11 @@ int train_fwd_pass(const fgnn_embed_params& p, const TrainPlan& tp, const TrainB
   const Geo& geo = tp.geo;
   const int G = tp.G, N = geo.N, C = tp.C, D = tp.D;
   const T* cur = xin;
-  int cur_c = tp.cin0;
+  int cur_c = tp.cin0, cur_real = tp.cin0;
   const float* cur_coef = nullptr;
   for (int b = 0; b < tp.nb; ++b) {
     const fgnn_block_params& bp = p.block[b];
+    const int co = bp.mlp1.c_out;
     const fgnn_mlp_params* mlps[3] = {&bp.mlp1, &bp.mlp2, &bp.mlp3};
     T* y12[2] = {reinterpret_cast<T*>(B.Y1[b]), reinterpret_cast<T*>(B.Y2[b])};
     const Layout mode12[2] = {kLayoutA, kLayoutB};
@@ -1134,7 +1151,8 @@ int train_fwd_pass(const fgnn_embed_params& p, const TrainPlan& tp, const TrainB
       if (l == 0) {   // mlp1 and mlp2 share the block input: one launch
         ConvCall<T> cc;
         cc.nmlp = 2;
-        cc.src[0] = cur; cc.c_src[0] = cur_c; cc.src_coef[0] = cur_coef; cc.nsrc = 1;
+        cc.src[0] = cur; cc.c_src[0] = cur_c; cc.cr_src[0] = cur_real; cc.src_coef[0] = cur_coef; cc.nsrc = 1;
+        cc.co_real = co;
         for (int m = 0; m < 2; ++m) {
           cc.w[m] = mlps[m]->w[0]; cc.b[m] = mlps[m]->b[0];
           cc.out[m] = last ? y12[m] : reinterpret_cast<T*>(B.H[b][m][0]);
@@ -1147,7 +1165,8 @@ int train_fwd_pass(const fgnn_embed_params& p, const TrainPlan& tp, const TrainB
       } else {
         for (int m = 0; m < 2; ++m) {
           ConvCall<T> cc;
-          cc.src[0] = reinterpret_cast<const T*>(B.H[b][m][l - 1]); cc.c_src[0] = C;
+          cc.src[0] = reinterpret_cast<const T*>(B.H[b][m][l - 1]); cc.c_src[0] = C; cc.cr_src[0] = co;
+          cc.co_real = co;
           cc.w[0] = mlps[m]->w[l]; cc.b[0] = mlps[m]->b[l];
           cc.out[0] = last ? y12[m] : reinterpret_cast<T*>(B.H[b][m][l]);
           cc.out_mode[0] = last ? mode12[m] : kLayoutC;
@@ -1164,11 +1183,12 @@ int train_fwd_pass(const fgnn_embed_params& p, const TrainPlan& tp, const TrainB
       const bool last = l == D - 1;
       ConvCall<T> cc;
       if (l == 0) {
-        cc.src[0] = mult; cc.c_src[0] = C; cc.src_coef[0] = nullptr;
-        cc.src[1] = cur; cc.c_src[1] = cur_c; cc.src_coef[1] = cur_coef; cc.nsrc = 2;
+        cc.src[0] = mult; cc.c_src[0] = C; cc.cr_src[0] = co; cc.src_coef[0] = nullptr;
+        cc.src[1] = cur; cc.c_src[1] = cur_c; cc.cr_src[1] = cur_real; cc.src_coef[1] = cur_coef; cc.nsrc = 2;
       } else {
-        cc.src[0] = reinterpret_cast<const T*>(B.H[b][2][l - 1]); cc.c_src[0] = C;
+        cc.src[0] = reinterpret_cast<const T*>(B.H[b][2][l - 1]); cc.c_src[0] = C; cc.cr_src[0] = co;
       }
+      cc.co_real = co;
       cc.w[0] = mlps[2]->w[l]; cc.b[0] = mlps[2]->b[l];
       cc.out[0] = last ? reinterpret_cast<T*>(B.Z3[b]) : reinterpret_cast<T*>(B.H[b][2][l]);
       if (last) { cc.gn[0] = mlps[2]; cc.coef[0] = B.coef[b][2]; cc.gnstat[0] = B.gnstat[b][2]; }
@@ -1177,11 +1197,12 @@ int train_fwd_pass(const fgnn_embed_params& p, const TrainPlan& tp, const TrainB
     }
     cur = reinterpret_cast<const T*>(B.Z3[b]);
     cur_c = C;
+    cur_real = co;
     cur_coef = B.coef[b][2];
   }
   {
     dim3 grid((unsigned)((N + 7) / 8), G * C);
-    colmax16_kernel<T><<<grid, 256, 0, st>>>(cur, cur_coef, emb, B.arg, C, geo, npg);
+    colmax16_kernel<T><<<grid, 256, 0, st>>>(cur, cur_coef, emb, B.arg, C, cur_real, geo, npg);
     FGNN_LAUNCHED();
   }
   return FGNN_OK;
@@ -1207,7 +1228,7 @@ int embed_fwd_train_t(const fgnn_embed_params& p, const float* x, float* emb, in
       to_planes_c_kernel<T><<<grid, 256, 0, st>>>(x, xin, tp.cin0, geo, npg);
       FGNN_LAUNCHED();
     }
-    if (int e = train_fwd_pass<T>(p, pp, B, xin + (size_t)g0 * tp.cin0 * geo.PSC, emb + (size_t)g0 * tp.C * N,
+    if (int e = train_fwd_pass<T>(p, pp, B, xin + (size_t)g0 * tp.cin0 * geo.PSC, emb + (size_t)g0 * tp.c_emb * N,
                                   npg ? npg + g0 : nullptr, st)) return e;
   }
   return FGNN_OK;
@@ -1227,8 +1248,10 @@ struct MlpBwd {
   const float* coef;
   const float* gnstat;
   void* const* H;               // hidden activations h_0 .. h_{D-2} (layout C)
+  int co_real;                  // real output channels (mp's c_out)
   const T* src[2];
-  int c_src[2];
+  int c_src[2];                 // channels of the source planes as stored
+  int cr_src[2];                // of which real
   const float* src_coef[2];
   int nsrc;
   T* bufs[2];
@@ -1246,7 +1269,7 @@ int mlp_bwd(const MlpBwd<T>& a, const TrainPlan& tp, const TrainBuf& B, const in
   FGNN_LAUNCHED();
   gn_bwd_coef_kernel<<<ceil_div(GC, 256), 256, 0, st>>>(B.gacc, a.coef, a.gnstat, B.bc, C, geo.N, npg, GC);
   FGNN_LAUNCHED();
-  gn_param_grad_kernel<<<ceil_div(C, 64), 64, 0, st>>>(B.gacc, a.gnstat, a.gr->gn_w, a.gr->gn_b, B.scale, G, C);
+  gn_param_grad_kernel<<<ceil_div(C, 64), 64, 0, st>>>(B.gacc, a.gnstat, a.gr->gn_w, a.gr->gn_b, B.scale, G, C, a.co_real);
   FGNN_LAUNCHED();
   int bi = 0;                                           // bsum[bi] = per-(graph, channel) sum of the current gradient
   FGNN_CUDA(cudaMemsetAsync(B.bsum[bi], 0, (size_t)GC * sizeof(float), st));
@@ -1260,10 +1283,10 @@ int mlp_bwd(const MlpBwd<T>& a, const TrainPlan& tp, const TrainBuf& B, const in
     FGNN_CUDA(cudaMemsetAsync(B.Pglob, 0, 128 * 128 * sizeof(float), st));
     if (int e = launch_wgrad<T>(curg, C, hin, C, nullptr, 0, B.Pglob, 0, G, geo, npg, st)) return e;
     wgrad_combine_hidden_kernel<<<ceil_div(C * C, 256), 256, 0, st>>>(B.Pglob, round_up(C, 16), B.bsum[bi], a.gr->w[l], a.gr->b[l],
-                                                                      B.scale, G, C, C);
+                                                                      B.scale, G, C, a.co_real, a.co_real);
     FGNN_LAUNCHED();
     // data gradient: pre = W_l^T g, then the ReLU mask of h_{l-1}
-    transpose_slice_kernel<<<ceil_div(C * C, 256), 256, 0, st>>>(a.mp->w[l], B.wt[0], C, C, 0, C, C, 0);
+    transpose_slice_kernel<<<ceil_div(C * C, 256), 256, 0, st>>>(a.mp->w[l], B.wt[0], C, a.co_real, a.co_real, 0, C, a.co_real, C, 0);
     FGNN_LAUNCHED();
     T* nxt = (curg == a.bufs[0]) ? a.bufs[1] : a.bufs[0];
     ConvCall<T> cc;
@@ -1293,11 +1316,14 @@ int mlp_bwd(const MlpBwd<T>& a, const TrainPlan& tp, const TrainBuf& B, const in
     ca.coef[1] = a.nsrc > 1 ? a.src_coef[1] : nullptr;
     ca.c[0] = a.c_src[0];
     ca.c[1] = a.nsrc > 1 ? a.c_src[1] : 0;
+    ca.cr[0] = a.cr_src[0];
+    ca.cr[1] = a.nsrc > 1 ? a.cr_src[1] : 0;
     ca.koff[0] = 0;
     ca.koff[1] = k0;
     ca.nsrc = a.nsrc;
     ca.G = G;
     ca.co = C;
+    ca.co_real = a.co_real;
     ca.ldp = Nw;
     ca.dW = a.gr->w[0];
     ca.db = a.gr->b[0];
@@ -1323,7 +1349,7 @@ int train_bwd_pass(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const
   FGNN_CUDA(cudaMemsetAsync(dOutA, 0, plane_bytes, st));
   {
     const long total = (long)GC * N;
-    pool_scatter_kernel<T><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(demb, B.arg, B.scale, dOutA, geo, total);
+    pool_scatter_kernel<T><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(demb, B.arg, B.scale, dOutA, C, tp.c_emb, geo, total);
     FGNN_LAUNCHED();
   }
   for (int b = tp.nb - 1; b >= 0; --b) {
@@ -1331,6 +1357,8 @@ int train_bwd_pass(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const
     const fgnn_block_grads& bg = gr.block[b];
     const T* cur = b > 0 ? reinterpret_cast<const T*>(B.Z3[b - 1]) : xin;
     const int cur_c = b > 0 ? C : tp.cin0;
+    const int cur_real = b > 0 ? p.block[b - 1].mlp3.c_out : tp.cin0;
+    const int co = bp.mlp1.c_out;
     const float* cur_coef = b > 0 ? B.coef[b - 1][2] : nullptr;
     T* A[2] = {reinterpret_cast<T*>(B.A0), reinterpret_cast<T*>(B.A1)};
     T* Bb[2] = {reinterpret_cast<T*>(B.B0), reinterpret_cast<T*>(B.B1)};
@@ -1346,20 +1374,21 @@ int train_bwd_pass(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const
       a.z = reinterpret_cast<const T*>(B.Z3[b]); a.zmode = kLayoutC;
       a.coef = B.coef[b][2]; a.gnstat = B.gnstat[b][2];
       a.H = B.H[b][2];
-      a.src[0] = reinterpret_cast<const T*>(B.MULT[b]); a.c_src[0] = C; a.src_coef[0] = nullptr;
-      a.src[1] = cur; a.c_src[1] = cur_c; a.src_coef[1] = cur_coef; a.nsrc = 2;
+      a.co_real = co;
+      a.src[0] = reinterpret_cast<const T*>(B.MULT[b]); a.c_src[0] = C; a.cr_src[0] = co; a.src_coef[0] = nullptr;
+      a.src[1] = cur; a.c_src[1] = cur_c; a.cr_src[1] = cur_real; a.src_coef[1] = cur_coef; a.nsrc = 2;
       a.bufs[0] = A[0]; a.bufs[1] = A[1];
       if (int e = mlp_bwd<T>(a, tp, B, npg, st, &g3)) return e;
-      // data gradients of the two sources: d mult = W0[:, :C]^T g, d cur = W0[:, C:]^T g (not needed for the raw input)
-      const int cin = C + cur_c;
-      transpose_slice_kernel<<<ceil_div(C * C, 256), 256, 0, st>>>(bp.mlp3.w[0], B.wt[0], C, cin, 0, C, C, 0);
+      // data gradients of the two sources: d mult = W0[:, :co]^T g, d cur = W0[:, co:]^T g (not needed for the raw input)
+      const int cin = co + cur_real;
+      transpose_slice_kernel<<<ceil_div(C * C, 256), 256, 0, st>>>(bp.mlp3.w[0], B.wt[0], C, co, cin, 0, C, co, C, 0);
       FGNN_LAUNCHED();
       ConvCall<T> cc;
       cc.src[0] = g3; cc.c_src[0] = C;
       cc.w[0] = B.wt[0];
       cc.out[0] = DM;
       if (b > 0) {
-        transpose_slice_kernel<<<ceil_div(C * C, 256), 256, 0, st>>>(bp.mlp3.w[0], B.wt[1], C, cin, C, C, C, 0);
+        transpose_slice_kernel<<<ceil_div(C * C, 256), 256, 0, st>>>(bp.mlp3.w[0], B.wt[1], C, co, cin, co, C, cur_real, C, 0);
         FGNN_LAUNCHED();
         cc.nmlp = 2;
         cc.w[1] = B.wt[1];
@@ -1392,16 +1421,17 @@ int train_bwd_pass(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const
       a.z = reinterpret_cast<const T*>(m == 0 ? B.Y1[b] : B.Y2[b]); a.zmode = m == 0 ? kLayoutA : kLayoutB;
       a.coef = B.coef[b][m]; a.gnstat = B.gnstat[b][m];
       a.H = B.H[b][m];
-      a.src[0] = cur; a.c_src[0] = cur_c; a.src_coef[0] = cur_coef; a.nsrc = 1;
+      a.co_real = co;
+      a.src[0] = cur; a.c_src[0] = cur_c; a.cr_src[0] = cur_real; a.src_coef[0] = cur_coef; a.nsrc = 1;
       a.bufs[0] = m == 0 ? A[0] : Bb[0];
       a.bufs[1] = m == 0 ? A[1] : Bb[1];
       if (int e = mlp_bwd<T>(a, tp, B, npg, st, &g12[m])) return e;
     }
     if (b > 0) {
       // d cur (through mlp1 and mlp2) = [W0_1^T | W0_2^T] [g1; g2]: one two-source conv
-      transpose_slice_kernel<<<ceil_div(C * C, 256), 256, 0, st>>>(bp.mlp1.w[0], B.wt[0], C, C, 0, C, 2 * C, 0);
+      transpose_slice_kernel<<<ceil_div(C * C, 256), 256, 0, st>>>(bp.mlp1.w[0], B.wt[0], C, co, cur_real, 0, C, cur_real, 2 * C, 0);
       FGNN_LAUNCHED();
-      transpose_slice_kernel<<<ceil_div(C * C, 256), 256, 0, st>>>(bp.mlp2.w[0], B.wt[0], C, C, 0, C, 2 * C, C);
+      transpose_slice_kernel<<<ceil_div(C * C, 256), 256, 0, st>>>(bp.mlp2.w[0], B.wt[0], C, co, cur_real, 0, C, cur_real, 2 * C, C);
       FGNN_LAUNCHED();
       ConvCall<T> cc;
       cc.src[0] = g12[0]; cc.c_src[0] = C;
@@ -1428,7 +1458,7 @@ int embed_bwd_t(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const fl
   if (need > ws_bytes) return fail(FGNN_ERR_WORKSPACE, "training workspace too small: %zu < %zu", ws_bytes, need);
   const Geo& geo = tp.geo;
   // one loss scale for the whole batch, whatever the passes
-  grad_scale_kernel<<<1, 1024, 0, st>>>(demb, (long)G * tp.C * N, B.scale, grad_scale_log2);
+  grad_scale_kernel<<<1, 1024, 0, st>>>(demb, (long)G * tp.c_emb * N, B.scale, grad_scale_log2);
   FGNN_LAUNCHED();
   const T* xin = reinterpret_cast<const T*>(B.xin);
   for (int g0 = 0; g0 < G; g0 += tp.G) {
@@ -1440,7 +1470,7 @@ int embed_bwd_t(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const fl
       if (int e = zero_pass(pp, B, ws, npg != nullptr, st)) return e;
       if (int e = train_fwd_pass<T>(p, pp, B, xin_p, B.rowsum, npg_p, st)) return e;
     }
-    if (int e = train_bwd_pass<T>(p, gr, pp, B, xin_p, demb + (size_t)g0 * tp.C * N, npg_p, st)) return e;
+    if (int e = train_bwd_pass<T>(p, gr, pp, B, xin_p, demb + (size_t)g0 * tp.c_emb * N, npg_p, st)) return e;
   }
   return FGNN_OK;
 }

@@ -142,79 +142,17 @@ class Network(nn.Module):
         return ('input', sfx[0], blocks)
 
     def _embed_params(self, keep):
+        """fgnn_embed_params of the fused embedder, real shapes: the C library zero-pads the widths it runs
+        (fgnn_tc.cu make_plan)."""
         p = L.EmbedParams()
         _, _, blocks = self._fused
         p.num_blocks = len(blocks)
-        padded = self._padded_widths()
         for i, trio in enumerate(blocks):
-            for j, (name, mlp) in enumerate(zip(('mlp1', 'mlp2', 'mlp3'), trio)):
-                if padded is None:
-                    ws, bs = [c.weight for c in mlp.convs], [c.bias for c in mlp.convs]
-                    gw, gb = mlp.gn.weight, mlp.gn.bias
-                else:
-                    ws, bs, gw, gb = padded[i][j]
-                mp = _ops.make_mlp_params(ws, bs, gw, gb, mlp.gn.eps, keep, bool(mlp.cst_vertices))
+            for name, mlp in zip(('mlp1', 'mlp2', 'mlp3'), trio):
+                mp = _ops.make_mlp_params([c.weight for c in mlp.convs], [c.bias for c in mlp.convs], mlp.gn.weight,
+                                          mlp.gn.bias, mlp.gn.eps, keep, bool(mlp.cst_vertices))
                 setattr(p.block[i], name, mp)
         return p
-
-    def _padded_widths(self):
-        """The tensor-core embedder runs ONE width C in {32, 64} through every block.  The reference lets in_features,
-        out_features be anything (models/blocks_emb.py:29-36: the last block maps in_features -> out_features), so other
-        widths up to 64 are run zero-padded to C: padded channels have zero conv weights and a zero GraphNorm weight / bias,
-        hence are exactly zero everywhere (a = 0, s = 0 in the fold, the matmul and the pooling) and are sliced off the
-        embeddings.  Inference only (the training path keeps the restriction).  Returns None when no padding is needed,
-        else per block / MLP (weights, biases, gn weight, gn bias); cached on the parameters' versions."""
-        blocks = self._fused[2]
-        widths = [m.convs[-1].weight.shape[0] for trio in blocks for m in trio]
-        cmax = max(widths)
-        if cmax > 64 or (all(w == widths[0] for w in widths) and widths[0] in (32, 64)):
-            return None                                   # uniform supported width, or too wide (the C side fails loudly)
-        C = 32 if cmax <= 32 else 64
-        params = [t for trio in blocks for m in trio for t in ([c.weight for c in m.convs] + [c.bias for c in m.convs] +
-                                                               [m.gn.weight, m.gn.bias])]
-        key = tuple((t.data_ptr(), t._version) for t in params if t is not None)
-        cache = getattr(self, "_pad_cache", None)
-        if cache is not None and cache[0] == key:
-            return cache[1]
-        out = []
-        with torch.no_grad():
-            cin_real = blocks[0][0].convs[0].weight.shape[1]      # block input: real channels / channels as stored (padded)
-            cin_store = cin_real
-            for trio in blocks:
-                row = []
-                co_real = trio[0].convs[-1].weight.shape[0]
-                for j, m in enumerate(trio):
-                    dev = m.convs[0].weight.device
-                    w0 = m.convs[0].weight.detach().reshape(m.convs[0].weight.shape[0], -1)
-                    if j < 2:                                  # mlp1 / mlp2 read the block input
-                        W0 = torch.zeros((C, cin_store), device=dev)
-                        W0[:w0.shape[0], :cin_real] = w0
-                    else:                                      # mlp3 reads cat[mult (C stored, co_real real), block input]
-                        W0 = torch.zeros((C, C + cin_store), device=dev)
-                        W0[:w0.shape[0], :co_real] = w0[:, :co_real]
-                        W0[:w0.shape[0], C:C + cin_real] = w0[:, co_real:co_real + cin_real]
-                    ws, bs = [W0], []
-                    for k, conv in enumerate(m.convs):
-                        if k > 0:
-                            wk = conv.weight.detach().reshape(conv.weight.shape[0], -1)
-                            Wk = torch.zeros((C, C), device=dev)
-                            Wk[:wk.shape[0], :wk.shape[1]] = wk
-                            ws.append(Wk)
-                        b = torch.zeros(C, device=dev)
-                        if conv.bias is not None:
-                            b[:conv.bias.shape[0]] = conv.bias.detach()
-                        bs.append(b)
-                    gw, gb = torch.zeros(C, device=dev), torch.zeros(C, device=dev)
-                    if m.gn.weight is not None:
-                        gw[:co_real] = m.gn.weight.detach().reshape(-1)
-                        gb[:co_real] = m.gn.bias.detach().reshape(-1)
-                    else:
-                        gw[:co_real] = 1.0
-                    row.append((ws, bs, gw, gb))
-                out.append(row)
-                cin_real, cin_store = co_real, C
-        self._pad_cache = (key, out)
-        return out
 
     def _flat_params(self):
         """(spec, tensors) of the fused embedder in the order _ops.embed_params_from_flat expects."""
@@ -258,10 +196,7 @@ class Network(nn.Module):
         keep = []
         params = self._embed_params(keep)
         c_out = self._fused[2][-1][2].convs[-1].weight.shape[0]
-        c_run = int(params.block[0].mlp1.c_out)               # the width the kernels run (zero-padded widths: see _padded_widths)
-        emb = _ops.embed_fwd(params, prec, plain, c_run, n_dev)
-        if c_run != c_out:
-            emb = emb[:, :c_out].contiguous()
+        emb = _ops.embed_fwd(params, prec, plain, c_out, n_dev)
         if isinstance(x, MaskedTensor):
             return rewrap(emb, x.tensor.names[:-1])
         return emb
@@ -279,9 +214,7 @@ class Network(nn.Module):
         keep = []
         params = self._embed_params(keep)
         c_out = self._fused[2][-1][2].convs[-1].weight.shape[0]
-        c_run = int(params.block[0].mlp1.c_out)
-        emb = _ops.embed_fwd_adjacency(params, L.PRECISIONS[prec_name], adj, c_run, sizes)
-        return emb if c_run == c_out else emb[:, :c_out].contiguous()
+        return _ops.embed_fwd_adjacency(params, L.PRECISIONS[prec_name], adj, c_out, sizes)
 
     # ---- reference-compatible execution ----------------------------------------------------------
     def forward(self, inputs):

@@ -219,7 +219,7 @@ int fgnn_lap_fwd(const float* scores, int32_t* col_of_row, int32_t* correct, dou
 
 /* ---- fused embedder (the hot path proper) ------------------------------------------------ */
 
-/* node_embedding forward for G graphs: x (G,c_in0,N,N) fp32 -> emb (G,C,N) fp32.
+/* node_embedding forward for G graphs: x (G,c_in0,N,N) fp32 -> emb (G,C,N) fp32, C = the last block's c_out.
  * Replaces Network.forward over the 4-block DAG + ColumnMaxPooling
  * (models/utils.py:63-69, models/blocks_emb.py:16-43, models/trainers.py:64-65).
  *   precision FGNN_FP32 : composition of the fp32 operators above.
@@ -227,6 +227,10 @@ int fgnn_lap_fwd(const float* scores, int32_t* col_of_row, int32_t* correct, dou
  *     16-bit pre-normalisation planes, GraphNorm is folded into the consumers (DESIGN.md).  N <= 4096; the
  *     batch is cut into passes of equal size, each within FGNN_TC_WS_GB (default 16) GB of planes when a graph
  *     fits (one graph takes 11.6 GB at N = 4096, C = 64, a pass is never less than one graph).
+ *     Widths: every block's c_out (shared by its three MLPs) is 1 .. 64 and c_in0 <= 64, with the parameters in
+ *     their real shapes.  The kernels run at width 32 when every c_out is <= 32, else 64, with the padded channels
+ *     exactly zero (the library pads the parameters itself); the workspace is that of the uniform model of that
+ *     width.  A c_out above 64 fails with FGNN_ERR_UNSUPPORTED.
  * workspace: fgnn_embed_workspace_bytes(...) bytes, 1024-byte aligned (0 when the shape is unsupported). */
 size_t fgnn_embed_workspace_bytes(const fgnn_embed_params* p, int32_t precision, int32_t G, int32_t N);
 int fgnn_embed_fwd(const fgnn_embed_params* p, int32_t precision, const float* x, float* emb,
@@ -244,14 +248,15 @@ int fgnn_embed_fwd_adjacency_u8(const fgnn_embed_params* p, int32_t precision, c
  * (models/trainers.py:70-76, commander_explore.py:120-123), with every contraction of both passes on tcgen05.
  * fgnn_embed_fwd_train computes the same embeddings as fgnn_embed_fwd (FGNN_BF16 / FGNN_FP16) and leaves in
  * `workspace` what backward needs (hidden activations, pre-norm planes, GraphNorm statistics, pooling arg-max);
- * fgnn_embed_bwd takes d loss / d emb (G,C,N) fp32 and ACCUMULATES d loss / d parameter into `grads` (fp32, same
- * shapes as the parameters; the last conv bias of every MLP receives its exact gradient, zero up to rounding, as
+ * fgnn_embed_bwd takes d loss / d emb (G,C,N) fp32 (C = the last block's c_out) and ACCUMULATES d loss / d parameter
+ * into `grads` (fp32, the real shapes of the parameters: widths as for fgnn_embed_fwd, padded entries are never written; the last conv bias of every MLP receives its exact gradient, zero up to rounding, as
  * in the reference).  16-bit gradient planes carry a power-of-two loss scale: the one that brings max |d emb| into
  * [2^(grad_scale_log2 - 1), 2^grad_scale_log2), chosen on the device; the parameter gradients come back un-scaled.
  * As with the reference's AMP GradScaler, fp16 gradient planes can overflow for a given scale: the parameter
  * gradients are then non-finite and the caller skips the step and lowers grad_scale_log2 (training.py does; 9 is
  * the default, -24 .. 15 accepted; bf16 never overflows).  The workspace must be the one the forward call filled
- * (same G, N, parameters), fgnn_embed_train_workspace_bytes(...) bytes, 1024-byte aligned.  N <= 1024.
+ * (same G, N, parameters), fgnn_embed_train_workspace_bytes(...) bytes, 1024-byte aligned.  N <= 1024, and every
+ * MLP has the same depth.
  * Two plans, picked from the shapes by all three calls alike:
  *   keep-all   the workspace keeps every activation of the batch from forward to backward (about 51 plane sets per
  *              graph at depth 3, 4 blocks: 107 GB for 64 graphs of N = 500, C = 64).  Used while that size is <= T.
