@@ -81,12 +81,21 @@ _SIGNATURES = {
     "fgnn_ce_argmax_fwd_f32": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _sz, _vp]),
     "fgnn_ce_bwd_f32": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp]),
     "fgnn_lap_fwd": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp]),
+    "fgnn_scores_pair_fwd_f32": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp]),
+    "fgnn_scores_pair_bwd_f32": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp]),
+    "fgnn_ce_pair_argmax_fwd_f32": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp, _vp, _sz, _vp]),
+    "fgnn_ce_pair_bwd_f32": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp, _vp]),
+    "fgnn_lap_pair_fwd": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp, _vp]),
     "fgnn_generate_workspace_bytes": (_sz, [_i32, _i32, _i32]),
     "fgnn_generate_pairs_u8": (C.c_int, [_vp, _vp, _i32, _i32, _vp, _i32, C.c_float, C.c_float, C.c_uint64, _vp, _sz, _vp]),
     "fgnn_head_workspace_bytes": (_sz, [_i32, _i32]),
     "fgnn_head_fwd": (C.c_int, [_i32, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp, _sz, _vp]),
     "fgnn_head_fwd_train": (C.c_int, [_i32, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp, _sz, _vp]),
     "fgnn_head_bwd": (C.c_int, [_i32, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp, _sz, _vp]),
+    "fgnn_head_pair_workspace_bytes": (_sz, [_i32, _i32]),
+    "fgnn_head_pair_fwd": (C.c_int, [_i32, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _sz, _vp]),
+    "fgnn_head_pair_fwd_train": (C.c_int, [_i32, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _sz, _vp]),
+    "fgnn_head_pair_bwd": (C.c_int, [_i32, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _sz, _vp]),
     "fgnn_embed_workspace_bytes": (_sz, [C.POINTER(EmbedParams), _i32, _i32, _i32]),
     "fgnn_embed_fwd": (C.c_int, [C.POINTER(EmbedParams), _i32, _vp, _vp, _i32, _i32, _vp, _vp, _sz, _vp]),
     "fgnn_embed_fwd_adjacency_u8": (C.c_int, [C.POINTER(EmbedParams), _i32, _vp, _vp, _i32, _i32, _vp, _vp, _sz, _vp]),

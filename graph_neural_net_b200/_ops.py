@@ -193,71 +193,99 @@ class ColMaxFunction(torch.autograd.Function):
         return dx, None
 
 
+def _save_sizes(*sizes):
+    """Size tensors for ctx.save_for_backward (an empty placeholder for None) and which of them were given."""
+    return [n if n is not None else torch.empty(0) for n in sizes], [n is not None for n in sizes]
+
+
+def _saved_sizes(saved, given):
+    return [n if g else None for n, g in zip(saved, given)]
+
+
+def _pair_shapes(e1: torch.Tensor, e2: torch.Tensor, what: str):
+    """(G, C, N1, N2) of graph 1's (G,C,N1) and graph 2's (G,C,N2) node vectors."""
+    if e1.dim() != 3 or e2.dim() != 3 or e1.shape[:2] != e2.shape[:2]:
+        raise L.FgnnError(f"{what}: embeddings must be (G,C,N1) and (G,C,N2) with the same G and C, got "
+                          f"{tuple(e1.shape)} and {tuple(e2.shape)}")
+    return e1.shape[0], e1.shape[1], e1.shape[2], e2.shape[2]
+
+
 class ScoresFunction(torch.autograd.Function):
-    """scores[b] = e1[b]^T e2[b] (reference models/trainers.py:67)."""
+    """scores[b] = e1[b]^T e2[b] (reference models/trainers.py:67): e1 (G,C,N1), e2 (G,C,N2) -> (G,N1,N2), zero outside
+    each graph's n1 x n2 block.  n2_dev (graph 2's sizes) defaults to n_dev."""
 
     @staticmethod
-    def forward(ctx, e1, e2, n_dev):
+    def forward(ctx, e1, e2, n_dev, n2_dev=None):
         lib = L.get_lib()
         e1 = L.require_cuda_f32(e1, "e1")
         e2 = L.require_cuda_f32(e2, "e2")
-        if e1.shape != e2.shape or e1.dim() != 3:
-            raise L.FgnnError(f"siamese head: expected two (B,C,N) tensors, got {tuple(e1.shape)} {tuple(e2.shape)}")
-        G, Cc, N = e1.shape
-        s = torch.empty((G, N, N), device=e1.device, dtype=torch.float32)
-        L.check(lib.fgnn_scores_fwd_f32(L.ptr(e1), L.ptr(e2), L.ptr(s), G, Cc, N, _npg(n_dev),
-                                        L.stream_ptr(e1.device)), "fgnn_scores_fwd_f32")
-        ctx.save_for_backward(e1, e2, n_dev if n_dev is not None else torch.empty(0))
-        ctx.has_n = n_dev is not None
+        G, Cc, N1, N2 = _pair_shapes(e1, e2, "siamese head")
+        n2_dev = n_dev if n2_dev is None else n2_dev
+        s = torch.empty((G, N1, N2), device=e1.device, dtype=torch.float32)
+        L.check(lib.fgnn_scores_pair_fwd_f32(L.ptr(e1), L.ptr(e2), L.ptr(s), G, Cc, N1, N2, _npg(n_dev, G), _npg(n2_dev, G),
+                                             L.stream_ptr(e1.device)), "fgnn_scores_pair_fwd_f32")
+        saved, ctx.given = _save_sizes(n_dev, n2_dev)
+        ctx.save_for_backward(e1, e2, *saved)
         return s
 
     @staticmethod
     def backward(ctx, ds):
         lib = L.get_lib()
-        e1, e2, n_dev = ctx.saved_tensors
-        n_dev = n_dev if ctx.has_n else None
+        e1, e2, *saved = ctx.saved_tensors
+        n_dev, n2_dev = _saved_sizes(saved, ctx.given)
         ds = L.require_cuda_f32(ds, "dscores")
-        G, Cc, N = e1.shape
+        G, Cc, N1, N2 = _pair_shapes(e1, e2, "siamese head")
         de1, de2 = torch.empty_like(e1), torch.empty_like(e2)
-        L.check(lib.fgnn_scores_bwd_f32(L.ptr(e1), L.ptr(e2), L.ptr(ds), L.ptr(de1), L.ptr(de2), G, Cc, N,
-                                        _npg(n_dev), L.stream_ptr(e1.device)), "fgnn_scores_bwd_f32")
-        return de1, de2, None
+        L.check(lib.fgnn_scores_pair_bwd_f32(L.ptr(e1), L.ptr(e2), L.ptr(ds), L.ptr(de1), L.ptr(de2), G, Cc, N1, N2,
+                                             _npg(n_dev), _npg(n2_dev), L.stream_ptr(e1.device)), "fgnn_scores_pair_bwd_f32")
+        return de1, de2, None, None
+
+
+def ce_argmax(scores: torch.Tensor, n_dev=None, n2_dev=None, want_argmax: bool = False):
+    """fgnn_ce_pair_argmax_fwd_f32 on (G,N1,N2) scores -> (ce_sum[G], correct[G], row_lse (G,N1), row_argmax (G,N1) or
+    None).  Row i's target is column i; rows i >= n2 have none.  n2_dev defaults to n_dev."""
+    lib = L.get_lib()
+    scores = L.require_cuda_f32(scores, "raw_scores")
+    if scores.dim() != 3:
+        raise L.FgnnError(f"raw_scores must be (B,N1,N2), got {tuple(scores.shape)}")
+    G, N1, N2 = scores.shape
+    n2_dev = n_dev if n2_dev is None else n2_dev
+    ce = torch.empty(G, device=scores.device, dtype=torch.float32)
+    correct = torch.empty(G, device=scores.device, dtype=torch.int32)
+    lse = torch.empty((G, N1), device=scores.device, dtype=torch.float32)
+    arg = torch.empty((G, N1), device=scores.device, dtype=torch.int32) if want_argmax else None
+    ws = L.workspace(scores.device, lib.fgnn_ce_workspace_bytes(G, N1))
+    L.check(lib.fgnn_ce_pair_argmax_fwd_f32(L.ptr(scores), L.ptr(ce), L.ptr(correct), L.ptr(lse), L.ptr(arg), G, N1, N2,
+                                            _npg(n_dev, G), _npg(n2_dev, G), L.ptr(ws), ws.numel(),
+                                            L.stream_ptr(scores.device)), "fgnn_ce_pair_argmax_fwd_f32")
+    return ce, correct, lse, arg
 
 
 class CrossEntropyIdentityFunction(torch.autograd.Function):
     """Per-graph sum_i CE(scores[i,:], i) (reference toolbox/losses.py:27-31), with the row argmax
-    count as a by-product (toolbox/metrics.py:125-134).  Returns (ce_sum[G], correct[G])."""
+    count as a by-product (toolbox/metrics.py:125-134).  Returns (ce_sum[G], correct[G]).  scores (G,N1,N2); the
+    softmax of row i runs over graph 2's n2 valid columns (n2_dev, default n_dev) and rows i >= n2 have no target."""
 
     @staticmethod
-    def forward(ctx, scores, n_dev):
-        lib = L.get_lib()
-        scores = L.require_cuda_f32(scores, "raw_scores")
-        G, N, M = scores.shape
-        if N != M:
-            raise L.FgnnError("raw_scores must be (B,N,N)")
-        ce = torch.empty(G, device=scores.device, dtype=torch.float32)
-        correct = torch.empty(G, device=scores.device, dtype=torch.int32)
-        lse = torch.empty((G, N), device=scores.device, dtype=torch.float32)
-        ws = L.workspace(scores.device, lib.fgnn_ce_workspace_bytes(G, N))
-        L.check(lib.fgnn_ce_argmax_fwd_f32(L.ptr(scores), L.ptr(ce), L.ptr(correct), L.ptr(lse), G, N,
-                                           _npg(n_dev), L.ptr(ws), ws.numel(), L.stream_ptr(scores.device)),
-                "fgnn_ce_argmax_fwd_f32")
-        ctx.save_for_backward(scores, lse, n_dev if n_dev is not None else torch.empty(0))
-        ctx.has_n = n_dev is not None
+    def forward(ctx, scores, n_dev, n2_dev=None):
+        n2_dev = n_dev if n2_dev is None else n2_dev
+        ce, correct, lse, _ = ce_argmax(scores, n_dev, n2_dev)
+        saved, ctx.given = _save_sizes(n_dev, n2_dev)
+        ctx.save_for_backward(scores, lse, *saved)
         ctx.mark_non_differentiable(correct)
         return ce, correct
 
     @staticmethod
     def backward(ctx, dce, _dcorrect):
         lib = L.get_lib()
-        scores, lse, n_dev = ctx.saved_tensors
-        n_dev = n_dev if ctx.has_n else None
-        G, N, _ = scores.shape
+        scores, lse, *saved = ctx.saved_tensors
+        n_dev, n2_dev = _saved_sizes(saved, ctx.given)
+        G, N1, N2 = scores.shape
         coef = L.require_cuda_f32(dce, "dce")
         ds = torch.empty_like(scores)
-        L.check(lib.fgnn_ce_bwd_f32(L.ptr(scores), L.ptr(lse), L.ptr(coef), L.ptr(ds), G, N, _npg(n_dev),
-                                    L.stream_ptr(scores.device)), "fgnn_ce_bwd_f32")
-        return ds, None
+        L.check(lib.fgnn_ce_pair_bwd_f32(L.ptr(scores), L.ptr(lse), L.ptr(coef), L.ptr(ds), G, N1, N2, _npg(n_dev),
+                                         _npg(n2_dev), L.stream_ptr(scores.device)), "fgnn_ce_pair_bwd_f32")
+        return ds, None, None
 
 
 def generate_pairs(generator: int, G: int, N: int, edge_density: float, noise: float, seed: int, n_dev=None, device="cuda"):
@@ -278,12 +306,11 @@ def generate_pairs(generator: int, G: int, N: int, edge_density: float, noise: f
 
 
 def _head_operands(e1: torch.Tensor, e2: torch.Tensor, precision: str, what: str):
-    """Checked (G,C,N) fp32 operands of the tensor-core head, C zero-padded to a multiple of 16 (K of the MMA; zero
-    channels add nothing to e1^T e2) -> (e1, e2, padded C)."""
+    """Checked (G,C,N1), (G,C,N2) fp32 operands of the tensor-core head, C zero-padded to a multiple of 16 (K of the
+    MMA; zero channels add nothing to e1^T e2) -> (e1, e2, padded C)."""
     e1 = L.require_cuda_f32(e1, "e1")
     e2 = L.require_cuda_f32(e2, "e2")
-    if e1.shape != e2.shape or e1.dim() != 3:
-        raise L.FgnnError(f"{what}: embeddings must both be (G,C,N), got {tuple(e1.shape)} and {tuple(e2.shape)}")
+    _pair_shapes(e1, e2, what)
     if precision not in ("bf16", "fp16"):
         raise L.FgnnError(f"{what} is the tensor-core head (bf16 / fp16 operand splitting); fp32 uses the CUDA-core operators")
     Cc = e1.shape[1]
@@ -295,61 +322,69 @@ def _head_operands(e1: torch.Tensor, e2: torch.Tensor, precision: str, what: str
     return e1, e2, Cc
 
 
-def head_fused(e1: torch.Tensor, e2: torch.Tensor, n_dev, precision: str = "fp16", want_scores: bool = False):
-    """Fused siamese head on tensor cores (fgnn_head_fwd): e1, e2 (G,C,N) -> (ce_sum[G], correct[G], scores or None).
-    scores = e1^T e2 (reference models/trainers.py:67), ce_sum / correct as CrossEntropyIdentityFunction
-    (toolbox/losses.py:27-33, toolbox/metrics.py:125-134); the (G,N,N) scores are only materialised on request.
-    Forward only: under autograd use HeadFunction (or ScoresFunction + CrossEntropyIdentityFunction)."""
+def head_fused(e1: torch.Tensor, e2: torch.Tensor, n_dev, precision: str = "fp16", want_scores: bool = False, n2_dev=None):
+    """Fused siamese head on tensor cores (fgnn_head_pair_fwd): e1 (G,C,N1), e2 (G,C,N2) -> (ce_sum[G], correct[G],
+    scores (G,N1,N2) or None).  scores = e1^T e2 (reference models/trainers.py:67), ce_sum / correct as
+    CrossEntropyIdentityFunction (toolbox/losses.py:27-33, toolbox/metrics.py:125-134); the scores are only materialised
+    on request.  n2_dev (graph 2's sizes) defaults to n_dev.  Forward only: under autograd use HeadFunction (or
+    ScoresFunction + CrossEntropyIdentityFunction)."""
     lib = L.get_lib()
     e1, e2, Cc = _head_operands(e1, e2, precision, "head_fused")
-    G, _, N = e1.shape
+    G, _, N1 = e1.shape
+    N2 = e2.shape[2]
+    n2_dev = n_dev if n2_dev is None else n2_dev
     ce = torch.empty(G, device=e1.device, dtype=torch.float32)
     correct = torch.empty(G, device=e1.device, dtype=torch.int32)
-    scores = torch.empty((G, N, N), device=e1.device, dtype=torch.float32) if want_scores else None
-    ws = L.workspace(e1.device, lib.fgnn_head_workspace_bytes(G, N))
-    L.check(lib.fgnn_head_fwd(L.PRECISIONS[precision], L.ptr(e1), L.ptr(e2), L.ptr(scores) if want_scores else None,
-                              L.ptr(ce), L.ptr(correct), G, Cc, N, _npg(n_dev, G), L.ptr(ws), ws.numel(),
-                              L.stream_ptr(e1.device)), "fgnn_head_fwd")
+    scores = torch.empty((G, N1, N2), device=e1.device, dtype=torch.float32) if want_scores else None
+    ws = L.workspace(e1.device, lib.fgnn_head_pair_workspace_bytes(G, N1))
+    L.check(lib.fgnn_head_pair_fwd(L.PRECISIONS[precision], L.ptr(e1), L.ptr(e2), L.ptr(scores) if want_scores else None,
+                                   L.ptr(ce), L.ptr(correct), G, Cc, N1, N2, _npg(n_dev, G), _npg(n2_dev, G), L.ptr(ws),
+                                   ws.numel(), L.stream_ptr(e1.device)), "fgnn_head_pair_fwd")
     return ce, correct, scores
 
 
 class HeadFunction(torch.autograd.Function):
-    """Differentiable fused head (fgnn_head_fwd_train / fgnn_head_bwd): e1, e2 (G,C,N) -> (ce_sum[G], correct[G]),
-    what ScoresFunction + CrossEntropyIdentityFunction compute (models/trainers.py:67, toolbox/losses.py:27-31,
-    toolbox/metrics.py:125-134) without the (G,N,N) scores or their gradient.  16-bit precisions only; correct is
-    not differentiable."""
+    """Differentiable fused head (fgnn_head_pair_fwd_train / fgnn_head_pair_bwd): e1 (G,C,N1), e2 (G,C,N2) ->
+    (ce_sum[G], correct[G]), what ScoresFunction + CrossEntropyIdentityFunction compute (models/trainers.py:67,
+    toolbox/losses.py:27-31, toolbox/metrics.py:125-134) without the (G,N1,N2) scores or their gradient.  16-bit
+    precisions only; correct is not differentiable; n2_dev (graph 2's sizes) defaults to n_dev."""
 
     @staticmethod
-    def forward(ctx, e1, e2, n_dev, precision):
+    def forward(ctx, e1, e2, n_dev, precision, n2_dev=None):
         lib = L.get_lib()
         c_in = e1.shape[1] if e1.dim() == 3 else None
         e1, e2, Cc = _head_operands(e1, e2, precision, "HeadFunction")
-        G, _, N = e1.shape
+        G, _, N1 = e1.shape
+        N2 = e2.shape[2]
+        n2_dev = n_dev if n2_dev is None else n2_dev
         ce = torch.empty(G, device=e1.device, dtype=torch.float32)
         correct = torch.empty(G, device=e1.device, dtype=torch.int32)
-        lse = torch.empty((G, N), device=e1.device, dtype=torch.float32)
-        ws = L.workspace(e1.device, lib.fgnn_head_workspace_bytes(G, N))
-        L.check(lib.fgnn_head_fwd_train(L.PRECISIONS[precision], L.ptr(e1), L.ptr(e2), L.ptr(ce), L.ptr(correct), L.ptr(lse),
-                                        G, Cc, N, _npg(n_dev, G), L.ptr(ws), ws.numel(), L.stream_ptr(e1.device)),
-                "fgnn_head_fwd_train")
-        ctx.save_for_backward(e1, e2, lse, n_dev if n_dev is not None else torch.empty(0))
-        ctx.has_n, ctx.precision, ctx.c_in = n_dev is not None, precision, c_in
+        lse = torch.empty((G, N1), device=e1.device, dtype=torch.float32)
+        ws = L.workspace(e1.device, lib.fgnn_head_pair_workspace_bytes(G, N1))
+        L.check(lib.fgnn_head_pair_fwd_train(L.PRECISIONS[precision], L.ptr(e1), L.ptr(e2), L.ptr(ce), L.ptr(correct),
+                                             L.ptr(lse), G, Cc, N1, N2, _npg(n_dev, G), _npg(n2_dev, G), L.ptr(ws),
+                                             ws.numel(), L.stream_ptr(e1.device)), "fgnn_head_pair_fwd_train")
+        saved, ctx.given = _save_sizes(n_dev, n2_dev)
+        ctx.save_for_backward(e1, e2, lse, *saved)
+        ctx.precision, ctx.c_in = precision, c_in
         ctx.mark_non_differentiable(correct)
         return ce, correct
 
     @staticmethod
     def backward(ctx, dce, _dcorrect):
         lib = L.get_lib()
-        e1, e2, lse, n_dev = ctx.saved_tensors
-        n_dev = n_dev if ctx.has_n else None
-        G, Cc, N = e1.shape
+        e1, e2, lse, *saved = ctx.saved_tensors
+        n_dev, n2_dev = _saved_sizes(saved, ctx.given)
+        G, Cc, N1 = e1.shape
+        N2 = e2.shape[2]
         coef = L.require_cuda_f32(dce, "dce")
         de1, de2 = torch.empty_like(e1), torch.empty_like(e2)
-        L.check(lib.fgnn_head_bwd(L.PRECISIONS[ctx.precision], L.ptr(e1), L.ptr(e2), L.ptr(lse), L.ptr(coef), L.ptr(de1),
-                                  L.ptr(de2), G, Cc, N, _npg(n_dev, G), None, 0, L.stream_ptr(e1.device)), "fgnn_head_bwd")
+        L.check(lib.fgnn_head_pair_bwd(L.PRECISIONS[ctx.precision], L.ptr(e1), L.ptr(e2), L.ptr(lse), L.ptr(coef),
+                                       L.ptr(de1), L.ptr(de2), G, Cc, N1, N2, _npg(n_dev, G), _npg(n2_dev, G), None, 0,
+                                       L.stream_ptr(e1.device)), "fgnn_head_pair_bwd")
         if Cc != ctx.c_in:
             de1, de2 = de1[:, :ctx.c_in], de2[:, :ctx.c_in]
-        return de1, de2, None, None
+        return de1, de2, None, None, None
 
 
 def graphnorm_fwd(x: torch.Tensor, n_dev, gn_w, gn_b, eps: float, constant_n: bool = True) -> torch.Tensor:

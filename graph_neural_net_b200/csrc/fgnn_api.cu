@@ -197,33 +197,60 @@ int fgnn_matmul_bwd_f32(const float* a, const float* b, const float* dout, float
   return FGNN_OK;
 }
 
-size_t fgnn_head_workspace_bytes(int32_t G, int32_t N) { return tc::head_workspace_bytes(G, N); }
+size_t fgnn_head_workspace_bytes(int32_t G, int32_t N) { return fgnn_head_pair_workspace_bytes(G, N); }
+size_t fgnn_head_pair_workspace_bytes(int32_t G, int32_t N1) { return tc::head_workspace_bytes(G, N1); }
 
 int fgnn_head_fwd(int32_t precision, const float* e1, const float* e2, float* scores, float* ce_sum, int32_t* correct,
                   int32_t G, int32_t C, int32_t N, const int32_t* n_per_graph, void* workspace, size_t workspace_bytes,
                   void* stream) {
-  return tc::head_fwd(precision, e1, e2, scores, ce_sum, correct, G, C, N, n_per_graph, workspace, workspace_bytes,
+  return fgnn_head_pair_fwd(precision, e1, e2, scores, ce_sum, correct, G, C, N, N, n_per_graph, n_per_graph, workspace,
+                            workspace_bytes, stream);
+}
+
+int fgnn_head_pair_fwd(int32_t precision, const float* e1, const float* e2, float* scores, float* ce_sum, int32_t* correct,
+                       int32_t G, int32_t C, int32_t N1, int32_t N2, const int32_t* n1, const int32_t* n2, void* workspace,
+                       size_t workspace_bytes, void* stream) {
+  return tc::head_fwd(precision, e1, e2, scores, ce_sum, correct, G, C, N1, N2, n1, n2, workspace, workspace_bytes,
                       (cudaStream_t)stream);
 }
 
 int fgnn_head_fwd_train(int32_t precision, const float* e1, const float* e2, float* ce_sum, int32_t* correct, float* row_lse,
                         int32_t G, int32_t C, int32_t N, const int32_t* n_per_graph, void* workspace, size_t workspace_bytes,
                         void* stream) {
-  return tc::head_fwd_train(precision, e1, e2, ce_sum, correct, row_lse, G, C, N, n_per_graph, workspace, workspace_bytes,
+  return fgnn_head_pair_fwd_train(precision, e1, e2, ce_sum, correct, row_lse, G, C, N, N, n_per_graph, n_per_graph,
+                                  workspace, workspace_bytes, stream);
+}
+
+int fgnn_head_pair_fwd_train(int32_t precision, const float* e1, const float* e2, float* ce_sum, int32_t* correct,
+                             float* row_lse, int32_t G, int32_t C, int32_t N1, int32_t N2, const int32_t* n1,
+                             const int32_t* n2, void* workspace, size_t workspace_bytes, void* stream) {
+  return tc::head_fwd_train(precision, e1, e2, ce_sum, correct, row_lse, G, C, N1, N2, n1, n2, workspace, workspace_bytes,
                             (cudaStream_t)stream);
 }
 
 int fgnn_head_bwd(int32_t precision, const float* e1, const float* e2, const float* row_lse, const float* coef, float* de1,
                   float* de2, int32_t G, int32_t C, int32_t N, const int32_t* n_per_graph, void* workspace,
                   size_t workspace_bytes, void* stream) {
+  return fgnn_head_pair_bwd(precision, e1, e2, row_lse, coef, de1, de2, G, C, N, N, n_per_graph, n_per_graph, workspace,
+                            workspace_bytes, stream);
+}
+
+int fgnn_head_pair_bwd(int32_t precision, const float* e1, const float* e2, const float* row_lse, const float* coef,
+                       float* de1, float* de2, int32_t G, int32_t C, int32_t N1, int32_t N2, const int32_t* n1,
+                       const int32_t* n2, void* workspace, size_t workspace_bytes, void* stream) {
   (void)workspace;
   (void)workspace_bytes;
-  return tc::head_bwd(precision, e1, e2, row_lse, coef, de1, de2, G, C, N, n_per_graph, (cudaStream_t)stream);
+  return tc::head_bwd(precision, e1, e2, row_lse, coef, de1, de2, G, C, N1, N2, n1, n2, (cudaStream_t)stream);
 }
 
 int fgnn_lap_fwd(const float* scores, int32_t* col_of_row, int32_t* correct, double* total_cost, int32_t G,
                  int32_t N, const int32_t* n_per_graph, void* stream) {
-  return lap::lap_fwd(scores, col_of_row, correct, total_cost, G, N, n_per_graph, (cudaStream_t)stream);
+  return fgnn_lap_pair_fwd(scores, col_of_row, correct, total_cost, G, N, N, n_per_graph, n_per_graph, stream);
+}
+
+int fgnn_lap_pair_fwd(const float* scores, int32_t* col_of_row, int32_t* correct, double* total_cost, int32_t G,
+                      int32_t N1, int32_t N2, const int32_t* n1, const int32_t* n2, void* stream) {
+  return lap::lap_fwd(scores, col_of_row, correct, total_cost, G, N1, N2, n1, n2, (cudaStream_t)stream);
 }
 
 int fgnn_features_from_adjacency_u8(const uint8_t* adj, float* out, int32_t G, int32_t N, const int32_t* n_per_graph,
@@ -245,13 +272,23 @@ int fgnn_colmax_bwd_f32(const float* dout, const int32_t* argmax, float* dx, int
 
 int fgnn_scores_fwd_f32(const float* e1, const float* e2, float* scores, int32_t G, int32_t C,
                         int32_t N, const int32_t* n_per_graph, void* stream) {
-  return f32::scores_fwd(e1, e2, scores, G, C, N, n_per_graph, (cudaStream_t)stream);
+  return fgnn_scores_pair_fwd_f32(e1, e2, scores, G, C, N, N, n_per_graph, n_per_graph, stream);
+}
+
+int fgnn_scores_pair_fwd_f32(const float* e1, const float* e2, float* scores, int32_t G, int32_t C, int32_t N1,
+                             int32_t N2, const int32_t* n1, const int32_t* n2, void* stream) {
+  return f32::scores_fwd(e1, e2, scores, G, C, N1, N2, n1, n2, (cudaStream_t)stream);
 }
 
 int fgnn_scores_bwd_f32(const float* e1, const float* e2, const float* dscores, float* de1,
                         float* de2, int32_t G, int32_t C, int32_t N, const int32_t* n_per_graph,
                         void* stream) {
-  return f32::scores_bwd(e1, e2, dscores, de1, de2, G, C, N, n_per_graph, (cudaStream_t)stream);
+  return fgnn_scores_pair_bwd_f32(e1, e2, dscores, de1, de2, G, C, N, N, n_per_graph, n_per_graph, stream);
+}
+
+int fgnn_scores_pair_bwd_f32(const float* e1, const float* e2, const float* dscores, float* de1, float* de2, int32_t G,
+                             int32_t C, int32_t N1, int32_t N2, const int32_t* n1, const int32_t* n2, void* stream) {
+  return f32::scores_bwd(e1, e2, dscores, de1, de2, G, C, N1, N2, n1, n2, (cudaStream_t)stream);
 }
 
 size_t fgnn_ce_workspace_bytes(int32_t G, int32_t N) { return (size_t)G * N * 8 + 1024; }
@@ -259,13 +296,25 @@ size_t fgnn_ce_workspace_bytes(int32_t G, int32_t N) { return (size_t)G * N * 8 
 int fgnn_ce_argmax_fwd_f32(const float* scores, float* ce_sum, int32_t* correct, float* row_lse,
                            int32_t G, int32_t N, const int32_t* n_per_graph, void* workspace,
                            size_t workspace_bytes, void* stream) {
-  return f32::ce_argmax_fwd(scores, ce_sum, correct, row_lse, G, N, n_per_graph, workspace, workspace_bytes,
+  return fgnn_ce_pair_argmax_fwd_f32(scores, ce_sum, correct, row_lse, nullptr, G, N, N, n_per_graph, n_per_graph,
+                                     workspace, workspace_bytes, stream);
+}
+
+int fgnn_ce_pair_argmax_fwd_f32(const float* scores, float* ce_sum, int32_t* correct, float* row_lse, int32_t* row_argmax,
+                                int32_t G, int32_t N1, int32_t N2, const int32_t* n1, const int32_t* n2, void* workspace,
+                                size_t workspace_bytes, void* stream) {
+  return f32::ce_argmax_fwd(scores, ce_sum, correct, row_lse, row_argmax, G, N1, N2, n1, n2, workspace, workspace_bytes,
                             (cudaStream_t)stream);
 }
 
 int fgnn_ce_bwd_f32(const float* scores, const float* row_lse, const float* coef, float* dscores,
                     int32_t G, int32_t N, const int32_t* n_per_graph, void* stream) {
-  return f32::ce_bwd(scores, row_lse, coef, dscores, G, N, n_per_graph, (cudaStream_t)stream);
+  return fgnn_ce_pair_bwd_f32(scores, row_lse, coef, dscores, G, N, N, n_per_graph, n_per_graph, stream);
+}
+
+int fgnn_ce_pair_bwd_f32(const float* scores, const float* row_lse, const float* coef, float* dscores, int32_t G,
+                         int32_t N1, int32_t N2, const int32_t* n1, const int32_t* n2, void* stream) {
+  return f32::ce_bwd(scores, row_lse, coef, dscores, G, N1, N2, n1, n2, (cudaStream_t)stream);
 }
 
 size_t fgnn_embed_workspace_bytes(const fgnn_embed_params* p, int32_t precision, int32_t G, int32_t N) {

@@ -276,12 +276,13 @@ __global__ void colmax_bwd_kernel(const float* __restrict__ dout, const int32_t*
 
 // ---------------------------------------------------------------------------------------
 // siamese scores[g,i,j] = sum_c e1[g,c,i] * e2[g,c,j]   (trainers.py:67)
+// graph 1 (rows i, e1 (G,C,N1)) has n1[g] vertices, graph 2 (columns j, e2 (G,C,N2)) n2[g]; scores (G,N1,N2)
 // ---------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
 scores_fwd_kernel(const float* __restrict__ e1, const float* __restrict__ e2, float* __restrict__ s,
-                  int C, int N, const int32_t* __restrict__ n_per_graph) {
+                  int C, int N1, int N2, const int32_t* __restrict__ n1p, const int32_t* __restrict__ n2p) {
   const int g = blockIdx.z;
-  const int n = graph_n(n_per_graph, g, N);
+  const int n1 = graph_n(n1p, g, N1), n2 = graph_n(n2p, g, N2);
   const int i = blockIdx.y * 16 + threadIdx.x / 16;
   const int j = blockIdx.x * 16 + threadIdx.x % 16;
   __shared__ float a[16][17], b[16][17];
@@ -290,59 +291,59 @@ scores_fwd_kernel(const float* __restrict__ e1, const float* __restrict__ e2, fl
     int cc = c0 + threadIdx.x / 16;
     int ii = blockIdx.y * 16 + threadIdx.x % 16;
     int jj = blockIdx.x * 16 + threadIdx.x % 16;
-    a[threadIdx.x / 16][threadIdx.x % 16] = (cc < C && ii < n) ? e1[((long)g * C + cc) * N + ii] : 0.f;
-    b[threadIdx.x / 16][threadIdx.x % 16] = (cc < C && jj < n) ? e2[((long)g * C + cc) * N + jj] : 0.f;
+    a[threadIdx.x / 16][threadIdx.x % 16] = (cc < C && ii < n1) ? e1[((long)g * C + cc) * N1 + ii] : 0.f;
+    b[threadIdx.x / 16][threadIdx.x % 16] = (cc < C && jj < n2) ? e2[((long)g * C + cc) * N2 + jj] : 0.f;
     __syncthreads();
 #pragma unroll
     for (int c = 0; c < 16; ++c) acc = fmaf(a[c][threadIdx.x / 16], b[c][threadIdx.x % 16], acc);
     __syncthreads();
   }
-  if (i < N && j < N) s[((long)g * N + i) * N + j] = (i < n && j < n) ? acc : 0.f;
+  if (i < N1 && j < N2) s[((long)g * N1 + i) * N2 + j] = (i < n1 && j < n2) ? acc : 0.f;
 }
 
 // de1[g,c,i] = sum_j ds[g,i,j] e2[g,c,j];  de2[g,c,j] = sum_i ds[g,i,j] e1[g,c,i]
 __global__ void __launch_bounds__(128)
 scores_bwd_kernel(const float* __restrict__ e1, const float* __restrict__ e2, const float* __restrict__ ds,
-                  float* __restrict__ de1, float* __restrict__ de2, int C, int N,
-                  const int32_t* __restrict__ n_per_graph) {
+                  float* __restrict__ de1, float* __restrict__ de2, int C, int N1, int N2,
+                  const int32_t* __restrict__ n1p, const int32_t* __restrict__ n2p) {
   const int g = blockIdx.z, c = blockIdx.y;
-  const int n = graph_n(n_per_graph, g, N);
+  const int n1 = graph_n(n1p, g, N1), n2 = graph_n(n2p, g, N2);
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;  // i for de1, j for de2
-  if (idx >= N) return;
-  const float* dsg = ds + (long)g * N * N;
-  const float* e1r = e1 + ((long)g * C + c) * N;
-  const float* e2r = e2 + ((long)g * C + c) * N;
+  if (idx >= N1 && idx >= N2) return;
+  const float* dsg = ds + (long)g * N1 * N2;
+  const float* e1r = e1 + ((long)g * C + c) * N1;
+  const float* e2r = e2 + ((long)g * C + c) * N2;
   float a1 = 0.f, a2 = 0.f;
-  if (idx < n) {
-    for (int q = 0; q < n; ++q) {
-      a1 = fmaf(dsg[(long)idx * N + q], e2r[q], a1);
-      a2 = fmaf(dsg[(long)q * N + idx], e1r[q], a2);
-    }
-  }
-  if (de1) de1[((long)g * C + c) * N + idx] = a1;
-  if (de2) de2[((long)g * C + c) * N + idx] = a2;
+  if (idx < n1)
+    for (int q = 0; q < n2; ++q) a1 = fmaf(dsg[(long)idx * N2 + q], e2r[q], a1);
+  if (idx < n2)
+    for (int q = 0; q < n1; ++q) a2 = fmaf(dsg[(long)q * N2 + idx], e1r[q], a2);
+  if (de1 && idx < N1) de1[((long)g * C + c) * N1 + idx] = a1;
+  if (de2 && idx < N2) de2[((long)g * C + c) * N2 + idx] = a2;
 }
 
 // ---------------------------------------------------------------------------------------
 // row softmax cross-entropy vs the identity matching + row argmax, one CTA per graph.
 // losses.py:27-34 / metrics.py:125-134 without the host loop.  Deterministic reduction.
+// scores (G,N1,N2); row i's target is column i, so rows i >= n2[g] have none (CE 0, not correct).
 // ---------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
 ce_argmax_rows_kernel(const float* __restrict__ s, float* __restrict__ row_ce, int32_t* __restrict__ row_ok,
-                      float* __restrict__ row_lse, int N, const int32_t* __restrict__ n_per_graph) {
+                      float* __restrict__ row_lse, int32_t* __restrict__ row_argmax, int N1, int N2,
+                      const int32_t* __restrict__ n1p, const int32_t* __restrict__ n2p) {
   // one warp per row: row_ce[g,i] = lse_i - s_ii, row_ok[g,i] = (argmax_j s_ij == i); padded rows -> 0
   const int g = blockIdx.y;
-  const int n = graph_n(n_per_graph, g, N);
+  const int n1 = graph_n(n1p, g, N1), n2 = graph_n(n2p, g, N2);
   const int lane = threadIdx.x % 32;
   const int i = blockIdx.x * (blockDim.x / 32) + threadIdx.x / 32;
-  if (i >= N) return;
+  if (i >= N1) return;
   float ce = 0.f, lse = 0.f;
-  int ok = 0;
-  if (i < n) {
-    const float* r = s + ((long)g * N + i) * N;
+  int ok = 0, am = -1;
+  if (i < n1) {
+    const float* r = s + ((long)g * N1 + i) * N2;
     float m = -INFINITY;
-    int am = 0;
-    for (int j = lane; j < n; j += 32) {
+    am = 0;
+    for (int j = lane; j < n2; j += 32) {
       float v = r[j];
       if (v > m) { m = v; am = j; }
     }
@@ -352,16 +353,19 @@ ce_argmax_rows_kernel(const float* __restrict__ s, float* __restrict__ row_ce, i
       if (ov > m || (ov == m && oi < am)) { m = ov; am = oi; }
     }
     float se = 0.f;
-    for (int j = lane; j < n; j += 32) se += expf(r[j] - m);
+    for (int j = lane; j < n2; j += 32) se += expf(r[j] - m);
     for (int o = 16; o > 0; o >>= 1) se += __shfl_xor_sync(0xffffffffu, se, o);
     lse = m + logf(se);
-    ce = lse - r[i];
-    ok = (am == i);
+    if (i < n2) {
+      ce = lse - r[i];
+      ok = (am == i);
+    }
   }
   if (lane == 0) {
-    row_ce[(long)g * N + i] = ce;
-    row_ok[(long)g * N + i] = ok;
-    if (row_lse) row_lse[(long)g * N + i] = lse;
+    row_ce[(long)g * N1 + i] = ce;
+    row_ok[(long)g * N1 + i] = ok;
+    if (row_lse) row_lse[(long)g * N1 + i] = lse;
+    if (row_argmax) row_argmax[(long)g * N1 + i] = am;
   }
 }
 
@@ -394,20 +398,21 @@ ce_argmax_reduce_kernel(const float* __restrict__ row_ce, const int32_t* __restr
   }
 }
 
+// rows without a target (i >= n2) are not in the CE sum: their gradient is zero
 __global__ void ce_bwd_kernel(const float* __restrict__ s, const float* __restrict__ row_lse,
-                              const float* __restrict__ coef, float* __restrict__ ds, int N,
-                              const int32_t* __restrict__ n_per_graph) {
+                              const float* __restrict__ coef, float* __restrict__ ds, int N1, int N2,
+                              const int32_t* __restrict__ n1p, const int32_t* __restrict__ n2p) {
   const int g = blockIdx.z;
-  const int n = graph_n(n_per_graph, g, N);
+  const int n1 = graph_n(n1p, g, N1), n2 = graph_n(n2p, g, N2);
   const int i = blockIdx.y;
   const float cf = coef[g];
-  for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < N; j += gridDim.x * blockDim.x) {
+  for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < N2; j += gridDim.x * blockDim.x) {
     float v = 0.f;
-    if (i < n && j < n) {
-      float sm = expf(s[((long)g * N + i) * N + j] - row_lse[(long)g * N + i]);
+    if (i < n1 && i < n2 && j < n2) {
+      float sm = expf(s[((long)g * N1 + i) * N2 + j] - row_lse[(long)g * N1 + i]);
       v = cf * (sm - (i == j ? 1.f : 0.f));
     }
-    ds[((long)g * N + i) * N + j] = v;
+    ds[((long)g * N1 + i) * N2 + j] = v;
   }
 }
 
@@ -575,51 +580,55 @@ int colmax_bwd(const float* dout, const int32_t* argmax, float* dx, int G, int C
   return FGNN_OK;
 }
 
-int scores_fwd(const float* e1, const float* e2, float* scores, int G, int C, int N,
-               const int32_t* n_per_graph, cudaStream_t st) {
-  if (int e = check_dims(G, C, N)) return e;
+int scores_fwd(const float* e1, const float* e2, float* scores, int G, int C, int N1, int N2,
+               const int32_t* n1, const int32_t* n2, cudaStream_t st) {
+  if (int e = check_dims(G, C, N1)) return e;
+  if (int e = check_dims(G, C, N2)) return e;
   FGNN_CHECK_ARG(e1 && e2 && scores, "null pointer");
   FGNN_CHECK_ARG(G <= 65535, "G=%d exceeds grid.z limit", G);
-  dim3 grid(ceil_div(N, 16), ceil_div(N, 16), G);
-  scores_fwd_kernel<<<grid, 256, 0, st>>>(e1, e2, scores, C, N, n_per_graph);
+  dim3 grid(ceil_div(N2, 16), ceil_div(N1, 16), G);
+  scores_fwd_kernel<<<grid, 256, 0, st>>>(e1, e2, scores, C, N1, N2, n1, n2);
   FGNN_LAUNCHED();
   return FGNN_OK;
 }
 
 int scores_bwd(const float* e1, const float* e2, const float* ds, float* de1, float* de2, int G, int C,
-               int N, const int32_t* n_per_graph, cudaStream_t st) {
-  if (int e = check_dims(G, C, N)) return e;
+               int N1, int N2, const int32_t* n1, const int32_t* n2, cudaStream_t st) {
+  if (int e = check_dims(G, C, N1)) return e;
+  if (int e = check_dims(G, C, N2)) return e;
   FGNN_CHECK_ARG(e1 && e2 && ds, "null pointer");
   FGNN_CHECK_ARG(G <= 65535 && C <= 65535, "G/C exceed grid limits");
-  dim3 grid(ceil_div(N, 128), C, G);
-  scores_bwd_kernel<<<grid, 128, 0, st>>>(e1, e2, ds, de1, de2, C, N, n_per_graph);
+  dim3 grid(ceil_div(std::max(N1, N2), 128), C, G);
+  scores_bwd_kernel<<<grid, 128, 0, st>>>(e1, e2, ds, de1, de2, C, N1, N2, n1, n2);
   FGNN_LAUNCHED();
   return FGNN_OK;
 }
 
-int ce_argmax_fwd(const float* scores, float* ce_sum, int32_t* correct, float* row_lse, int G, int N,
-                  const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
-  if (int e = check_dims(G, 1, N)) return e;
+int ce_argmax_fwd(const float* scores, float* ce_sum, int32_t* correct, float* row_lse, int32_t* row_argmax, int G,
+                  int N1, int N2, const int32_t* n1, const int32_t* n2, void* ws, size_t ws_bytes, cudaStream_t st) {
+  if (int e = check_dims(G, 1, N1)) return e;
+  if (int e = check_dims(G, 1, N2)) return e;
   FGNN_CHECK_ARG(scores && ce_sum && ws, "null pointer");
   FGNN_CHECK_ARG(G <= 65535, "G=%d exceeds grid.y limit", G);
   Arena ar(ws, ws_bytes);
-  float* row_ce = ar.take<float>((size_t)G * N);
-  int32_t* row_ok = ar.take<int32_t>((size_t)G * N);
+  float* row_ce = ar.take<float>((size_t)G * N1);
+  int32_t* row_ok = ar.take<int32_t>((size_t)G * N1);
   if (!ar.ok()) return fail(FGNN_ERR_WORKSPACE, "ce workspace too small");
-  ce_argmax_rows_kernel<<<dim3(ceil_div(N, 8), G), 256, 0, st>>>(scores, row_ce, row_ok, row_lse, N, n_per_graph);
+  ce_argmax_rows_kernel<<<dim3(ceil_div(N1, 8), G), 256, 0, st>>>(scores, row_ce, row_ok, row_lse, row_argmax, N1, N2, n1, n2);
   FGNN_LAUNCHED();
-  ce_argmax_reduce_kernel<<<G, 256, 0, st>>>(row_ce, row_ok, ce_sum, correct, N);
+  ce_argmax_reduce_kernel<<<G, 256, 0, st>>>(row_ce, row_ok, ce_sum, correct, N1);
   FGNN_LAUNCHED();
   return FGNN_OK;
 }
 
-int ce_bwd(const float* scores, const float* row_lse, const float* coef, float* ds, int G, int N,
-           const int32_t* n_per_graph, cudaStream_t st) {
-  if (int e = check_dims(G, 1, N)) return e;
+int ce_bwd(const float* scores, const float* row_lse, const float* coef, float* ds, int G, int N1, int N2,
+           const int32_t* n1, const int32_t* n2, cudaStream_t st) {
+  if (int e = check_dims(G, 1, N1)) return e;
+  if (int e = check_dims(G, 1, N2)) return e;
   FGNN_CHECK_ARG(scores && row_lse && coef && ds, "null pointer");
-  FGNN_CHECK_ARG(G <= 65535 && N <= 65535, "G/N exceed grid limits");
-  dim3 grid(ceil_div(N, 256), N, G);
-  ce_bwd_kernel<<<grid, 256, 0, st>>>(scores, row_lse, coef, ds, N, n_per_graph);
+  FGNN_CHECK_ARG(G <= 65535 && N1 <= 65535, "G/N exceed grid limits");
+  dim3 grid(ceil_div(N2, 256), N1, G);
+  ce_bwd_kernel<<<grid, 256, 0, st>>>(scores, row_lse, coef, ds, N1, N2, n1, n2);
   FGNN_LAUNCHED();
   return FGNN_OK;
 }

@@ -26,14 +26,15 @@ int colmax_fwd(const float* x, float* out, int32_t* argmax, int G, int C, int N,
                const int32_t* n_per_graph, cudaStream_t st);
 int colmax_bwd(const float* dout, const int32_t* argmax, float* dx, int G, int C, int N,
                const int32_t* n_per_graph, cudaStream_t st);
-int scores_fwd(const float* e1, const float* e2, float* scores, int G, int C, int N,
-               const int32_t* n_per_graph, cudaStream_t st);
+// siamese head, graph 1 padded to N1 with sizes n1, graph 2 to N2 with sizes n2 (null: the padded size)
+int scores_fwd(const float* e1, const float* e2, float* scores, int G, int C, int N1, int N2,
+               const int32_t* n1, const int32_t* n2, cudaStream_t st);
 int scores_bwd(const float* e1, const float* e2, const float* ds, float* de1, float* de2, int G, int C,
-               int N, const int32_t* n_per_graph, cudaStream_t st);
-int ce_argmax_fwd(const float* scores, float* ce_sum, int32_t* correct, float* row_lse, int G, int N,
-                  const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st);
-int ce_bwd(const float* scores, const float* row_lse, const float* coef, float* ds, int G, int N,
-           const int32_t* n_per_graph, cudaStream_t st);
+               int N1, int N2, const int32_t* n1, const int32_t* n2, cudaStream_t st);
+int ce_argmax_fwd(const float* scores, float* ce_sum, int32_t* correct, float* row_lse, int32_t* row_argmax, int G,
+                  int N1, int N2, const int32_t* n1, const int32_t* n2, void* ws, size_t ws_bytes, cudaStream_t st);
+int ce_bwd(const float* scores, const float* row_lse, const float* coef, float* ds, int G, int N1, int N2,
+           const int32_t* n1, const int32_t* n2, cudaStream_t st);
 // out (G,Ca+Cb,N,N) = cat(a (G,Ca,N,N), b (G,Cb,N,N)) along channels  (models/layers.py:145-146)
 int concat_channels(const float* a, const float* b, float* out, int G, int Ca, int Cb, int N,
                     cudaStream_t st);

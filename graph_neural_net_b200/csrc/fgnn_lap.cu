@@ -12,9 +12,12 @@
 // list, else the FIRST assigned one; the kernel keeps the same list in shared memory and reduces over list
 // POSITIONS with that preference.  One CTA per graph: the scan of every Dijkstra step is spread over the CTA's
 // threads and closed by a block-wide arg-min; duals, path and matching arrays live in shared memory: 53 bytes per
-// column (smem_bytes), so the padded size N is limited by the device's opt-in shared memory per block -- N <= 4380 with
-// the 227 KB of an sm_100 device, 217 104 bytes at N = 4096.  Indices into the (G,N,N) scores are 64-bit; the rest are
-// column / row numbers < N.
+// column (smem_bytes), so the solver's column count M = max(N1, N2) is limited by the device's opt-in shared memory per
+// block -- M <= 4380 with the 227 KB of an sm_100 device, 217 104 bytes at M = 4096.  Indices into the (G,N1,N2) scores
+// are 64-bit; the rest are column / row numbers < M.
+// Rectangular problems (graph 1 with n1 rows, graph 2 with n2 columns) are solved as scipy's rectangular_lsap solves
+// them: as they are when n1 <= n2, transposed when n1 > n2 (solver rows = graph-2 vertices), with the cost of each entry
+// always formed from its ORIGINAL row's log-softmax constants.  Rows left without a column get -1.
 #include "fgnn_common.cuh"
 
 #include <cfloat>
@@ -43,10 +46,13 @@ __device__ __forceinline__ bool better(const Best& a, const Best& b) {   // is a
 
 __global__ void __launch_bounds__(kThreads)
 lap_kernel(const float* __restrict__ scores, int32_t* __restrict__ col_of_row, int32_t* __restrict__ correct,
-           double* __restrict__ total_cost, int N, const int32_t* __restrict__ n_per_graph) {
+           double* __restrict__ total_cost, int N1, int N2, const int32_t* __restrict__ n1p, const int32_t* __restrict__ n2p) {
   extern __shared__ __align__(16) unsigned char lap_smem[];
   const int g = blockIdx.x;
-  const int n = n_per_graph ? n_per_graph[g] : N;
+  const int n1 = n1p ? n1p[g] : N1, n2 = n2p ? n2p[g] : N2;
+  const bool tr = n1 > n2;                              // solve the transposed problem
+  const int nr = tr ? n2 : n1, nc = tr ? n1 : n2;       // solver rows <= solver columns
+  const int N = max(N1, N2);                            // capacity of every shared array
   double* u = reinterpret_cast<double*>(lap_smem);      // row duals
   double* v = u + N;                                    // column duals
   double* spc = v + N;                                  // shortest path cost to each column
@@ -61,7 +67,12 @@ lap_kernel(const float* __restrict__ scores, int32_t* __restrict__ col_of_row, i
   __shared__ Best s_best[kWarps];
   __shared__ Best s_pick;
   const int tid = threadIdx.x, lane = tid % 32, warp = tid / 32;
-  const float* S = scores + (long)g * N * N;
+  const float* S = scores + (long)g * N1 * N2;
+  // weight of solver entry (i, j): log_softmax of the original row, fp32 as torch forms it
+  auto weight = [&](int i, int j) -> float {
+    const int r = tr ? j : i, c = tr ? i : j;
+    return (S[(long)r * N2 + c] - rmx[r]) - rlg[r];
+  };
 
   for (int k = tid; k < N; k += kThreads) {
     u[k] = 0.0;
@@ -69,37 +80,35 @@ lap_kernel(const float* __restrict__ scores, int32_t* __restrict__ col_of_row, i
     col4row[k] = -1;
     row4col[k] = -1;
   }
-  for (int r = warp; r < n; r += kWarps) {               // row constants of the log-softmax over the valid columns
-    const float* row = S + (long)r * N;
+  for (int r = warp; r < n1; r += kWarps) {              // row constants of the log-softmax over the valid columns
+    const float* row = S + (long)r * N2;
     float mx = -INFINITY;
-    for (int j = lane; j < n; j += 32) mx = fmaxf(mx, row[j]);
+    for (int j = lane; j < n2; j += 32) mx = fmaxf(mx, row[j]);
     for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
     float sum = 0.f;
-    for (int j = lane; j < n; j += 32) sum += expf(row[j] - mx);
+    for (int j = lane; j < n2; j += 32) sum += expf(row[j] - mx);
     for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
     if (lane == 0) { rmx[r] = mx; rlg[r] = logf(sum); }
   }
   __syncthreads();
 
-  for (int cur = 0; cur < n; ++cur) {
-    for (int j = tid; j < n; j += kThreads) {
+  for (int cur = 0; cur < nr; ++cur) {
+    for (int j = tid; j < nc; j += kThreads) {
       spc[j] = INFINITY;
       sc[j] = 0;
-      remaining[j] = n - j - 1;
+      remaining[j] = nc - j - 1;
     }
     __syncthreads();
     double min_val = 0.0;
-    int i = cur, sink = -1, nvis = 0, num_remaining = n;
+    int i = cur, sink = -1, nvis = 0, num_remaining = nc;
     while (sink < 0) {
       if (tid == 0) vis[nvis] = i;
       ++nvis;
       const double ui = u[i];
-      const float* row = S + (long)i * N;
-      const float mxi = rmx[i], lgi = rlg[i];
       Best b{INFINITY, 0x7fffffff, 0};
       for (int it = tid; it < num_remaining; it += kThreads) {
         const int j = remaining[it];
-        const double r = min_val + (-(double)((row[j] - mxi) - lgi)) - ui - v[j];   // cost = -weight, scipy's operation order
+        const double r = min_val + (-(double)weight(i, j)) - ui - v[j];   // cost = -weight, scipy's operation order
         double cur_cost = spc[j];
         if (r < cur_cost) {
           spc[j] = r;
@@ -142,7 +151,7 @@ lap_kernel(const float* __restrict__ scores, int32_t* __restrict__ col_of_row, i
       if (r == cur) u[r] += min_val;
       else u[r] += min_val - spc[col4row[r]];
     }
-    for (int j = tid; j < n; j += kThreads)
+    for (int j = tid; j < nc; j += kThreads)
       if (sc[j]) v[j] -= min_val - spc[j];
     __syncthreads();
     if (tid == 0) {
@@ -162,12 +171,12 @@ lap_kernel(const float* __restrict__ scores, int32_t* __restrict__ col_of_row, i
   // outputs: matching, #fixed points (the identity is the ground truth, metrics.py:103), optimal cost
   int hits = 0;
   double cost = 0.0;
-  for (int r = tid; r < N; r += kThreads) {
-    const int c = r < n ? col4row[r] : -1;
-    if (col_of_row) col_of_row[(long)g * N + r] = c;
-    if (r < n) {
+  for (int r = tid; r < N1; r += kThreads) {            // r: an original row; transposed, its column is row4col[r]
+    const int c = r < n1 ? (tr ? row4col[r] : col4row[r]) : -1;
+    if (col_of_row) col_of_row[(long)g * N1 + r] = c;
+    if (c >= 0) {
       hits += (c == r);
-      cost -= (double)((S[(long)r * N + c] - rmx[r]) - rlg[r]);
+      cost -= (double)((S[(long)r * N2 + c] - rmx[r]) - rlg[r]);
     }
   }
   for (int o = 16; o > 0; o >>= 1) {
@@ -201,10 +210,11 @@ int max_n(size_t limit) {
 
 }  // namespace
 
-int lap_fwd(const float* scores, int32_t* col_of_row, int32_t* correct, double* total_cost, int G, int N,
-            const int32_t* n_per_graph, cudaStream_t st) {
+int lap_fwd(const float* scores, int32_t* col_of_row, int32_t* correct, double* total_cost, int G, int N1, int N2,
+            const int32_t* n1, const int32_t* n2, cudaStream_t st) {
   FGNN_CHECK_ARG(scores && correct, "null pointer");
-  FGNN_CHECK_ARG(G >= 1 && N >= 1, "bad sizes G=%d N=%d", G, N);
+  FGNN_CHECK_ARG(G >= 1 && N1 >= 1 && N2 >= 1, "bad sizes G=%d N1=%d N2=%d", G, N1, N2);
+  const int N = std::max(N1, N2);
   const size_t smem = smem_bytes(N);
   int dev = 0, optin = 0;
   FGNN_CUDA(cudaGetDevice(&dev));
@@ -213,10 +223,10 @@ int lap_fwd(const float* scores, int32_t* col_of_row, int32_t* correct, double* 
   FGNN_CUDA(cudaFuncGetAttributes(&fa, lap_kernel));
   const size_t limit = (size_t)optin > fa.sharedSizeBytes ? (size_t)optin - fa.sharedSizeBytes : 0;
   if (smem > limit)
-    return fail(FGNN_ERR_UNSUPPORTED, "linear assignment supports N <= %d on this device (%d bytes of shared memory per block; got %d)",
-                max_n(limit), optin, N);
+    return fail(FGNN_ERR_UNSUPPORTED, "linear assignment supports N <= %d, N = max(N1, N2), on this device (%d bytes of shared "
+                "memory per block; got N1=%d N2=%d)", max_n(limit), optin, N1, N2);
   FGNN_CUDA(cudaFuncSetAttribute(lap_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  lap_kernel<<<G, kThreads, smem, st>>>(scores, col_of_row, correct, total_cost, N, n_per_graph);
+  lap_kernel<<<G, kThreads, smem, st>>>(scores, col_of_row, correct, total_cost, N1, N2, n1, n2);
   FGNN_LAUNCHED();
   return FGNN_OK;
 }

@@ -1329,14 +1329,18 @@ tc_matmul_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
 // (coef p falls below fp16's normal range at coef = 1 / #rows).  One CTA per (pair, 128-row tile) walks the column
 // tiles for d E1, one per (pair, 128-column tile) walks the row tiles for d E2: every output is written once.
 // =============================================================================================
+// Graph 1 (rows i) has n_per_graph[g] <= N vertices, graph 2 (columns j) n2[g] <= N2; N2 == N, n2 == n_per_graph is the
+// square head.  Row i's target is column i: rows i >= n2[g] have none and add nothing to (sum CE, #correct).
 struct HeadArgs {
   const float* e1;       // (G,C,N)
-  const float* e2;
-  float* scores;         // (G,N,N) or null
+  const float* e2;       // (G,C,N2)
+  float* scores;         // (G,N,N2) or null
   float* partial;        // [G][MT][2] = (sum CE, #correct) of the row tile
   int G, C, N, MT;
   const int32_t* n_per_graph;
   float* row_lse;        // (G,N), kRowLse only: log sum_j exp(s_ij) of valid rows, 0 elsewhere
+  int N2;
+  const int32_t* n2;     // null: every graph 2 has N2 vertices
 };
 
 template <typename T, bool kRowLse>
@@ -1354,9 +1358,10 @@ __global__ void __launch_bounds__(160, 1) tc_head_kernel(const HeadArgs a) {
   float* red = reinterpret_cast<float*>(tmem_slot + 2);     // [4 warps][2]
   const int warp = uniform_warp_idx(), lane = threadIdx.x % 32;
   const int mt = blockIdx.x, b = blockIdx.y;
-  const int n = graph_n(a.n_per_graph, b, N);
+  const int N2 = a.N2;
+  const int n = graph_n(a.n_per_graph, b, N), n2 = graph_n(a.n2, b, N2);
   const float* e1 = a.e1 + (size_t)b * C * N;
-  const float* e2 = a.e2 + (size_t)b * C * N;
+  const float* e2 = a.e2 + (size_t)b * C * N2;
   const int i0 = mt * 128;
   const bool want_scores = a.scores != nullptr;
   if (i0 >= n && !want_scores) {                            // nothing valid in this row tile
@@ -1396,12 +1401,12 @@ __global__ void __launch_bounds__(160, 1) tc_head_kernel(const HeadArgs a) {
   float run_m = -INFINITY, run_l = 0.f, diag = 0.f, best = -INFINITY;
   int best_j = -1;
   uint32_t phase = 0;
-  const int ncol = want_scores ? N : n;
+  const int ncol = want_scores ? N2 : n2;
   for (int j0 = 0; j0 < ncol; j0 += 256) {
-    if (j0 < n) {
+    if (j0 < n2) {
       for (int idx = threadIdx.x; idx < C * 32; idx += blockDim.x) {    // B: columns j0 .. j0+255 of E2
         const int c = idx / 32, q = idx % 32;
-        put8(e2 + (size_t)c * N, j0 + q * 8, n, sBhi, sBlo, c, q * 8);
+        put8(e2 + (size_t)c * N2, j0 + q * 8, n2, sBhi, sBlo, c, q * 8);
       }
       fence_proxy_async_smem();
       tc_fence_before();
@@ -1424,21 +1429,21 @@ __global__ void __launch_bounds__(160, 1) tc_head_kernel(const HeadArgs a) {
       }
     }
     if (warp < 4) {
-      if (j0 < n) { mbar_wait(bar, phase); phase ^= 1u; tc_fence_after(); }
+      if (j0 < n2) { mbar_wait(bar, phase); phase ^= 1u; tc_fence_after(); }
       const uint32_t taddr = tmem_base + ((uint32_t)(warp * 32) << 16);
-      float* srow = want_scores && i < N ? a.scores + ((size_t)b * N + i) * N : nullptr;
+      float* srow = want_scores && i < N ? a.scores + ((size_t)b * N + i) * N2 : nullptr;
 #pragma unroll 1
       for (int c0 = 0; c0 < 256; c0 += 32) {
         if (j0 + c0 >= ncol) break;
         uint32_t v[32];
-        if (j0 < n) { tmem_ld32(taddr + (uint32_t)c0, v); tmem_wait_ld(); }
-        if (row_ok && j0 + c0 < n) {
+        if (j0 < n2) { tmem_ld32(taddr + (uint32_t)c0, v); tmem_wait_ld(); }
+        if (row_ok && j0 + c0 < n2) {
           float cmax = -INFINITY;
 #pragma unroll
           for (int u = 0; u < 32; ++u) {
             const int j = j0 + c0 + u;
             const float x = __uint_as_float(v[u]);
-            if (j < n) {
+            if (j < n2) {
               cmax = fmaxf(cmax, x);
               if (x > best) { best = x; best_j = j; }
               if (j == i) diag = x;
@@ -1448,7 +1453,7 @@ __global__ void __launch_bounds__(160, 1) tc_head_kernel(const HeadArgs a) {
           float acc = 0.f;
 #pragma unroll
           for (int u = 0; u < 32; ++u)
-            if (j0 + c0 + u < n) acc += __expf(__uint_as_float(v[u]) - m_new);
+            if (j0 + c0 + u < n2) acc += __expf(__uint_as_float(v[u]) - m_new);
           run_l = run_l * __expf(run_m - m_new) + acc;
           run_m = m_new;
         }
@@ -1456,7 +1461,7 @@ __global__ void __launch_bounds__(160, 1) tc_head_kernel(const HeadArgs a) {
 #pragma unroll
           for (int u = 0; u < 32; ++u) {
             const int j = j0 + c0 + u;
-            if (j < N) srow[j] = (row_ok && j < n) ? __uint_as_float(v[u]) : 0.f;
+            if (j < N2) srow[j] = (row_ok && j < n2) ? __uint_as_float(v[u]) : 0.f;
           }
         }
       }
@@ -1467,8 +1472,9 @@ __global__ void __launch_bounds__(160, 1) tc_head_kernel(const HeadArgs a) {
   if (warp < 4) {
     if constexpr (kRowLse)
       if (i < N) a.row_lse[(size_t)b * N + i] = row_ok ? run_m + logf(run_l) : 0.f;
-    float ce = row_ok ? (run_m + logf(run_l) - diag) : 0.f;
-    float ok = (row_ok && best_j == i) ? 1.f : 0.f;
+    const bool has_target = row_ok && i < n2;
+    float ce = has_target ? (run_m + logf(run_l) - diag) : 0.f;
+    float ok = (has_target && best_j == i) ? 1.f : 0.f;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
       ce += __shfl_xor_sync(0xffffffffu, ce, o);
@@ -1504,22 +1510,24 @@ __global__ void head_finalize_kernel(const float* __restrict__ partial, float* _
 //   as 16-bit (hi, lo) K-major tiles  ->  D (TMEM cols [128, 128 + C)) += P Y_t^T.
 // The y tile is stored MN-major (K = channel) for the first product; the same bytes are the K-major B operand
 // (K = position, N = channel) of the second.  The steps of one tile are serialised (commit / wait): the kernel is
-// bound by the exponentials of the epilogue, not by the MMAs.
+// bound by the exponentials of the epilogue, not by the MMAs.  Rows i >= n2 have no target (forward): their dS row is
+// zero, so the kRows CTA owns rows i < min(n1, n2) and the column CTA walks those rows only.
 struct HeadBwdArgs {
-  const float* x;        // (G,C,N): the side whose gradient this launch writes
-  const float* y;        // (G,C,N): the other side
-  const float* row_lse;  // (G,N)
+  const float* x;        // (G,C,Nx): the side whose gradient this launch writes
+  const float* y;        // (G,C,Ny): the other side
+  const float* row_lse;  // (G,N1), N1 = Nx (kRows) or Ny
   const float* coef;     // [G]
-  float* dx;             // (G,C,N)
-  int C, N;
-  const int32_t* n_per_graph;
+  float* dx;             // (G,C,Nx)
+  int C, Nx, Ny;
+  const int32_t* nx;     // sizes of x's graphs (null: Nx) ...
+  const int32_t* ny;     // ... and of y's (null: Ny)
 };
 
 template <typename T, bool kRows>
 __global__ void __launch_bounds__(160, 1) tc_head_bwd_kernel(const HeadBwdArgs a) {
   extern __shared__ uint8_t smem_head_bwd[];
   uint8_t* smem = smem_head_bwd + ((1024u - (smem_u32(smem_head_bwd) & 1023u)) & 1023u);
-  const int C = a.C, N = a.N;
+  const int C = a.C, Nx = a.Nx, Ny = a.Ny;
   const uint32_t xy_bytes = (uint32_t)C * 256u;             // 128 positions x C x 2 bytes
   uint8_t* sXhi = smem;
   uint8_t* sXlo = sXhi + xy_bytes;
@@ -1532,25 +1540,28 @@ __global__ void __launch_bounds__(160, 1) tc_head_bwd_kernel(const HeadBwdArgs a
   float* s_lse = reinterpret_cast<float*>(tmem_slot + 2);   // [128] lse of the walked rows (!kRows)
   const int warp = uniform_warp_idx(), lane = threadIdx.x % 32;
   const int t0 = blockIdx.x * 128, b = blockIdx.y;
-  const int n = graph_n(a.n_per_graph, b, N);
-  const float* xg = a.x + (size_t)b * C * N;
-  const float* yg = a.y + (size_t)b * C * N;
-  float* dxg = a.dx + (size_t)b * C * N;
-  if (t0 >= n) {                                            // no valid position: exact zeros
+  const int nx = graph_n(a.nx, b, Nx), ny = graph_n(a.ny, b, Ny);
+  const int n_own = kRows ? min(nx, ny) : nx;               // owned positions with a nonzero gradient
+  const int n_walk = kRows ? ny : min(nx, ny);              // walked positions with a nonzero dS
+  const int N1 = kRows ? Nx : Ny;                           // pitch of row_lse
+  const float* xg = a.x + (size_t)b * C * Nx;
+  const float* yg = a.y + (size_t)b * C * Ny;
+  float* dxg = a.dx + (size_t)b * C * Nx;
+  if (t0 >= n_own || n_walk == 0) {                         // no valid position: exact zeros
     for (int idx = threadIdx.x; idx < C * 128; idx += blockDim.x) {
       const int c = idx / 128, p = t0 + idx % 128;
-      if (p < N) dxg[(size_t)c * N + p] = 0.f;
+      if (p < Nx) dxg[(size_t)c * Nx + p] = 0.f;
     }
     return;
   }
   if (threadIdx.x == 0) { mbar_init(&bar[0], 1); mbar_init(&bar[1], 1); fence_barrier_init(); }
   if (warp == 4) tmem_alloc(tmem_slot, 256);
-  auto put8 = [&](const float* src_row, int first, uint8_t* hi_tile, uint8_t* lo_tile, int c, int pos) {
+  auto put8 = [&](const float* src_row, int first, int limit, uint8_t* hi_tile, uint8_t* lo_tile, int c, int pos) {
     uint32_t hw[4], lw[4];
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
       const int x0 = first + 2 * u, x1 = x0 + 1;
-      const float v0 = x0 < n ? src_row[x0] : 0.f, v1 = x1 < n ? src_row[x1] : 0.f;
+      const float v0 = x0 < limit ? src_row[x0] : 0.f, v1 = x1 < limit ? src_row[x1] : 0.f;
       const float h0 = Elem<T>::to_float(Elem<T>::from_float(v0)), h1 = Elem<T>::to_float(Elem<T>::from_float(v1));
       hw[u] = Elem<T>::pack(v0, v1);
       lw[u] = Elem<T>::pack(v0 - h0, v1 - h1);
@@ -1561,7 +1572,7 @@ __global__ void __launch_bounds__(160, 1) tc_head_bwd_kernel(const HeadBwdArgs a
   };
   for (int idx = threadIdx.x; idx < C * 16; idx += blockDim.x) {
     const int c = idx / 16, q = idx % 16;
-    put8(xg + (size_t)c * N, t0 + q * 8, sXhi, sXlo, c, q * 8);
+    put8(xg + (size_t)c * Nx, t0 + q * 8, n_own, sXhi, sXlo, c, q * 8);
   }
   tc_fence_before();
   __syncthreads();
@@ -1569,16 +1580,16 @@ __global__ void __launch_bounds__(160, 1) tc_head_bwd_kernel(const HeadBwdArgs a
   const uint32_t tmem_base = *tmem_slot;
   const int r = warp * 32 + lane;                           // row of the CTA's tile (epilogue warps)
   const int p_own = t0 + r;                                 // its position: i (kRows) or j
-  const bool own_ok = warp < 4 && p_own < n;
-  const float lse_own = (kRows && own_ok) ? a.row_lse[(size_t)b * N + p_own] : 0.f;
+  const bool own_ok = warp < 4 && p_own < n_own;
+  const float lse_own = (kRows && own_ok) ? a.row_lse[(size_t)b * N1 + p_own] : 0.f;
   uint32_t phase = 0;
-  for (int w0 = 0; w0 < n; w0 += 128) {
+  for (int w0 = 0; w0 < n_walk; w0 += 128) {
     if (w0 > 0) { mbar_wait(&bar[1], phase ^ 1u); tc_fence_after(); }   // previous P Y^T has read sY and sP
     for (int idx = threadIdx.x; idx < C * 16; idx += blockDim.x) {
       const int c = idx / 16, q = idx % 16;
-      put8(yg + (size_t)c * N, w0 + q * 8, sYhi, sYlo, c, q * 8);
+      put8(yg + (size_t)c * Ny, w0 + q * 8, n_walk, sYhi, sYlo, c, q * 8);
     }
-    if (!kRows && threadIdx.x < 128) s_lse[threadIdx.x] = w0 + (int)threadIdx.x < n ? a.row_lse[(size_t)b * N + w0 + threadIdx.x] : 0.f;
+    if (!kRows && threadIdx.x < 128) s_lse[threadIdx.x] = w0 + (int)threadIdx.x < n_walk ? a.row_lse[(size_t)b * N1 + w0 + threadIdx.x] : 0.f;
     fence_proxy_async_smem();
     tc_fence_before();
     __syncthreads();
@@ -1612,7 +1623,7 @@ __global__ void __launch_bounds__(160, 1) tc_head_bwd_kernel(const HeadBwdArgs a
         for (int u = 0; u < 32; ++u) {
           const int q = w0 + c0 + u;                        // the walked position: j (kRows) or i
           const float lse = kRows ? lse_own : s_lse[c0 + u];
-          pv[u] = (own_ok && q < n) ? __expf(__uint_as_float(v[u]) - lse) - (q == p_own ? 1.f : 0.f) : 0.f;
+          pv[u] = (own_ok && q < n_walk) ? __expf(__uint_as_float(v[u]) - lse) - (q == p_own ? 1.f : 0.f) : 0.f;
         }
 #pragma unroll
         for (int s8 = 0; s8 < 4; ++s8) {
@@ -1663,9 +1674,9 @@ __global__ void __launch_bounds__(160, 1) tc_head_bwd_kernel(const HeadBwdArgs a
       uint32_t v[16];
       tmem_ld16(taddr + (uint32_t)c0, v);
       tmem_wait_ld();
-      if (p_own < N) {
+      if (p_own < Nx) {
 #pragma unroll
-        for (int u = 0; u < 16; ++u) dxg[(size_t)(c0 + u) * N + p_own] = own_ok ? cf * __uint_as_float(v[u]) : 0.f;
+        for (int u = 0; u < 16; ++u) dxg[(size_t)(c0 + u) * Nx + p_own] = own_ok ? cf * __uint_as_float(v[u]) : 0.f;
       }
     }
     tc_fence_before();
@@ -2235,13 +2246,14 @@ size_t head_workspace_bytes(int G, int N) { return align_up((size_t)G * ((N + 12
 
 template <typename T, bool kRowLse>
 int head_fwd_t(const float* e1, const float* e2, float* scores, float* ce_sum, int32_t* correct, float* row_lse, int G, int C,
-               int N, const int32_t* npg, void* ws, cudaStream_t st) {
+               int N1, int N2, const int32_t* n1, const int32_t* n2, void* ws, cudaStream_t st) {
   HeadArgs a{};
   a.e1 = e1; a.e2 = e2; a.scores = scores;
   a.partial = static_cast<float*>(ws);
-  a.G = G; a.C = C; a.N = N; a.MT = (N + 127) / 128;
-  a.n_per_graph = npg;
+  a.G = G; a.C = C; a.N = N1; a.MT = (N1 + 127) / 128;
+  a.n_per_graph = n1;
   a.row_lse = row_lse;
+  a.N2 = N2; a.n2 = n2;
   const size_t smem = 1024 + (size_t)C * 256 * 2 + (size_t)C * 512 * 2 + 128;
   FGNN_CUDA(cudaFuncSetAttribute(tc_head_kernel<T, kRowLse>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   prof::begin(prof::kGlue, st);
@@ -2254,47 +2266,46 @@ int head_fwd_t(const float* e1, const float* e2, float* scores, float* ce_sum, i
 }
 
 // the shapes every fused-head entry point accepts
-int check_head_shape(int G, int C, int N) {
-  FGNN_CHECK_ARG(G >= 1 && G <= 65535 && N >= 1 && N <= kMaxN, "fused head supports G <= 65535 and N <= %d (got G=%d N=%d)",
-                 kMaxN, G, N);
+int check_head_shape(int G, int C, int N1, int N2) {
+  FGNN_CHECK_ARG(G >= 1 && G <= 65535 && N1 >= 1 && N1 <= kMaxN && N2 >= 1 && N2 <= kMaxN,
+                 "fused head supports G <= 65535 and N1, N2 <= %d (got G=%d N1=%d N2=%d)", kMaxN, G, N1, N2);
   FGNN_CHECK_ARG(C >= 16 && C <= 128 && C % 16 == 0, "the fused head needs an embedding width that is a multiple of 16, at most 128 (got %d)", C);
   return FGNN_OK;
 }
 
 int head_fwd(int precision, const float* e1, const float* e2, float* scores, float* ce_sum, int32_t* correct, int G, int C,
-             int N, const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
-  return with_16bit(precision, "fgnn_head_fwd", [&](auto t) -> int {
+             int N1, int N2, const int32_t* n1, const int32_t* n2, void* ws, size_t ws_bytes, cudaStream_t st) {
+  return with_16bit(precision, "fgnn_head_pair_fwd", [&](auto t) -> int {
     FGNN_CHECK_ARG(e1 && e2 && ce_sum && correct && ws, "null pointer");
-    if (int e = check_head_shape(G, C, N)) return e;
-    if (ws_bytes < head_workspace_bytes(G, N)) return fail(FGNN_ERR_WORKSPACE, "head workspace too small");
-    return head_fwd_t<decltype(t), false>(e1, e2, scores, ce_sum, correct, nullptr, G, C, N, n_per_graph, ws, st);
+    if (int e = check_head_shape(G, C, N1, N2)) return e;
+    if (ws_bytes < head_workspace_bytes(G, N1)) return fail(FGNN_ERR_WORKSPACE, "head workspace too small");
+    return head_fwd_t<decltype(t), false>(e1, e2, scores, ce_sum, correct, nullptr, G, C, N1, N2, n1, n2, ws, st);
   });
 }
 
 int head_fwd_train(int precision, const float* e1, const float* e2, float* ce_sum, int32_t* correct, float* row_lse, int G,
-                   int C, int N, const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
-  return with_16bit(precision, "fgnn_head_fwd_train", [&](auto t) -> int {
+                   int C, int N1, int N2, const int32_t* n1, const int32_t* n2, void* ws, size_t ws_bytes, cudaStream_t st) {
+  return with_16bit(precision, "fgnn_head_pair_fwd_train", [&](auto t) -> int {
     FGNN_CHECK_ARG(e1 && e2 && ce_sum && correct && row_lse && ws, "null pointer");
-    if (int e = check_head_shape(G, C, N)) return e;
-    if (ws_bytes < head_workspace_bytes(G, N)) return fail(FGNN_ERR_WORKSPACE, "head workspace too small");
-    return head_fwd_t<decltype(t), true>(e1, e2, nullptr, ce_sum, correct, row_lse, G, C, N, n_per_graph, ws, st);
+    if (int e = check_head_shape(G, C, N1, N2)) return e;
+    if (ws_bytes < head_workspace_bytes(G, N1)) return fail(FGNN_ERR_WORKSPACE, "head workspace too small");
+    return head_fwd_t<decltype(t), true>(e1, e2, nullptr, ce_sum, correct, row_lse, G, C, N1, N2, n1, n2, ws, st);
   });
 }
 
 int head_bwd(int precision, const float* e1, const float* e2, const float* row_lse, const float* coef, float* de1, float* de2,
-             int G, int C, int N, const int32_t* n_per_graph, cudaStream_t st) {
-  return with_16bit(precision, "fgnn_head_bwd", [&](auto t) -> int {
+             int G, int C, int N1, int N2, const int32_t* n1, const int32_t* n2, cudaStream_t st) {
+  return with_16bit(precision, "fgnn_head_pair_bwd", [&](auto t) -> int {
     using T = decltype(t);
     FGNN_CHECK_ARG(e1 && e2 && row_lse && coef && de1 && de2, "null pointer");
-    if (int e = check_head_shape(G, C, N)) return e;
+    if (int e = check_head_shape(G, C, N1, N2)) return e;
     const size_t smem = 1024 + (size_t)C * 256 * 4 + 2 * 32768 + 16 + 8 + 128 * sizeof(float);
-    const dim3 grid((N + 127) / 128, G);
     prof::begin(prof::kGlue, st);
     FGNN_CUDA(cudaFuncSetAttribute(tc_head_bwd_kernel<T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    tc_head_bwd_kernel<T, true><<<grid, 160, smem, st>>>(HeadBwdArgs{e1, e2, row_lse, coef, de1, C, N, n_per_graph});
+    tc_head_bwd_kernel<T, true><<<dim3((N1 + 127) / 128, G), 160, smem, st>>>(HeadBwdArgs{e1, e2, row_lse, coef, de1, C, N1, N2, n1, n2});
     FGNN_LAUNCHED();
     FGNN_CUDA(cudaFuncSetAttribute(tc_head_bwd_kernel<T, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    tc_head_bwd_kernel<T, false><<<grid, 160, smem, st>>>(HeadBwdArgs{e2, e1, row_lse, coef, de2, C, N, n_per_graph});
+    tc_head_bwd_kernel<T, false><<<dim3((N2 + 127) / 128, G), 160, smem, st>>>(HeadBwdArgs{e2, e1, row_lse, coef, de2, C, N2, N1, n2, n1});
     prof::end(prof::kGlue, st);
     FGNN_LAUNCHED();
     return FGNN_OK;

@@ -81,6 +81,8 @@ class MaskedTensor:
         self.device = self.tensor.device
         self._sizes_cache = None
         self._sizes_dev = None        # int32 device copy of the sizes, uploaded once per batch
+        self._dim_sizes = {}          # per-dim sizes_host(name) / sizes_i32(name=name)
+        self._dim_sizes_dev = {}
         if adjust_mask:
             self._adjust_mask_()
         if apply_mask:
@@ -107,23 +109,41 @@ class MaskedTensor:
     def mask(self):
         return MaskedTensor(self.tensor, self.mask_dict, adjust_mask=False, apply_mask=True, copy=True)
 
-    def sizes_host(self) -> List[int]:
-        """True size of each graph (all masked dims of one graph share it for from_list data)."""
+    @staticmethod
+    def _prefix_sizes(m: torch.Tensor) -> torch.Tensor:
+        """(B, size) mask -> int64 sizes; the CUDA operators address padding by size: masks must be prefix masks."""
+        m = m.rename(None)
+        sz = m.sum(dim=1).round().to(torch.int64)
+        pref = (torch.arange(m.shape[1], device=m.device)[None, :] < sz[:, None]).to(m.dtype)
+        if not torch.equal(pref, m):
+            raise ValueError("fgnn_b200 supports prefix masks only (as built by from_list)")
+        return sz
+
+    def sizes_host(self, name: Optional[str] = None) -> List[int]:
+        """True size of each graph along the masked dim `name`.  Without a name: the one size all masked dims of a graph
+        share (from_list data); scores of graphs of unequal sizes have one size per dim, ask for each by name."""
+        if name is not None:
+            if name not in self._dim_sizes:
+                if name not in self.mask_dict:
+                    raise KeyError(f"no mask for dim {name!r} (masked dims: {list(self.mask_dict)})")
+                self._dim_sizes[name] = [int(v) for v in self._prefix_sizes(self.mask_dict[name]).tolist()]
+            return self._dim_sizes[name]
         if self._sizes_cache is None:
-            m = next(iter(self.mask_dict.values())).rename(None)
-            sz = m.sum(dim=1).round().to(torch.int64)
-            # the CUDA operators address padding by size: masks must be prefix masks
-            pref = (torch.arange(m.shape[1], device=m.device)[None, :] < sz[:, None]).to(m.dtype)
-            if not torch.equal(pref, m):
-                raise ValueError("fgnn_b200 supports prefix masks only (as built by from_list)")
+            sz = self._prefix_sizes(next(iter(self.mask_dict.values())))
             for other in self.mask_dict.values():
                 if not torch.equal(other.rename(None).sum(dim=1).round().to(torch.int64), sz):
                     raise ValueError("all masked dims of a graph must have the same size")
             self._sizes_cache = [int(v) for v in sz.tolist()]
         return self._sizes_cache
 
-    def sizes_i32(self, device=None) -> torch.Tensor:
+    def sizes_i32(self, device=None, name: Optional[str] = None) -> torch.Tensor:
+        """sizes_host(name) as an int32 tensor on `device` (default: the data's), uploaded once."""
         dev = torch.device(self.device if device is None else device)
+        if name is not None:
+            t = self._dim_sizes_dev.get(name)
+            if t is None or t.device != dev:
+                t = self._dim_sizes_dev[name] = torch.tensor(self.sizes_host(name), dtype=torch.int32, device=dev)
+            return t
         if self._sizes_dev is None or self._sizes_dev.device != dev:
             self._sizes_dev = torch.tensor(self.sizes_host(), dtype=torch.int32, device=dev)
         return self._sizes_dev

@@ -8,7 +8,7 @@ import torch
 import torch.nn as nn
 
 from .. import _ops
-from ..toolbox.losses import triplet_loss, _as_batch
+from ..toolbox.losses import triplet_loss, _as_batch, check_loss_sizes
 from ..toolbox.metrics import accuracy_max, accuracy_linear_assignment
 from ..maskedtensors.maskedtensor import MaskedTensor
 from .blocks_emb import node_embedding, block_emb, block
@@ -31,6 +31,17 @@ def _lookup(table, key, what):
     if key not in table:
         raise NotImplementedError(f"{what} {key} is not implemented")
     return table[key]
+
+
+def _head_sizes(e1, e2):
+    """Embeddings of both sides -> (graph 1's sizes, graph 2's sizes (int32 device tensors or None), float sizes of
+    graph 1 (B,)), after refusing pairs the identity loss is not defined on (n1 > n2)."""
+    if isinstance(e1, MaskedTensor):
+        check_loss_sizes(e1.sizes_host(), e2.sizes_host())
+        n_dev = e1.sizes_i32()
+        return n_dev, e2.sizes_i32(), n_dev.to(torch.float32)
+    check_loss_sizes([e1.shape[-1]], [e2.shape[-1]])
+    return None, None, torch.full((e1.shape[0],), float(e1.shape[-1]), device=e1.device)
 
 
 class Siamese_Node_Exp(_Base):
@@ -68,58 +79,69 @@ class Siamese_Node_Exp(_Base):
         return self.node_embedder(x)['ne/suffix']
 
     def forward(self, x1, x2):
+        """Graph 1 padded to N1, graph 2 to N2 (the two may differ) -> (B,N1,N2) scores, zero outside each pair's n1 x n2
+        block; for MaskedTensor inputs the rows carry graph 1's mask and the columns graph 2's."""
         e1 = self.embed(x1)
         e2 = self.embed(x2)
-        # inference in a 16-bit mode: E1^T E2 on tensor cores (fgnn_head_fwd with the scores requested)
+        # inference in a 16-bit mode: E1^T E2 on tensor cores (fgnn_head_pair_fwd with the scores requested)
         fused = (not torch.is_grad_enabled()) and self.precision != "fp32"
         if isinstance(e1, MaskedTensor):
-            # both sides must describe the same graphs sizes; the result is masked on (N, N_)
-            n_dev = e1.sizes_i32()
+            n_dev, n2_dev = e1.sizes_i32(), e2.sizes_i32()
+            t1, t2 = e1.tensor.rename(None), e2.tensor.rename(None)
             if fused:
-                s = _ops.head_fused(e1.tensor.rename(None), e2.tensor.rename(None), n_dev, self.precision, want_scores=True)[2]
+                s = _ops.head_fused(t1, t2, n_dev, self.precision, want_scores=True, n2_dev=n2_dev)[2]
             else:
-                s = _ops.ScoresFunction.apply(e1.tensor.rename(None), e2.tensor.rename(None), n_dev)
+                s = _ops.ScoresFunction.apply(t1, t2, n_dev, n2_dev)
             bname, nname = e1.tensor.names[0], e1.tensor.names[2]
-            m = e1.mask_dict[nname]
-            masks = {nname: m, nname + '_': m.rename(None).rename(bname, nname + '_')}
-            return MaskedTensor(s.rename(bname, nname, nname + '_'), masks, adjust_mask=False, apply_mask=False)
+            masks = {nname: e1.mask_dict[nname],
+                     nname + '_': e2.mask_dict[e2.tensor.names[2]].rename(None).rename(bname, nname + '_')}
+            out = MaskedTensor(s.rename(bname, nname, nname + '_'), masks, adjust_mask=False, apply_mask=False)
+            # the embedders validated and uploaded both sides' sizes already
+            out._dim_sizes = {nname: e1.sizes_host(), nname + '_': e2.sizes_host()}
+            out._dim_sizes_dev = {nname: n_dev, nname + '_': n2_dev}
+            return out
         if fused:
             return _ops.head_fused(e1, e2, None, self.precision, want_scores=True)[2]
         return _ops.ScoresFunction.apply(e1, e2, None)
 
     @torch.no_grad()
     def loss_and_accuracy(self, x1, x2):
-        """Inference step without materialising the (B,N,N) scores: both embedders, then the fused tensor-core head
+        """Inference step without materialising the (B,N1,N2) scores: both embedders, then the fused tensor-core head
         (E1^T E2, row softmax cross-entropy against the identity matching, row argmax; models/trainers.py:67 +
         toolbox/losses.py:27-34 + toolbox/metrics.py:118-141 in one pass).  Returns device tensors
-        (loss 'mean' = sum CE / sum n, #correct rows, #rows).  16-bit precisions; fp32 goes through forward()."""
+        (loss 'mean' = sum CE / sum n1, #correct rows, #rows = sum n1).  Graph 2's sizes come from x2; every pair needs
+        n1 <= n2.  16-bit precisions; fp32 goes through forward()."""
         if self.precision == "fp32":
             scores = self(x1, x2)
-            plain, n_dev, sizes = _as_batch(scores)
-            ce, correct = _ops.CrossEntropyIdentityFunction.apply(plain, n_dev)
+            plain, n_dev, n2_dev, sizes = _as_batch(scores, loss=True)
+            ce, correct = _ops.CrossEntropyIdentityFunction.apply(plain, n_dev, n2_dev)
         else:
             e1, e2 = self.embed(x1), self.embed(x2)
-            n_dev, sizes = None, None
+            n_dev, n2_dev, sizes = _head_sizes(e1, e2)
             if isinstance(e1, MaskedTensor):
-                n_dev, sizes = e1.sizes_i32(), e1.sizes_i32().to(torch.float32)
                 e1, e2 = e1.tensor.rename(None), e2.tensor.rename(None)
-            else:
-                sizes = torch.full((e1.shape[0],), float(e1.shape[-1]), device=e1.device)
-            ce, correct, _ = _ops.head_fused(e1, e2, n_dev, self.precision)
+            ce, correct, _ = _ops.head_fused(e1, e2, n_dev, self.precision, n2_dev=n2_dev)
         rows = sizes.sum()
         return ce.sum() / rows, correct.sum(), rows
 
     @torch.no_grad()
-    def loss_and_accuracy_from_adjacency(self, adj1, adj2, sizes=None):
-        """loss_and_accuracy fed from two CUDA (B,N,N) uint8 / bool adjacency batches (`sizes`: optional CUDA int32 vertex counts
-        of a padded ragged batch): the reference's input construction (loaders/data_generator.py:118-125) happens on the device,
-        so a step ships 1 byte per matrix entry instead of the 8 bytes of the (B,2,N,N) fp32 features.  16-bit precisions."""
+    def loss_and_accuracy_from_adjacency(self, adj1, adj2, sizes=None, sizes2=None):
+        """loss_and_accuracy fed from two CUDA (B,N1,N1) and (B,N2,N2) uint8 / bool adjacency batches (`sizes`, `sizes2`:
+        optional CUDA int32 vertex counts of graph 1 and graph 2 in a padded ragged batch; `sizes2` defaults to `sizes`):
+        the reference's input construction (loaders/data_generator.py:118-125) happens on the device, so a step ships
+        1 byte per matrix entry instead of the 8 bytes of the (B,2,N,N) fp32 features.  16-bit precisions."""
         if self.precision == "fp32":
             raise _ops.L.FgnnError("loss_and_accuracy_from_adjacency needs precision 'fp16' or 'bf16'")
+        sizes2 = sizes if sizes2 is None else sizes2
         e1 = self.node_embedder.forward_fused_adjacency(adj1, sizes=sizes)
-        e2 = self.node_embedder.forward_fused_adjacency(adj2, sizes=sizes)
-        ce, correct, _ = _ops.head_fused(e1, e2, sizes, self.precision)
-        rows = sizes.sum().to(torch.float32) if sizes is not None else torch.tensor(float(e1.shape[0] * e1.shape[-1]), device=e1.device)
+        e2 = self.node_embedder.forward_fused_adjacency(adj2, sizes=sizes2)
+        B, N1, N2 = e1.shape[0], e1.shape[-1], e2.shape[-1]
+        if sizes2 is not sizes or N1 != N2:
+            n1 = sizes.tolist() if sizes is not None else [N1] * B
+            n2 = sizes2.tolist() if sizes2 is not None else [N2] * B
+            check_loss_sizes(n1, n2)
+        ce, correct, _ = _ops.head_fused(e1, e2, sizes, self.precision, n2_dev=sizes2)
+        rows = sizes.sum().to(torch.float32) if sizes is not None else torch.tensor(float(B * N1), device=e1.device)
         return ce.sum() / rows, correct.sum(), rows
 
     def _step(self, batch, tag):

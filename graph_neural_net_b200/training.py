@@ -121,6 +121,7 @@ def train_step_flat(model, opt: "FlatAdam", x1, x2, group: Optional[dist.Process
     from . import _ops
     from .maskedtensors.maskedtensor import MaskedTensor
     from .toolbox.losses import _as_batch
+    from .models.trainers import _head_sizes
 
     if fused_head and getattr(model, "precision", "fp32") == "fp32":
         raise _ops.L.FgnnError("fused_head is the tensor-core head of the 16-bit precisions; fp32 trains through the "
@@ -129,18 +130,14 @@ def train_step_flat(model, opt: "FlatAdam", x1, x2, group: Optional[dist.Process
     try:
         if fused_head:
             e1, e2 = model.embed(x1), model.embed(x2)
+            n_dev, n2_dev, sizes = _head_sizes(e1, e2)
             if isinstance(e1, MaskedTensor):
-                n_dev = e1.sizes_i32()
-                sizes = n_dev.to(torch.float32)
                 e1, e2 = e1.tensor.rename(None), e2.tensor.rename(None)
-            else:
-                n_dev = None
-                sizes = torch.full((e1.shape[0],), float(e1.shape[-1]), device=e1.device)
-            ce, correct = _ops.HeadFunction.apply(e1, e2, n_dev, model.precision)
+            ce, correct = _ops.HeadFunction.apply(e1, e2, n_dev, model.precision, n2_dev)
         else:
             scores = model(x1, x2)
-            plain, n_dev, sizes = _as_batch(scores)
-            ce, correct = _ops.CrossEntropyIdentityFunction.apply(plain, n_dev)
+            plain, n_dev, n2_dev, sizes = _as_batch(scores, loss=True)
+            ce, correct = _ops.CrossEntropyIdentityFunction.apply(plain, n_dev, n2_dev)
         local_sum = ce.sum()
         local_sum.backward()                                   # gradients land in opt.flat_g (in place)
     finally:
@@ -181,8 +178,8 @@ def train_step(model, optimizer, x1, x2, group: Optional[dist.ProcessGroup] = No
 
     optimizer.zero_grad(set_to_none=True)
     scores = model(x1, x2)
-    plain, n_dev, sizes = _as_batch(scores)
-    ce, correct = _ops.CrossEntropyIdentityFunction.apply(plain, n_dev)
+    plain, n_dev, n2_dev, sizes = _as_batch(scores, loss=True)
+    ce, correct = _ops.CrossEntropyIdentityFunction.apply(plain, n_dev, n2_dev)
     local_sum = ce.sum()
     local_sum.backward()                                   # un-normalised: d(sum CE_local)/d theta
     extras = torch.stack((local_sum.detach(), sizes.sum(), correct.sum().to(torch.float32)))

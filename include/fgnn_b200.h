@@ -14,6 +14,12 @@
  *   - n_per_graph: int32[G] true vertex counts (prefix masks of maskedtensor.from_list,
  *     maskedtensors/maskedtensor.py:40-46), or NULL when every graph has exactly N vertices;
  *     padded positions of every output are written as exact zeros (maskedtensor.py:87-90);
+ *   - graph pairs of unequal sizes: the *_pair_* entry points take graph 1 (rows i) padded to N1 with sizes n1 and
+ *     graph 2 (columns j) padded to N2 with sizes n2 (either NULL when every graph has its padded size): e1 (G,C,N1),
+ *     e2 (G,C,N2), scores (G,N1,N2), zero outside the n1 x n2 block.  The loss keeps the reference's ground truth,
+ *     row i <-> column i: rows i >= n2[g] carry no target and add nothing to ce_sum, correct or the gradient (the
+ *     loss is meant for n1 <= n2, where CrossEntropyLoss(out, arange(n1)) is defined).  Each square entry point is
+ *     its pair form with N1 = N2 = N and n1 = n2 = n_per_graph;
  *   - stream: a cudaStream_t passed as void*; all work is enqueued there, no hidden syncs;
  *   - the library never allocates device memory: callers size scratch with the *_workspace_bytes
  *     query and own every buffer;
@@ -162,6 +168,11 @@ int fgnn_scores_fwd_f32(const float* e1, const float* e2, float* scores, int32_t
 int fgnn_scores_bwd_f32(const float* e1, const float* e2, const float* dscores, float* de1,
                         float* de2, int32_t G, int32_t C, int32_t N, const int32_t* n_per_graph,
                         void* stream);
+/* Pair forms: e1 (G,C,N1), e2 (G,C,N2) -> scores (G,N1,N2); de1 (G,C,N1), de2 (G,C,N2). */
+int fgnn_scores_pair_fwd_f32(const float* e1, const float* e2, float* scores, int32_t G, int32_t C, int32_t N1,
+                             int32_t N2, const int32_t* n1, const int32_t* n2, void* stream);
+int fgnn_scores_pair_bwd_f32(const float* e1, const float* e2, const float* dscores, float* de1, float* de2, int32_t G,
+                             int32_t C, int32_t N1, int32_t N2, const int32_t* n1, const int32_t* n2, void* stream);
 
 /* Row-softmax cross-entropy against the identity matching + row argmax, one pass
  * (toolbox/losses.py:20-34 and toolbox/metrics.py:118-141 without the per-graph host loop).
@@ -176,6 +187,14 @@ int fgnn_ce_argmax_fwd_f32(const float* scores, float* ce_sum, int32_t* correct,
  * reduction and the upstream gradient. */
 int fgnn_ce_bwd_f32(const float* scores, const float* row_lse, const float* coef, float* dscores,
                     int32_t G, int32_t N, const int32_t* n_per_graph, void* stream);
+/* Pair forms: scores (G,N1,N2), the softmax of row i over its n2[g] valid columns; row_lse (G,N1); workspace:
+ * fgnn_ce_workspace_bytes(G, N1).  row_argmax (G,N1) int32 may be NULL: the arg-max column of every row i < n1[g]
+ * (ties: the lowest column), -1 on padded rows. */
+int fgnn_ce_pair_argmax_fwd_f32(const float* scores, float* ce_sum, int32_t* correct, float* row_lse, int32_t* row_argmax,
+                                int32_t G, int32_t N1, int32_t N2, const int32_t* n1, const int32_t* n2, void* workspace,
+                                size_t workspace_bytes, void* stream);
+int fgnn_ce_pair_bwd_f32(const float* scores, const float* row_lse, const float* coef, float* dscores, int32_t G,
+                         int32_t N1, int32_t N2, const int32_t* n1, const int32_t* n2, void* stream);
 
 /* Fused siamese head on tensor cores (FGNN_BF16 / FGNN_FP16): scores = e1^T e2 (models/trainers.py:67) with the
  * row-softmax cross-entropy against the identity matching (toolbox/losses.py:27-33) and the row argmax
@@ -205,6 +224,19 @@ int fgnn_head_fwd_train(int32_t precision, const float* e1, const float* e2, flo
 int fgnn_head_bwd(int32_t precision, const float* e1, const float* e2, const float* row_lse, const float* coef, float* de1,
                   float* de2, int32_t G, int32_t C, int32_t N, const int32_t* n_per_graph, void* workspace,
                   size_t workspace_bytes, void* stream);
+/* Pair forms of the fused head: e1 (G,C,N1), e2 (G,C,N2), scores (G,N1,N2), row_lse (G,N1), de1 (G,C,N1), de2 (G,C,N2);
+ * N1, N2 <= 4096.  The workspace depends on N1 only: fgnn_head_pair_workspace_bytes(G, N1) ==
+ * fgnn_head_workspace_bytes(G, N1). */
+size_t fgnn_head_pair_workspace_bytes(int32_t G, int32_t N1);
+int fgnn_head_pair_fwd(int32_t precision, const float* e1, const float* e2, float* scores, float* ce_sum, int32_t* correct,
+                       int32_t G, int32_t C, int32_t N1, int32_t N2, const int32_t* n1, const int32_t* n2, void* workspace,
+                       size_t workspace_bytes, void* stream);
+int fgnn_head_pair_fwd_train(int32_t precision, const float* e1, const float* e2, float* ce_sum, int32_t* correct,
+                             float* row_lse, int32_t G, int32_t C, int32_t N1, int32_t N2, const int32_t* n1,
+                             const int32_t* n2, void* workspace, size_t workspace_bytes, void* stream);
+int fgnn_head_pair_bwd(int32_t precision, const float* e1, const float* e2, const float* row_lse, const float* coef,
+                       float* de1, float* de2, int32_t G, int32_t C, int32_t N1, int32_t N2, const int32_t* n1,
+                       const int32_t* n2, void* workspace, size_t workspace_bytes, void* stream);
 
 /* accuracy_linear_assignment (toolbox/metrics.py:92-116), the metric training_step / validation_step call
  * (models/trainers.py:53,74): per graph the assignment scipy.optimize.linear_sum_assignment returns on
@@ -216,6 +248,11 @@ int fgnn_head_bwd(int32_t precision, const float* e1, const float* e2, const flo
  * with FGNN_ERR_UNSUPPORTED and states the limit. */
 int fgnn_lap_fwd(const float* scores, int32_t* col_of_row, int32_t* correct, double* total_cost, int32_t G,
                  int32_t N, const int32_t* n_per_graph, void* stream);
+/* Rectangular form, as scipy's rectangular_lsap: scores (G,N1,N2), cost = -log_softmax over each row's n2[g] valid
+ * columns; min(n1, n2) pairs are matched (the problem is solved transposed when n1 > n2).  col_of_row (G,N1): -1 on
+ * padded rows and on rows left without a column.  The shared-memory limit above applies to max(N1, N2). */
+int fgnn_lap_pair_fwd(const float* scores, int32_t* col_of_row, int32_t* correct, double* total_cost, int32_t G,
+                      int32_t N1, int32_t N2, const int32_t* n1, const int32_t* n2, void* stream);
 
 /* ---- fused embedder (the hot path proper) ------------------------------------------------ */
 
