@@ -20,6 +20,7 @@ FGNN_MAX_DEPTH = 8
 FGNN_MAX_BLOCKS = 16
 FP32, BF16, FP16 = 0, 1, 2
 PRECISIONS = {"fp32": FP32, "bf16": BF16, "fp16": FP16}
+FGNN_DETERMINISTIC = 0x100   # ORed into `precision` / passed as `flags`: fixed-order sums instead of atomics
 
 c_float_p = C.POINTER(C.c_float)
 
@@ -69,6 +70,9 @@ _SIGNATURES = {
     "fgnn_mlp_fwd_f32": (C.c_int, [C.POINTER(MlpParams), _vp, _vp, _vp, _i32, _i32, _vp, _vp, _sz, _vp]),
     "fgnn_mlp_bwd_f32": (C.c_int, [C.POINTER(MlpParams), C.POINTER(MlpGrads), _vp, _vp, _vp, _vp, _i32, _i32,
                                    _vp, _vp, _sz, _vp]),
+    "fgnn_mlp_workspace_bytes_ex": (_sz, [_i32] * 6),
+    "fgnn_mlp_bwd_f32_ex": (C.c_int, [C.POINTER(MlpParams), C.POINTER(MlpGrads), _vp, _vp, _vp, _vp, _i32, _i32,
+                                      _vp, _vp, _sz, _vp, _i32]),
     "fgnn_graphnorm_fwd_f32": (C.c_int, [_vp, _vp, _vp, _vp, _vp, C.c_float, _i32, _i32, _i32, _i32, _vp, _vp]),
     "fgnn_matmul_fwd_f32": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp]),
     "fgnn_matmul_bwd_f32": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp]),
@@ -162,6 +166,19 @@ def require_cuda_f32(t: torch.Tensor, name: str) -> torch.Tensor:
 _workspaces = {}
 
 
+def _scratch(nbytes: int, device) -> torch.Tensor:
+    """torch.empty of nbytes uint8.  Under torch.use_deterministic_algorithms PyTorch fills new memory by default; the
+    library never relies on its scratch's initial contents, so that fill (tens of GB for a training workspace) is
+    skipped."""
+    import torch.utils.deterministic as D
+    fill = D.fill_uninitialized_memory
+    D.fill_uninitialized_memory = False
+    try:
+        return torch.empty(int(nbytes), dtype=torch.uint8, device=device)
+    finally:
+        D.fill_uninitialized_memory = fill
+
+
 def workspace(device, nbytes: int) -> torch.Tensor:
     """A reusable uint8 scratch tensor of at least nbytes on `device`, 1 KiB aligned (TMA / swizzled
     shared-memory tiles want 1024-byte aligned bases; torch only guarantees 512)."""
@@ -170,7 +187,7 @@ def workspace(device, nbytes: int) -> torch.Tensor:
     if buf is None or buf.numel() < nbytes:
         buf = None
         _workspaces.pop(key, None)
-        raw = torch.empty(max(int(nbytes), 1 << 20) + 1024, dtype=torch.uint8, device=device)
+        raw = _scratch(max(int(nbytes), 1 << 20) + 1024, device)
         off = (-raw.data_ptr()) % 1024
         buf = raw[off:off + raw.numel() - 1024]
         _workspaces[key] = buf
@@ -180,7 +197,7 @@ def workspace(device, nbytes: int) -> torch.Tensor:
 def private_workspace(device, nbytes: int) -> torch.Tensor:
     """A 1 KiB-aligned uint8 tensor of nbytes that is NOT shared with other calls (the 16-bit training forward keeps
     its activations there until backward)."""
-    raw = torch.empty(int(nbytes) + 1024, dtype=torch.uint8, device=device)
+    raw = _scratch(int(nbytes) + 1024, device)
     off = (-raw.data_ptr()) % 1024
     return raw[off:off + int(nbytes)]
 

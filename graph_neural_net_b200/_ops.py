@@ -6,11 +6,20 @@ stream.  Inputs must be CUDA float32 tensors; anything else raises (no CPU fallb
 from __future__ import annotations
 
 import ctypes as C
+import os
 from typing import Optional, Sequence, Tuple
 
 import torch
 
 from . import _lib as L
+
+
+def deterministic_bit() -> int:
+    """FGNN_DETERMINISTIC when this call must be bit-reproducible: torch.use_deterministic_algorithms(True) is on, or
+    the environment sets FGNN_DETERMINISTIC=1 (lets a script that cannot change, such as a benchmark, ask for it);
+    else 0.  Decided per call; a backward reuses the mode of its forward."""
+    on = torch.are_deterministic_algorithms_enabled() or os.environ.get("FGNN_DETERMINISTIC", "0") == "1"
+    return L.FGNN_DETERMINISTIC if on else 0
 
 
 def _npg(n_dev: Optional[torch.Tensor], G: Optional[int] = None):
@@ -93,6 +102,7 @@ class MlpFunction(torch.autograd.Function):
                                      L.ptr(ws), ws.numel(), L.stream_ptr(x.device)), "fgnn_mlp_fwd_f32")
         ctx.save_for_backward(x, stats, n_dev if n_dev is not None else torch.empty(0), gn_w, gn_b, *wb)
         ctx.has_n = n_dev is not None
+        ctx.flags = deterministic_bit()
         ctx.eps, ctx.depth, ctx.constant_n = eps, depth, constant_n
         return y
 
@@ -117,11 +127,11 @@ class MlpFunction(torch.autograd.Function):
         G, Ci, N, _ = x.shape
         dy = L.require_cuda_f32(dy, "dy")
         dx = torch.empty_like(x) if ctx.needs_input_grad[0] else None
-        nbytes = lib.fgnn_mlp_workspace_bytes(G, p.c_in, p.c_out, p.depth, N)
+        nbytes = lib.fgnn_mlp_workspace_bytes_ex(G, p.c_in, p.c_out, p.depth, N, ctx.flags)
         ws = L.workspace(x.device, nbytes)
-        L.check(lib.fgnn_mlp_bwd_f32(C.byref(p), C.byref(g), L.ptr(x), L.ptr(stats), L.ptr(dy), L.ptr(dx),
-                                     G, N, _npg(n_dev), L.ptr(ws), ws.numel(), L.stream_ptr(x.device)),
-                "fgnn_mlp_bwd_f32")
+        L.check(lib.fgnn_mlp_bwd_f32_ex(C.byref(p), C.byref(g), L.ptr(x), L.ptr(stats), L.ptr(dy), L.ptr(dx),
+                                        G, N, _npg(n_dev), L.ptr(ws), ws.numel(), L.stream_ptr(x.device), ctx.flags),
+                "fgnn_mlp_bwd_f32_ex")
         grads_w = [dws[k].reshape(weights[k].shape) for k in range(depth)]
         grads_b = [dbs[k] if biases[k] is not None else None for k in range(depth)]
         return (dx, None, None, None, None,
@@ -337,7 +347,7 @@ def head_fused(e1: torch.Tensor, e2: torch.Tensor, n_dev, precision: str = "fp16
     correct = torch.empty(G, device=e1.device, dtype=torch.int32)
     scores = torch.empty((G, N1, N2), device=e1.device, dtype=torch.float32) if want_scores else None
     ws = L.workspace(e1.device, lib.fgnn_head_pair_workspace_bytes(G, N1))
-    L.check(lib.fgnn_head_pair_fwd(L.PRECISIONS[precision], L.ptr(e1), L.ptr(e2), L.ptr(scores) if want_scores else None,
+    L.check(lib.fgnn_head_pair_fwd(L.PRECISIONS[precision] | deterministic_bit(), L.ptr(e1), L.ptr(e2), L.ptr(scores) if want_scores else None,
                                    L.ptr(ce), L.ptr(correct), G, Cc, N1, N2, _npg(n_dev, G), _npg(n2_dev, G), L.ptr(ws),
                                    ws.numel(), L.stream_ptr(e1.device)), "fgnn_head_pair_fwd")
     return ce, correct, scores
@@ -361,12 +371,13 @@ class HeadFunction(torch.autograd.Function):
         correct = torch.empty(G, device=e1.device, dtype=torch.int32)
         lse = torch.empty((G, N1), device=e1.device, dtype=torch.float32)
         ws = L.workspace(e1.device, lib.fgnn_head_pair_workspace_bytes(G, N1))
-        L.check(lib.fgnn_head_pair_fwd_train(L.PRECISIONS[precision], L.ptr(e1), L.ptr(e2), L.ptr(ce), L.ptr(correct),
+        prec = L.PRECISIONS[precision] | deterministic_bit()
+        L.check(lib.fgnn_head_pair_fwd_train(prec, L.ptr(e1), L.ptr(e2), L.ptr(ce), L.ptr(correct),
                                              L.ptr(lse), G, Cc, N1, N2, _npg(n_dev, G), _npg(n2_dev, G), L.ptr(ws),
                                              ws.numel(), L.stream_ptr(e1.device)), "fgnn_head_pair_fwd_train")
         saved, ctx.given = _save_sizes(n_dev, n2_dev)
         ctx.save_for_backward(e1, e2, lse, *saved)
-        ctx.precision, ctx.c_in = precision, c_in
+        ctx.precision, ctx.c_in = prec, c_in
         ctx.mark_non_differentiable(correct)
         return ce, correct
 
@@ -379,7 +390,7 @@ class HeadFunction(torch.autograd.Function):
         N2 = e2.shape[2]
         coef = L.require_cuda_f32(dce, "dce")
         de1, de2 = torch.empty_like(e1), torch.empty_like(e2)
-        L.check(lib.fgnn_head_pair_bwd(L.PRECISIONS[ctx.precision], L.ptr(e1), L.ptr(e2), L.ptr(lse), L.ptr(coef),
+        L.check(lib.fgnn_head_pair_bwd(ctx.precision, L.ptr(e1), L.ptr(e2), L.ptr(lse), L.ptr(coef),
                                        L.ptr(de1), L.ptr(de2), G, Cc, N1, N2, _npg(n_dev, G), _npg(n2_dev, G), None, 0,
                                        L.stream_ptr(e1.device)), "fgnn_head_pair_bwd")
         if Cc != ctx.c_in:
@@ -432,6 +443,7 @@ def embed_fwd(params: L.EmbedParams, precision: int, x: torch.Tensor, c_out: int
     if N != M:
         raise L.FgnnError("input must be (B,F,N,N)")
     emb = torch.empty((G, c_out, N), device=x.device, dtype=torch.float32)
+    precision |= deterministic_bit()
     nbytes = lib.fgnn_embed_workspace_bytes(C.byref(params), precision, G, N)
     if nbytes == 0:
         raise L.FgnnError("fgnn_embed_workspace_bytes returned 0: " + lib.fgnn_last_error().decode())
@@ -455,6 +467,7 @@ def embed_fwd_adjacency(params: L.EmbedParams, precision: int, adj: torch.Tensor
     adj = adj.contiguous()
     G, N, _ = adj.shape
     emb = torch.empty((G, c_out, N), device=adj.device, dtype=torch.float32)
+    precision |= deterministic_bit()
     nbytes = lib.fgnn_embed_workspace_bytes(C.byref(params), precision, G, N)
     if nbytes == 0:
         raise L.FgnnError("fgnn_embed_workspace_bytes returned 0: " + lib.fgnn_last_error().decode())
@@ -524,6 +537,7 @@ class EmbedTrainFunction(torch.autograd.Function):
             raise L.FgnnError("input must be (B,F,N,N)")
         keep = []
         params = embed_params_from_flat(spec, flat, keep)
+        precision |= deterministic_bit()              # kept in ctx.precision: the backward runs in the forward's mode
         nbytes = lib.fgnn_embed_train_workspace_bytes(C.byref(params), precision, G, N)
         if nbytes == 0:
             raise L.FgnnError("fgnn_embed_train_workspace_bytes returned 0: " + lib.fgnn_last_error().decode())

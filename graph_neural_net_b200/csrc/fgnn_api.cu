@@ -129,6 +129,14 @@ int f32_embed_fwd(const fgnn_embed_params& p, const float* x, float* emb, int G,
   return FGNN_OK;
 }
 
+// `precision` argument of the embedder entry points: an fgnn_precision in the low byte, optionally | FGNN_DETERMINISTIC.
+// false for any other bit.
+bool split_precision(int32_t arg, int* precision, bool* det) {
+  *precision = arg & 0xFF;
+  *det = (arg & FGNN_DETERMINISTIC) != 0;
+  return (arg & ~(0xFF | FGNN_DETERMINISTIC)) == 0;
+}
+
 int check_embed(const fgnn_embed_params* p, int G, int N) {
   FGNN_CHECK_ARG(p != nullptr, "null params");
   FGNN_CHECK_ARG(p->num_blocks >= 1 && p->num_blocks <= FGNN_MAX_BLOCKS, "num_blocks %d out of range", p->num_blocks);
@@ -157,7 +165,12 @@ int fgnn_device_supports_tcgen05(void) {
 }
 
 size_t fgnn_mlp_workspace_bytes(int32_t G, int32_t c_in, int32_t c_out, int32_t depth, int32_t N) {
-  return f32::mlp_workspace_bytes(G, c_in, c_out, depth, N);
+  return fgnn_mlp_workspace_bytes_ex(G, c_in, c_out, depth, N, 0);
+}
+
+size_t fgnn_mlp_workspace_bytes_ex(int32_t G, int32_t c_in, int32_t c_out, int32_t depth, int32_t N, int32_t flags) {
+  if (flags & ~FGNN_DETERMINISTIC) return 0;
+  return f32::mlp_workspace_bytes(G, c_in, c_out, depth, N, flags != 0);
 }
 
 int fgnn_mlp_fwd_f32(const fgnn_mlp_params* p, const float* x, float* y, float* stats, int32_t G,
@@ -171,9 +184,16 @@ int fgnn_mlp_bwd_f32(const fgnn_mlp_params* p, const fgnn_mlp_grads* g, const fl
                      const float* stats, const float* dy, float* dx, int32_t G, int32_t N,
                      const int32_t* n_per_graph, void* workspace, size_t workspace_bytes,
                      void* stream) {
+  return fgnn_mlp_bwd_f32_ex(p, g, x, stats, dy, dx, G, N, n_per_graph, workspace, workspace_bytes, stream, 0);
+}
+
+int fgnn_mlp_bwd_f32_ex(const fgnn_mlp_params* p, const fgnn_mlp_grads* g, const float* x, const float* stats,
+                        const float* dy, float* dx, int32_t G, int32_t N, const int32_t* n_per_graph, void* workspace,
+                        size_t workspace_bytes, void* stream, int32_t flags) {
   FGNN_CHECK_ARG(p != nullptr && g != nullptr, "null params");
-  return f32::mlp_bwd(*p, *g, x, stats, dy, dx, G, N, n_per_graph, workspace, workspace_bytes,
-                      (cudaStream_t)stream);
+  FGNN_CHECK_ARG((flags & ~FGNN_DETERMINISTIC) == 0, "unknown flags 0x%x", (unsigned)flags);
+  return f32::mlp_bwd(*p, *g, x, stats, dy, dx, G, N, n_per_graph, workspace, workspace_bytes, (cudaStream_t)stream,
+                      flags != 0);
 }
 
 int fgnn_graphnorm_fwd_f32(const float* x, float* y, float* stats, const float* gn_w,
@@ -210,7 +230,7 @@ int fgnn_head_fwd(int32_t precision, const float* e1, const float* e2, float* sc
 int fgnn_head_pair_fwd(int32_t precision, const float* e1, const float* e2, float* scores, float* ce_sum, int32_t* correct,
                        int32_t G, int32_t C, int32_t N1, int32_t N2, const int32_t* n1, const int32_t* n2, void* workspace,
                        size_t workspace_bytes, void* stream) {
-  return tc::head_fwd(precision, e1, e2, scores, ce_sum, correct, G, C, N1, N2, n1, n2, workspace, workspace_bytes,
+  return tc::head_fwd(precision & ~FGNN_DETERMINISTIC, e1, e2, scores, ce_sum, correct, G, C, N1, N2, n1, n2, workspace, workspace_bytes,
                       (cudaStream_t)stream);
 }
 
@@ -224,7 +244,7 @@ int fgnn_head_fwd_train(int32_t precision, const float* e1, const float* e2, flo
 int fgnn_head_pair_fwd_train(int32_t precision, const float* e1, const float* e2, float* ce_sum, int32_t* correct,
                              float* row_lse, int32_t G, int32_t C, int32_t N1, int32_t N2, const int32_t* n1,
                              const int32_t* n2, void* workspace, size_t workspace_bytes, void* stream) {
-  return tc::head_fwd_train(precision, e1, e2, ce_sum, correct, row_lse, G, C, N1, N2, n1, n2, workspace, workspace_bytes,
+  return tc::head_fwd_train(precision & ~FGNN_DETERMINISTIC, e1, e2, ce_sum, correct, row_lse, G, C, N1, N2, n1, n2, workspace, workspace_bytes,
                             (cudaStream_t)stream);
 }
 
@@ -240,7 +260,7 @@ int fgnn_head_pair_bwd(int32_t precision, const float* e1, const float* e2, cons
                        const int32_t* n2, void* workspace, size_t workspace_bytes, void* stream) {
   (void)workspace;
   (void)workspace_bytes;
-  return tc::head_bwd(precision, e1, e2, row_lse, coef, de1, de2, G, C, N1, N2, n1, n2, (cudaStream_t)stream);
+  return tc::head_bwd(precision & ~FGNN_DETERMINISTIC, e1, e2, row_lse, coef, de1, de2, G, C, N1, N2, n1, n2, (cudaStream_t)stream);
 }
 
 int fgnn_lap_fwd(const float* scores, int32_t* col_of_row, int32_t* correct, double* total_cost, int32_t G,
@@ -317,51 +337,69 @@ int fgnn_ce_pair_bwd_f32(const float* scores, const float* row_lse, const float*
   return f32::ce_bwd(scores, row_lse, coef, dscores, G, N1, N2, n1, n2, (cudaStream_t)stream);
 }
 
-size_t fgnn_embed_workspace_bytes(const fgnn_embed_params* p, int32_t precision, int32_t G, int32_t N) {
+size_t fgnn_embed_workspace_bytes(const fgnn_embed_params* p, int32_t precision_flags, int32_t G, int32_t N) {
+  int precision;
+  bool det;
+  if (!split_precision(precision_flags, &precision, &det)) return 0;
   if (!p || p->num_blocks < 1 || p->num_blocks > FGNN_MAX_BLOCKS || G < 1 || N < 1) return 0;
-  if (precision == FGNN_FP32) return f32_embed_ws(*p, G, N);
-  return tc::embed_workspace_bytes(*p, G, N);
+  if (precision == FGNN_FP32) return f32_embed_ws(*p, G, N);   // the fp32 forward has no cross-CTA sums
+  return tc::embed_workspace_bytes(*p, G, N, det);
 }
 
-int fgnn_embed_fwd(const fgnn_embed_params* p, int32_t precision, const float* x, float* emb,
+int fgnn_embed_fwd(const fgnn_embed_params* p, int32_t precision_flags, const float* x, float* emb,
                    int32_t G, int32_t N, const int32_t* n_per_graph, void* workspace, size_t workspace_bytes,
                    void* stream) {
+  int precision;
+  bool det;
+  FGNN_CHECK_ARG(split_precision(precision_flags, &precision, &det), "unknown precision flags 0x%x", (unsigned)precision_flags);
   if (int e = check_embed(p, G, N)) return e;
   FGNN_CHECK_ARG(x && emb && workspace, "null pointer");
   cudaStream_t st = (cudaStream_t)stream;
   if (precision == FGNN_FP32)
     return f32_embed_fwd(*p, x, emb, G, N, n_per_graph, workspace, workspace_bytes, st);
   if (precision == FGNN_BF16 || precision == FGNN_FP16)
-    return tc::embed_fwd(*p, precision, x, emb, G, N, n_per_graph, workspace, workspace_bytes, st);
+    return tc::embed_fwd(*p, precision, det, x, emb, G, N, n_per_graph, workspace, workspace_bytes, st);
   return fail(FGNN_ERR_INVALID, "unknown precision %d", precision);
 }
 
-int fgnn_embed_fwd_adjacency_u8(const fgnn_embed_params* p, int32_t precision, const uint8_t* adj, float* emb,
+int fgnn_embed_fwd_adjacency_u8(const fgnn_embed_params* p, int32_t precision_flags, const uint8_t* adj, float* emb,
                                 int32_t G, int32_t N, const int32_t* n_per_graph, void* workspace,
                                 size_t workspace_bytes, void* stream) {
+  int precision;
+  bool det;
+  FGNN_CHECK_ARG(split_precision(precision_flags, &precision, &det), "unknown precision flags 0x%x", (unsigned)precision_flags);
   if (int e = check_embed(p, G, N)) return e;
   FGNN_CHECK_ARG(adj && emb && workspace, "null pointer");
-  return tc::embed_fwd_adjacency(*p, precision, adj, emb, G, N, n_per_graph, workspace, workspace_bytes,
+  return tc::embed_fwd_adjacency(*p, precision, det, adj, emb, G, N, n_per_graph, workspace, workspace_bytes,
                                  (cudaStream_t)stream);
 }
 
-size_t fgnn_embed_train_workspace_bytes(const fgnn_embed_params* p, int32_t precision, int32_t G, int32_t N) {
+size_t fgnn_embed_train_workspace_bytes(const fgnn_embed_params* p, int32_t precision_flags, int32_t G, int32_t N) {
+  int precision;
+  bool det;
+  if (!split_precision(precision_flags, &precision, &det)) return 0;
   if (!p || p->num_blocks < 1 || p->num_blocks > FGNN_MAX_BLOCKS || G < 1 || N < 1) return 0;
   if (precision != FGNN_BF16 && precision != FGNN_FP16) return 0;
-  return tc::embed_train_workspace_bytes(*p, G, N);
+  return tc::embed_train_workspace_bytes(*p, G, N, det);
 }
 
-int fgnn_embed_fwd_train(const fgnn_embed_params* p, int32_t precision, const float* x, float* emb, int32_t G,
+int fgnn_embed_fwd_train(const fgnn_embed_params* p, int32_t precision_flags, const float* x, float* emb, int32_t G,
                          int32_t N, const int32_t* n_per_graph, void* workspace, size_t workspace_bytes,
                          void* stream) {
+  int precision;
+  bool det;
+  FGNN_CHECK_ARG(split_precision(precision_flags, &precision, &det), "unknown precision flags 0x%x", (unsigned)precision_flags);
   if (int e = check_embed(p, G, N)) return e;
   FGNN_CHECK_ARG(x && emb && workspace, "null pointer");
-  return tc::embed_fwd_train(*p, precision, x, emb, G, N, n_per_graph, workspace, workspace_bytes, (cudaStream_t)stream);
+  return tc::embed_fwd_train(*p, precision, det, x, emb, G, N, n_per_graph, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
-int fgnn_embed_bwd(const fgnn_embed_params* p, const fgnn_embed_grads* grads, int32_t precision, const float* demb,
+int fgnn_embed_bwd(const fgnn_embed_params* p, const fgnn_embed_grads* grads, int32_t precision_flags, const float* demb,
                    int32_t grad_scale_log2, int32_t G, int32_t N, const int32_t* n_per_graph, void* workspace,
                    size_t workspace_bytes, void* stream) {
+  int precision;
+  bool det;
+  FGNN_CHECK_ARG(split_precision(precision_flags, &precision, &det), "unknown precision flags 0x%x", (unsigned)precision_flags);
   if (int e = check_embed(p, G, N)) return e;
   FGNN_CHECK_ARG(grads && demb && workspace, "null pointer");
   FGNN_CHECK_ARG(grads->num_blocks == p->num_blocks, "grads describe %d blocks, params %d", grads->num_blocks, p->num_blocks);
@@ -372,7 +410,7 @@ int fgnn_embed_bwd(const fgnn_embed_params* p, const fgnn_embed_grads* grads, in
       for (int l = 0; l < mp[m]->depth; ++l)
         FGNN_CHECK_ARG(mg[m]->w[l] != nullptr, "block %d mlp%d: missing weight-gradient buffer of layer %d", b, m + 1, l);
   }
-  return tc::embed_bwd(*p, *grads, precision, demb, grad_scale_log2, G, N, n_per_graph, workspace, workspace_bytes,
+  return tc::embed_bwd(*p, *grads, precision, det, demb, grad_scale_log2, G, N, n_per_graph, workspace, workspace_bytes,
                        (cudaStream_t)stream);
 }
 

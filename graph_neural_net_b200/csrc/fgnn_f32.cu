@@ -474,7 +474,7 @@ int run_conv1x1(const float* w, const float* b, int c_in, int c_out, bool transp
 // ---------------------------------------------------------------------------------------
 // host launchers
 // ---------------------------------------------------------------------------------------
-size_t mlp_workspace_bytes(int G, int c_in, int c_out, int depth, int N) {
+size_t mlp_workspace_bytes(int G, int c_in, int c_out, int depth, int N, bool det) {
   Arena ar(nullptr, 0);
   const int cop = (c_out + 7) / 8 * 8;
   for (int k = 0; k < depth; ++k) ar.take<float>((size_t)(k == 0 ? c_in : c_out) * cop);
@@ -487,6 +487,7 @@ size_t mlp_workspace_bytes(int G, int c_in, int c_out, int depth, int N) {
   if (graphs < 1) graphs = 1;
   if (graphs > (size_t)G) graphs = G;
   ar.take<char>(graphs * per_graph + 4096);
+  if (det) mlp_bwd_records(ar, G, c_out, cmax);
   return align_up(ar.off, 256);
 }
 

@@ -10,14 +10,29 @@ namespace f32 {
 int run_conv1x1(const float* w, const float* b, int c_in, int c_out, bool transpose_w, bool relu, const float* x,
                 float* y, float* wt_scratch, int G, int N, const int32_t* n_per_graph, cudaStream_t st);
 
-// workspace layout helper for one MLP call
-size_t mlp_workspace_bytes(int G, int c_in, int c_out, int depth, int N);
+// OrderedSum records of the fp32 MLP backward (deterministic mode): the GraphNorm affine-gradient terms of every
+// (graph, channel) [2][G][c_out], and the weight / bias gradient of every pixel split [kMaxWgradSplits][c_out][cmax] /
+// [kMaxWgradSplits][c_out]
+constexpr int kMaxWgradSplits = 64;
+struct MlpBwdRecords {
+  float *gn, *w, *b;
+};
+inline MlpBwdRecords mlp_bwd_records(Arena& ar, int G, int c_out, int cmax) {
+  MlpBwdRecords r;
+  r.gn = ar.take<float>((size_t)2 * G * c_out);
+  r.w = ar.take<float>((size_t)kMaxWgradSplits * c_out * cmax);
+  r.b = ar.take<float>((size_t)kMaxWgradSplits * c_out);
+  return r;
+}
+
+// workspace layout helper for one MLP call (det: room for the backward's OrderedSum records)
+size_t mlp_workspace_bytes(int G, int c_in, int c_out, int depth, int N, bool det = false);
 
 int mlp_fwd(const fgnn_mlp_params& p, const float* x, float* y, float* stats, int G, int N,
             const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st);
 int mlp_bwd(const fgnn_mlp_params& p, const fgnn_mlp_grads& g, const float* x, const float* stats,
             const float* dy, float* dx, int G, int N, const int32_t* n_per_graph, void* ws,
-            size_t ws_bytes, cudaStream_t st);
+            size_t ws_bytes, cudaStream_t st, bool det = false);
 int graphnorm_fwd(const float* x, float* y, float* stats, const float* gw, const float* gb, float eps,
                   int constant_n, int G, int C, int N, const int32_t* n_per_graph, cudaStream_t st);
 int matmul_fwd(const float* a, const float* b, float* out, int G, int C, int N,

@@ -19,6 +19,8 @@ __device__ __forceinline__ int graph_n(const int32_t* n_per_graph, int g, int N)
 }
 
 // per plane (g,c): a1 = sum dy, a2 = sum dy (z - mu) over valid pixels; dgw += inv * a2, dgb += a1
+// (OrderedSum: the two terms go to rec[0][gc] / rec[1][gc] instead, rec = dgw, and the caller sums them over g)
+template <typename Sum>
 __global__ void __launch_bounds__(256)
 gn_bwd_stats_kernel(const float* __restrict__ dy, const float* __restrict__ z, const float* __restrict__ stats,
                     float* __restrict__ sums, float* __restrict__ dgw, float* __restrict__ dgb, int C, int N,
@@ -50,8 +52,13 @@ gn_bwd_stats_kernel(const float* __restrict__ dy, const float* __restrict__ z, c
   if (threadIdx.x == 0) {
     sums[2 * gc] = (float)sh[0][0];
     sums[2 * gc + 1] = (float)sh[1][0];
-    if (dgw) atomicAdd(dgw + c, (float)(sh[1][0] * (double)inv));
-    if (dgb) atomicAdd(dgb + c, (float)sh[0][0]);
+    if constexpr (Sum::kOrdered) {
+      dgw[gc] = (float)(sh[1][0] * (double)inv);
+      dgw[(long)gridDim.x + gc] = (float)sh[0][0];
+    } else {
+      if (dgw) atomicAdd(dgw + c, (float)(sh[1][0] * (double)inv));
+      if (dgb) atomicAdd(dgb + c, (float)sh[0][0]);
+    }
   }
 }
 
@@ -85,6 +92,8 @@ __global__ void relu_mask_kernel(float* __restrict__ d, const float* __restrict_
 
 // dW[co][ci] += sum_{g,p} d[g,co,p] in[g,ci,p];  db[co] += sum_{g,p} d[g,co,p]
 // grid: (ci tiles of 16, co tiles of 16, pixel splits); block 16x16; K chunk 64 pixels staged in smem.
+// OrderedSum: split z stores its partials to dW[z][co][ci] / db[z][co] (records) and the caller sums them over z.
+template <typename Sum>
 __global__ void __launch_bounds__(256)
 wgrad_kernel(const float* __restrict__ d, const float* __restrict__ in, float* __restrict__ dW, float* __restrict__ db,
              int Co, int Ci, long P, int G) {
@@ -117,15 +126,20 @@ wgrad_kernel(const float* __restrict__ d, const float* __restrict__ in, float* _
     }
     __syncthreads();
   }
-  if (co0 + ty < Co && ci0 + tx < Ci) atomicAdd(dW + (long)(co0 + ty) * Ci + ci0 + tx, acc);
-  if (db && blockIdx.x == 0 && tx == 0 && co0 + ty < Co) atomicAdd(db + co0 + ty, bacc);
+  if constexpr (Sum::kOrdered) {
+    if (co0 + ty < Co && ci0 + tx < Ci) dW[((long)blockIdx.z * Co + co0 + ty) * Ci + ci0 + tx] = acc;
+    if (db && blockIdx.x == 0 && tx == 0 && co0 + ty < Co) db[(long)blockIdx.z * Co + co0 + ty] = bacc;
+  } else {
+    if (co0 + ty < Co && ci0 + tx < Ci) atomicAdd(dW + (long)(co0 + ty) * Ci + ci0 + tx, acc);
+    if (db && blockIdx.x == 0 && tx == 0 && co0 + ty < Co) atomicAdd(db + co0 + ty, bacc);
+  }
 }
 
 }  // namespace
 
 int mlp_bwd(const fgnn_mlp_params& p, const fgnn_mlp_grads& gr, const float* x, const float* stats,
             const float* dy, float* dx, int G, int N, const int32_t* n_per_graph, void* ws, size_t ws_bytes,
-            cudaStream_t st) {
+            cudaStream_t st, bool det) {
   FGNN_CHECK_ARG(x && stats && dy && ws, "null pointer");
   FGNN_CHECK_ARG(p.depth >= 1 && p.depth <= FGNN_MAX_DEPTH, "depth %d out of range", p.depth);
   const int Co = p.c_out, Ci = p.c_in, depth = p.depth;
@@ -135,6 +149,7 @@ int mlp_bwd(const fgnn_mlp_params& p, const fgnn_mlp_grads& gr, const float* x, 
   Arena ar(ws, ws_bytes);
   float* wt = ar.take<float>((size_t)(Ci > Co ? Ci : Co) * ((cmax + 7) / 8 * 8));
   float* sums = ar.take<float>((size_t)G * Co * 2);
+  const MlpBwdRecords rec = det ? mlp_bwd_records(ar, G, Co, cmax) : MlpBwdRecords{};
   const size_t fixed = align_up(ar.off, 256);
   if (fixed >= ws_bytes) return fail(FGNN_ERR_WORKSPACE, "mlp backward workspace too small");
   const size_t per_graph = (size_t)(depth + 2) * cmax * P * sizeof(float) + 256 * (depth + 2);
@@ -161,8 +176,16 @@ int mlp_bwd(const fgnn_mlp_params& p, const fgnn_mlp_grads& gr, const float* x, 
         return e;
     }
     // 2. GraphNorm backward -> dz
-    gn_bwd_stats_kernel<<<gc * Co, 256, 0, st>>>(dyc, h[depth - 1], stc, smc, gr.gn_w, gr.gn_b, Co, N, n_c);
-    FGNN_LAUNCHED();
+    if (det) {
+      // records [2][gc * Co], then dgw[c] / dgb[c] += their sum over the chunk's graphs in ascending order
+      gn_bwd_stats_kernel<OrderedSum><<<gc * Co, 256, 0, st>>>(dyc, h[depth - 1], stc, smc, rec.gn, nullptr, Co, N, n_c);
+      FGNN_LAUNCHED();
+      if (gr.gn_w) if (int e = sum_records(rec.gn, gr.gn_w, Co, gc, Co, true, st)) return e;
+      if (gr.gn_b) if (int e = sum_records(rec.gn + (long)gc * Co, gr.gn_b, Co, gc, Co, true, st)) return e;
+    } else {
+      gn_bwd_stats_kernel<AtomicSum><<<gc * Co, 256, 0, st>>>(dyc, h[depth - 1], stc, smc, gr.gn_w, gr.gn_b, Co, N, n_c);
+      FGNN_LAUNCHED();
+    }
     {
       dim3 grid((unsigned)std::min<long>(64, (P + 255) / 256), gc * Co);
       gn_bwd_apply_kernel<<<grid, 256, 0, st>>>(dyc, h[depth - 1], stc, smc, p.gn_w, dcur, Co, N, n_c, p.constant_n);
@@ -173,10 +196,17 @@ int mlp_bwd(const fgnn_mlp_params& p, const fgnn_mlp_grads& gr, const float* x, 
       const int cin = (k == 0) ? Ci : Co;
       const float* in = (k == 0) ? xc : h[k - 1];
       if (gr.w[k]) {
-        const int splits = (int)std::min<long>(64, std::max<long>(1, (long)gc * P / 4096));
+        const int splits = (int)std::min<long>(kMaxWgradSplits, std::max<long>(1, (long)gc * P / 4096));
         dim3 grid(ceil_div(cin, 16), ceil_div(Co, 16), splits);
-        wgrad_kernel<<<grid, 256, 0, st>>>(dcur, in, gr.w[k], gr.b[k], Co, cin, P, gc);
-        FGNN_LAUNCHED();
+        if (det) {
+          wgrad_kernel<OrderedSum><<<grid, 256, 0, st>>>(dcur, in, rec.w, gr.b[k] ? rec.b : nullptr, Co, cin, P, gc);
+          FGNN_LAUNCHED();
+          if (int e = sum_records(rec.w, gr.w[k], (long)Co * cin, splits, Co * cin, true, st)) return e;
+          if (gr.b[k]) if (int e = sum_records(rec.b, gr.b[k], Co, splits, Co, true, st)) return e;
+        } else {
+          wgrad_kernel<AtomicSum><<<grid, 256, 0, st>>>(dcur, in, gr.w[k], gr.b[k], Co, cin, P, gc);
+          FGNN_LAUNCHED();
+        }
       }
       if (k == 0 && dx == nullptr) break;
       float* dst = (k == 0) ? dx + (long)g0 * Ci * P : dnxt;

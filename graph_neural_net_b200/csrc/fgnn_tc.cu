@@ -378,7 +378,7 @@ __global__ void finalize_coef_kernel(CoefArgs a, int total) {
 //           memory with stmatrix.trans (16x256b accumulator fragments, four rounds of 16 registers), stored by TMA;
 //           per-(graph, channel) sum and sum of squares are taken from the fp32 accumulators in the same pass (register
 //           partials per thread in the fragment layout, folded across lanes and added with double atomics on a graph
-//           change).  POOL = true (last block): the tile is not stored; the group reads its staged tile back
+//           change; Sum = OrderedSum stores them to records instead, see stat_records_reduce_kernel).  POOL = true (last block): the tile is not stored; the group reads its staged tile back
 //           (thread = channel) for the statistics and the row-wise max / min of the fused column-max pooling.
 // Warp roles: warps 0-15 = four epilogue groups (group = warp / 4 = TMEM slot, lane quadrant = warp % 4), warp 16 = TMA
 // producer, warp 17 = first-layer MMA issuer (the only consumer of the input ring: it sees every phase of every
@@ -400,7 +400,7 @@ struct MlpArgs {
   T* out[2];                                 // per MLP output planes (direct stores of the ones row only)
   Layout out_mode[2];                        // output plane layout
   int ones[2];                               // kLayoutA: write the ones rows; kLayoutB: holes hold ones
-  double* stat_acc;                          // [G][NMLP][COUT][2]
+  double* stat_acc;                          // [G][NMLP][COUT][2]; OrderedSum: the records of stat_records_reduce_kernel
   // Fused column-max pooling (last block): when rowenc[m] is set, MLP m's tile is NOT stored; the statistics pass
   // folds the row-wise max and min of its valid pixels into rowenc[m][g][c][i][2] (order-preserving unsigned codes
   // of max(y) and max(-y), buffer zeroed by the caller) and pool_finalize_kernel applies the GraphNorm affine.
@@ -409,6 +409,78 @@ struct MlpArgs {
 };
 
 constexpr int kSlots = 4;                    // TMEM slots = epilogue groups
+
+// Deterministic conv-chain statistics (Sum = OrderedSum).  A CTA owns a contiguous range of the launch's flat
+// (graph, tile) list, so each of its (TMEM slot, lane quadrant or pixel part) partial sums is flushed at most once per
+// graph.  CTA b flushes graph g into record g + b: the CTAs that touch a graph form a contiguous run, and both ends of
+// the run never decrease from one graph to the next, so (g, b) -> g + b is one-to-one on the pairs that occur and a
+// launch of G graphs on `grid` CTAs fills at most G + grid records of [kSlots][4][COUT][2] doubles (zeroed beforehand:
+// slots that saw no tile of the graph write nothing).
+constexpr int kStatSubs = 4;   // lane quadrants (register statistics) or pixel parts (POOL, 128 / COUT <= 4) per slot
+__host__ __device__ inline long stat_record_doubles(int COUT) { return (long)kSlots * kStatSubs * COUT * 2; }
+__device__ __forceinline__ long stat_record(int g, int slot, int sub, int ch, int COUT) {
+  return (long)(g + (int)blockIdx.x) * stat_record_doubles(COUT) + (((long)slot * kStatSubs + sub) * COUT + ch) * 2;
+}
+// CTAs of a tc_mlp_kernel launch: one per SM, at most one per tile (upper bound on the tiles of a ragged launch)
+int mlp_grid(int G, const Geo& geo);
+
+// acc[g][m][c][2] = the records of graph g summed in double over its CTAs, the slots of MLP m (slot % NMLP == m) and
+// their sub-partials.  One block per (g, m, c): thread t adds records t, t + 256, ... of the graph's run in ascending
+// order, then a fixed tree adds the 256 thread sums -- the same order on every run, spread over enough SMs that a
+// launch of one large graph (148 CTAs x 16 records per channel) is not one SM's serial loop.
+constexpr int kStatReduceThreads = 256;
+__global__ void __launch_bounds__(kStatReduceThreads)
+stat_records_reduce_kernel(const double* __restrict__ rec, double* __restrict__ acc, int G, int nmlp, int C, int grid,
+                           Geo geo, const int32_t* __restrict__ n_per_graph) {
+  __shared__ unsigned long long s_base, s_total;
+  __shared__ int s_b0, s_b1;
+  __shared__ double s_red[2][kStatReduceThreads];
+  const int c = blockIdx.x % C, m = (blockIdx.x / C) % nmlp, g = blockIdx.x / (C * nmlp);
+  if (threadIdx.x == 0) { s_base = 0; s_total = 0; s_b0 = INT_MAX; s_b1 = -1; }
+  __syncthreads();
+  unsigned long long base = 0, total = 0;        // tiles of graphs < g, of all graphs (integer sums: any order)
+  for (int h = threadIdx.x; h < G; h += blockDim.x) {
+    const unsigned long long t = mlp_tiles(n_per_graph, h, geo);
+    total += t;
+    if (h < g) base += t;
+  }
+  atomicAdd(&s_base, base);
+  atomicAdd(&s_total, total);
+  __syncthreads();
+  // the run of CTAs whose tile range meets the graph's (the kernel's partition of the tiles); CTAs without tiles inside
+  // the run flushed nothing and their records are zero
+  const long t0 = (long)s_base, t1 = t0 + mlp_tiles(n_per_graph, g, geo), tot = (long)s_total;
+  for (int b = threadIdx.x; b < grid; b += blockDim.x) {
+    const long tb = tot * b / grid, te = tot * (b + 1) / grid;
+    if (te > tb && tb < t1 && te > t0) { atomicMin(&s_b0, b); atomicMax(&s_b1, b); }
+  }
+  __syncthreads();
+  const int spm = kSlots / nmlp, per_cta = spm * kStatSubs;
+  const int nrec = s_b1 >= s_b0 ? (s_b1 - s_b0 + 1) * per_cta : 0;
+  double v0 = 0.0, v1 = 0.0;
+  for (int k = threadIdx.x; k < nrec; k += blockDim.x) {
+    const int b = s_b0 + k / per_cta, slot = m + nmlp * ((k % per_cta) / kStatSubs), sub = k % kStatSubs;
+    const double* r = rec + (long)(g + b) * stat_record_doubles(C) + (((long)slot * kStatSubs + sub) * C + c) * 2;
+    v0 += r[0];
+    v1 += r[1];
+  }
+  s_red[0][threadIdx.x] = v0;
+  s_red[1][threadIdx.x] = v1;
+  __syncthreads();
+  for (int o = kStatReduceThreads / 2; o > 0; o >>= 1) {
+    if (threadIdx.x < o) {
+      s_red[0][threadIdx.x] += s_red[0][threadIdx.x + o];
+      s_red[1][threadIdx.x] += s_red[1][threadIdx.x + o];
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) {
+    double* a = acc + (((long)g * nmlp + m) * C + c) * 2;
+    a[0] = s_red[0][0];
+    a[1] = s_red[1][0];
+  }
+}
+
 constexpr int kWProd = 4 * kSlots, kWL1 = kWProd + 1;
 // 18 warps; registers are allocated in units of four warps, so the kernel gets 96 registers per thread (as 20 warps would).
 // (setmaxnreg hand-over from the control warps to the epilogue groups was tried: ptxas 12.9 then allocates the WHOLE
@@ -440,7 +512,7 @@ struct MlpSmem {
   }
 };
 
-template <typename T, int COUT, int NMLP, bool POOL, bool RELU_OUT>
+template <typename T, int COUT, int NMLP, bool POOL, bool RELU_OUT, typename Sum>
 __global__ void __launch_bounds__(kMlpThreads, 1)
 tc_mlp_kernel(const __grid_constant__ CUtensorMap map_x0, const __grid_constant__ CUtensorMap map_x1,
               const __grid_constant__ CUtensorMap map_w1, const __grid_constant__ CUtensorMap map_wh,
@@ -719,9 +791,15 @@ tc_mlp_kernel(const __grid_constant__ CUtensorMap map_x0, const __grid_constant_
         }
         if (lane < 4) {
           const int ch = 8 * (i >> 1) + 2 * lane + (i & 1);
-          double* dst = args.stat_acc + (((long)acc_g * NMLP + m) * COUT + ch) * 2;
-          atomicAdd(dst, (double)sv);
-          atomicAdd(dst + 1, (double)qv);
+          if constexpr (Sum::kOrdered) {
+            double* dst = args.stat_acc + stat_record(acc_g, s, quad, ch, COUT);
+            dst[0] = (double)sv;
+            dst[1] = (double)qv;
+          } else {
+            double* dst = args.stat_acc + (((long)acc_g * NMLP + m) * COUT + ch) * 2;
+            atomicAdd(dst, (double)sv);
+            atomicAdd(dst + 1, (double)qv);
+          }
         }
         st_S[i] = 0.f;
         st_Q[i] = 0.f;
@@ -729,9 +807,15 @@ tc_mlp_kernel(const __grid_constant__ CUtensorMap map_x0, const __grid_constant_
     };
     auto flush = [&]() {
       if (acc_g < 0) return;
-      double* dst = args.stat_acc + (((long)acc_g * NMLP + m) * COUT + c) * 2;
-      atomicAdd(dst, (double)acc_s);
-      atomicAdd(dst + 1, (double)acc_q);
+      if constexpr (Sum::kOrdered) {
+        double* dst = args.stat_acc + stat_record(acc_g, s, part, c, COUT);
+        dst[0] = (double)acc_s;
+        dst[1] = (double)acc_q;
+      } else {
+        double* dst = args.stat_acc + (((long)acc_g * NMLP + m) * COUT + c) * 2;
+        atomicAdd(dst, (double)acc_s);
+        atomicAdd(dst + 1, (double)acc_q);
+      }
       acc_s = 0.f;
       acc_q = 0.f;
     };
@@ -1816,12 +1900,21 @@ struct MlpGroup {
   int ones[2];
   float* coef[2];
   double* stat_acc;  // [G][nmlp][C][2], zeroed by the launch
+  double* stat_rec;  // deterministic mode: room for (G + mlp_grid) conv-chain statistics records (null: atomics)
   unsigned int* rowenc[2];   // fused max pooling of this MLP's output instead of storing it (see MlpArgs), or null
   // training path (depth-1 launches, see fgnn_tc_train.cuh)
   int relu_out;              // out = relu(conv + bias) instead of the raw accumulator
   int no_coef;               // skip the GraphNorm coefficient finalisation (hidden layers, backward convs)
   float* gnstat[2];          // statistics kept for backward (or null)
 };
+
+int mlp_grid(int G, const Geo& geo) {
+  const long total_tiles = (long)G * ((geo.PSC + kTileM - 1) / kTileM);
+  return (int)std::max<long>(1, std::min<long>((long)num_sms(), total_tiles));
+}
+
+// doubles of the conv-chain statistics records a launch of G graphs at width C may fill (deterministic mode)
+size_t stat_rec_doubles(int G, int C, const Geo& geo) { return (size_t)(G + mlp_grid(G, geo)) * stat_record_doubles(C); }
 
 template <typename T, int COUT, int NMLP>
 int launch_mlp_t(const MlpGroup<T>& M, int G, const Geo& geo, const int32_t* npg, cudaStream_t st) {
@@ -1871,21 +1964,29 @@ int launch_mlp_t(const MlpGroup<T>& M, int G, const Geo& geo, const int32_t* npg
   const bool pool = a.rowenc[0] != nullptr;
   FGNN_CHECK_ARG(!pool || NMLP == 1, "fused pooling is only built for single-MLP launches");
   FGNN_CHECK_ARG(!M.relu_out || (a.depth == 1 && !pool), "relu_out is a depth-1, non-pooled launch");
-  auto kernel = M.relu_out ? tc_mlp_kernel<T, COUT, NMLP, false, true> : tc_mlp_kernel<T, COUT, NMLP, false, false>;
-  if constexpr (NMLP == 1) {
-    if (pool) kernel = tc_mlp_kernel<T, COUT, NMLP, true, false>;
+  const int grid = mlp_grid(G, geo);
+  auto launch = [&](auto sum) -> int {
+    using S = decltype(sum);
+    auto kernel = M.relu_out ? tc_mlp_kernel<T, COUT, NMLP, false, true, S> : tc_mlp_kernel<T, COUT, NMLP, false, false, S>;
+    if constexpr (NMLP == 1) {
+      if (pool) kernel = tc_mlp_kernel<T, COUT, NMLP, true, false, S>;
+    }
+    // the opt-in is per device and cheap: set on every call
+    FGNN_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    prof::begin(prof::kMlp, st);
+    kernel<<<grid, kMlpThreads, smem, st>>>(mx0, mx1, mw1, mwh, mo[0], mo[1], a);
+    prof::end(prof::kMlp, st);
+    FGNN_LAUNCHED();
+    return FGNN_OK;
+  };
+  if (!M.stat_rec) {
+    FGNN_CUDA(cudaMemsetAsync(M.stat_acc, 0, (size_t)G * NMLP * COUT * 2 * sizeof(double), st));
+    return launch(AtomicSum{});
   }
-  // the opt-in is per device and cheap: set on every call
-  FGNN_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  FGNN_CUDA(cudaMemsetAsync(M.stat_acc, 0, (size_t)G * NMLP * COUT * 2 * sizeof(double), st));
-  long total_tiles = (long)G * ((geo.PSC + kTileM - 1) / kTileM);
-  int grid = (int)std::min<long>((long)num_sms(), total_tiles);
-  if (grid < 1) grid = 1;
-  prof::begin(prof::kMlp, st);
-  kernel<<<grid, kMlpThreads, smem, st>>>(mx0, mx1, mw1, mwh, mo[0], mo[1], a);
-  prof::end(prof::kMlp, st);
-  FGNN_LAUNCHED();
-  return FGNN_OK;
+  // records of the launch (their statistics are only read when the coefficients are finalised)
+  a.stat_acc = M.stat_rec;
+  if (!M.no_coef) FGNN_CUDA(cudaMemsetAsync(M.stat_rec, 0, (size_t)(G + grid) * stat_record_doubles(COUT) * sizeof(double), st));
+  return launch(OrderedSum{});
 }
 
 template <typename T>
@@ -1939,6 +2040,13 @@ int run_mlp_group(const MlpGroup<T>& M, int C, int G, const Geo& geo, const int3
   }
   if (int e = launch_mlp<T>(P, C, G, geo, npg, st)) return e;
   if (M.no_coef) return FGNN_OK;
+  if (M.stat_rec) {
+    prof::begin(prof::kStats, st);
+    stat_records_reduce_kernel<<<G * M.nmlp * C, kStatReduceThreads, 0, st>>>(M.stat_rec, M.stat_acc, G, M.nmlp, C,
+                                                                               mlp_grid(G, geo), geo, npg);
+    prof::end(prof::kStats, st);
+    FGNN_LAUNCHED();
+  }
   CoefArgs ca{};
   ca.acc = M.stat_acc;
   ca.nmlp = M.nmlp;
@@ -2037,9 +2145,10 @@ struct Buffers {
   double* stat_acc;                            // [chunk][2][C][2]
   void* wh;                                    // [blocks][3][depth-1][C][Kh]
   unsigned int* rowenc;                        // [chunk][C][N][2] row max / min codes of the last block's output
+  double* stat_rec;                            // deterministic mode: conv-chain statistics records (else null)
 };
 
-size_t carve(const Plan& pl, int num_blocks, Arena& ar, Buffers& B) {
+size_t carve(const Plan& pl, int num_blocks, bool det, Arena& ar, Buffers& B) {
   const size_t actC = (size_t)pl.chunk * pl.C * pl.geo.stride(kLayoutC);
   B.xin = ar.take<uint16_t>((size_t)pl.chunk * pl.cin0 * pl.geo.stride(kLayoutC), 1024);
   B.xa = ar.take<uint16_t>(actC, 1024);
@@ -2062,17 +2171,18 @@ size_t carve(const Plan& pl, int num_blocks, Arena& ar, Buffers& B) {
   const int Kh = pl.C < 64 ? 64 : pl.C;
   B.wh = ar.take<uint16_t>((size_t)num_blocks * 3 * std::max(pl.depth_max - 1, 1) * pl.C * Kh, 1024);
   B.rowenc = ar.take<unsigned int>(nc * pl.geo.N * 2, 1024);
+  B.stat_rec = det ? ar.take<double>(stat_rec_doubles(pl.chunk, pl.C, pl.geo)) : nullptr;
   return align_up(ar.off, 1024);
 }
 
 template <typename T>
-int embed_fwd_t(const fgnn_embed_params& p, const float* x, const uint8_t* adj, float* emb, int G, int N,
+int embed_fwd_t(const fgnn_embed_params& p, bool det, const float* x, const uint8_t* adj, float* emb, int G, int N,
                 const int32_t* npg, void* ws, size_t ws_bytes, cudaStream_t st) {
   Plan pl;
   if (int e = make_plan(p, G, N, pl)) return e;
   Arena ar(ws, ws_bytes);
   Buffers B;
-  size_t need = carve(pl, p.num_blocks, ar, B);
+  size_t need = carve(pl, p.num_blocks, det, ar, B);
   if (need > ws_bytes) return fail(FGNN_ERR_WORKSPACE, "embed workspace too small: %zu < %zu", ws_bytes, need);
   const int C = pl.C;
   const Geo& geo = pl.geo;
@@ -2140,6 +2250,7 @@ int embed_fwd_t(const fgnn_embed_params& p, const float* x, const uint8_t* adj, 
         M.out[0] = y1; M.out_mode[0] = kLayoutA; M.ones[0] = 1; M.coef[0] = B.coef1;
         M.out[1] = y2; M.out_mode[1] = kLayoutB; M.ones[1] = 1; M.coef[1] = B.coef2;
         M.stat_acc = B.stat_acc;
+        M.stat_rec = B.stat_rec;
         if (int e = run_mlp_group<T>(M, C, gc, geo, n_c, st)) return e;
       }
       if (int e = launch_matmul<T>(y1, y2, mult, B.coef1, B.coef2, gc, C, geo, n_c, st)) return e;
@@ -2154,6 +2265,7 @@ int embed_fwd_t(const fgnn_embed_params& p, const float* x, const uint8_t* adj, 
         M.bias_pad = static_cast<float*>(B.wf12);
         M.out[0] = nxt; M.out_mode[0] = kLayoutC; M.ones[0] = 0; M.coef[0] = nxt_coef;
         M.stat_acc = B.stat_acc;
+        M.stat_rec = B.stat_rec;
         if (b == p.num_blocks - 1) {
           // the last block's output is only ever max-pooled: keep its row max / min and never write the planes
           M.rowenc[0] = B.rowenc;
@@ -2191,54 +2303,54 @@ int with_16bit(int precision, const char* what, F&& f) {
 
 }  // namespace
 
-size_t embed_train_workspace_bytes(const fgnn_embed_params& p, int G, int N) {
+size_t embed_train_workspace_bytes(const fgnn_embed_params& p, int G, int N, bool det) {
   TrainPlan tp;
-  if (make_train_plan(p, G, N, tp)) return 0;
+  if (make_train_plan(p, G, N, det, tp)) return 0;
   Arena ar(nullptr, 0);
   TrainBuf B;
   return carve_train(tp, ar, B);
 }
 
-int embed_fwd_train(const fgnn_embed_params& p, int precision, const float* x, float* emb, int G, int N,
+int embed_fwd_train(const fgnn_embed_params& p, int precision, bool det, const float* x, float* emb, int G, int N,
                     const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
   return with_16bit(precision, "fgnn_embed_fwd_train", [&](auto t) -> int {
     if (reinterpret_cast<uintptr_t>(ws) & 1023) return fail(FGNN_ERR_INVALID, "workspace must be 1024-byte aligned");
-    return embed_fwd_train_t<decltype(t)>(p, x, emb, G, N, n_per_graph, ws, ws_bytes, st);
+    return embed_fwd_train_t<decltype(t)>(p, det, x, emb, G, N, n_per_graph, ws, ws_bytes, st);
   });
 }
 
-int embed_bwd(const fgnn_embed_params& p, const fgnn_embed_grads& g, int precision, const float* demb, int grad_scale_log2,
+int embed_bwd(const fgnn_embed_params& p, const fgnn_embed_grads& g, int precision, bool det, const float* demb, int grad_scale_log2,
               int G, int N, const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
   return with_16bit(precision, "fgnn_embed_bwd", [&](auto t) -> int {
     if (reinterpret_cast<uintptr_t>(ws) & 1023) return fail(FGNN_ERR_INVALID, "workspace must be 1024-byte aligned");
     if (grad_scale_log2 < -24 || grad_scale_log2 > 15) return fail(FGNN_ERR_INVALID, "grad_scale_log2 %d outside [-24, 15]", grad_scale_log2);
-    return embed_bwd_t<decltype(t)>(p, g, demb, grad_scale_log2, G, N, n_per_graph, ws, ws_bytes, st);
+    return embed_bwd_t<decltype(t)>(p, g, det, demb, grad_scale_log2, G, N, n_per_graph, ws, ws_bytes, st);
   });
 }
 
-size_t embed_workspace_bytes(const fgnn_embed_params& p, int G, int N) {
+size_t embed_workspace_bytes(const fgnn_embed_params& p, int G, int N, bool det) {
   Plan pl;
   if (make_plan(p, G, N, pl)) return 0;
   Arena ar(nullptr, 0);
   Buffers B;
-  return carve(pl, p.num_blocks, ar, B);
+  return carve(pl, p.num_blocks, det, ar, B);
 }
 
-int embed_fwd(const fgnn_embed_params& p, int precision, const float* x, float* emb, int G, int N,
+int embed_fwd(const fgnn_embed_params& p, int precision, bool det, const float* x, float* emb, int G, int N,
               const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
   return with_16bit(precision, "fgnn_embed_fwd", [&](auto t) -> int {
     if (reinterpret_cast<uintptr_t>(ws) & 1023) return fail(FGNN_ERR_INVALID, "workspace must be 1024-byte aligned");
-    return embed_fwd_t<decltype(t)>(p, x, nullptr, emb, G, N, n_per_graph, ws, ws_bytes, st);
+    return embed_fwd_t<decltype(t)>(p, det, x, nullptr, emb, G, N, n_per_graph, ws, ws_bytes, st);
   });
 }
 
-int embed_fwd_adjacency(const fgnn_embed_params& p, int precision, const uint8_t* adj, float* emb, int G, int N,
+int embed_fwd_adjacency(const fgnn_embed_params& p, int precision, bool det, const uint8_t* adj, float* emb, int G, int N,
                         const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
   return with_16bit(precision, "fgnn_embed_fwd_adjacency_u8", [&](auto t) -> int {
     if (reinterpret_cast<uintptr_t>(ws) & 1023) return fail(FGNN_ERR_INVALID, "workspace must be 1024-byte aligned");
     FGNN_CHECK_ARG(p.num_blocks >= 1 && p.block[0].mlp1.c_in == 2,
                    "the adjacency input builds exactly the reference's 2 features (W, diag(deg))");
-    return embed_fwd_t<decltype(t)>(p, nullptr, adj, emb, G, N, n_per_graph, ws, ws_bytes, st);
+    return embed_fwd_t<decltype(t)>(p, det, nullptr, adj, emb, G, N, n_per_graph, ws, ws_bytes, st);
   });
 }
 

@@ -5,18 +5,19 @@
 namespace fgnn {
 namespace tc {
 
-size_t embed_workspace_bytes(const fgnn_embed_params& p, int G, int N);
-int embed_fwd(const fgnn_embed_params& p, int precision, const float* x, float* emb, int G, int N,
+// det: deterministic mode (FGNN_DETERMINISTIC): OrderedSum kernels, and a workspace with room for their records
+size_t embed_workspace_bytes(const fgnn_embed_params& p, int G, int N, bool det);
+int embed_fwd(const fgnn_embed_params& p, int precision, bool det, const float* x, float* emb, int G, int N,
               const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st);
 
-int embed_fwd_adjacency(const fgnn_embed_params& p, int precision, const uint8_t* adj, float* emb, int G, int N,
+int embed_fwd_adjacency(const fgnn_embed_params& p, int precision, bool det, const uint8_t* adj, float* emb, int G, int N,
                         const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st);
 
 // 16-bit training path (fgnn_tc_train.cuh): forward keeping what backward needs in `ws`, and the backward of the stack
-size_t embed_train_workspace_bytes(const fgnn_embed_params& p, int G, int N);
-int embed_fwd_train(const fgnn_embed_params& p, int precision, const float* x, float* emb, int G, int N,
+size_t embed_train_workspace_bytes(const fgnn_embed_params& p, int G, int N, bool det);
+int embed_fwd_train(const fgnn_embed_params& p, int precision, bool det, const float* x, float* emb, int G, int N,
                     const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st);
-int embed_bwd(const fgnn_embed_params& p, const fgnn_embed_grads& g, int precision, const float* demb, int grad_scale_log2,
+int embed_bwd(const fgnn_embed_params& p, const fgnn_embed_grads& g, int precision, bool det, const float* demb, int grad_scale_log2,
               int G, int N, const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st);
 
 // fused head: scores (optional) + row-softmax CE + row argmax on tensor cores.  Graph 1 (rows) is padded to N1 with

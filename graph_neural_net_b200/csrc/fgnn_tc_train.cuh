@@ -43,6 +43,13 @@ __device__ __forceinline__ uint32_t valid8(int pj0, int n, const Geo& geo) {
   return m;
 }
 
+// bias-gradient partial of CTA (x, gc): added to bsum[gc] (AtomicSum) or stored to bsum[gc][x] (OrderedSum records)
+template <typename Sum>
+__device__ __forceinline__ void add_bsum(float* bsum, int gc, float t) {
+  if constexpr (Sum::kOrdered) bsum[(long)gc * gridDim.x + blockIdx.x] = t;
+  else atomicAdd(bsum + gc, t);
+}
+
 __device__ __forceinline__ float block_sum(float v, float* s_red) {
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   const int warp = threadIdx.x / 32, lane = threadIdx.x % 32;
@@ -57,8 +64,9 @@ __device__ __forceinline__ float block_sum(float v, float* s_red) {
   return t;   // valid in warp 0
 }
 
-// acc[gc] += (sum dy, sum dy z) over the valid n x n block; dy = dya (+ dyb), layout C; z in layout zmode
-template <typename T>
+// acc[gc] += (sum dy, sum dy z) over the valid n x n block; dy = dya (+ dyb), layout C; z in layout zmode.
+// OrderedSum: CTA (x, gc) stores its pair to acc[gc][x] (records, reduced by the caller).
+template <typename T, typename Sum>
 __global__ void __launch_bounds__(256)
 gn_bwd_stats_kernel(const T* __restrict__ dya, const T* __restrict__ dyb, const T* __restrict__ z, Layout zmode,
                     double* __restrict__ acc, int C, Geo geo, const int32_t* __restrict__ npg) {
@@ -90,8 +98,14 @@ gn_bwd_stats_kernel(const T* __restrict__ dya, const T* __restrict__ dyb, const 
   const float t1 = block_sum(s1, s_red);
   const float t2 = block_sum(s2, s_red);
   if (threadIdx.x == 0) {
-    atomicAdd(acc + 2 * (long)gc, (double)t1);
-    atomicAdd(acc + 2 * (long)gc + 1, (double)t2);
+    if constexpr (Sum::kOrdered) {
+      double* r = acc + 2 * ((long)gc * gridDim.x + blockIdx.x);
+      r[0] = (double)t1;
+      r[1] = (double)t2;
+    } else {
+      atomicAdd(acc + 2 * (long)gc, (double)t1);
+      atomicAdd(acc + 2 * (long)gc + 1, (double)t2);
+    }
   }
 }
 
@@ -132,7 +146,7 @@ __global__ void gn_param_grad_kernel(const double* __restrict__ acc, const float
 
 // dz = a dy + beta z + gamma on the valid block, 0 elsewhere (layout C out, covered rows only);
 // bsum[gc] += sum of the ROUNDED dz (the last conv's bias gradient: zero up to rounding, as in the reference)
-template <typename T>
+template <typename T, typename Sum>
 __global__ void __launch_bounds__(256)
 gn_bwd_apply_kernel(const T* __restrict__ dya, const T* __restrict__ dyb, const T* __restrict__ z, Layout zmode,
                     const float* __restrict__ bc, T* __restrict__ out, float* __restrict__ bsum, int C, Geo geo,
@@ -174,11 +188,11 @@ gn_bwd_apply_kernel(const T* __restrict__ dya, const T* __restrict__ dyb, const 
     }
   }
   const float t = block_sum(ssum, s_red);
-  if (threadIdx.x == 0) atomicAdd(bsum + gc, t);
+  if (threadIdx.x == 0) add_bsum<Sum>(bsum, gc, t);
 }
 
 // ReLU backward in place: pre <- pre * [h > 0]; bsum[gc] += sum of the result (bias gradient of the layer below)
-template <typename T>
+template <typename T, typename Sum>
 __global__ void __launch_bounds__(256)
 relu_mask_kernel(T* __restrict__ pre, const T* __restrict__ h, float* __restrict__ bsum, int C, Geo geo,
                  const int32_t* __restrict__ npg) {
@@ -200,11 +214,11 @@ relu_mask_kernel(T* __restrict__ pre, const T* __restrict__ h, float* __restrict
     *reinterpret_cast<uint4*>(pre + oc) = pack8<T>(p);
   }
   const float t = block_sum(s, s_red);
-  if (threadIdx.x == 0) atomicAdd(bsum + gc, t);
+  if (threadIdx.x == 0) add_bsum<Sum>(bsum, gc, t);
 }
 
 // bsum[gc] = sum of a layout-C plane (bias gradient of a layer whose output gradient needs no mask)
-template <typename T>
+template <typename T, typename Sum>
 __global__ void __launch_bounds__(256)
 plane_sum_kernel(const T* __restrict__ x, float* __restrict__ bsum, int C, Geo geo, const int32_t* __restrict__ npg) {
   __shared__ float s_red[8];
@@ -218,7 +232,7 @@ plane_sum_kernel(const T* __restrict__ x, float* __restrict__ bsum, int C, Geo g
     for (int e = 0; e < 8; ++e) s += p[e];
   }
   const float t = block_sum(s, s_red);
-  if (threadIdx.x == 0) atomicAdd(bsum + gc, t);
+  if (threadIdx.x == 0) add_bsum<Sum>(bsum, gc, t);
 }
 
 // rowsum[gc][i] = sum_j x[i][j] (valid block), one warp per row
@@ -409,6 +423,8 @@ __global__ void wgrad_combine_first_kernel(CombineFirstArgs a) {
 //   64 pixels x channels, rows beyond the channel count zero-filled by the tensor map), M = 128, N = Nw, fp32
 //   accumulation in TMEM over the CTA's pixel range, atomicAdd of the accumulator tile at the end.
 //   Work item = (graph, split of its pixel range); out_stride_g = 0 accumulates all graphs into one matrix.
+//   OrderedSum: every item stores its tile to its own record out[item][co][Nw] (zeros for an empty pixel range) with
+//   plain stores, and launch_wgrad sums the records in item order.
 // Warp roles: warp 0 = TMA producer, warp 1 = MMA issuer, warps 2-5 = epilogue.
 // =============================================================================================
 struct WgradArgs {
@@ -427,7 +443,7 @@ constexpr int kWgMaxStages = 16;
 constexpr size_t kWgRingBytes = 160 * 1024;
 constexpr size_t kWgSmemBytes = kWgRingBytes + 128 * 128 + (2 * kWgMaxStages + 4) * 8 + 16;   // + slack the last stage's 128-row read may touch
 
-template <typename T>
+template <typename T, typename Sum>
 __global__ void __launch_bounds__(192, 1)
 tc_wgrad_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b0,
                 const __grid_constant__ CUtensorMap map_b1, const WgradArgs args) {
@@ -533,7 +549,26 @@ tc_wgrad_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant
       mbar_wait(&tmem_full[as], aphase);
       tc_fence_after();
       const int r = quad * 32 + lane;
-      if (hi > lo && quad * 32 < args.co) {          // warp-uniform
+      if constexpr (Sum::kOrdered) {
+        if (quad * 32 < args.co) {                   // warp-uniform
+          const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(as * 128);
+          float4* dst = reinterpret_cast<float4*>(args.out + ((long)item * args.co + r) * Nw);
+#pragma unroll 1
+          for (int c0 = 0; c0 < Nw; c0 += 16) {
+            uint32_t rr[16] = {0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u};
+            if (hi > lo) {                           // warp-uniform; an empty range leaves the accumulator unwritten
+              tmem_ld16(taddr + (uint32_t)c0, rr);
+              tmem_wait_ld();
+            }
+            if (r < args.co) {
+#pragma unroll
+              for (int u = 0; u < 4; ++u)
+                dst[c0 / 4 + u] = make_float4(__uint_as_float(rr[4 * u]), __uint_as_float(rr[4 * u + 1]),
+                                              __uint_as_float(rr[4 * u + 2]), __uint_as_float(rr[4 * u + 3]));
+            }
+          }
+        }
+      } else if (hi > lo && quad * 32 < args.co) {          // warp-uniform
         const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(as * 128);
         float* dst = args.out + (long)g * args.out_stride_g + (long)r * Nw;
 #pragma unroll 1
@@ -808,9 +843,18 @@ tc_bmm_bwd_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
 // =============================================================================================
 // host side of the training path
 // =============================================================================================
+// pixel splits per graph of the weight-gradient GEMM (about two work items per SM)
+int wgrad_splits(int G, const Geo& geo) {
+  const int steps = (int)((geo.PSC + 63) / 64);
+  return std::max(1, std::min(steps / 8, ceil_div(2 * num_sms(), G)));
+}
+
+// out (+)= the weight-gradient GEMM; rec: deterministic mode, room for G * wgrad_splits(G) records of co x Nw floats
+// (the kernel stores each work item's tile there and out is OVERWRITTEN with their fixed-order sum), or null (atomics
+// into out, which the caller has zeroed)
 template <typename T>
 int launch_wgrad(const T* gplanes, int co, const T* src0, int c0, const T* src1, int c1, float* out, long out_stride_g,
-                 int G, const Geo& geo, const int32_t* npg, cudaStream_t st) {
+                 int G, const Geo& geo, const int32_t* npg, float* rec, cudaStream_t st) {
   const int k0 = round_up(c0, 16), k1 = src1 ? round_up(c1, 16) : 0;
   FGNN_CHECK_ARG(co <= 128 && k0 + k1 <= 128, "weight-gradient GEMM supports <= 128 channels per side (got %d x %d)", co, k0 + k1);
   CUtensorMap ma, mb0, mb1;
@@ -823,23 +867,33 @@ int launch_wgrad(const T* gplanes, int co, const T* src0, int c0, const T* src1,
   }
   WgradArgs a{};
   a.G = G;
-  const int steps = (int)((geo.PSC + 63) / 64);
-  a.S = std::max(1, std::min(steps / 8, ceil_div(2 * num_sms(), G)));
+  a.S = wgrad_splits(G, geo);
   a.co = co;
   a.Nw = k0 + k1;
   a.k0 = k0;
   a.nsrc = src1 ? 2 : 1;
-  a.out = out;
+  a.out = rec ? rec : out;
   a.out_stride_g = out_stride_g;
   a.geo = geo;
   a.n_per_graph = npg;
-  FGNN_CUDA(cudaFuncSetAttribute(tc_wgrad_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWgSmemBytes));
   const int grid = std::min(num_sms(), G * a.S);
+  if (!rec) {
+    FGNN_CUDA(cudaFuncSetAttribute(tc_wgrad_kernel<T, AtomicSum>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWgSmemBytes));
+    prof::begin(prof::kGlue, st);
+    tc_wgrad_kernel<T, AtomicSum><<<grid, 192, kWgSmemBytes, st>>>(ma, mb0, mb1, a);
+    prof::end(prof::kGlue, st);
+    FGNN_LAUNCHED();
+    return FGNN_OK;
+  }
+  FGNN_CUDA(cudaFuncSetAttribute(tc_wgrad_kernel<T, OrderedSum>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWgSmemBytes));
   prof::begin(prof::kGlue, st);
-  tc_wgrad_kernel<T><<<grid, 192, kWgSmemBytes, st>>>(ma, mb0, mb1, a);
-  prof::end(prof::kGlue, st);
+  tc_wgrad_kernel<T, OrderedSum><<<grid, 192, kWgSmemBytes, st>>>(ma, mb0, mb1, a);
   FGNN_LAUNCHED();
-  return FGNN_OK;
+  // per graph over its splits (first layers: out [G][co][Nw]), or over all items in (graph, split) order (one matrix)
+  const int w = co * a.Nw;
+  const int ret = out_stride_g ? sum_records(rec, out, (long)G * w, a.S, w, false, st) : sum_records(rec, out, w, G * a.S, w, false, st);
+  prof::end(prof::kGlue, st);
+  return ret;
 }
 
 // mode 1: out = alpha (a b^T) + beta rowsum, a = dM (layout C), b = Y2 (layout B);  mode 2: out = alpha (a^T b) + beta colsum,
@@ -895,6 +949,7 @@ struct TrainPlan {
   int G;            // graphs of one pass: the whole batch on keep-all, `chunk` on recompute (pass_plan lowers it for a short last pass)
   int batch;        // graphs of the call
   bool recompute;
+  bool det;         // deterministic mode: OrderedSum kernels, and room for their records in the carve
 };
 
 // 16-bit training keeps every activation of a pass in its workspace, and a pass holds at least one graph (some 15 GB
@@ -921,7 +976,14 @@ struct TrainBuf {
   size_t bwd_begin, bwd_end;
   double* gacc;
   float *bc, *bsum[2], *rowsum, *colsum, *P, *Pglob, *scale;
+  // deterministic mode only (else null): OrderedSum records of the conv-chain statistics, the GraphNorm backward
+  // sums [GC][kPlaneCtas][2], the bias-gradient sums [GC][kPlaneCtas] and the weight-gradient GEMM [items][C][128]
+  double *stat_rec, *gacc_rec;
+  float *bsum_rec, *wg_rec;
 };
+
+// CTAs per plane of the plane reductions (gn_bwd_stats / gn_bwd_apply / relu_mask)
+constexpr int kPlaneCtas = 32;
 
 size_t carve_train(const TrainPlan& tp, Arena& ar, TrainBuf& B) {
   const Geo& geo = tp.geo;
@@ -965,6 +1027,11 @@ size_t carve_train(const TrainPlan& tp, Arena& ar, TrainBuf& B) {
   B.P = ar.take<float>(G * C * 128);
   B.Pglob = ar.take<float>(128 * 128);
   B.scale = ar.take<float>(4);
+  B.stat_rec = tp.det ? ar.take<double>(stat_rec_doubles(tp.G, tp.C, geo)) : nullptr;
+  B.gacc_rec = tp.det ? ar.take<double>(G * C * kPlaneCtas * 2) : nullptr;
+  B.bsum_rec = tp.det ? ar.take<float>(G * C * kPlaneCtas) : nullptr;
+  // a pass of g <= G graphs has g * wgrad_splits(g) < g + 2 num_sms() work items, each at most C x 128
+  B.wg_rec = tp.det ? ar.take<float>((G + 2 * (size_t)num_sms()) * C * 128) : nullptr;
   return align_up(ar.off, 1024);
 }
 
@@ -994,7 +1061,7 @@ size_t keep_all_limit() {
   return t;
 }
 
-int make_train_plan(const fgnn_embed_params& p, int G, int N, TrainPlan& tp) {
+int make_train_plan(const fgnn_embed_params& p, int G, int N, bool det, TrainPlan& tp) {
   if (N > kMaxTrainN)
     return fail(FGNN_ERR_UNSUPPORTED, "16-bit training supports N <= %d (got %d): its workspace holds every activation of at "
                 "least one graph; embed larger graphs with the inference path (N <= %d)", kMaxTrainN, N, kMaxN);
@@ -1008,6 +1075,7 @@ int make_train_plan(const fgnn_embed_params& p, int G, int N, TrainPlan& tp) {
   tp.G = G;
   tp.batch = G;
   tp.recompute = false;
+  tp.det = det;
   tp.D = p.block[0].mlp1.depth;
   for (int b = 0; b < p.num_blocks; ++b) {
     const fgnn_block_params& bp = p.block[b];
@@ -1125,6 +1193,7 @@ int run_conv(const ConvCall<T>& cc, const TrainPlan& tp, const TrainBuf& B, cons
   M.bf = B.bf;
   M.wh = nullptr;
   M.stat_acc = B.stat_acc;
+  M.stat_rec = B.stat_rec;
   M.relu_out = cc.relu;
   M.no_coef = cc.gn[0] == nullptr;
   return run_mlp_group<T>(M, tp.C, tp.G, tp.geo, npg, st);
@@ -1209,10 +1278,10 @@ int train_fwd_pass(const fgnn_embed_params& p, const TrainPlan& tp, const TrainB
 }
 
 template <typename T>
-int embed_fwd_train_t(const fgnn_embed_params& p, const float* x, float* emb, int G, int N, const int32_t* npg, void* ws,
+int embed_fwd_train_t(const fgnn_embed_params& p, bool det, const float* x, float* emb, int G, int N, const int32_t* npg, void* ws,
                       size_t ws_bytes, cudaStream_t st) {
   TrainPlan tp;
-  if (int e = make_train_plan(p, G, N, tp)) return e;
+  if (int e = make_train_plan(p, G, N, det, tp)) return e;
   Arena ar(ws, ws_bytes);
   TrainBuf B;
   const size_t need = carve_train(tp, ar, B);
@@ -1262,26 +1331,41 @@ int mlp_bwd(const MlpBwd<T>& a, const TrainPlan& tp, const TrainBuf& B, const in
   const Geo& geo = tp.geo;
   const int G = tp.G, C = tp.C, D = tp.D;
   const int GC = G * C;
-  const dim3 pgrid((unsigned)std::max<long>(1, std::min<long>(32, (geo.PSC / 8 + 255) / 256)), GC);
-  FGNN_CUDA(cudaMemsetAsync(B.gacc, 0, (size_t)GC * 2 * sizeof(double), st));
+  const dim3 pgrid((unsigned)std::max<long>(1, std::min<long>(kPlaneCtas, (geo.PSC / 8 + 255) / 256)), GC);
+  const bool det = tp.det;
+  // bias-gradient sums of the plane kernels: atomics into bsum[bi] (zeroed), or records reduced into it
+  auto bsum_begin = [&](int bi) -> int {
+    if (!det) FGNN_CUDA(cudaMemsetAsync(B.bsum[bi], 0, (size_t)GC * sizeof(float), st));
+    return FGNN_OK;
+  };
+  auto bsum_end = [&](int bi) -> int { return det ? sum_records(B.bsum_rec, B.bsum[bi], GC, (int)pgrid.x, 1, false, st) : FGNN_OK; };
   prof::begin(prof::kStats, st);
-  gn_bwd_stats_kernel<T><<<pgrid, 256, 0, st>>>(a.dya, a.dyb, a.z, a.zmode, B.gacc, C, geo, npg);
-  FGNN_LAUNCHED();
+  if (det) {
+    gn_bwd_stats_kernel<T, OrderedSum><<<pgrid, 256, 0, st>>>(a.dya, a.dyb, a.z, a.zmode, B.gacc_rec, C, geo, npg);
+    FGNN_LAUNCHED();
+    if (int e = sum_records(B.gacc_rec, B.gacc, (long)GC * 2, (int)pgrid.x, 2, false, st)) return e;
+  } else {
+    FGNN_CUDA(cudaMemsetAsync(B.gacc, 0, (size_t)GC * 2 * sizeof(double), st));
+    gn_bwd_stats_kernel<T, AtomicSum><<<pgrid, 256, 0, st>>>(a.dya, a.dyb, a.z, a.zmode, B.gacc, C, geo, npg);
+    FGNN_LAUNCHED();
+  }
   gn_bwd_coef_kernel<<<ceil_div(GC, 256), 256, 0, st>>>(B.gacc, a.coef, a.gnstat, B.bc, C, geo.N, npg, GC);
   FGNN_LAUNCHED();
   gn_param_grad_kernel<<<ceil_div(C, 64), 64, 0, st>>>(B.gacc, a.gnstat, a.gr->gn_w, a.gr->gn_b, B.scale, G, C, a.co_real);
   FGNN_LAUNCHED();
   int bi = 0;                                           // bsum[bi] = per-(graph, channel) sum of the current gradient
-  FGNN_CUDA(cudaMemsetAsync(B.bsum[bi], 0, (size_t)GC * sizeof(float), st));
-  gn_bwd_apply_kernel<T><<<pgrid, 256, 0, st>>>(a.dya, a.dyb, a.z, a.zmode, B.bc, a.bufs[0], B.bsum[bi], C, geo, npg);
+  if (int e = bsum_begin(bi)) return e;
+  if (det) gn_bwd_apply_kernel<T, OrderedSum><<<pgrid, 256, 0, st>>>(a.dya, a.dyb, a.z, a.zmode, B.bc, a.bufs[0], B.bsum_rec, C, geo, npg);
+  else gn_bwd_apply_kernel<T, AtomicSum><<<pgrid, 256, 0, st>>>(a.dya, a.dyb, a.z, a.zmode, B.bc, a.bufs[0], B.bsum[bi], C, geo, npg);
   FGNN_LAUNCHED();
+  if (int e = bsum_end(bi)) return e;
   prof::end(prof::kStats, st);
   T* curg = a.bufs[0];
   for (int l = D - 1; l >= 1; --l) {
     const T* hin = reinterpret_cast<const T*>(a.H[l - 1]);
     // weight / bias gradient of layer l (all graphs into one matrix)
-    FGNN_CUDA(cudaMemsetAsync(B.Pglob, 0, 128 * 128 * sizeof(float), st));
-    if (int e = launch_wgrad<T>(curg, C, hin, C, nullptr, 0, B.Pglob, 0, G, geo, npg, st)) return e;
+    if (!det) FGNN_CUDA(cudaMemsetAsync(B.Pglob, 0, 128 * 128 * sizeof(float), st));
+    if (int e = launch_wgrad<T>(curg, C, hin, C, nullptr, 0, B.Pglob, 0, G, geo, npg, B.wg_rec, st)) return e;
     wgrad_combine_hidden_kernel<<<ceil_div(C * C, 256), 256, 0, st>>>(B.Pglob, round_up(C, 16), B.bsum[bi], a.gr->w[l], a.gr->b[l],
                                                                       B.scale, G, C, a.co_real, a.co_real);
     FGNN_LAUNCHED();
@@ -1295,20 +1379,22 @@ int mlp_bwd(const MlpBwd<T>& a, const TrainPlan& tp, const TrainBuf& B, const in
     cc.out[0] = nxt;
     if (int e = run_conv<T>(cc, tp, B, npg, st)) return e;
     bi ^= 1;
-    FGNN_CUDA(cudaMemsetAsync(B.bsum[bi], 0, (size_t)GC * sizeof(float), st));
+    if (int e = bsum_begin(bi)) return e;
     prof::begin(prof::kStats, st);
-    relu_mask_kernel<T><<<pgrid, 256, 0, st>>>(nxt, hin, B.bsum[bi], C, geo, npg);
-    prof::end(prof::kStats, st);
+    if (det) relu_mask_kernel<T, OrderedSum><<<pgrid, 256, 0, st>>>(nxt, hin, B.bsum_rec, C, geo, npg);
+    else relu_mask_kernel<T, AtomicSum><<<pgrid, 256, 0, st>>>(nxt, hin, B.bsum[bi], C, geo, npg);
     FGNN_LAUNCHED();
+    if (int e = bsum_end(bi)) return e;
+    prof::end(prof::kStats, st);
     curg = nxt;
   }
   // first layer: per-graph pixel GEMM, combined through the per-graph GraphNorm fold of the sources
   {
     const int k0 = round_up(a.c_src[0], 16), k1 = a.nsrc > 1 ? round_up(a.c_src[1], 16) : 0;
     const int Nw = k0 + k1;
-    FGNN_CUDA(cudaMemsetAsync(B.P, 0, (size_t)G * C * Nw * sizeof(float), st));
+    if (!det) FGNN_CUDA(cudaMemsetAsync(B.P, 0, (size_t)G * C * Nw * sizeof(float), st));
     if (int e = launch_wgrad<T>(curg, C, a.src[0], a.c_src[0], a.nsrc > 1 ? a.src[1] : nullptr, a.c_src[1], B.P, (long)C * Nw, G, geo,
-                                npg, st)) return e;
+                                npg, B.wg_rec, st)) return e;
     CombineFirstArgs ca{};
     ca.P = B.P;
     ca.bsum = B.bsum[bi];
@@ -1448,10 +1534,10 @@ int train_bwd_pass(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const
 }
 
 template <typename T>
-int embed_bwd_t(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const float* demb, int grad_scale_log2, int G, int N,
+int embed_bwd_t(const fgnn_embed_params& p, const fgnn_embed_grads& gr, bool det, const float* demb, int grad_scale_log2, int G, int N,
                 const int32_t* npg, void* ws, size_t ws_bytes, cudaStream_t st) {
   TrainPlan tp;
-  if (int e = make_train_plan(p, G, N, tp)) return e;
+  if (int e = make_train_plan(p, G, N, det, tp)) return e;
   Arena ar(ws, ws_bytes);
   TrainBuf B;
   const size_t need = carve_train(tp, ar, B);

@@ -49,6 +49,19 @@ typedef enum {
   FGNN_FP16 = 2   /* same kernels and speed with fp16 operands (8x smaller rounding error)     */
 } fgnn_precision;
 
+/* Deterministic mode: ORed into the `precision` argument of the embedder entry points (fgnn_embed_workspace_bytes,
+ * fgnn_embed_fwd, fgnn_embed_fwd_adjacency_u8, fgnn_embed_train_workspace_bytes, fgnn_embed_fwd_train, fgnn_embed_bwd)
+ * and passed as `flags` to fgnn_mlp_workspace_bytes_ex / fgnn_mlp_bwd_f32_ex.  Every sum whose partials come from
+ * several CTAs (GraphNorm statistics, bias and weight gradients) is then formed from per-CTA records added in a fixed
+ * order instead of floating-point atomics, so that, for the same build, device model, inputs, batch composition,
+ * FGNN_TC_* variables and parameters, the embeddings and parameter gradients are bit-identical from run to run.  Not
+ * covered: a graph alone vs inside a batch, keep-all vs recompute plans (the reduction partitions differ), multi-GPU
+ * all-reduce order.  The workspaces are larger (they hold the records): the workspace query, the forward and the
+ * backward of one training call must all take the same flag, as they must see the same FGNN_TC_* variables.  The fused
+ * head (fgnn_head_*) accepts the bit and ignores it: it is deterministic in both modes.  Any other bit outside the
+ * precision's low byte is rejected (FGNN_ERR_INVALID; workspace queries return 0). */
+#define FGNN_DETERMINISTIC 0x100
+
 #define FGNN_MAX_DEPTH 8
 #define FGNN_MAX_BLOCKS 16
 
@@ -120,6 +133,12 @@ int fgnn_mlp_bwd_f32(const fgnn_mlp_params* p, const fgnn_mlp_grads* g, const fl
                      const float* stats, const float* dy, float* dx, int32_t G, int32_t N,
                      const int32_t* n_per_graph, void* workspace, size_t workspace_bytes,
                      void* stream);
+/* The same with flags: 0 or FGNN_DETERMINISTIC (fixed-order parameter-gradient sums; the backward's workspace must be
+ * sized by fgnn_mlp_workspace_bytes_ex with the same flags).  The two functions above are these with flags 0. */
+size_t fgnn_mlp_workspace_bytes_ex(int32_t G, int32_t c_in, int32_t c_out, int32_t depth, int32_t N, int32_t flags);
+int fgnn_mlp_bwd_f32_ex(const fgnn_mlp_params* p, const fgnn_mlp_grads* g, const float* x, const float* stats,
+                        const float* dy, float* dx, int32_t G, int32_t N, const int32_t* n_per_graph, void* workspace,
+                        size_t workspace_bytes, void* stream, int32_t flags);
 
 /* GraphNorm.forward / normalize (models/layers.py:68-80).  gn_w/gn_b may be NULL (plain
  * normalize).  stats as above (may be NULL).  constant_n: see fgnn_mlp_params. */
