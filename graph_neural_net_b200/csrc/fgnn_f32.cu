@@ -31,12 +31,13 @@ __global__ void transpose_pad_kernel(const float* __restrict__ w, float* __restr
   wt[idx] = (o < co) ? w[o * ci + i] : 0.f;
 }
 
-// out[i][o] = w[i * co + o] for o < co, 0 for the padding columns (row-padded copy)
-__global__ void pad_rows_kernel(const float* __restrict__ w, float* __restrict__ out, int rows, int co, int cop) {
+// out[i][o] = w[i * ld + o] for o < co, 0 for the padding columns (row-padded copy of co columns of a row-major
+// matrix with ld columns)
+__global__ void pad_rows_kernel(const float* __restrict__ w, float* __restrict__ out, int rows, int co, int ld, int cop) {
   int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= rows * cop) return;
   int i = idx / cop, o = idx % cop;
-  out[idx] = (o < co) ? w[i * co + o] : 0.f;
+  out[idx] = (o < co) ? w[i * ld + o] : 0.f;
 }
 
 struct ChainArgs {
@@ -45,6 +46,7 @@ struct ChainArgs {
   int c_in;
   int c_out;
   int cop;                          // padded c_out (multiple of 8)
+  int out_ch, out_off;              // z holds out_ch channels per graph; this chain writes [out_off, out_off + c_out)
   const float* wt[FGNN_MAX_DEPTH];  // (cin_k, cop)
   const float* b[FGNN_MAX_DEPTH];   // (c_out)
 };
@@ -101,7 +103,7 @@ conv_chain_fwd_kernel(ChainArgs a, const float* __restrict__ x, float* __restric
 #pragma unroll
         for (int u = 0; u < 8; ++u)
           if (co0 + u < a.c_out)
-            z[((long)g * a.c_out + co0 + u) * P + p] = valid ? (a.relu_last ? fmaxf(acc[u], 0.f) : acc[u]) : 0.f;
+            z[((long)g * a.out_ch + a.out_off + co0 + u) * P + p] = valid ? (a.relu_last ? fmaxf(acc[u], 0.f) : acc[u]) : 0.f;
       }
     }
     in = out;
@@ -148,80 +150,83 @@ plane_stats_kernel(const float* __restrict__ z, float* __restrict__ stats, int C
   }
 }
 
-// y = gw * (z - mean) * inv + gb on valid positions, 0 elsewhere (in place allowed)
+// y = gw * (z - mean) * inv + gb on valid positions, 0 elsewhere (in place allowed).  blockIdx.y strides over the
+// planes (grid.y is limited to 65535).
 __global__ void normalize_apply_kernel(const float* __restrict__ z, float* __restrict__ y,
                                        const float* __restrict__ stats, const float* __restrict__ gw,
-                                       const float* __restrict__ gb, int C, int N,
+                                       const float* __restrict__ gb, int C, int N, long planes,
                                        const int32_t* __restrict__ n_per_graph) {
-  const int gc = blockIdx.y;
-  const int g = gc / C, c = gc % C;
-  const int n = graph_n(n_per_graph, g, N);
   const long P = (long)N * N;
-  const float mean = stats[2 * gc], inv = stats[2 * gc + 1];
-  const float w = gw ? gw[c] : 1.f, b = gb ? gb[c] : 0.f;
-  for (long p = (long)blockIdx.x * blockDim.x + threadIdx.x; p < P; p += (long)gridDim.x * blockDim.x) {
-    int i = (int)(p / N), j = (int)(p % N);
-    float v = 0.f;
-    if (i < n && j < n) v = w * ((z[(long)gc * P + p] - mean) * inv) + b;
-    y[(long)gc * P + p] = v;
+  for (long gc = blockIdx.y; gc < planes; gc += gridDim.y) {
+    const int g = (int)(gc / C), c = (int)(gc % C);
+    const int n = graph_n(n_per_graph, g, N);
+    const float mean = stats[2 * gc], inv = stats[2 * gc + 1];
+    const float w = gw ? gw[c] : 1.f, b = gb ? gb[c] : 0.f;
+    for (long p = (long)blockIdx.x * blockDim.x + threadIdx.x; p < P; p += (long)gridDim.x * blockDim.x) {
+      int i = (int)(p / N), j = (int)(p % N);
+      float v = 0.f;
+      if (i < n && j < n) v = w * ((z[gc * P + p] - mean) * inv) + b;
+      y[gc * P + p] = v;
+    }
   }
 }
 
 // ---------------------------------------------------------------------------------------
 // batched matmul out[g,c] = op(a[g,c]) @ op(b[g,c]) over the valid corner (layers.py:161-162)
-// 64x64 tile, 256 threads, 4x4 per thread.
+// 64x64 tile, 256 threads, 4x4 per thread.  blockIdx.z strides over the planes (grid.z is limited to 65535).
 // ---------------------------------------------------------------------------------------
 template <bool TA, bool TB>
 __global__ void __launch_bounds__(256)
 matmul_kernel(const float* __restrict__ A, const float* __restrict__ B, float* __restrict__ Cout, int Cch,
-              int N, const int32_t* __restrict__ n_per_graph) {
-  const int gc = blockIdx.z;
-  const int g = gc / Cch;
-  const int n = graph_n(n_per_graph, g, N);
-  const int row0 = blockIdx.y * 64, col0 = blockIdx.x * 64;
-  const float* a = A + (long)gc * N * N;
-  const float* b = B + (long)gc * N * N;
-  float* c = Cout + (long)gc * N * N;
+              int N, long planes, const int32_t* __restrict__ n_per_graph) {
   __shared__ float As[16][64 + 1];
   __shared__ float Bs[16][64 + 1];
   const int tx = threadIdx.x % 16, ty = threadIdx.x / 16;
-  float acc[4][4] = {};
-  if (row0 < n && col0 < n) {
-    for (int k0 = 0; k0 < n; k0 += 16) {
-      for (int e = threadIdx.x; e < 16 * 64; e += 256) {
-        int kk = e / 64, m = e % 64;
-        int r = row0 + m, k = k0 + kk;
-        float v = 0.f;
-        if (r < n && k < n) v = TA ? a[(long)k * N + r] : a[(long)r * N + k];
-        As[kk][m] = v;
-        int cc = col0 + m;
-        float w = 0.f;
-        if (cc < n && k < n) w = TB ? b[(long)cc * N + k] : b[(long)k * N + cc];
-        Bs[kk][m] = w;
+  const int row0 = blockIdx.y * 64, col0 = blockIdx.x * 64;
+  for (long gc = blockIdx.z; gc < planes; gc += gridDim.z) {
+    const int g = (int)(gc / Cch);
+    const int n = graph_n(n_per_graph, g, N);
+    const float* a = A + gc * N * N;
+    const float* b = B + gc * N * N;
+    float* c = Cout + gc * N * N;
+    float acc[4][4] = {};
+    if (row0 < n && col0 < n) {
+      for (int k0 = 0; k0 < n; k0 += 16) {
+        for (int e = threadIdx.x; e < 16 * 64; e += 256) {
+          int kk = e / 64, m = e % 64;
+          int r = row0 + m, k = k0 + kk;
+          float v = 0.f;
+          if (r < n && k < n) v = TA ? a[(long)k * N + r] : a[(long)r * N + k];
+          As[kk][m] = v;
+          int cc = col0 + m;
+          float w = 0.f;
+          if (cc < n && k < n) w = TB ? b[(long)cc * N + k] : b[(long)k * N + cc];
+          Bs[kk][m] = w;
+        }
+        __syncthreads();
+#pragma unroll
+        for (int kk = 0; kk < 16; ++kk) {
+          float av[4], bv[4];
+#pragma unroll
+          for (int u = 0; u < 4; ++u) av[u] = As[kk][ty * 4 + u];
+#pragma unroll
+          for (int u = 0; u < 4; ++u) bv[u] = Bs[kk][tx * 4 + u];
+#pragma unroll
+          for (int u = 0; u < 4; ++u)
+#pragma unroll
+            for (int v = 0; v < 4; ++v) acc[u][v] = fmaf(av[u], bv[v], acc[u][v]);
+        }
+        __syncthreads();
       }
-      __syncthreads();
-#pragma unroll
-      for (int kk = 0; kk < 16; ++kk) {
-        float av[4], bv[4];
-#pragma unroll
-        for (int u = 0; u < 4; ++u) av[u] = As[kk][ty * 4 + u];
-#pragma unroll
-        for (int u = 0; u < 4; ++u) bv[u] = Bs[kk][tx * 4 + u];
-#pragma unroll
-        for (int u = 0; u < 4; ++u)
-#pragma unroll
-          for (int v = 0; v < 4; ++v) acc[u][v] = fmaf(av[u], bv[v], acc[u][v]);
-      }
-      __syncthreads();
     }
+#pragma unroll
+    for (int u = 0; u < 4; ++u)
+#pragma unroll
+      for (int v = 0; v < 4; ++v) {
+        int r = row0 + ty * 4 + u, cc = col0 + tx * 4 + v;
+        if (r < N && cc < N) c[(long)r * N + cc] = (r < n && cc < n) ? acc[u][v] : 0.f;
+      }
   }
-#pragma unroll
-  for (int u = 0; u < 4; ++u)
-#pragma unroll
-    for (int v = 0; v < 4; ++v) {
-      int r = row0 + ty * 4 + u, cc = col0 + tx * 4 + v;
-      if (r < N && cc < N) c[(long)r * N + cc] = (r < n && cc < n) ? acc[u][v] : 0.f;
-    }
 }
 
 // ---------------------------------------------------------------------------------------
@@ -440,34 +445,38 @@ int run_conv1x1(const float* w, const float* b, int c_in, int c_out, bool transp
                 float* y, float* wt_scratch, int G, int N, const int32_t* n_per_graph, cudaStream_t st) {
   // y[g,co,p] = sum_ci W'[co,ci] x[g,ci,p] (+ b[co]) (optionally ReLU) on valid pixels, 0 elsewhere.
   // transpose_w: W' = w^T where w is stored (c_in, c_out) row-major, i.e. the backward-data conv.
-  ChainArgs a;
-  a.relu_last = relu ? 1 : 0;
-  a.depth = 1;
-  a.c_in = c_in;
-  a.c_out = c_out;
-  a.cop = (c_out + 7) / 8 * 8;
-  const int total = c_in * a.cop;
-  if (!transpose_w) {
-    transpose_pad_kernel<<<ceil_div(total, 256), 256, 0, st>>>(w, wt_scratch, c_out, c_in, a.cop);
-  } else {
-    // w is (c_in rows, c_out cols): already "wt" up to row padding -> transpose_pad of its transpose == pad rows
-    // implemented as transpose_pad with swapped roles: out[i][o] = w[i*c_out + o]
-    pad_rows_kernel<<<ceil_div(total, 256), 256, 0, st>>>(w, wt_scratch, c_in, c_out, a.cop);
-  }
-  FGNN_LAUNCHED();
-  a.wt[0] = wt_scratch;
-  a.b[0] = b;
-  const size_t smem = (size_t)2 * a.cop * kPixThreads * sizeof(float);
+  // The chain kernel keeps at most kMaxC output channels in shared memory, so a wider c_out (the backward-data conv of
+  // an MLP whose input is wider than kMaxC) runs in slices of kMaxC output channels.  Each output channel's sum is
+  // formed alone, in ascending ci, so the slicing does not change a single bit.
   // set on every call: the attribute is per device and the call is cheap (a process may drive several GPUs)
-  {
-    FGNN_CUDA(cudaFuncSetAttribute(conv_chain_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                   2 * kMaxC * kPixThreads * (int)sizeof(float)));
+  FGNN_CUDA(cudaFuncSetAttribute(conv_chain_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 2 * kMaxC * kPixThreads * (int)sizeof(float)));
+  const long P = (long)N * N;
+  const dim3 grid((unsigned)((P + kPixThreads - 1) / kPixThreads), G);
+  for (int s0 = 0; s0 < c_out; s0 += kMaxC) {
+    ChainArgs a;
+    a.relu_last = relu ? 1 : 0;
+    a.depth = 1;
+    a.c_in = c_in;
+    a.c_out = std::min(kMaxC, c_out - s0);
+    a.cop = (a.c_out + 7) / 8 * 8;
+    a.out_ch = c_out;
+    a.out_off = s0;
+    const int total = c_in * a.cop;
+    if (!transpose_w) {
+      // rows [s0, s0 + a.c_out) of w (c_out, c_in)
+      transpose_pad_kernel<<<ceil_div(total, 256), 256, 0, st>>>(w + (long)s0 * c_in, wt_scratch, a.c_out, c_in, a.cop);
+    } else {
+      // w is (c_in rows, c_out cols): its columns [s0, s0 + a.c_out) are already "wt" up to the row padding
+      pad_rows_kernel<<<ceil_div(total, 256), 256, 0, st>>>(w + s0, wt_scratch, c_in, a.c_out, c_out, a.cop);
+    }
+    FGNN_LAUNCHED();
+    a.wt[0] = wt_scratch;
+    a.b[0] = b ? b + s0 : nullptr;
+    const size_t smem = (size_t)2 * a.cop * kPixThreads * sizeof(float);
+    conv_chain_fwd_kernel<<<grid, kPixThreads, smem, st>>>(a, x, y, N, n_per_graph);
+    FGNN_LAUNCHED();
   }
-  FGNN_CHECK_ARG(c_out <= kMaxC, "conv1x1: c_out %d unsupported (max %d)", c_out, kMaxC);
-  long P = (long)N * N;
-  dim3 grid((unsigned)((P + kPixThreads - 1) / kPixThreads), G);
-  conv_chain_fwd_kernel<<<grid, kPixThreads, smem, st>>>(a, x, y, N, n_per_graph);
-  FGNN_LAUNCHED();
   return FGNN_OK;
 }
 
@@ -500,6 +509,8 @@ static int prepare_chain(const fgnn_mlp_params& p, ChainArgs& a, Arena& ar, cuda
   a.c_in = p.c_in;
   a.c_out = p.c_out;
   a.cop = (p.c_out + 7) / 8 * 8;
+  a.out_ch = p.c_out;
+  a.out_off = 0;
   for (int k = 0; k < p.depth; ++k) {
     FGNN_CHECK_ARG(p.w[k] && p.b[k], "null weight/bias for layer %d", k);
     const int cin = (k == 0) ? p.c_in : p.c_out;
@@ -521,8 +532,9 @@ int graphnorm_fwd(const float* x, float* y, float* stats, const float* gw, const
   plane_stats_kernel<<<G * C, 256, 0, st>>>(x, stats, C, N, n_per_graph, eps, constant_n);
   FGNN_LAUNCHED();
   long P = (long)N * N;
-  dim3 grid((unsigned)min((long)64, (P + 255) / 256), G * C);
-  normalize_apply_kernel<<<grid, 256, 0, st>>>(x, y, stats, gw, gb, C, N, n_per_graph);
+  const long planes = (long)G * C;
+  dim3 grid((unsigned)min((long)64, (P + 255) / 256), (unsigned)min(planes, 65535L));
+  normalize_apply_kernel<<<grid, 256, 0, st>>>(x, y, stats, gw, gb, C, N, planes, n_per_graph);
   FGNN_LAUNCHED();
   return FGNN_OK;
 }
@@ -551,12 +563,12 @@ int matmul_fwd(const float* a, const float* b, float* out, int G, int C, int N,
                const int32_t* n_per_graph, cudaStream_t st, bool ta, bool tb) {
   if (int e = check_dims(G, C, N)) return e;
   FGNN_CHECK_ARG(a && b && out, "null pointer");
-  FGNN_CHECK_ARG((long)G * C <= 65535L * 1, "G*C=%ld exceeds grid.z limit; split the batch", (long)G * C);
-  dim3 grid(ceil_div(N, 64), ceil_div(N, 64), G * C);
-  if (!ta && !tb) matmul_kernel<false, false><<<grid, 256, 0, st>>>(a, b, out, C, N, n_per_graph);
-  else if (ta && !tb) matmul_kernel<true, false><<<grid, 256, 0, st>>>(a, b, out, C, N, n_per_graph);
-  else if (!ta && tb) matmul_kernel<false, true><<<grid, 256, 0, st>>>(a, b, out, C, N, n_per_graph);
-  else matmul_kernel<true, true><<<grid, 256, 0, st>>>(a, b, out, C, N, n_per_graph);
+  const long planes = (long)G * C;
+  dim3 grid(ceil_div(N, 64), ceil_div(N, 64), (unsigned)min(planes, 65535L));
+  if (!ta && !tb) matmul_kernel<false, false><<<grid, 256, 0, st>>>(a, b, out, C, N, planes, n_per_graph);
+  else if (ta && !tb) matmul_kernel<true, false><<<grid, 256, 0, st>>>(a, b, out, C, N, planes, n_per_graph);
+  else if (!ta && tb) matmul_kernel<false, true><<<grid, 256, 0, st>>>(a, b, out, C, N, planes, n_per_graph);
+  else matmul_kernel<true, true><<<grid, 256, 0, st>>>(a, b, out, C, N, planes, n_per_graph);
   FGNN_LAUNCHED();
   return FGNN_OK;
 }

@@ -6,7 +6,8 @@
 namespace fgnn {
 namespace f32 {
 
-// single 1x1 conv layer (shared by forward recomputation and backward-data in fgnn_f32_bwd.cu)
+// single 1x1 conv layer (shared by forward recomputation and backward-data in fgnn_f32_bwd.cu); any c_out, run in
+// slices of at most 128 output channels.  wt_scratch: c_in * round_up(min(c_out, 128), 8) floats.
 int run_conv1x1(const float* w, const float* b, int c_in, int c_out, bool transpose_w, bool relu, const float* x,
                 float* y, float* wt_scratch, int G, int N, const int32_t* n_per_graph, cudaStream_t st);
 

@@ -62,25 +62,27 @@ gn_bwd_stats_kernel(const float* __restrict__ dy, const float* __restrict__ z, c
   }
 }
 
-// dz = gw * inv * (dy - a1/cnt - (z - mu) * (a2/cnt) * 4 n inv^2) on valid pixels, 0 elsewhere (in place on dy ok)
+// dz = gw * inv * (dy - a1/cnt - (z - mu) * (a2/cnt) * 4 n inv^2) on valid pixels, 0 elsewhere (in place on dy ok).
+// blockIdx.y strides over the planes (grid.y is limited to 65535).
 __global__ void gn_bwd_apply_kernel(const float* __restrict__ dy, const float* __restrict__ z,
                                     const float* __restrict__ stats, const float* __restrict__ sums,
-                                    const float* __restrict__ gw, float* __restrict__ dz, int C, int N,
+                                    const float* __restrict__ gw, float* __restrict__ dz, int C, int N, long planes,
                                     const int32_t* __restrict__ n_per_graph, int constant_n) {
-  const int gc = blockIdx.y;
-  const int g = gc / C, c = gc % C;
-  const int n = graph_n(n_per_graph, g, N);
   const long P = (long)N * N;
-  const float mu = stats[2 * gc], inv = stats[2 * gc + 1];
-  const float cnt = (float)n * (float)n;
-  const float m1 = sums[2 * gc] / cnt;
-  const float m2 = sums[2 * gc + 1] / cnt * 4.f * (float)(constant_n ? N : n) * inv * inv;   // mean(g (z-mu)) / (var + eps)
-  const float w = (gw ? gw[c] : 1.f) * inv;
-  for (long p = (long)blockIdx.x * blockDim.x + threadIdx.x; p < P; p += (long)gridDim.x * blockDim.x) {
-    int i = (int)(p / N), j = (int)(p % N);
-    float v = 0.f;
-    if (i < n && j < n) v = w * (dy[(long)gc * P + p] - m1 - (z[(long)gc * P + p] - mu) * m2);
-    dz[(long)gc * P + p] = v;
+  for (long gc = blockIdx.y; gc < planes; gc += gridDim.y) {
+    const int g = (int)(gc / C), c = (int)(gc % C);
+    const int n = graph_n(n_per_graph, g, N);
+    const float mu = stats[2 * gc], inv = stats[2 * gc + 1];
+    const float cnt = (float)n * (float)n;
+    const float m1 = sums[2 * gc] / cnt;
+    const float m2 = sums[2 * gc + 1] / cnt * 4.f * (float)(constant_n ? N : n) * inv * inv;   // mean(g (z-mu)) / (var + eps)
+    const float w = (gw ? gw[c] : 1.f) * inv;
+    for (long p = (long)blockIdx.x * blockDim.x + threadIdx.x; p < P; p += (long)gridDim.x * blockDim.x) {
+      int i = (int)(p / N), j = (int)(p % N);
+      float v = 0.f;
+      if (i < n && j < n) v = w * (dy[gc * P + p] - m1 - (z[gc * P + p] - mu) * m2);
+      dz[gc * P + p] = v;
+    }
   }
 }
 
@@ -187,8 +189,9 @@ int mlp_bwd(const fgnn_mlp_params& p, const fgnn_mlp_grads& gr, const float* x, 
       FGNN_LAUNCHED();
     }
     {
-      dim3 grid((unsigned)std::min<long>(64, (P + 255) / 256), gc * Co);
-      gn_bwd_apply_kernel<<<grid, 256, 0, st>>>(dyc, h[depth - 1], stc, smc, p.gn_w, dcur, Co, N, n_c, p.constant_n);
+      const long planes = (long)gc * Co;
+      dim3 grid((unsigned)std::min<long>(64, (P + 255) / 256), (unsigned)std::min<long>(planes, 65535));
+      gn_bwd_apply_kernel<<<grid, 256, 0, st>>>(dyc, h[depth - 1], stc, smc, p.gn_w, dcur, Co, N, planes, n_c, p.constant_n);
       FGNN_LAUNCHED();
     }
     // 3. layers in reverse

@@ -141,7 +141,7 @@ int fgnn_mlp_bwd_f32_ex(const fgnn_mlp_params* p, const fgnn_mlp_grads* g, const
                         size_t workspace_bytes, void* stream, int32_t flags);
 
 /* GraphNorm.forward / normalize (models/layers.py:68-80).  gn_w/gn_b may be NULL (plain
- * normalize).  stats as above (may be NULL).  constant_n: see fgnn_mlp_params. */
+ * normalize).  stats (G,C,2) as above, required: the normalisation reads it back.  constant_n: see fgnn_mlp_params. */
 int fgnn_graphnorm_fwd_f32(const float* x, float* y, float* stats, const float* gn_w,
                            const float* gn_b, float eps, int32_t constant_n, int32_t G, int32_t C, int32_t N,
                            const int32_t* n_per_graph, void* stream);
