@@ -21,6 +21,7 @@ FGNN_MAX_BLOCKS = 16
 FP32, BF16, FP16 = 0, 1, 2
 PRECISIONS = {"fp32": FP32, "bf16": BF16, "fp16": FP16}
 FGNN_DETERMINISTIC = 0x100   # ORed into `precision` / passed as `flags`: fixed-order sums instead of atomics
+FGNN_CHECKPOINT_BLOCKS = 0x400   # ORed into `precision` of the 16-bit training calls: block-level checkpoints
 
 c_float_p = C.POINTER(C.c_float)
 

@@ -137,6 +137,12 @@ bool split_precision(int32_t arg, int* precision, bool* det) {
   return (arg & ~(0xFF | FGNN_DETERMINISTIC)) == 0;
 }
 
+// the same for the 16-bit training entry points, which also take FGNN_CHECKPOINT_BLOCKS
+bool split_train_precision(int32_t arg, int* precision, bool* det, bool* ckpt) {
+  *ckpt = (arg & FGNN_CHECKPOINT_BLOCKS) != 0;
+  return split_precision(arg & ~FGNN_CHECKPOINT_BLOCKS, precision, det);
+}
+
 int check_embed(const fgnn_embed_params* p, int G, int N) {
   FGNN_CHECK_ARG(p != nullptr, "null params");
   FGNN_CHECK_ARG(p->num_blocks >= 1 && p->num_blocks <= FGNN_MAX_BLOCKS, "num_blocks %d out of range", p->num_blocks);
@@ -376,30 +382,32 @@ int fgnn_embed_fwd_adjacency_u8(const fgnn_embed_params* p, int32_t precision_fl
 
 size_t fgnn_embed_train_workspace_bytes(const fgnn_embed_params* p, int32_t precision_flags, int32_t G, int32_t N) {
   int precision;
-  bool det;
-  if (!split_precision(precision_flags, &precision, &det)) return 0;
+  bool det, ckpt;
+  if (!split_train_precision(precision_flags, &precision, &det, &ckpt)) return 0;
   if (!p || p->num_blocks < 1 || p->num_blocks > FGNN_MAX_BLOCKS || G < 1 || N < 1) return 0;
   if (precision != FGNN_BF16 && precision != FGNN_FP16) return 0;
-  return tc::embed_train_workspace_bytes(*p, G, N, det);
+  return tc::embed_train_workspace_bytes(*p, G, N, det, ckpt);
 }
 
 int fgnn_embed_fwd_train(const fgnn_embed_params* p, int32_t precision_flags, const float* x, float* emb, int32_t G,
                          int32_t N, const int32_t* n_per_graph, void* workspace, size_t workspace_bytes,
                          void* stream) {
   int precision;
-  bool det;
-  FGNN_CHECK_ARG(split_precision(precision_flags, &precision, &det), "unknown precision flags 0x%x", (unsigned)precision_flags);
+  bool det, ckpt;
+  FGNN_CHECK_ARG(split_train_precision(precision_flags, &precision, &det, &ckpt), "unknown precision flags 0x%x",
+                 (unsigned)precision_flags);
   if (int e = check_embed(p, G, N)) return e;
   FGNN_CHECK_ARG(x && emb && workspace, "null pointer");
-  return tc::embed_fwd_train(*p, precision, det, x, emb, G, N, n_per_graph, workspace, workspace_bytes, (cudaStream_t)stream);
+  return tc::embed_fwd_train(*p, precision, det, ckpt, x, emb, G, N, n_per_graph, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 int fgnn_embed_bwd(const fgnn_embed_params* p, const fgnn_embed_grads* grads, int32_t precision_flags, const float* demb,
                    int32_t grad_scale_log2, int32_t G, int32_t N, const int32_t* n_per_graph, void* workspace,
                    size_t workspace_bytes, void* stream) {
   int precision;
-  bool det;
-  FGNN_CHECK_ARG(split_precision(precision_flags, &precision, &det), "unknown precision flags 0x%x", (unsigned)precision_flags);
+  bool det, ckpt;
+  FGNN_CHECK_ARG(split_train_precision(precision_flags, &precision, &det, &ckpt), "unknown precision flags 0x%x",
+                 (unsigned)precision_flags);
   if (int e = check_embed(p, G, N)) return e;
   FGNN_CHECK_ARG(grads && demb && workspace, "null pointer");
   FGNN_CHECK_ARG(grads->num_blocks == p->num_blocks, "grads describe %d blocks, params %d", grads->num_blocks, p->num_blocks);
@@ -410,7 +418,7 @@ int fgnn_embed_bwd(const fgnn_embed_params* p, const fgnn_embed_grads* grads, in
       for (int l = 0; l < mp[m]->depth; ++l)
         FGNN_CHECK_ARG(mg[m]->w[l] != nullptr, "block %d mlp%d: missing weight-gradient buffer of layer %d", b, m + 1, l);
   }
-  return tc::embed_bwd(*p, *grads, precision, det, demb, grad_scale_log2, G, N, n_per_graph, workspace, workspace_bytes,
+  return tc::embed_bwd(*p, *grads, precision, det, ckpt, demb, grad_scale_log2, G, N, n_per_graph, workspace, workspace_bytes,
                        (cudaStream_t)stream);
 }
 

@@ -39,7 +39,8 @@ namespace {
 
 // Largest padded graph size of the 16-bit inference path (embedder, fused head).  At N = 4096 a plane holds
 // 4096 x 4352 = 17.8 M pixels and one graph 139 264 conv-chain tiles: per-graph pixel and tile indices fit in int,
-// and make_plan checks the per-launch tile count (see there).  Training keeps its own, lower limit (kMaxTrainN).
+// and make_plan checks the per-launch tile count (see there).  Training keeps a lower limit (kMaxTrainN) except
+// on its checkpoint plan.
 constexpr int kMaxN = 4096;
 constexpr int kTileM = 128;  // pixels per MLP tile / physical rows per matmul tile
 constexpr int kTM1 = 127;    // logical rows per matmul tile
@@ -2303,28 +2304,28 @@ int with_16bit(int precision, const char* what, F&& f) {
 
 }  // namespace
 
-size_t embed_train_workspace_bytes(const fgnn_embed_params& p, int G, int N, bool det) {
+size_t embed_train_workspace_bytes(const fgnn_embed_params& p, int G, int N, bool det, bool ckpt) {
   TrainPlan tp;
-  if (make_train_plan(p, G, N, det, tp)) return 0;
+  if (make_train_plan(p, G, N, det, ckpt, tp)) return 0;
   Arena ar(nullptr, 0);
   TrainBuf B;
   return carve_train(tp, ar, B);
 }
 
-int embed_fwd_train(const fgnn_embed_params& p, int precision, bool det, const float* x, float* emb, int G, int N,
+int embed_fwd_train(const fgnn_embed_params& p, int precision, bool det, bool ckpt, const float* x, float* emb, int G, int N,
                     const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
   return with_16bit(precision, "fgnn_embed_fwd_train", [&](auto t) -> int {
     if (reinterpret_cast<uintptr_t>(ws) & 1023) return fail(FGNN_ERR_INVALID, "workspace must be 1024-byte aligned");
-    return embed_fwd_train_t<decltype(t)>(p, det, x, emb, G, N, n_per_graph, ws, ws_bytes, st);
+    return embed_fwd_train_t<decltype(t)>(p, det, ckpt, x, emb, G, N, n_per_graph, ws, ws_bytes, st);
   });
 }
 
-int embed_bwd(const fgnn_embed_params& p, const fgnn_embed_grads& g, int precision, bool det, const float* demb, int grad_scale_log2,
-              int G, int N, const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
+int embed_bwd(const fgnn_embed_params& p, const fgnn_embed_grads& g, int precision, bool det, bool ckpt, const float* demb,
+              int grad_scale_log2, int G, int N, const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st) {
   return with_16bit(precision, "fgnn_embed_bwd", [&](auto t) -> int {
     if (reinterpret_cast<uintptr_t>(ws) & 1023) return fail(FGNN_ERR_INVALID, "workspace must be 1024-byte aligned");
     if (grad_scale_log2 < -24 || grad_scale_log2 > 15) return fail(FGNN_ERR_INVALID, "grad_scale_log2 %d outside [-24, 15]", grad_scale_log2);
-    return embed_bwd_t<decltype(t)>(p, g, det, demb, grad_scale_log2, G, N, n_per_graph, ws, ws_bytes, st);
+    return embed_bwd_t<decltype(t)>(p, g, det, ckpt, demb, grad_scale_log2, G, N, n_per_graph, ws, ws_bytes, st);
   });
 }
 

@@ -13,12 +13,13 @@ int embed_fwd(const fgnn_embed_params& p, int precision, bool det, const float* 
 int embed_fwd_adjacency(const fgnn_embed_params& p, int precision, bool det, const uint8_t* adj, float* emb, int G, int N,
                         const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st);
 
-// 16-bit training path (fgnn_tc_train.cuh): forward keeping what backward needs in `ws`, and the backward of the stack
-size_t embed_train_workspace_bytes(const fgnn_embed_params& p, int G, int N, bool det);
-int embed_fwd_train(const fgnn_embed_params& p, int precision, bool det, const float* x, float* emb, int G, int N,
+// 16-bit training path (fgnn_tc_train.cuh): forward keeping what backward needs in `ws`, and the backward of the stack.
+// ckpt: block-level checkpoints (FGNN_CHECKPOINT_BLOCKS), the plan that trains up to N = 4096
+size_t embed_train_workspace_bytes(const fgnn_embed_params& p, int G, int N, bool det, bool ckpt);
+int embed_fwd_train(const fgnn_embed_params& p, int precision, bool det, bool ckpt, const float* x, float* emb, int G, int N,
                     const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st);
-int embed_bwd(const fgnn_embed_params& p, const fgnn_embed_grads& g, int precision, bool det, const float* demb, int grad_scale_log2,
-              int G, int N, const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st);
+int embed_bwd(const fgnn_embed_params& p, const fgnn_embed_grads& g, int precision, bool det, bool ckpt, const float* demb,
+              int grad_scale_log2, int G, int N, const int32_t* n_per_graph, void* ws, size_t ws_bytes, cudaStream_t st);
 
 // fused head: scores (optional) + row-softmax CE + row argmax on tensor cores.  Graph 1 (rows) is padded to N1 with
 // sizes n1, graph 2 (columns) to N2 with sizes n2 (null: every graph has the padded size); the workspace follows N1.

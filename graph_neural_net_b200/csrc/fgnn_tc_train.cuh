@@ -927,7 +927,7 @@ int launch_bmm_bwd(int mode, const T* a, const T* b, T* out, const float* coef, 
   });
 }
 
-// Two plans for the 16-bit training entry points.
+// Three plans for the 16-bit training entry points.
 //   KEEP-ALL   one pass over the whole batch: the forward leaves every activation in the workspace until the backward
 //              (carve_train: about 51 plane sets per graph at depth 3, 4 blocks; 107 GB for 64 graphs at N = 500, C = 64).
 //   RECOMPUTE  chosen only when the keep-all workspace exceeds T.  The workspace holds the 16-bit input planes of the
@@ -935,29 +935,40 @@ int launch_bmm_bwd(int mode, const T* a, const T* b, T* out, const float* coef, 
 //              the backward computes the loss scale once over the whole d emb, then per pass re-runs that pass's
 //              forward from the input planes and runs the block-stack backward on it (about one extra training forward
 //              per step).  Parameter gradients accumulate across passes as they do across calls.
+//   CHECKPOINT chosen by the caller (FGNN_CHECKPOINT_BLOCKS), and then the only plan.  The workspace holds, for the whole
+//              batch, the input planes, every block's pre-norm output Z3[b], every MLP's GraphNorm coefficients and
+//              statistics and the pooling arg-max; and, for one pass of `chunk` graphs, ONE block's intermediates (H, Y1,
+//              Y2, MULT, shared by all blocks) and the backward scratch: about nb + 3 D + 11 plane sets per graph instead
+//              of 51.  The forward runs pass by pass, block by block.  The backward, per pass and for b = nb-1 .. 0,
+//              re-runs block b's forward from Z3[b-1] (the input planes for b = 0) up to, not including, mlp3's last conv,
+//              whose output Z3[b] and statistics are kept, then runs block b's backward (about one extra forward per step).
 // T = FGNN_TC_TRAIN_WS_GB GiB when set; otherwise half the current device's memory, because a siamese step holds two
 // embedder workspaces (x1, x2) until backward; unlimited when no device can be queried (host-only workspace queries).
-// chunk = FGNN_TC_CHUNK when set (as for inference), else the largest pass whose carve fits FGNN_TC_WS_GB (default 16)
-// GiB, never less than one graph; the passes are equal, the last one may be shorter.
-// The plan is a pure function of (parameter shapes, G, N, T, FGNN_TC_WS_GB, FGNN_TC_CHUNK).  fgnn_embed_bwd derives it
-// again from the same arguments and must reach the forward call's answer: neither the variables nor the device may
+// chunk = FGNN_TC_CHUNK when set (as for inference), else the largest pass whose own part of the carve fits FGNN_TC_WS_GB
+// (default 16) GiB, never less than one graph; the passes are equal, the last one may be shorter.
+// The plan is a pure function of (parameter shapes, G, N, flags, T, FGNN_TC_WS_GB, FGNN_TC_CHUNK).  fgnn_embed_bwd derives
+// it again from the same arguments and must reach the forward call's answer: neither the variables nor the device may
 // change between the two calls.
 struct TrainPlan {
   Geo geo;
   int C, cin0, D, nb;
   int c_emb;        // real channels of the embeddings (the last block's c_out)
-  int G;            // graphs of one pass: the whole batch on keep-all, `chunk` on recompute (pass_plan lowers it for a short last pass)
+  int G;            // graphs of one pass: the whole batch on keep-all, `chunk` otherwise (pass_plan lowers it for a short last pass)
   int batch;        // graphs of the call
   bool recompute;
+  bool checkpoint;  // FGNN_CHECKPOINT_BLOCKS: block-level checkpoints, one block's intermediates at a time
   bool det;         // deterministic mode: OrderedSum kernels, and room for their records in the carve
 };
 
-// 16-bit training keeps every activation of a pass in its workspace, and a pass holds at least one graph (some 15 GB
-// at N = 2048, C = 32), so it stops at the padded size the inference path had before it was extended to kMaxN.
+// The keep-all and recompute plans keep every activation of a pass in their workspace, and a pass holds at least one
+// graph (some 15 GB at N = 2048, C = 32), so they stop at the padded size the inference path had before it was extended
+// to kMaxN.  The checkpoint plan (about 55 GB for one graph at N = 4096, C = 64) trains up to kMaxN.
 constexpr int kMaxTrainN = 1024;
 
 struct TrainBuf {
-  // kept from forward to backward (recompute: xin for the whole call, the rest for the current pass)
+  // kept from forward to backward (recompute: xin for the whole call, the rest for the current pass; checkpoint: xin,
+  // Z3, coef, gnstat and arg for the whole call, the other planes for one block of the current pass, H[b] .. MULT[b]
+  // the same buffers for every b)
   void* xin;
   void* H[FGNN_MAX_BLOCKS][3][FGNN_MAX_DEPTH];
   void *Y1[FGNN_MAX_BLOCKS], *Y2[FGNN_MAX_BLOCKS], *MULT[FGNN_MAX_BLOCKS], *Z3[FGNN_MAX_BLOCKS];
@@ -989,25 +1000,45 @@ size_t carve_train(const TrainPlan& tp, Arena& ar, TrainBuf& B) {
   const Geo& geo = tp.geo;
   const size_t G = tp.G, C = tp.C;
   const size_t actC = G * C * geo.stride(kLayoutC);
-  // recompute: the batch's input planes come first, outside the plane range that every pass zeroes
-  if (tp.recompute) B.xin = ar.take<uint16_t>((size_t)tp.batch * tp.cin0 * geo.stride(kLayoutC), 1024);
+  // recompute / checkpoint: the batch's input planes come first, outside the plane range that every pass zeroes
+  if (tp.recompute || tp.checkpoint) B.xin = ar.take<uint16_t>((size_t)tp.batch * tp.cin0 * geo.stride(kLayoutC), 1024);
+  if (tp.checkpoint) {   // the block checkpoints of the whole batch, also outside that range
+    const size_t BC = (size_t)tp.batch * C;
+    for (int b = 0; b < tp.nb; ++b) B.Z3[b] = ar.take<uint16_t>(BC * geo.stride(kLayoutC), 1024);
+    for (int b = 0; b < tp.nb; ++b)
+      for (int m = 0; m < 3; ++m) {
+        B.coef[b][m] = ar.take<float>(BC * 2);
+        B.gnstat[b][m] = ar.take<float>(BC * 4);
+      }
+    B.arg = ar.take<int32_t>(BC * geo.N);
+  }
   B.planes_begin = align_up(ar.off, 1024);
-  if (!tp.recompute) B.xin = ar.take<uint16_t>(G * tp.cin0 * geo.stride(kLayoutC), 1024);
-  for (int b = 0; b < tp.nb; ++b) {
+  if (!tp.recompute && !tp.checkpoint) B.xin = ar.take<uint16_t>(G * tp.cin0 * geo.stride(kLayoutC), 1024);
+  const int sets = tp.checkpoint ? 1 : tp.nb;
+  for (int b = 0; b < sets; ++b) {
     for (int m = 0; m < 3; ++m)
       for (int l = 0; l < tp.D - 1; ++l) B.H[b][m][l] = ar.take<uint16_t>(actC, 1024);
     B.Y1[b] = ar.take<uint16_t>(G * C * geo.stride(kLayoutA), 1024);
     B.Y2[b] = ar.take<uint16_t>(G * C * geo.stride(kLayoutB), 1024);
     B.MULT[b] = ar.take<uint16_t>(actC, 1024);
-    B.Z3[b] = ar.take<uint16_t>(actC, 1024);
+    if (!tp.checkpoint) B.Z3[b] = ar.take<uint16_t>(actC, 1024);
+  }
+  for (int b = sets; b < tp.nb; ++b) {
+    for (int m = 0; m < 3; ++m)
+      for (int l = 0; l < tp.D - 1; ++l) B.H[b][m][l] = B.H[0][m][l];
+    B.Y1[b] = B.Y1[0];
+    B.Y2[b] = B.Y2[0];
+    B.MULT[b] = B.MULT[0];
   }
   B.planes_end = ar.off;
-  for (int b = 0; b < tp.nb; ++b)
-    for (int m = 0; m < 3; ++m) {
-      B.coef[b][m] = ar.take<float>(G * C * 2);
-      B.gnstat[b][m] = ar.take<float>(G * C * 4);
-    }
-  B.arg = ar.take<int32_t>(G * C * geo.N);
+  if (!tp.checkpoint) {
+    for (int b = 0; b < tp.nb; ++b)
+      for (int m = 0; m < 3; ++m) {
+        B.coef[b][m] = ar.take<float>(G * C * 2);
+        B.gnstat[b][m] = ar.take<float>(G * C * 4);
+      }
+    B.arg = ar.take<int32_t>(G * C * geo.N);
+  }
   B.wf = ar.take<uint16_t>(G * 2 * C * 256, 1024);
   B.bf = ar.take<float>(G * 2 * C);
   B.stat_acc = ar.take<double>(G * 2 * C * 2);
@@ -1061,10 +1092,13 @@ size_t keep_all_limit() {
   return t;
 }
 
-int make_train_plan(const fgnn_embed_params& p, int G, int N, bool det, TrainPlan& tp) {
-  if (N > kMaxTrainN)
+int make_train_plan(const fgnn_embed_params& p, int G, int N, bool det, bool ckpt, TrainPlan& tp) {
+  if (ckpt && N > kMaxN)
+    return fail(FGNN_ERR_UNSUPPORTED, "16-bit training with block checkpoints supports N <= %d (got %d)", kMaxN, N);
+  if (!ckpt && N > kMaxTrainN)
     return fail(FGNN_ERR_UNSUPPORTED, "16-bit training supports N <= %d (got %d): its workspace holds every activation of at "
-                "least one graph; embed larger graphs with the inference path (N <= %d)", kMaxTrainN, N, kMaxN);
+                "least one graph; embed larger graphs with the inference path (N <= %d), or train them with block "
+                "checkpoints (FGNN_CHECKPOINT_BLOCKS, Network.set_checkpoint_blocks)", kMaxTrainN, N, kMaxN);
   Plan pl;
   if (int e = make_plan(p, G, N, pl)) return e;
   tp.geo = pl.geo;
@@ -1075,6 +1109,7 @@ int make_train_plan(const fgnn_embed_params& p, int G, int N, bool det, TrainPla
   tp.G = G;
   tp.batch = G;
   tp.recompute = false;
+  tp.checkpoint = false;
   tp.det = det;
   tp.D = p.block[0].mlp1.depth;
   for (int b = 0; b < p.num_blocks; ++b) {
@@ -1085,10 +1120,14 @@ int make_train_plan(const fgnn_embed_params& p, int G, int N, bool det, TrainPla
   if (tp.D < 1 || tp.D > FGNN_MAX_DEPTH) return fail(FGNN_ERR_INVALID, "bad depth %d", tp.D);
   if (tp.cin0 > 64) return fail(FGNN_ERR_UNSUPPORTED, "original_features_num %d > 64 unsupported", tp.cin0);
   if ((long)G * tp.C > 65535) return fail(FGNN_ERR_UNSUPPORTED, "16-bit training: G * C = %ld planes exceed one call's grid (split the batch)", (long)G * tp.C);
-  if (train_workspace_bytes(tp) <= keep_all_limit()) return FGNN_OK;
-  tp.recompute = true;
+  if (ckpt) {
+    tp.checkpoint = true;
+  } else {
+    if (train_workspace_bytes(tp) <= keep_all_limit()) return FGNN_OK;
+    tp.recompute = true;
+  }
   int chunk = env_int("FGNN_TC_CHUNK", 0);
-  if (chunk <= 0) {   // the largest pass whose own carve (batch = 0: without the input planes) fits the budget, or 1
+  if (chunk <= 0) {   // the largest pass whose own carve (batch = 0: without the batch-wide part) fits the budget, or 1
     const size_t budget = (size_t)std::max(1, env_int("FGNN_TC_WS_GB", 16)) << 30;
     TrainPlan q = tp;
     q.batch = 0;
@@ -1112,10 +1151,27 @@ TrainPlan pass_plan(const TrainPlan& tp, int g0) {
   return pp;
 }
 
+// the buffers of the pass that starts at graph g0: on the checkpoint plan its graphs' part of the batch-wide buffers,
+// on the other plans B itself (their buffers hold one pass)
+TrainBuf pass_bufs(const TrainPlan& tp, const TrainBuf& B, int g0) {
+  TrainBuf V = B;
+  if (!tp.checkpoint) return V;
+  const size_t gc = (size_t)g0 * tp.C;
+  for (int b = 0; b < tp.nb; ++b) {
+    V.Z3[b] = static_cast<uint16_t*>(B.Z3[b]) + gc * tp.geo.PSC;
+    for (int m = 0; m < 3; ++m) {
+      V.coef[b][m] = B.coef[b][m] + gc * 2;
+      V.gnstat[b][m] = B.gnstat[b][m] + gc * 4;
+    }
+  }
+  V.arg = B.arg + gc * tp.geo.N;
+  return V;
+}
+
 // Zero what a pass's producers never write but later reads cover, before every pass's forward.  Ragged batch: all the
 // kept planes and the backward scratch (rows beyond a graph's covered range are never written, the GEMM K loops read
 // them, and an earlier pass's larger graph leaves data there).  Otherwise: the physical rows / column chunks the
-// producers skip.  The recompute plan's input planes lie before planes_begin and are not touched.
+// producers skip.  The batch-wide part of the recompute and checkpoint plans lies before planes_begin and is not touched.
 int zero_pass(const TrainPlan& tp, const TrainBuf& B, void* ws, bool ragged, cudaStream_t st) {
   const Geo& geo = tp.geo;
   const size_t GC = (size_t)tp.G * tp.C;
@@ -1124,7 +1180,7 @@ int zero_pass(const TrainPlan& tp, const TrainBuf& B, void* ws, bool ragged, cud
     FGNN_CUDA(cudaMemsetAsync(base + B.planes_begin, 0, B.planes_end - B.planes_begin, st));
     FGNN_CUDA(cudaMemsetAsync(base + B.bwd_begin, 0, B.bwd_end - B.bwd_begin, st));
   } else {
-    for (int b = 0; b < tp.nb; ++b) {
+    for (int b = 0; b < (tp.checkpoint ? 1 : tp.nb); ++b) {   // checkpoint: one set of planes shared by all blocks
       FGNN_CUDA(cudaMemsetAsync(B.Y1[b], 0, GC * geo.PSA * 2, st));
       FGNN_CUDA(cudaMemsetAsync(B.Y2[b], 0, GC * geo.PSB * 2, st));
       FGNN_CUDA(cudaMemsetAsync(B.MULT[b], 0, GC * geo.PSC * 2, st));
@@ -1199,89 +1255,110 @@ int run_conv(const ConvCall<T>& cc, const TrainPlan& tp, const TrainBuf& B, cons
   return run_mlp_group<T>(M, tp.C, tp.G, tp.geo, npg, st);
 }
 
+// input of block b: the input planes xin for b = 0, else the previous block's pre-norm output and its GraphNorm fold
+template <typename T>
+struct BlockIn {
+  const T* x;
+  int c, c_real;
+  const float* coef;
+};
+template <typename T>
+BlockIn<T> block_in(const fgnn_embed_params& p, const TrainPlan& tp, const TrainBuf& B, int b, const T* xin) {
+  if (b == 0) return {xin, tp.cin0, tp.cin0, nullptr};
+  return {reinterpret_cast<const T*>(B.Z3[b - 1]), tp.C, p.block[b - 1].mlp3.c_out, B.coef[b - 1][2]};
+}
+
+// training forward of block b of one pass (tp.G graphs): writes its hidden activations, Y1, Y2, MULT, Z3[b] and the
+// GraphNorm statistics of its MLPs into B.  z3 = false stops before mlp3's last conv (the checkpoint plan's backward:
+// Z3[b] and its statistics are kept, never rewritten).
+template <typename T>
+int train_fwd_block(const fgnn_embed_params& p, const TrainPlan& tp, const TrainBuf& B, int b, const T* xin, bool z3,
+                    const int32_t* npg, cudaStream_t st) {
+  const Geo& geo = tp.geo;
+  const int G = tp.G, C = tp.C, D = tp.D;
+  const BlockIn<T> in = block_in<T>(p, tp, B, b, xin);
+  const T* cur = in.x;
+  const int cur_c = in.c, cur_real = in.c_real;
+  const float* cur_coef = in.coef;
+  const fgnn_block_params& bp = p.block[b];
+  const int co = bp.mlp1.c_out;
+  const fgnn_mlp_params* mlps[3] = {&bp.mlp1, &bp.mlp2, &bp.mlp3};
+  T* y12[2] = {reinterpret_cast<T*>(B.Y1[b]), reinterpret_cast<T*>(B.Y2[b])};
+  const Layout mode12[2] = {kLayoutA, kLayoutB};
+  for (int l = 0; l < D; ++l) {
+    const bool last = l == D - 1;
+    if (l == 0) {   // mlp1 and mlp2 share the block input: one launch
+      ConvCall<T> cc;
+      cc.nmlp = 2;
+      cc.src[0] = cur; cc.c_src[0] = cur_c; cc.cr_src[0] = cur_real; cc.src_coef[0] = cur_coef; cc.nsrc = 1;
+      cc.co_real = co;
+      for (int m = 0; m < 2; ++m) {
+        cc.w[m] = mlps[m]->w[0]; cc.b[m] = mlps[m]->b[0];
+        cc.out[m] = last ? y12[m] : reinterpret_cast<T*>(B.H[b][m][0]);
+        cc.out_mode[m] = last ? mode12[m] : kLayoutC;
+        cc.ones[m] = last ? 1 : 0;
+        if (last) { cc.gn[m] = mlps[m]; cc.coef[m] = B.coef[b][m]; cc.gnstat[m] = B.gnstat[b][m]; }
+      }
+      cc.relu = last ? 0 : 1;
+      if (int e = run_conv<T>(cc, tp, B, npg, st)) return e;
+    } else {
+      for (int m = 0; m < 2; ++m) {
+        ConvCall<T> cc;
+        cc.src[0] = reinterpret_cast<const T*>(B.H[b][m][l - 1]); cc.c_src[0] = C; cc.cr_src[0] = co;
+        cc.co_real = co;
+        cc.w[0] = mlps[m]->w[l]; cc.b[0] = mlps[m]->b[l];
+        cc.out[0] = last ? y12[m] : reinterpret_cast<T*>(B.H[b][m][l]);
+        cc.out_mode[0] = last ? mode12[m] : kLayoutC;
+        cc.ones[0] = last ? 1 : 0;
+        if (last) { cc.gn[0] = mlps[m]; cc.coef[0] = B.coef[b][m]; cc.gnstat[0] = B.gnstat[b][m]; }
+        cc.relu = last ? 0 : 1;
+        if (int e = run_conv<T>(cc, tp, B, npg, st)) return e;
+      }
+    }
+  }
+  T* mult = reinterpret_cast<T*>(B.MULT[b]);
+  if (int e = launch_matmul<T>(y12[0], y12[1], mult, B.coef[b][0], B.coef[b][1], G, C, geo, npg, st)) return e;
+  for (int l = 0; l < (z3 ? D : D - 1); ++l) {
+    const bool last = l == D - 1;
+    ConvCall<T> cc;
+    if (l == 0) {
+      cc.src[0] = mult; cc.c_src[0] = C; cc.cr_src[0] = co; cc.src_coef[0] = nullptr;
+      cc.src[1] = cur; cc.c_src[1] = cur_c; cc.cr_src[1] = cur_real; cc.src_coef[1] = cur_coef; cc.nsrc = 2;
+    } else {
+      cc.src[0] = reinterpret_cast<const T*>(B.H[b][2][l - 1]); cc.c_src[0] = C; cc.cr_src[0] = co;
+    }
+    cc.co_real = co;
+    cc.w[0] = mlps[2]->w[l]; cc.b[0] = mlps[2]->b[l];
+    cc.out[0] = last ? reinterpret_cast<T*>(B.Z3[b]) : reinterpret_cast<T*>(B.H[b][2][l]);
+    if (last) { cc.gn[0] = mlps[2]; cc.coef[0] = B.coef[b][2]; cc.gnstat[0] = B.gnstat[b][2]; }
+    cc.relu = last ? 0 : 1;
+    if (int e = run_conv<T>(cc, tp, B, npg, st)) return e;
+  }
+  return FGNN_OK;
+}
+
 // training forward of one pass (tp.G graphs): their input planes xin -> emb (tp.G, C, N), and in B everything the
 // backward reads
 template <typename T>
 int train_fwd_pass(const fgnn_embed_params& p, const TrainPlan& tp, const TrainBuf& B, const T* xin, float* emb,
                    const int32_t* npg, cudaStream_t st) {
   const Geo& geo = tp.geo;
-  const int G = tp.G, N = geo.N, C = tp.C, D = tp.D;
-  const T* cur = xin;
-  int cur_c = tp.cin0, cur_real = tp.cin0;
-  const float* cur_coef = nullptr;
-  for (int b = 0; b < tp.nb; ++b) {
-    const fgnn_block_params& bp = p.block[b];
-    const int co = bp.mlp1.c_out;
-    const fgnn_mlp_params* mlps[3] = {&bp.mlp1, &bp.mlp2, &bp.mlp3};
-    T* y12[2] = {reinterpret_cast<T*>(B.Y1[b]), reinterpret_cast<T*>(B.Y2[b])};
-    const Layout mode12[2] = {kLayoutA, kLayoutB};
-    for (int l = 0; l < D; ++l) {
-      const bool last = l == D - 1;
-      if (l == 0) {   // mlp1 and mlp2 share the block input: one launch
-        ConvCall<T> cc;
-        cc.nmlp = 2;
-        cc.src[0] = cur; cc.c_src[0] = cur_c; cc.cr_src[0] = cur_real; cc.src_coef[0] = cur_coef; cc.nsrc = 1;
-        cc.co_real = co;
-        for (int m = 0; m < 2; ++m) {
-          cc.w[m] = mlps[m]->w[0]; cc.b[m] = mlps[m]->b[0];
-          cc.out[m] = last ? y12[m] : reinterpret_cast<T*>(B.H[b][m][0]);
-          cc.out_mode[m] = last ? mode12[m] : kLayoutC;
-          cc.ones[m] = last ? 1 : 0;
-          if (last) { cc.gn[m] = mlps[m]; cc.coef[m] = B.coef[b][m]; cc.gnstat[m] = B.gnstat[b][m]; }
-        }
-        cc.relu = last ? 0 : 1;
-        if (int e = run_conv<T>(cc, tp, B, npg, st)) return e;
-      } else {
-        for (int m = 0; m < 2; ++m) {
-          ConvCall<T> cc;
-          cc.src[0] = reinterpret_cast<const T*>(B.H[b][m][l - 1]); cc.c_src[0] = C; cc.cr_src[0] = co;
-          cc.co_real = co;
-          cc.w[0] = mlps[m]->w[l]; cc.b[0] = mlps[m]->b[l];
-          cc.out[0] = last ? y12[m] : reinterpret_cast<T*>(B.H[b][m][l]);
-          cc.out_mode[0] = last ? mode12[m] : kLayoutC;
-          cc.ones[0] = last ? 1 : 0;
-          if (last) { cc.gn[0] = mlps[m]; cc.coef[0] = B.coef[b][m]; cc.gnstat[0] = B.gnstat[b][m]; }
-          cc.relu = last ? 0 : 1;
-          if (int e = run_conv<T>(cc, tp, B, npg, st)) return e;
-        }
-      }
-    }
-    T* mult = reinterpret_cast<T*>(B.MULT[b]);
-    if (int e = launch_matmul<T>(y12[0], y12[1], mult, B.coef[b][0], B.coef[b][1], G, C, geo, npg, st)) return e;
-    for (int l = 0; l < D; ++l) {
-      const bool last = l == D - 1;
-      ConvCall<T> cc;
-      if (l == 0) {
-        cc.src[0] = mult; cc.c_src[0] = C; cc.cr_src[0] = co; cc.src_coef[0] = nullptr;
-        cc.src[1] = cur; cc.c_src[1] = cur_c; cc.cr_src[1] = cur_real; cc.src_coef[1] = cur_coef; cc.nsrc = 2;
-      } else {
-        cc.src[0] = reinterpret_cast<const T*>(B.H[b][2][l - 1]); cc.c_src[0] = C; cc.cr_src[0] = co;
-      }
-      cc.co_real = co;
-      cc.w[0] = mlps[2]->w[l]; cc.b[0] = mlps[2]->b[l];
-      cc.out[0] = last ? reinterpret_cast<T*>(B.Z3[b]) : reinterpret_cast<T*>(B.H[b][2][l]);
-      if (last) { cc.gn[0] = mlps[2]; cc.coef[0] = B.coef[b][2]; cc.gnstat[0] = B.gnstat[b][2]; }
-      cc.relu = last ? 0 : 1;
-      if (int e = run_conv<T>(cc, tp, B, npg, st)) return e;
-    }
-    cur = reinterpret_cast<const T*>(B.Z3[b]);
-    cur_c = C;
-    cur_real = co;
-    cur_coef = B.coef[b][2];
-  }
+  for (int b = 0; b < tp.nb; ++b)
+    if (int e = train_fwd_block<T>(p, tp, B, b, xin, true, npg, st)) return e;
   {
-    dim3 grid((unsigned)((N + 7) / 8), G * C);
-    colmax16_kernel<T><<<grid, 256, 0, st>>>(cur, cur_coef, emb, B.arg, C, cur_real, geo, npg);
+    const BlockIn<T> out = block_in<T>(p, tp, B, tp.nb, xin);
+    dim3 grid((unsigned)((geo.N + 7) / 8), tp.G * tp.C);
+    colmax16_kernel<T><<<grid, 256, 0, st>>>(out.x, out.coef, emb, B.arg, tp.C, out.c_real, geo, npg);
     FGNN_LAUNCHED();
   }
   return FGNN_OK;
 }
 
 template <typename T>
-int embed_fwd_train_t(const fgnn_embed_params& p, bool det, const float* x, float* emb, int G, int N, const int32_t* npg, void* ws,
-                      size_t ws_bytes, cudaStream_t st) {
+int embed_fwd_train_t(const fgnn_embed_params& p, bool det, bool ckpt, const float* x, float* emb, int G, int N,
+                      const int32_t* npg, void* ws, size_t ws_bytes, cudaStream_t st) {
   TrainPlan tp;
-  if (int e = make_train_plan(p, G, N, det, tp)) return e;
+  if (int e = make_train_plan(p, G, N, det, ckpt, tp)) return e;
   Arena ar(ws, ws_bytes);
   TrainBuf B;
   const size_t need = carve_train(tp, ar, B);
@@ -1289,6 +1366,8 @@ int embed_fwd_train_t(const fgnn_embed_params& p, bool det, const float* x, floa
   const Geo& geo = tp.geo;
   T* xin = reinterpret_cast<T*>(B.xin);
   FGNN_CUDA(cudaMemsetAsync(B.zeros, 0, 512 * sizeof(float), st));
+  if (tp.checkpoint && npg)   // ragged: the batch's checkpoints once, as zero_pass does for a pass's planes
+    for (int b = 0; b < tp.nb; ++b) FGNN_CUDA(cudaMemsetAsync(B.Z3[b], 0, (size_t)G * tp.C * geo.PSC * sizeof(T), st));
   for (int g0 = 0; g0 < G; g0 += tp.G) {
     const TrainPlan pp = pass_plan(tp, g0);
     if (int e = zero_pass(pp, B, ws, npg != nullptr, st)) return e;
@@ -1297,8 +1376,8 @@ int embed_fwd_train_t(const fgnn_embed_params& p, bool det, const float* x, floa
       to_planes_c_kernel<T><<<grid, 256, 0, st>>>(x, xin, tp.cin0, geo, npg);
       FGNN_LAUNCHED();
     }
-    if (int e = train_fwd_pass<T>(p, pp, B, xin + (size_t)g0 * tp.cin0 * geo.PSC, emb + (size_t)g0 * tp.c_emb * N,
-                                  npg ? npg + g0 : nullptr, st)) return e;
+    if (int e = train_fwd_pass<T>(p, pp, pass_bufs(tp, B, g0), xin + (size_t)g0 * tp.cin0 * geo.PSC,
+                                  emb + (size_t)g0 * tp.c_emb * N, npg ? npg + g0 : nullptr, st)) return e;
   }
   return FGNN_OK;
 }
@@ -1422,7 +1501,8 @@ int mlp_bwd(const MlpBwd<T>& a, const TrainPlan& tp, const TrainBuf& B, const in
   return FGNN_OK;
 }
 
-// block-stack backward of one pass (tp.G graphs) whose forward state is in B: demb (tp.G, C, N), scaled by *B.scale
+// block-stack backward of one pass (tp.G graphs) whose forward state is in B: demb (tp.G, C, N), scaled by *B.scale.
+// On the checkpoint plan B holds the pass's checkpoints, and each block's forward is re-run just before its backward.
 template <typename T>
 int train_bwd_pass(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const TrainPlan& tp, const TrainBuf& B,
                    const T* xin, const float* demb, const int32_t* npg, cudaStream_t st) {
@@ -1439,13 +1519,16 @@ int train_bwd_pass(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const
     FGNN_LAUNCHED();
   }
   for (int b = tp.nb - 1; b >= 0; --b) {
+    // checkpoint plan: block b's intermediates, re-derived from its kept input into the planes all blocks share
+    if (tp.checkpoint)
+      if (int e = train_fwd_block<T>(p, tp, B, b, xin, false, npg, st)) return e;
     const fgnn_block_params& bp = p.block[b];
     const fgnn_block_grads& bg = gr.block[b];
-    const T* cur = b > 0 ? reinterpret_cast<const T*>(B.Z3[b - 1]) : xin;
-    const int cur_c = b > 0 ? C : tp.cin0;
-    const int cur_real = b > 0 ? p.block[b - 1].mlp3.c_out : tp.cin0;
+    const BlockIn<T> in = block_in<T>(p, tp, B, b, xin);
+    const T* cur = in.x;
+    const int cur_c = in.c, cur_real = in.c_real;
     const int co = bp.mlp1.c_out;
-    const float* cur_coef = b > 0 ? B.coef[b - 1][2] : nullptr;
+    const float* cur_coef = in.coef;
     T* A[2] = {reinterpret_cast<T*>(B.A0), reinterpret_cast<T*>(B.A1)};
     T* Bb[2] = {reinterpret_cast<T*>(B.B0), reinterpret_cast<T*>(B.B1)};
     T* DM = reinterpret_cast<T*>(B.DM);
@@ -1534,10 +1617,10 @@ int train_bwd_pass(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const
 }
 
 template <typename T>
-int embed_bwd_t(const fgnn_embed_params& p, const fgnn_embed_grads& gr, bool det, const float* demb, int grad_scale_log2, int G, int N,
-                const int32_t* npg, void* ws, size_t ws_bytes, cudaStream_t st) {
+int embed_bwd_t(const fgnn_embed_params& p, const fgnn_embed_grads& gr, bool det, bool ckpt, const float* demb, int grad_scale_log2,
+                int G, int N, const int32_t* npg, void* ws, size_t ws_bytes, cudaStream_t st) {
   TrainPlan tp;
-  if (int e = make_train_plan(p, G, N, det, tp)) return e;
+  if (int e = make_train_plan(p, G, N, det, ckpt, tp)) return e;
   Arena ar(ws, ws_bytes);
   TrainBuf B;
   const size_t need = carve_train(tp, ar, B);
@@ -1555,8 +1638,11 @@ int embed_bwd_t(const fgnn_embed_params& p, const fgnn_embed_grads& gr, bool det
       // re-derive the pass's activations; its embeddings land in rowsum, which the backward rewrites before reading it
       if (int e = zero_pass(pp, B, ws, npg != nullptr, st)) return e;
       if (int e = train_fwd_pass<T>(p, pp, B, xin_p, B.rowsum, npg_p, st)) return e;
+    } else if (tp.checkpoint) {
+      // the shared block planes and the backward scratch hold another pass's data: zero them as the forward did
+      if (int e = zero_pass(pp, B, ws, npg != nullptr, st)) return e;
     }
-    if (int e = train_bwd_pass<T>(p, gr, pp, B, xin_p, demb + (size_t)g0 * tp.c_emb * N, npg_p, st)) return e;
+    if (int e = train_bwd_pass<T>(p, gr, pp, pass_bufs(tp, B, g0), xin_p, demb + (size_t)g0 * tp.c_emb * N, npg_p, st)) return e;
   }
   return FGNN_OK;
 }

@@ -75,6 +75,11 @@ class Siamese_Node_Exp(_Base):
         self.node_embedder.set_precision(precision)
         return self
 
+    def set_checkpoint_blocks(self, on=True):
+        """Train the 16-bit embedder with block-level activation checkpoints (Network.set_checkpoint_blocks)."""
+        self.node_embedder.set_checkpoint_blocks(on)
+        return self
+
     def embed(self, x):
         return self.node_embedder(x)['ne/suffix']
 

@@ -98,12 +98,21 @@ class Network(nn.Module):
         for path, (val, _) in self.graph.items():
             setattr(self, path.replace(sep, '_'), val)
         self.precision = _DEFAULT_PRECISION
+        self.checkpoint_blocks = False
         self._fused = self._match_embedder()
 
     def set_precision(self, precision: str):
         if precision not in L.PRECISIONS:
             raise ValueError(f"precision must be one of {sorted(L.PRECISIONS)}")
         self.precision = precision
+        return self
+
+    def set_checkpoint_blocks(self, on: bool = True):
+        """16-bit training with block-level activation checkpoints (FGNN_CHECKPOINT_BLOCKS): the forward keeps each
+        block's output only, the backward re-runs each block's forward just before its backward.  About one more
+        forward per step for less than half the memory, and training on graphs of up to 4096 vertices instead of 1024.
+        Inference and the fp32 mode (which trains any size) are unaffected."""
+        self.checkpoint_blocks = bool(on)
         return self
 
     def nodes(self):
@@ -180,7 +189,8 @@ class Network(nn.Module):
         if any(t is None for t in flat):
             raise L.FgnnError("the fused training path needs conv biases and an affine GraphNorm (the reference's modules)")
         c_out = self._fused[2][-1][2].convs[-1].weight.shape[0]
-        emb = _ops.EmbedTrainFunction.apply(plain, n_dev, spec, L.PRECISIONS[prec_name], c_out, *flat)
+        prec = L.PRECISIONS[prec_name] | (L.FGNN_CHECKPOINT_BLOCKS if self.checkpoint_blocks else 0)
+        emb = _ops.EmbedTrainFunction.apply(plain, n_dev, spec, prec, c_out, *flat)
         if isinstance(x, MaskedTensor):
             return rewrap(emb, x.tensor.names[:-1])
         return emb

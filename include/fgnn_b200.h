@@ -62,6 +62,12 @@ typedef enum {
  * precision's low byte is rejected (FGNN_ERR_INVALID; workspace queries return 0). */
 #define FGNN_DETERMINISTIC 0x100
 
+/* Block-level activation checkpointing of 16-bit training: ORed into the `precision` argument of
+ * fgnn_embed_train_workspace_bytes, fgnn_embed_fwd_train and fgnn_embed_bwd (all three alike, as for
+ * FGNN_DETERMINISTIC, with which it combines).  It selects the checkpoint plan described there, which trains graphs
+ * of up to N = 4096.  Every other entry point rejects it as an unknown flag. */
+#define FGNN_CHECKPOINT_BLOCKS 0x400
+
 #define FGNN_MAX_DEPTH 8
 #define FGNN_MAX_BLOCKS 16
 
@@ -311,9 +317,9 @@ int fgnn_embed_fwd_adjacency_u8(const fgnn_embed_params* p, int32_t precision, c
  * As with the reference's AMP GradScaler, fp16 gradient planes can overflow for a given scale: the parameter
  * gradients are then non-finite and the caller skips the step and lowers grad_scale_log2 (training.py does; 9 is
  * the default, -24 .. 15 accepted; bf16 never overflows).  The workspace must be the one the forward call filled
- * (same G, N, parameters), fgnn_embed_train_workspace_bytes(...) bytes, 1024-byte aligned.  N <= 1024, and every
- * MLP has the same depth.
- * Two plans, picked from the shapes by all three calls alike:
+ * (same G, N, parameters), fgnn_embed_train_workspace_bytes(...) bytes, 1024-byte aligned.  Every MLP has the same
+ * depth, and N <= 1024 (N <= 4096 with FGNN_CHECKPOINT_BLOCKS).
+ * Three plans, picked by all three calls alike:
  *   keep-all   the workspace keeps every activation of the batch from forward to backward (about 51 plane sets per
  *              graph at depth 3, 4 blocks: 107 GB for 64 graphs of N = 500, C = 64).  Used while that size is <= T.
  *   recompute  the workspace keeps the 16-bit input planes of the batch plus the activations of one pass of graphs;
@@ -321,6 +327,12 @@ int fgnn_embed_fwd_adjacency_u8(const fgnn_embed_params* p, int32_t precision, c
  *              backward (about one more forward per step; the loss scale is still chosen once over all of d emb).
  *              Passes are equal and as large as fit FGNN_TC_WS_GB (default 16) GiB, never less than one graph
  *              (FGNN_TC_CHUNK graphs when set, as for fgnn_embed_fwd).
+ *   checkpoint used when `precision` carries FGNN_CHECKPOINT_BLOCKS, and then always (T plays no part).  The workspace
+ *              keeps, for the whole batch, the input planes, every block's output and GraphNorm statistics and the
+ *              pooling arg-max, plus one block's activations and the backward scratch for one pass of graphs (passes
+ *              cut as for recompute): about nb + 3 depth + 11 plane sets per graph, 55 GB for one graph of N = 4096,
+ *              C = 64, 4 blocks of depth 3.  The backward re-runs each block's forward from its kept input just before
+ *              that block's backward (about one more forward per step).
  * T is FGNN_TC_TRAIN_WS_GB GiB when set (0 always picks recompute); otherwise half the current device's memory, because
  * a siamese step holds two workspaces (x1 and x2) until backward; unlimited when no device can be queried.  The plan
  * must not change between fgnn_embed_fwd_train and fgnn_embed_bwd: keep these variables and the current device as
