@@ -2307,9 +2307,7 @@ int with_16bit(int precision, const char* what, F&& f) {
 size_t embed_train_workspace_bytes(const fgnn_embed_params& p, int G, int N, bool det, bool ckpt) {
   TrainPlan tp;
   if (make_train_plan(p, G, N, det, ckpt, tp)) return 0;
-  Arena ar(nullptr, 0);
-  TrainBuf B;
-  return carve_train(tp, ar, B);
+  return train_workspace_bytes(tp);
 }
 
 int embed_fwd_train(const fgnn_embed_params& p, int precision, bool det, bool ckpt, const float* x, float* emb, int G, int N,

@@ -217,24 +217,6 @@ relu_mask_kernel(T* __restrict__ pre, const T* __restrict__ h, float* __restrict
   if (threadIdx.x == 0) add_bsum<Sum>(bsum, gc, t);
 }
 
-// bsum[gc] = sum of a layout-C plane (bias gradient of a layer whose output gradient needs no mask)
-template <typename T, typename Sum>
-__global__ void __launch_bounds__(256)
-plane_sum_kernel(const T* __restrict__ x, float* __restrict__ bsum, int C, Geo geo, const int32_t* __restrict__ npg) {
-  __shared__ float s_red[8];
-  const int gc = blockIdx.y, g = gc / C;
-  const long tot = (long)rows_cover(npg, g, geo) * (geo.NPC / 8);
-  float s = 0.f;
-  for (long idx = (long)blockIdx.x * blockDim.x + threadIdx.x; idx < tot; idx += (long)gridDim.x * blockDim.x) {
-    float p[8];
-    unpack8<T>(*reinterpret_cast<const uint4*>(x + (long)gc * geo.PSC + idx * 8), p);
-#pragma unroll
-    for (int e = 0; e < 8; ++e) s += p[e];
-  }
-  const float t = block_sum(s, s_red);
-  if (threadIdx.x == 0) add_bsum<Sum>(bsum, gc, t);
-}
-
 // rowsum[gc][i] = sum_j x[i][j] (valid block), one warp per row
 template <typename T>
 __global__ void __launch_bounds__(256)
@@ -927,23 +909,26 @@ int launch_bmm_bwd(int mode, const T* a, const T* b, T* out, const float* coef, 
   });
 }
 
-// Three plans for the 16-bit training entry points.
-//   KEEP-ALL   one pass over the whole batch: the forward leaves every activation in the workspace until the backward
-//              (carve_train: about 51 plane sets per graph at depth 3, 4 blocks; 107 GB for 64 graphs at N = 500, C = 64).
-//   RECOMPUTE  chosen only when the keep-all workspace exceeds T.  The workspace holds the 16-bit input planes of the
-//              whole batch and one keep-all carve of `chunk` graphs.  The forward runs pass by pass and keeps only emb;
-//              the backward computes the loss scale once over the whole d emb, then per pass re-runs that pass's
-//              forward from the input planes and runs the block-stack backward on it (about one extra training forward
-//              per step).  Parameter gradients accumulate across passes as they do across calls.
-//   CHECKPOINT chosen by the caller (FGNN_CHECKPOINT_BLOCKS), and then the only plan.  The workspace holds, for the whole
-//              batch, the input planes, every block's pre-norm output Z3[b], every MLP's GraphNorm coefficients and
-//              statistics and the pooling arg-max; and, for one pass of `chunk` graphs, ONE block's intermediates (H, Y1,
-//              Y2, MULT, shared by all blocks) and the backward scratch: about nb + 3 D + 11 plane sets per graph instead
-//              of 51.  The forward runs pass by pass, block by block.  The backward, per pass and for b = nb-1 .. 0,
-//              re-runs block b's forward from Z3[b-1] (the input planes for b = 0) up to, not including, mlp3's last conv,
-//              whose output Z3[b] and statistics are kept, then runs block b's backward (about one extra forward per step).
-// T = FGNN_TC_TRAIN_WS_GB GiB when set; otherwise half the current device's memory, because a siamese step holds two
-// embedder workspaces (x1, x2) until backward; unlimited when no device can be queried (host-only workspace queries).
+// Two workspace layouts for the 16-bit training entry points.  Both hold the 16-bit input planes of the whole batch
+// first, outside the range that every pass zeroes, and cut the batch into passes of tp.G graphs.
+//   PASSES     the workspace holds every activation of one pass (carve_train: about 51 plane sets per graph at depth 3,
+//              4 blocks; 107 GB for 64 graphs at N = 500, C = 64).  When the whole batch fits T as one pass, it is one
+//              pass: the forward leaves every activation in the workspace until the backward.  Otherwise the passes are
+//              `chunk` graphs.  The forward runs pass by pass and keeps only emb; the backward computes the loss scale
+//              once over the whole d emb, then per pass re-runs that pass's forward from the input planes and runs the
+//              block-stack backward on it (about one extra training forward per step).  Parameter gradients accumulate
+//              across passes as they do across calls.
+//   CHECKPOINT chosen by the caller (FGNN_CHECKPOINT_BLOCKS), and then always in passes of `chunk` graphs.  The
+//              workspace holds, for the whole batch, the input planes, every block's pre-norm output Z3[b], every MLP's
+//              GraphNorm coefficients and statistics and the pooling arg-max; and, for one pass, ONE block's
+//              intermediates (H, Y1, Y2, MULT, shared by all blocks) and the backward scratch: about nb + 3 D + 11 plane
+//              sets per graph instead of 51.  The forward runs pass by pass, block by block.  The backward, per pass and
+//              for b = nb-1 .. 0, re-runs block b's forward from Z3[b-1] (the input planes for b = 0) up to, not
+//              including, mlp3's last conv, whose output Z3[b] and statistics are kept, then runs block b's backward
+//              (about one extra forward per step).
+// T = FGNN_TC_TRAIN_WS_GB GiB when set (0: the batch is always cut into passes of `chunk`, and one that fits a single
+// pass is not re-run); otherwise half the current device's memory, because a siamese step holds two embedder
+// workspaces (x1, x2) until backward; unlimited when no device can be queried (host-only workspace queries).
 // chunk = FGNN_TC_CHUNK when set (as for inference), else the largest pass whose own part of the carve fits FGNN_TC_WS_GB
 // (default 16) GiB, never less than one graph; the passes are equal, the last one may be shorter.
 // The plan is a pure function of (parameter shapes, G, N, flags, T, FGNN_TC_WS_GB, FGNN_TC_CHUNK).  fgnn_embed_bwd derives
@@ -953,22 +938,21 @@ struct TrainPlan {
   Geo geo;
   int C, cin0, D, nb;
   int c_emb;        // real channels of the embeddings (the last block's c_out)
-  int G;            // graphs of one pass: the whole batch on keep-all, `chunk` otherwise (pass_plan lowers it for a short last pass)
+  int G;            // graphs of one pass: the whole batch or `chunk` (pass_plan lowers it for a short last pass)
   int batch;        // graphs of the call
-  bool recompute;
   bool checkpoint;  // FGNN_CHECKPOINT_BLOCKS: block-level checkpoints, one block's intermediates at a time
   bool det;         // deterministic mode: OrderedSum kernels, and room for their records in the carve
 };
 
-// The keep-all and recompute plans keep every activation of a pass in their workspace, and a pass holds at least one
-// graph (some 15 GB at N = 2048, C = 32), so they stop at the padded size the inference path had before it was extended
-// to kMaxN.  The checkpoint plan (about 55 GB for one graph at N = 4096, C = 64) trains up to kMaxN.
+// Without checkpoints the workspace keeps every activation of a pass, and a pass holds at least one graph (some 15 GB
+// at N = 2048, C = 32), so training stops at the padded size the inference path had before it was extended to kMaxN.
+// The checkpoint plan (about 55 GB for one graph at N = 4096, C = 64) trains up to kMaxN.
 constexpr int kMaxTrainN = 1024;
 
 struct TrainBuf {
-  // kept from forward to backward (recompute: xin for the whole call, the rest for the current pass; checkpoint: xin,
-  // Z3, coef, gnstat and arg for the whole call, the other planes for one block of the current pass, H[b] .. MULT[b]
-  // the same buffers for every b)
+  // kept from forward to backward (xin for the whole call; the rest for the current pass, except on the checkpoint
+  // plan: Z3, coef, gnstat and arg for the whole call, the other planes for one block of the current pass, H[b] ..
+  // MULT[b] the same buffers for every b)
   void* xin;
   void* H[FGNN_MAX_BLOCKS][3][FGNN_MAX_DEPTH];
   void *Y1[FGNN_MAX_BLOCKS], *Y2[FGNN_MAX_BLOCKS], *MULT[FGNN_MAX_BLOCKS], *Z3[FGNN_MAX_BLOCKS];
@@ -1000,8 +984,8 @@ size_t carve_train(const TrainPlan& tp, Arena& ar, TrainBuf& B) {
   const Geo& geo = tp.geo;
   const size_t G = tp.G, C = tp.C;
   const size_t actC = G * C * geo.stride(kLayoutC);
-  // recompute / checkpoint: the batch's input planes come first, outside the plane range that every pass zeroes
-  if (tp.recompute || tp.checkpoint) B.xin = ar.take<uint16_t>((size_t)tp.batch * tp.cin0 * geo.stride(kLayoutC), 1024);
+  // the batch's input planes come first, outside the plane range that every pass zeroes
+  B.xin = ar.take<uint16_t>((size_t)tp.batch * tp.cin0 * geo.stride(kLayoutC), 1024);
   if (tp.checkpoint) {   // the block checkpoints of the whole batch, also outside that range
     const size_t BC = (size_t)tp.batch * C;
     for (int b = 0; b < tp.nb; ++b) B.Z3[b] = ar.take<uint16_t>(BC * geo.stride(kLayoutC), 1024);
@@ -1013,7 +997,6 @@ size_t carve_train(const TrainPlan& tp, Arena& ar, TrainBuf& B) {
     B.arg = ar.take<int32_t>(BC * geo.N);
   }
   B.planes_begin = align_up(ar.off, 1024);
-  if (!tp.recompute && !tp.checkpoint) B.xin = ar.take<uint16_t>(G * tp.cin0 * geo.stride(kLayoutC), 1024);
   const int sets = tp.checkpoint ? 1 : tp.nb;
   for (int b = 0; b < sets; ++b) {
     for (int m = 0; m < 3; ++m)
@@ -1073,7 +1056,7 @@ size_t train_workspace_bytes(const TrainPlan& tp) {
 }
 
 // T of the plan selection, in bytes (see TrainPlan)
-size_t keep_all_limit() {
+size_t one_pass_limit() {
   if (const char* v = getenv("FGNN_TC_TRAIN_WS_GB")) return (size_t)(std::min(std::max(atof(v), 0.0), 1e9) * (double)(1ull << 30));
   static size_t cache[64] = {0};   // per device: the query is not free and runs three times per embedder call
   int dev = 0;
@@ -1108,8 +1091,7 @@ int make_train_plan(const fgnn_embed_params& p, int G, int N, bool det, bool ckp
   tp.c_emb = p.block[p.num_blocks - 1].mlp3.c_out;
   tp.G = G;
   tp.batch = G;
-  tp.recompute = false;
-  tp.checkpoint = false;
+  tp.checkpoint = ckpt;
   tp.det = det;
   tp.D = p.block[0].mlp1.depth;
   for (int b = 0; b < p.num_blocks; ++b) {
@@ -1120,12 +1102,7 @@ int make_train_plan(const fgnn_embed_params& p, int G, int N, bool det, bool ckp
   if (tp.D < 1 || tp.D > FGNN_MAX_DEPTH) return fail(FGNN_ERR_INVALID, "bad depth %d", tp.D);
   if (tp.cin0 > 64) return fail(FGNN_ERR_UNSUPPORTED, "original_features_num %d > 64 unsupported", tp.cin0);
   if ((long)G * tp.C > 65535) return fail(FGNN_ERR_UNSUPPORTED, "16-bit training: G * C = %ld planes exceed one call's grid (split the batch)", (long)G * tp.C);
-  if (ckpt) {
-    tp.checkpoint = true;
-  } else {
-    if (train_workspace_bytes(tp) <= keep_all_limit()) return FGNN_OK;
-    tp.recompute = true;
-  }
+  if (!ckpt && train_workspace_bytes(tp) <= one_pass_limit()) return FGNN_OK;   // the whole batch in one pass
   int chunk = env_int("FGNN_TC_CHUNK", 0);
   if (chunk <= 0) {   // the largest pass whose own carve (batch = 0: without the batch-wide part) fits the budget, or 1
     const size_t budget = (size_t)std::max(1, env_int("FGNN_TC_WS_GB", 16)) << 30;
@@ -1151,10 +1128,11 @@ TrainPlan pass_plan(const TrainPlan& tp, int g0) {
   return pp;
 }
 
-// the buffers of the pass that starts at graph g0: on the checkpoint plan its graphs' part of the batch-wide buffers,
-// on the other plans B itself (their buffers hold one pass)
+// the buffers of the pass that starts at graph g0: its graphs' part of the batch-wide buffers (the input planes, and on
+// the checkpoint plan the checkpoints), B's own for the rest (they hold one pass)
 TrainBuf pass_bufs(const TrainPlan& tp, const TrainBuf& B, int g0) {
   TrainBuf V = B;
+  V.xin = static_cast<uint16_t*>(B.xin) + (size_t)g0 * tp.cin0 * tp.geo.PSC;
   if (!tp.checkpoint) return V;
   const size_t gc = (size_t)g0 * tp.C;
   for (int b = 0; b < tp.nb; ++b) {
@@ -1171,7 +1149,7 @@ TrainBuf pass_bufs(const TrainPlan& tp, const TrainBuf& B, int g0) {
 // Zero what a pass's producers never write but later reads cover, before every pass's forward.  Ragged batch: all the
 // kept planes and the backward scratch (rows beyond a graph's covered range are never written, the GEMM K loops read
 // them, and an earlier pass's larger graph leaves data there).  Otherwise: the physical rows / column chunks the
-// producers skip.  The batch-wide part of the recompute and checkpoint plans lies before planes_begin and is not touched.
+// producers skip.  The batch-wide part of the workspace lies before planes_begin and is not touched.
 int zero_pass(const TrainPlan& tp, const TrainBuf& B, void* ws, bool ragged, cudaStream_t st) {
   const Geo& geo = tp.geo;
   const size_t GC = (size_t)tp.G * tp.C;
@@ -1263,8 +1241,8 @@ struct BlockIn {
   const float* coef;
 };
 template <typename T>
-BlockIn<T> block_in(const fgnn_embed_params& p, const TrainPlan& tp, const TrainBuf& B, int b, const T* xin) {
-  if (b == 0) return {xin, tp.cin0, tp.cin0, nullptr};
+BlockIn<T> block_in(const fgnn_embed_params& p, const TrainPlan& tp, const TrainBuf& B, int b) {
+  if (b == 0) return {reinterpret_cast<const T*>(B.xin), tp.cin0, tp.cin0, nullptr};
   return {reinterpret_cast<const T*>(B.Z3[b - 1]), tp.C, p.block[b - 1].mlp3.c_out, B.coef[b - 1][2]};
 }
 
@@ -1272,11 +1250,11 @@ BlockIn<T> block_in(const fgnn_embed_params& p, const TrainPlan& tp, const Train
 // GraphNorm statistics of its MLPs into B.  z3 = false stops before mlp3's last conv (the checkpoint plan's backward:
 // Z3[b] and its statistics are kept, never rewritten).
 template <typename T>
-int train_fwd_block(const fgnn_embed_params& p, const TrainPlan& tp, const TrainBuf& B, int b, const T* xin, bool z3,
+int train_fwd_block(const fgnn_embed_params& p, const TrainPlan& tp, const TrainBuf& B, int b, bool z3,
                     const int32_t* npg, cudaStream_t st) {
   const Geo& geo = tp.geo;
   const int G = tp.G, C = tp.C, D = tp.D;
-  const BlockIn<T> in = block_in<T>(p, tp, B, b, xin);
+  const BlockIn<T> in = block_in<T>(p, tp, B, b);
   const T* cur = in.x;
   const int cur_c = in.c, cur_real = in.c_real;
   const float* cur_coef = in.coef;
@@ -1337,16 +1315,16 @@ int train_fwd_block(const fgnn_embed_params& p, const TrainPlan& tp, const Train
   return FGNN_OK;
 }
 
-// training forward of one pass (tp.G graphs): their input planes xin -> emb (tp.G, C, N), and in B everything the
+// training forward of one pass (tp.G graphs): their input planes B.xin -> emb (tp.G, C, N), and in B everything the
 // backward reads
 template <typename T>
-int train_fwd_pass(const fgnn_embed_params& p, const TrainPlan& tp, const TrainBuf& B, const T* xin, float* emb,
-                   const int32_t* npg, cudaStream_t st) {
+int train_fwd_pass(const fgnn_embed_params& p, const TrainPlan& tp, const TrainBuf& B, float* emb, const int32_t* npg,
+                   cudaStream_t st) {
   const Geo& geo = tp.geo;
   for (int b = 0; b < tp.nb; ++b)
-    if (int e = train_fwd_block<T>(p, tp, B, b, xin, true, npg, st)) return e;
+    if (int e = train_fwd_block<T>(p, tp, B, b, true, npg, st)) return e;
   {
-    const BlockIn<T> out = block_in<T>(p, tp, B, tp.nb, xin);
+    const BlockIn<T> out = block_in<T>(p, tp, B, tp.nb);
     dim3 grid((unsigned)((geo.N + 7) / 8), tp.G * tp.C);
     colmax16_kernel<T><<<grid, 256, 0, st>>>(out.x, out.coef, emb, B.arg, tp.C, out.c_real, geo, npg);
     FGNN_LAUNCHED();
@@ -1364,20 +1342,19 @@ int embed_fwd_train_t(const fgnn_embed_params& p, bool det, bool ckpt, const flo
   const size_t need = carve_train(tp, ar, B);
   if (need > ws_bytes) return fail(FGNN_ERR_WORKSPACE, "training workspace too small: %zu < %zu", ws_bytes, need);
   const Geo& geo = tp.geo;
-  T* xin = reinterpret_cast<T*>(B.xin);
   FGNN_CUDA(cudaMemsetAsync(B.zeros, 0, 512 * sizeof(float), st));
   if (tp.checkpoint && npg)   // ragged: the batch's checkpoints once, as zero_pass does for a pass's planes
     for (int b = 0; b < tp.nb; ++b) FGNN_CUDA(cudaMemsetAsync(B.Z3[b], 0, (size_t)G * tp.C * geo.PSC * sizeof(T), st));
+  {   // the whole batch's input planes, every pixel (padding and holes included) written
+    dim3 grid((unsigned)std::min(N, 256), G * tp.cin0);
+    to_planes_c_kernel<T><<<grid, 256, 0, st>>>(x, reinterpret_cast<T*>(B.xin), tp.cin0, geo, npg);
+    FGNN_LAUNCHED();
+  }
   for (int g0 = 0; g0 < G; g0 += tp.G) {
     const TrainPlan pp = pass_plan(tp, g0);
     if (int e = zero_pass(pp, B, ws, npg != nullptr, st)) return e;
-    if (g0 == 0) {   // the whole batch, after the first zeroing: on keep-all the zeroed range holds xin
-      dim3 grid((unsigned)std::min(N, 256), G * tp.cin0);
-      to_planes_c_kernel<T><<<grid, 256, 0, st>>>(x, xin, tp.cin0, geo, npg);
-      FGNN_LAUNCHED();
-    }
-    if (int e = train_fwd_pass<T>(p, pp, pass_bufs(tp, B, g0), xin + (size_t)g0 * tp.cin0 * geo.PSC,
-                                  emb + (size_t)g0 * tp.c_emb * N, npg ? npg + g0 : nullptr, st)) return e;
+    if (int e = train_fwd_pass<T>(p, pp, pass_bufs(tp, B, g0), emb + (size_t)g0 * tp.c_emb * N, npg ? npg + g0 : nullptr,
+                                  st)) return e;
   }
   return FGNN_OK;
 }
@@ -1505,7 +1482,7 @@ int mlp_bwd(const MlpBwd<T>& a, const TrainPlan& tp, const TrainBuf& B, const in
 // On the checkpoint plan B holds the pass's checkpoints, and each block's forward is re-run just before its backward.
 template <typename T>
 int train_bwd_pass(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const TrainPlan& tp, const TrainBuf& B,
-                   const T* xin, const float* demb, const int32_t* npg, cudaStream_t st) {
+                   const float* demb, const int32_t* npg, cudaStream_t st) {
   const Geo& geo = tp.geo;
   const int G = tp.G, N = geo.N, C = tp.C, GC = G * C;
   const size_t plane_bytes = (size_t)GC * geo.PSC * sizeof(T);
@@ -1521,10 +1498,10 @@ int train_bwd_pass(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const
   for (int b = tp.nb - 1; b >= 0; --b) {
     // checkpoint plan: block b's intermediates, re-derived from its kept input into the planes all blocks share
     if (tp.checkpoint)
-      if (int e = train_fwd_block<T>(p, tp, B, b, xin, false, npg, st)) return e;
+      if (int e = train_fwd_block<T>(p, tp, B, b, false, npg, st)) return e;
     const fgnn_block_params& bp = p.block[b];
     const fgnn_block_grads& bg = gr.block[b];
-    const BlockIn<T> in = block_in<T>(p, tp, B, b, xin);
+    const BlockIn<T> in = block_in<T>(p, tp, B, b);
     const T* cur = in.x;
     const int cur_c = in.c, cur_real = in.c_real;
     const int co = bp.mlp1.c_out;
@@ -1625,24 +1602,22 @@ int embed_bwd_t(const fgnn_embed_params& p, const fgnn_embed_grads& gr, bool det
   TrainBuf B;
   const size_t need = carve_train(tp, ar, B);
   if (need > ws_bytes) return fail(FGNN_ERR_WORKSPACE, "training workspace too small: %zu < %zu", ws_bytes, need);
-  const Geo& geo = tp.geo;
   // one loss scale for the whole batch, whatever the passes
   grad_scale_kernel<<<1, 1024, 0, st>>>(demb, (long)G * tp.c_emb * N, B.scale, grad_scale_log2);
   FGNN_LAUNCHED();
-  const T* xin = reinterpret_cast<const T*>(B.xin);
+  const bool passes = tp.G < G;   // else the forward's single pass is still in the workspace
   for (int g0 = 0; g0 < G; g0 += tp.G) {
     const TrainPlan pp = pass_plan(tp, g0);
-    const T* xin_p = xin + (size_t)g0 * tp.cin0 * geo.PSC;
+    const TrainBuf V = pass_bufs(tp, B, g0);
     const int32_t* npg_p = npg ? npg + g0 : nullptr;
-    if (tp.recompute) {
-      // re-derive the pass's activations; its embeddings land in rowsum, which the backward rewrites before reading it
+    // the pass's planes (on the checkpoint plan: the shared block planes) and the backward scratch hold other data than
+    // this pass's forward left: zero them as the forward did
+    if (passes || tp.checkpoint)
       if (int e = zero_pass(pp, B, ws, npg != nullptr, st)) return e;
-      if (int e = train_fwd_pass<T>(p, pp, B, xin_p, B.rowsum, npg_p, st)) return e;
-    } else if (tp.checkpoint) {
-      // the shared block planes and the backward scratch hold another pass's data: zero them as the forward did
-      if (int e = zero_pass(pp, B, ws, npg != nullptr, st)) return e;
-    }
-    if (int e = train_bwd_pass<T>(p, gr, pp, pass_bufs(tp, B, g0), xin_p, demb + (size_t)g0 * tp.c_emb * N, npg_p, st)) return e;
+    // re-derive the pass's activations; its embeddings land in rowsum, which the backward rewrites before reading it
+    if (passes && !tp.checkpoint)
+      if (int e = train_fwd_pass<T>(p, pp, V, V.rowsum, npg_p, st)) return e;
+    if (int e = train_bwd_pass<T>(p, gr, pp, V, demb + (size_t)g0 * tp.c_emb * N, npg_p, st)) return e;
   }
   return FGNN_OK;
 }

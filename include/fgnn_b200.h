@@ -55,8 +55,8 @@ typedef enum {
  * several CTAs (GraphNorm statistics, bias and weight gradients) is then formed from per-CTA records added in a fixed
  * order instead of floating-point atomics, so that, for the same build, device model, inputs, batch composition,
  * FGNN_TC_* variables and parameters, the embeddings and parameter gradients are bit-identical from run to run.  Not
- * covered: a graph alone vs inside a batch, keep-all vs recompute plans (the reduction partitions differ), multi-GPU
- * all-reduce order.  The workspaces are larger (they hold the records): the workspace query, the forward and the
+ * covered: a graph alone vs inside a batch, one batch cut into different passes (the reduction partitions differ),
+ * multi-GPU all-reduce order.  The workspaces are larger (they hold the records): the workspace query, the forward and the
  * backward of one training call must all take the same flag, as they must see the same FGNN_TC_* variables.  The fused
  * head (fgnn_head_*) accepts the bit and ignores it: it is deterministic in both modes.  Any other bit outside the
  * precision's low byte is rejected (FGNN_ERR_INVALID; workspace queries return 0). */
@@ -319,24 +319,26 @@ int fgnn_embed_fwd_adjacency_u8(const fgnn_embed_params* p, int32_t precision, c
  * the default, -24 .. 15 accepted; bf16 never overflows).  The workspace must be the one the forward call filled
  * (same G, N, parameters), fgnn_embed_train_workspace_bytes(...) bytes, 1024-byte aligned.  Every MLP has the same
  * depth, and N <= 1024 (N <= 4096 with FGNN_CHECKPOINT_BLOCKS).
- * Three plans, picked by all three calls alike:
- *   keep-all   the workspace keeps every activation of the batch from forward to backward (about 51 plane sets per
- *              graph at depth 3, 4 blocks: 107 GB for 64 graphs of N = 500, C = 64).  Used while that size is <= T.
- *   recompute  the workspace keeps the 16-bit input planes of the batch plus the activations of one pass of graphs;
- *              the forward runs pass by pass and keeps only emb, the backward re-runs each pass's forward before its
- *              backward (about one more forward per step; the loss scale is still chosen once over all of d emb).
- *              Passes are equal and as large as fit FGNN_TC_WS_GB (default 16) GiB, never less than one graph
- *              (FGNN_TC_CHUNK graphs when set, as for fgnn_embed_fwd).
+ * Two workspace layouts, picked by all three calls alike.  Both keep the 16-bit input planes of the whole batch and
+ * cut the batch into passes of graphs.
+ *   passes     the workspace keeps every activation of one pass (about 51 plane sets per graph at depth 3, 4 blocks:
+ *              107 GB for 64 graphs of N = 500, C = 64).  While that size for the whole batch is <= T, the batch is
+ *              one pass and the forward's activations stay in the workspace until the backward.  Otherwise passes are
+ *              equal and as large as fit FGNN_TC_WS_GB (default 16) GiB, never less than one graph (FGNN_TC_CHUNK
+ *              graphs when set, as for fgnn_embed_fwd); the forward runs pass by pass and keeps only emb, the backward
+ *              re-runs each pass's forward before its backward (about one more forward per step; the loss scale is
+ *              still chosen once over all of d emb).
  *   checkpoint used when `precision` carries FGNN_CHECKPOINT_BLOCKS, and then always (T plays no part).  The workspace
  *              keeps, for the whole batch, the input planes, every block's output and GraphNorm statistics and the
  *              pooling arg-max, plus one block's activations and the backward scratch for one pass of graphs (passes
- *              cut as for recompute): about nb + 3 depth + 11 plane sets per graph, 55 GB for one graph of N = 4096,
- *              C = 64, 4 blocks of depth 3.  The backward re-runs each block's forward from its kept input just before
- *              that block's backward (about one more forward per step).
- * T is FGNN_TC_TRAIN_WS_GB GiB when set (0 always picks recompute); otherwise half the current device's memory, because
- * a siamese step holds two workspaces (x1 and x2) until backward; unlimited when no device can be queried.  The plan
- * must not change between fgnn_embed_fwd_train and fgnn_embed_bwd: keep these variables and the current device as
- * they were for the workspace query. */
+ *              cut by FGNN_TC_WS_GB / FGNN_TC_CHUNK as above): about nb + 3 depth + 11 plane sets per graph, 55 GB for
+ *              one graph of N = 4096, C = 64, 4 blocks of depth 3.  The backward re-runs each block's forward from its
+ *              kept input just before that block's backward (about one more forward per step).
+ * T is FGNN_TC_TRAIN_WS_GB GiB when set (0: the batch is always cut by FGNN_TC_WS_GB / FGNN_TC_CHUNK, and a batch that
+ * fits one pass is not re-run); otherwise half the current device's memory, because a siamese step holds two workspaces
+ * (x1 and x2) until backward; unlimited when no device can be queried.  The passes must not change between
+ * fgnn_embed_fwd_train and fgnn_embed_bwd: keep these variables and the current device as they were for the workspace
+ * query. */
 size_t fgnn_embed_train_workspace_bytes(const fgnn_embed_params* p, int32_t precision, int32_t G, int32_t N);
 int fgnn_embed_fwd_train(const fgnn_embed_params* p, int32_t precision, const float* x, float* emb, int32_t G,
                          int32_t N, const int32_t* n_per_graph, void* workspace, size_t workspace_bytes,

@@ -1,5 +1,5 @@
 """CPU tests of the deterministic mode (FGNN_DETERMINISTIC): flag handling of the C ABI, the workspaces it asks for,
-the plan choice that follows them, and a SASS audit of which kernels may add with floating-point atomics (nothing here
+how the batch is cut into passes by them, and a SASS audit of which kernels may add with floating-point atomics (nothing here
 touches a device)."""
 import ctypes
 import os
@@ -54,8 +54,8 @@ def test_default_sizes_unchanged_and_deterministic_sizes_larger(prec, plan_env):
 
 
 def test_plan_choice_follows_the_deterministic_size(plan_env):
-    """A keep-all threshold between the default and the deterministic keep-all sizes: the default keeps everything,
-    the deterministic mode cuts the batch into recompute passes (of FGNN_TC_CHUNK graphs: smaller than keep-all)."""
+    """A threshold between the default and the deterministic one-pass sizes: the default runs the batch as one pass,
+    the deterministic mode cuts it into passes (of FGNN_TC_CHUNK graphs: smaller than one pass)."""
     c, g, n = 32, 16, 200
     p = L.PRECISIONS["fp16"]
     plan_env.setenv("FGNN_TC_TRAIN_WS_GB", "1000")

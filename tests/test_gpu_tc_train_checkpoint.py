@@ -1,9 +1,9 @@
 """GPU tests of the checkpoint plan of 16-bit training (FGNN_CHECKPOINT_BLOCKS, Network.set_checkpoint_blocks): the
 forward keeps each block's output, the backward re-runs each block's forward just before its backward.
 
-Against the recompute plan with the same passes the plan runs the same kernels on the same graphs: in the deterministic
-mode both give the same loss, embeddings and gradients bit for bit, up to N = 1024.  Above, where no other 16-bit plan
-trains, the loss is checked against the fp32 mode (see fp32_vs_checkpoint for the gradients).
+Against training without checkpoints on the same passes the plan runs the same kernels on the same graphs: in the
+deterministic mode both give the same loss, embeddings and gradients bit for bit, up to N = 1024.  Above, where nothing
+else trains in 16 bits, the loss is checked against the fp32 mode (see fp32_vs_checkpoint for the gradients).
 """
 import contextlib
 
@@ -66,7 +66,8 @@ def device_pair(n, seed, pairs=1):
 
 
 def both_plans(make_model, x1, x2, monkeypatch, chunk):
-    """(recompute, checkpoint) train_once results on the same passes of `chunk` graphs."""
+    """(without, with checkpoints) train_once results on the same passes of `chunk` graphs (FGNN_TC_TRAIN_WS_GB=0: a
+    batch of more than `chunk` graphs is re-derived pass by pass in backward, one that fits a single pass is not)."""
     use_plan(monkeypatch, True, chunk)
     rc = train_once(make_model(), {"input": x1}, {"input": x2})
     ck = train_once(make_model().set_checkpoint_blocks(), {"input": x1}, {"input": x2})
@@ -76,8 +77,8 @@ def both_plans(make_model, x1, x2, monkeypatch, chunk):
 @pytest.mark.parametrize("prec", ["fp16", "bf16"])
 @pytest.mark.parametrize("name", ["cfg1_er50_c32", "cfg2_er200_c32"])
 def test_checkpoint_matches_recompute_on_goldens(name, prec, monkeypatch):
-    """cfg1 (4 pairs) in passes of one graph, cfg2 (1 pair) in one pass: bit-identical to the recompute plan in the
-    deterministic mode, within the recompute tests' golden envelope without it."""
+    """cfg1 (4 pairs) in passes of one graph, cfg2 (1 pair) in one pass: bit-identical to the same passes without
+    checkpoints in the deterministic mode, within the recompute tests' golden envelope without it."""
     z = load_golden(name)
     x1, x2 = golden_inputs(z)
     with deterministic():
@@ -103,7 +104,7 @@ def test_checkpoint_matches_recompute_shallow_models(nb, depth, monkeypatch):
 
 def test_checkpoint_gradients_match_oracles(monkeypatch):
     """The checkpoint gradients against the emulated-16-bit autograd and the reference's fp32 autograd, as the
-    recompute plan's are checked."""
+    gradients of passes without checkpoints are checked."""
     for v in ("FGNN_TC_TRAIN_WS_GB", "FGNN_TC_WS_GB", "FGNN_TC_CHUNK"):
         monkeypatch.delenv(v, raising=False)
     for name in ("cfg1_er50_c32", "cfg2_er200_c32"):
@@ -142,18 +143,19 @@ def test_checkpoint_ragged_matches_recompute(cst, monkeypatch):
 
 
 def test_checkpoint_matches_recompute_at_1024(monkeypatch):
-    """The largest size both plans train: one pair at N = 1024, C = 64, 4 blocks of depth 3."""
+    """The largest size trained with and without checkpoints: one pair at N = 1024, C = 64, 4 blocks of depth 3, one
+    pass (which the backward does not re-run without checkpoints; the ragged tests cover the re-run in passes of 2)."""
     x1, x2 = device_pair(1024, 7)
     with deterministic():
         rc, ck = both_plans(lambda: random_model(4, 3, 64, seed=64), x1, x2, monkeypatch, None)
-    assert_bit_identical("checkpoint vs recompute N = 1024 C = 64 deterministic", ck, rc)
+    assert_bit_identical("checkpoint vs one pass N = 1024 C = 64 deterministic", ck, rc)
 
 
 # Above N = 1024 against the fp32 mode.  Only the loss is held to a bound.  The parameter gradients of the 16-bit
 # backward leave the fp32 gradients at large N on every plan, not only this one.  Measured on one B200 (1000 W) for one
 # ErdosRenyi pair, 2 blocks of depth 2, C = 32, fp16, all parameters together:
 #   - 2.8e-2 at N = 256 (cosine 0.9996);
-#   - 0.45 at N = 1024 on the default plan and on the checkpoint plan alike (bit-identical gradients, cosine 0.94);
+#   - 0.45 at N = 1024 without checkpoints and with them alike (bit-identical gradients, cosine 0.94);
 #   - 0.48 at N = 4096 (cosine 0.89).
 # No test pinned 16-bit gradients beyond n = 500 before, so this is a limit of the 16-bit backward at these sizes, not
 # of the checkpoints.  These tests print the gradient parity, and hold the loss, finiteness, and the mathematically

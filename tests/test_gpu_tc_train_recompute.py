@@ -1,15 +1,15 @@
-"""GPU tests of the recompute plan of 16-bit training (fgnn_embed_fwd_train / fgnn_embed_bwd cut into passes whose
-activations the backward re-derives from the input planes).
+"""GPU tests of 16-bit training in passes (fgnn_embed_fwd_train / fgnn_embed_bwd cut into passes whose activations the
+backward re-derives from the input planes).
 
-The plan is chosen from the keep-all workspace size against FGNN_TC_TRAIN_WS_GB (default: half the device's memory),
-so the tests force it with FGNN_TC_TRAIN_WS_GB=0 and set the pass with FGNN_TC_CHUNK; the keep-all runs they are
-compared with set a threshold no batch here reaches.  Both plans run the same kernels per graph, and the forward is
-deterministic: a recompute plan of one pass gives keep-all's embeddings bit for bit (measured).  What differs is how
-many graphs share a launch.  That changes how the conv-chain kernel's CTAs split the (graph, tile) work, so the
-GraphNorm statistics are summed in another order and 16-bit activations round differently from the first block on.
-The inference path shows the same when FGNN_TC_CHUNK cuts a ragged batch into passes (2.0e-3 to 3.0e-3 on the
-embeddings of the batches below).  Weight-gradient reductions are fp32 atomics in any order (a few 1e-7 between two
-runs of the same plan).
+A batch is cut into passes when its one-pass workspace exceeds FGNN_TC_TRAIN_WS_GB (default: half the device's
+memory), so the tests force passes with FGNN_TC_TRAIN_WS_GB=0 and set them with FGNN_TC_CHUNK; the one-pass runs
+("keep-all") they are compared with set a threshold no batch here reaches.  Every pass runs the same kernels per graph,
+and the forward is deterministic: a batch that fits one pass gives the same embeddings bit for bit whatever the
+threshold (measured), and its backward re-runs nothing.  What differs with several passes is how many graphs share a
+launch.  That changes how the conv-chain kernel's CTAs split the (graph, tile) work, so the GraphNorm statistics are
+summed in another order and 16-bit activations round differently from the first block on.  The inference path shows
+the same when FGNN_TC_CHUNK cuts a ragged batch into passes (2.0e-3 to 3.0e-3 on the embeddings of the batches below).
+Weight-gradient reductions are fp32 atomics in any order (a few 1e-7 between two runs on the same passes).
 """
 import numpy as np
 import pytest
@@ -85,7 +85,8 @@ RAGGED_PASSES_TOL = (1e-6, 1e-6, 1e-6)
 @pytest.mark.parametrize("prec", ["fp16", "bf16"])
 @pytest.mark.parametrize("name", ["cfg1_er50_c32", "cfg2_er200_c32"])
 def test_recompute_gradients_match_oracles_and_keep_all(name, prec, monkeypatch):
-    """cfg1 (4 pairs) runs as 4 passes of one graph; cfg2 (1 pair) as one pass, recomputed in backward."""
+    """cfg1 (4 pairs) runs as 4 passes of one graph, each re-derived in backward; cfg2 (1 pair) as one pass, which the
+    backward does not re-run (the same work as the one-pass run it is compared with)."""
     z = load_golden(name)
     n = int(z["meta"][0])
     if "W1" in z:
@@ -106,6 +107,39 @@ def test_recompute_gradients_match_oracles_and_keep_all(name, prec, monkeypatch)
         compare_grads(model, egrads, EMUL_TOL[prec], f"{name} {prec} recompute vs emulated-16-bit-forward autograd", depth, nb)
     finally:
         compare_grads(model, ref, REF_TOL[prec], f"{name} {prec} recompute vs reference fp32 autograd", depth, nb)
+
+
+def test_backward_re_runs_the_forward_only_for_several_passes(monkeypatch):
+    """Kernel launches of each fgnn_embed_bwd call (x1's and x2's) on cfg1's 4 pairs: with FGNN_TC_TRAIN_WS_GB=0 and
+    FGNN_TC_CHUNK >= G the batch is one pass whose activations the forward left in place, so the backward launches
+    exactly what it does below the threshold; in two passes it launches more (each pass's forward again)."""
+    z = load_golden("cfg1_er50_c32")
+    x1, x2 = feats(z["W1"]).to(DEV), feats(z["W2"]).to(DEV)
+    G = x1.shape[0]
+    lib = pkg.get_lib()
+    embed_bwd, counts = lib.fgnn_embed_bwd, []
+
+    def counted(*args):      # runs on autograd's thread: the launch counter is thread-local
+        lib.fgnn_reset_launch_count()
+        status = embed_bwd(*args)
+        counts.append(lib.fgnn_launch_count())
+        return status
+
+    monkeypatch.setattr(lib, "fgnn_embed_bwd", counted)
+
+    def launches(recompute, chunk):
+        counts.clear()
+        use_plan(monkeypatch, recompute, chunk)
+        train_once(build_model(z, "fp16"), {"input": x1}, {"input": x2})
+        assert len(counts) == 2, counts
+        return list(counts)
+
+    one_pass = launches(False, None)
+    assert launches(True, G) == one_pass
+    assert launches(True, 2 * G) == one_pass
+    two = launches(True, G // 2)
+    print(f"PARITY fgnn_embed_bwd launches: one pass {one_pass}, two passes {two}")
+    assert all(t > o for t, o in zip(two, one_pass)), (two, one_pass)
 
 
 def ragged_runs(sizes, cst, plans, monkeypatch):

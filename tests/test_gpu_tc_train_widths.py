@@ -94,21 +94,11 @@ def head_loss(e1, e2, n_dev):
     return ce.sum() / n_dev.to(torch.float32).sum()
 
 
-@pytest.mark.parametrize("prec", ["fp16", "bf16"])
-@pytest.mark.parametrize("in_f,out_f,depth", CASES)
-def test_padded_widths_match_the_uniform_twin(in_f, out_f, depth, prec, twin):
-    _ops.GRAD_SINK.clear()
-    model = make_model(in_f, out_f, depth).to(DEV).set_precision(prec)
-    tw, C = twin(model, in_f, out_f, depth)
-    x1, x2 = ragged_pair()
+def twin_training_parity(label, model, tw, C, out_f, x1, x2):
+    """One training forward + backward of the model and of its twin: embeddings and loss bitwise equal, the twin's
+    gradients exact zeros on the padded entries, the model's as close to the twin's as two runs of the twin are."""
     n_dev = x1.sizes_i32(DEV)
     net, tnet = model.node_embedder, tw.node_embedder
-    with torch.no_grad():
-        for x in (x1, x2):
-            e, et = plain(net.forward_fused(x)), plain(tnet.forward_fused(x))
-            assert e.shape == (len(SIZES), out_f, max(SIZES)) and et.shape[1] == C
-            assert torch.equal(e, et[:, :out_f])
-            assert not et[:, out_f:].any()
     e1, e2 = plain(net.forward_fused_train(x1)), plain(net.forward_fused_train(x2))
     t1, t2 = plain(tnet.forward_fused_train(x1)), plain(tnet.forward_fused_train(x2))
     assert torch.equal(e1.detach(), t1.detach()[:, :out_f]) and torch.equal(e2.detach(), t2.detach()[:, :out_f])
@@ -135,9 +125,26 @@ def test_padded_widths_match_the_uniform_twin(in_f, out_f, depth, prec, twin):
     mine, twin_a, twin_b = torch.cat(mine), torch.cat(twin_a), torch.cat(twin_b)
     d_model = float((mine - twin_a).norm() / twin_a.norm())
     d_twin = float((twin_b - twin_a).norm() / twin_a.norm())
-    print(f"PARITY {prec} in={in_f} out={out_f} depth={depth}: embeddings and loss {float(loss):.6f} bitwise equal to the "
-          f"C={C} twin; gradients {d_model:.2e} from the twin's (two runs of the twin: {d_twin:.2e})")
+    print(f"PARITY {label}: embeddings and loss {float(loss):.6f} bitwise equal to the C={C} twin; gradients "
+          f"{d_model:.2e} from the twin's (two runs of the twin: {d_twin:.2e})")
     assert d_model <= 4 * d_twin + 2e-6, (d_model, d_twin)
+
+
+@pytest.mark.parametrize("prec", ["fp16", "bf16"])
+@pytest.mark.parametrize("in_f,out_f,depth", CASES)
+def test_padded_widths_match_the_uniform_twin(in_f, out_f, depth, prec, twin):
+    _ops.GRAD_SINK.clear()
+    model = make_model(in_f, out_f, depth).to(DEV).set_precision(prec)
+    tw, C = twin(model, in_f, out_f, depth)
+    x1, x2 = ragged_pair()
+    net, tnet = model.node_embedder, tw.node_embedder
+    with torch.no_grad():
+        for x in (x1, x2):
+            e, et = plain(net.forward_fused(x)), plain(tnet.forward_fused(x))
+            assert e.shape == (len(SIZES), out_f, max(SIZES)) and et.shape[1] == C
+            assert torch.equal(e, et[:, :out_f])
+            assert not et[:, out_f:].any()
+    twin_training_parity(f"{prec} in={in_f} out={out_f} depth={depth}", model, tw, C, out_f, x1, x2)
 
 
 @pytest.mark.parametrize("cst", [False, True])
@@ -191,31 +198,16 @@ def test_flat_train_step_at_padded_widths(fused_head):
     assert losses[-1] < losses[0]
 
 
-def test_recompute_plan_reproduces_keep_all_at_padded_widths(monkeypatch):
+def test_recompute_passes_match_the_uniform_twin_at_padded_widths(monkeypatch, twin):
+    """The batch cut into passes of two graphs ([50, 23], [37, 64], [130]), each re-derived from its input planes in
+    backward: the model and its twin on the same passes."""
     _ops.GRAD_SINK.clear()
-    model = make_model(24, 40, 3).to(DEV).set_precision("fp16")
-    x1, x2 = ragged_pair()
-    n_dev = x1.sizes_i32(DEV)
-    net = model.node_embedder
-
-    def run():
-        model.zero_grad(set_to_none=True)
-        e1, e2 = plain(net.forward_fused_train(x1)), plain(net.forward_fused_train(x2))
-        loss = head_loss(e1, e2, n_dev)
-        loss.backward()
-        return [loss.detach(), e1.detach().clone(), e2.detach().clone()], torch.cat([p.grad.flatten() for p in model.parameters()])
-
-    monkeypatch.delenv("FGNN_TC_CHUNK", raising=False)
-    monkeypatch.setenv("FGNN_TC_TRAIN_WS_GB", "1000")
-    ref, gref = run()
-    _, gref2 = run()                                                    # run-to-run spread of the atomics
     monkeypatch.setenv("FGNN_TC_TRAIN_WS_GB", "0")
-    monkeypatch.setenv("FGNN_TC_CHUNK", str(len(SIZES)))             # one recompute pass
-    got, g = run()
-    assert all(torch.equal(a, b) for a, b in zip(ref, got))             # loss and embeddings bit for bit
-    d, d_ka = float((g - gref).norm() / gref.norm()), float((gref2 - gref).norm() / gref.norm())
-    print(f"PARITY recompute (one pass) vs keep-all in=24 out=40: gradients {d:.2e} (two keep-all runs: {d_ka:.2e})")
-    assert d <= 4 * d_ka + 2e-6, (d, d_ka)
+    monkeypatch.setenv("FGNN_TC_CHUNK", "2")
+    model = make_model(24, 40, 3).to(DEV).set_precision("fp16")
+    tw, C = twin(model, 24, 40, 3)
+    x1, x2 = ragged_pair()
+    twin_training_parity("passes of 2, fp16 in=24 out=40 depth=3", model, tw, C, 40, x1, x2)
 
 
 @pytest.mark.parametrize("in_f,out_f", [(65, 65), (32, 65), (128, 128)])

@@ -1,5 +1,5 @@
-"""CPU tests of the 16-bit training plans (keep-all / recompute in passes): which plan a shape gets, the workspace each
-plan asks for, and the limits that stay (nothing here touches a device)."""
+"""CPU tests of how 16-bit training cuts a batch into passes (one pass, or several the backward re-runs): which passes a
+shape gets, the workspace they ask for, and the limits that stay (nothing here touches a device)."""
 import ctypes
 import os
 
@@ -8,7 +8,7 @@ import pytest
 from graph_neural_net_b200 import _lib as L
 
 GIB = 2**30
-# keep-all workspaces (fp16 and bf16, 4 blocks of depth 3), byte for byte what the single-plan version returned:
+# one-pass workspaces (fp16 and bf16, 4 blocks of depth 3), byte for byte what they were before passes existed:
 # (N, C, G) -> bytes
 KEEP_ALL = {
     (200, 32, 1): 171_729_920,          # cfg2 golden: one pair of n = 200
@@ -56,14 +56,14 @@ def keep_all(monkeypatch, c, G, N):
 
 
 def input_planes(G, N, cin=2):
-    """Bytes of G graphs' 16-bit layout-C input planes (the recompute plan keeps them for the whole batch)."""
+    """Bytes of G graphs' 16-bit layout-C input planes (the workspace keeps them for the whole batch)."""
     bn = 64 if N <= 63 else (128 if N <= 127 else 256)
     npc = bn * -(-N // (bn - 1))
     return -(-G * cin * N * npc * 2 // 1024) * 1024
 
 
 def pass_bytes(monkeypatch, c, G, N):
-    """One pass of G graphs on the recompute plan: their keep-all carve without their input planes."""
+    """The part of the workspace that holds one pass of G graphs: their one-pass carve without their input planes."""
     return keep_all(monkeypatch, c, G, N) - input_planes(G, N)
 
 
@@ -98,7 +98,7 @@ def test_pass_is_never_less_than_one_graph(plan_env):
     assert one > GIB
     for g in (1, 3, 8):
         assert ws(64, g, 1024) == one + input_planes(g, 1024)
-    assert ws(64, 1, 1024) == KEEP_ALL[(1024, 64, 1)]    # one graph: the same bytes as keep-all, laid out differently
+    assert ws(64, 1, 1024) == KEEP_ALL[(1024, 64, 1)]    # one graph: one pass, whatever T
 
 
 def test_passes_are_equal(plan_env):

@@ -1,5 +1,5 @@
-"""Time and memory of the 16-bit training step on its three plans (keep-all / recompute in passes / block checkpoints),
-as one JSON document.
+"""Time and memory of the 16-bit training step in one pass, in passes the backward re-runs ("keep-all" and "recompute"
+below) and with block checkpoints, as one JSON document.
 
   python tools/train_memory_bench.py --out train_memory.json
 
@@ -144,7 +144,7 @@ def main():
         torch.cuda.empty_cache()
         return {plan: statistics.median(v) for plan, v in ms.items()}
 
-    # cfg2: the three plans alternated on the same model and batch
+    # cfg2: one pass, re-run passes and checkpoints alternated on the same model and batch
     med = alternate("cfg2", 200, 32, 128, ("keep-all", "recompute", "checkpoint"), args.rounds)
     res["cfg2_recompute_overhead"] = {"keep_all_ms_median": med["keep-all"], "recompute_ms_median": med["recompute"],
                                       "ratio": med["recompute"] / med["keep-all"]}
