@@ -1880,17 +1880,35 @@ int launch_matmul(const T* y1, const T* y2, T* out, const float* coef_a, const f
   });
 }
 
-// fold + conv chain(s) + statistics finalisation for 1 or 2 MLPs sharing their input.  The MLPs' parameters have their
-// real shapes (mp[m]->c_out <= C output channels, cr_src[s] <= c_src[s] channels read from source s); see make_plan.
+// a conv's source: planes of c stored channels, the first c_real real, through the GraphNorm fold coef (null: identity)
+template <typename T>
+struct Src {
+  const T* x;
+  int c, c_real;
+  const float* coef;   // [G][c][2] = {a, s}
+};
+
+// what a launch reads of one MLP: real shapes, first-layer weight w0 (co_real, the sources' c_real summed), b[l] of layer l
+struct MlpLayers {
+  const float* w0;
+  const float* b[FGNN_MAX_DEPTH];
+  int depth, co_real;
+  const fgnn_mlp_params* gn;   // GraphNorm whose coefficients the launch finalises, or null (hidden layers, backward convs)
+};
+
+// mp's layers as one fused conv chain
+MlpLayers chain(const fgnn_mlp_params& mp) {
+  MlpLayers d{mp.w[0], {}, mp.depth, mp.c_out, &mp};
+  for (int l = 0; l < mp.depth; ++l) d.b[l] = mp.b[l];
+  return d;
+}
+
+// fold + conv chain(s) + statistics finalisation for 1 or 2 MLPs sharing their sources; see make_plan for the widths.
 template <typename T>
 struct MlpGroup {
-  int nmlp;
-  const fgnn_mlp_params* mp[2];
-  const T* src[2];
-  int c_src[2];              // channels of the source planes as stored
-  int cr_src[2];             // of which real
-  const float* src_coef[2];
-  int nsrc;
+  int nmlp, nsrc;
+  MlpLayers mlp[2];
+  Src<T> src[2];
   T* wf;             // [G][nmlp][C][K1g] folded first-layer weights
   float* bf;         // [G][nmlp][C] folded first-layer bias
   T* bt;             // [G][nmlp][C][16] folded first-layer bias as an MMA step (may be null for depth-1 launches)
@@ -1905,7 +1923,6 @@ struct MlpGroup {
   unsigned int* rowenc[2];   // fused max pooling of this MLP's output instead of storing it (see MlpArgs), or null
   // training path (depth-1 launches, see fgnn_tc_train.cuh)
   int relu_out;              // out = relu(conv + bias) instead of the raw accumulator
-  int no_coef;               // skip the GraphNorm coefficient finalisation (hidden layers, backward convs)
   float* gnstat[2];          // statistics kept for backward (or null)
 };
 
@@ -1923,18 +1940,17 @@ int launch_mlp_t(const MlpGroup<T>& M, int G, const Geo& geo, const int32_t* npg
   a.G = G;
   a.geo = geo;
   a.nsrc = M.nsrc;
-  a.k_src[0] = round_up(M.c_src[0], 16);
-  a.k_src[1] = M.nsrc > 1 ? round_up(M.c_src[1], 16) : 0;
+  for (int s = 0; s < M.nsrc; ++s) a.k_src[s] = round_up(M.src[s].c, 16);
   a.K1 = a.k_src[0] + a.k_src[1];
   a.K1g = round_up(a.K1, 64);
-  a.depth = M.mp[0]->depth;
+  a.depth = M.mlp[0].depth;
   a.Kh = COUT < 64 ? 64 : COUT;
   a.bias1 = M.bf;
   a.bias1_tile = M.bt;
   FGNN_CHECK_ARG(a.depth == 1 || M.bt != nullptr, "conv chains with hidden layers need the folded bias tile");
   for (int m = 0; m < NMLP; ++m) {
-    FGNN_CHECK_ARG(M.mp[m]->depth == a.depth, "MLPs fused in one launch must have the same depth");
-    for (int l = 0; l < a.depth; ++l) a.bias[m][l] = M.mp[m]->b[l];
+    FGNN_CHECK_ARG(M.mlp[m].depth == a.depth, "MLPs fused in one launch must have the same depth");
+    for (int l = 0; l < a.depth; ++l) a.bias[m][l] = M.mlp[m].b[l];
     a.out[m] = M.out[m];
     a.out_mode[m] = M.out_mode[m];
     a.ones[m] = M.ones[m];
@@ -1943,16 +1959,13 @@ int launch_mlp_t(const MlpGroup<T>& M, int G, const Geo& geo, const int32_t* npg
   a.stat_acc = M.stat_acc;
   a.n_per_graph = npg;
   FGNN_CHECK_ARG(a.K1 <= 256, "first-layer K=%d too wide for the tensor-core MLP kernel", a.K1);
-  CUtensorMap mx0, mx1, mw1, mwh, mo[2];
+  CUtensorMap mx[2], mw1, mwh, mo[2];
   for (int m = 0; m < NMLP; ++m)   // one 64-pixel row piece of all COUT channels per store
     if (int e = plane_map(&mo[m], M.out[m], M.out_mode[m], geo, (uint64_t)G * COUT, 1, COUT)) return e;
   if (NMLP == 1) mo[1] = mo[0];
-  if (int e = pixel_map(&mx0, M.src[0], M.c_src[0], G, geo, a.k_src[0])) return e;
-  if (M.nsrc > 1) {
-    if (int e = pixel_map(&mx1, M.src[1], M.c_src[1], G, geo, a.k_src[1])) return e;
-  } else {
-    mx1 = mx0;
-  }
+  for (int s = 0; s < M.nsrc; ++s)
+    if (int e = pixel_map(&mx[s], M.src[s].x, M.src[s].c, G, geo, a.k_src[s])) return e;
+  if (M.nsrc == 1) mx[1] = mx[0];
   constexpr int is_bf16 = Elem<T>::kFmt;
   if (int e = make_map3(&mw1, is_bf16, M.wf, a.K1g, COUT, (uint64_t)G * NMLP, a.K1g, (uint64_t)COUT * a.K1g, 64, COUT)) return e;
   if (a.depth > 1) {
@@ -1975,7 +1988,7 @@ int launch_mlp_t(const MlpGroup<T>& M, int G, const Geo& geo, const int32_t* npg
     // the opt-in is per device and cheap: set on every call
     FGNN_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     prof::begin(prof::kMlp, st);
-    kernel<<<grid, kMlpThreads, smem, st>>>(mx0, mx1, mw1, mwh, mo[0], mo[1], a);
+    kernel<<<grid, kMlpThreads, smem, st>>>(mx[0], mx[1], mw1, mwh, mo[0], mo[1], a);
     prof::end(prof::kMlp, st);
     FGNN_LAUNCHED();
     return FGNN_OK;
@@ -1986,7 +1999,7 @@ int launch_mlp_t(const MlpGroup<T>& M, int G, const Geo& geo, const int32_t* npg
   }
   // records of the launch (their statistics are only read when the coefficients are finalised)
   a.stat_acc = M.stat_rec;
-  if (!M.no_coef) FGNN_CUDA(cudaMemsetAsync(M.stat_rec, 0, (size_t)(G + grid) * stat_record_doubles(COUT) * sizeof(double), st));
+  if (M.mlp[0].gn) FGNN_CUDA(cudaMemsetAsync(M.stat_rec, 0, (size_t)(G + grid) * stat_record_doubles(COUT) * sizeof(double), st));
   return launch(OrderedSum{});
 }
 
@@ -2000,47 +2013,37 @@ int launch_mlp(const MlpGroup<T>& M, int C, int G, const Geo& geo, const int32_t
 }
 
 template <typename T>
-int run_mlp_group(const MlpGroup<T>& M, int C, int G, const Geo& geo, const int32_t* npg, cudaStream_t st) {
-  const int co_real = M.mp[0]->c_out;
+int run_mlp_group(MlpGroup<T> M, int C, int G, const Geo& geo, const int32_t* npg, cudaStream_t st) {
+  const int co_real = M.mlp[0].co_real;
   FoldArgs fa{};
   fa.nmlp = M.nmlp;
   fa.nsrc = M.nsrc;
-  for (int m = 0; m < M.nmlp; ++m) { fa.w[m] = M.mp[m]->w[0]; fa.b[m] = M.mp[m]->b[0]; }
-  fa.c[0] = M.c_src[0];
-  fa.c[1] = M.nsrc > 1 ? M.c_src[1] : 0;
-  fa.cr[0] = M.cr_src[0];
-  fa.cr[1] = M.nsrc > 1 ? M.cr_src[1] : 0;
-  fa.coef[0] = M.src_coef[0];
-  fa.coef[1] = M.nsrc > 1 ? M.src_coef[1] : nullptr;
+  for (int m = 0; m < M.nmlp; ++m) { fa.w[m] = M.mlp[m].w0; fa.b[m] = M.mlp[m].b[0]; }
+  for (int s = 0; s < M.nsrc; ++s) { fa.c[s] = M.src[s].c; fa.cr[s] = M.src[s].c_real; fa.coef[s] = M.src[s].coef; }
   fa.koff[0] = 0;
-  fa.koff[1] = round_up(M.c_src[0], 16);
+  fa.koff[1] = round_up(fa.c[0], 16);
   fa.c_out = C;
   fa.co_real = co_real;
-  fa.K1g = round_up(round_up(M.c_src[0], 16) + (M.nsrc > 1 ? round_up(M.c_src[1], 16) : 0), 64);
+  fa.K1g = round_up(fa.koff[1] + round_up(fa.c[1], 16), 64);
   FGNN_CHECK_ARG(fa.c[0] + fa.c[1] <= 512, "too many input channels for the fold kernel");
   fold_weights_kernel<T><<<dim3(G, M.nmlp, 8), 256, 0, st>>>(fa, M.wf, M.bf, M.bt);
   FGNN_LAUNCHED();
-  // the conv-chain kernel reads C entries of every hidden bias that feeds a ReLU: give it zero-padded copies
-  const int depth = M.mp[0]->depth;
-  MlpGroup<T> P = M;
-  fgnn_mlp_params padded[2];
+  // the conv-chain kernel reads C entries of every hidden bias that feeds a ReLU: point it at zero-padded copies
+  const int depth = M.mlp[0].depth;
   if (co_real < C && depth > 2) {
     FGNN_CHECK_ARG(M.bias_pad != nullptr, "zero-padded hidden layers need room for their biases");
     PadBatch pb{};
-    for (int m = 0; m < M.nmlp; ++m) {
-      padded[m] = *M.mp[m];
+    for (int m = 0; m < M.nmlp; ++m)
       for (int l = 1; l < depth - 1; ++l) {
         const int v = m * (depth - 2) + l - 1;
-        pb.src[v] = M.mp[m]->b[l];
-        padded[m].b[l] = M.bias_pad + (size_t)v * C;
+        pb.src[v] = M.mlp[m].b[l];
+        M.mlp[m].b[l] = M.bias_pad + (size_t)v * C;
       }
-      P.mp[m] = &padded[m];
-    }
     pad_vectors_kernel<<<dim3(1, M.nmlp * (depth - 2)), 64, 0, st>>>(pb, M.bias_pad, C, co_real);
     FGNN_LAUNCHED();
   }
-  if (int e = launch_mlp<T>(P, C, G, geo, npg, st)) return e;
-  if (M.no_coef) return FGNN_OK;
+  if (int e = launch_mlp<T>(M, C, G, geo, npg, st)) return e;
+  if (!M.mlp[0].gn) return FGNN_OK;
   if (M.stat_rec) {
     prof::begin(prof::kStats, st);
     stat_records_reduce_kernel<<<G * M.nmlp * C, kStatReduceThreads, 0, st>>>(M.stat_rec, M.stat_acc, G, M.nmlp, C,
@@ -2056,11 +2059,11 @@ int run_mlp_group(const MlpGroup<T>& M, int C, int G, const Geo& geo, const int3
   ca.n_per_graph = npg;
   for (int m = 0; m < M.nmlp; ++m) {
     ca.coef[m] = M.coef[m];
-    ca.gw[m] = M.mp[m]->gn_w;
-    ca.gb[m] = M.mp[m]->gn_b;
-    ca.eps[m] = M.mp[m]->eps;
-    ca.constant_n[m] = M.mp[m]->constant_n;
-    ca.co_real[m] = M.mp[m]->c_out;
+    ca.gw[m] = M.mlp[m].gn->gn_w;
+    ca.gb[m] = M.mlp[m].gn->gn_b;
+    ca.eps[m] = M.mlp[m].gn->eps;
+    ca.constant_n[m] = M.mlp[m].gn->constant_n;
+    ca.co_real[m] = M.mlp[m].co_real;
     ca.gnstat[m] = M.gnstat[m];
   }
   const int total = G * M.nmlp * C;
@@ -2226,9 +2229,7 @@ int embed_fwd_t(const fgnn_embed_params& p, bool det, const float* x, const uint
       zero_inserted_rows_kernel<T><<<grid, 256, 0, st>>>(reinterpret_cast<T*>(B.y2), geo, kLayoutB);
       FGNN_LAUNCHED();
     }
-    const T* cur = reinterpret_cast<const T*>(B.xin);
-    int cur_c = pl.cin0, cur_real = pl.cin0;
-    const float* cur_coef = nullptr;
+    Src<T> cur{reinterpret_cast<const T*>(B.xin), pl.cin0, pl.cin0, nullptr};
     T* nxt = reinterpret_cast<T*>(B.xa);
     float* nxt_coef = B.coef3a;
     T* y1 = reinterpret_cast<T*>(B.y1);
@@ -2243,8 +2244,8 @@ int embed_fwd_t(const fgnn_embed_params& p, bool det, const float* x, const uint
       {
         MlpGroup<T> M{};
         M.nmlp = 2;
-        M.mp[0] = &bp.mlp1; M.mp[1] = &bp.mlp2;
-        M.src[0] = cur; M.c_src[0] = cur_c; M.cr_src[0] = cur_real; M.src_coef[0] = cur_coef; M.nsrc = 1;
+        M.mlp[0] = chain(bp.mlp1); M.mlp[1] = chain(bp.mlp2);
+        M.src[0] = cur; M.nsrc = 1;
         M.wf = reinterpret_cast<T*>(B.wf12); M.bf = B.bf12; M.bt = reinterpret_cast<T*>(B.bt12);
         M.wh = whb;
         M.bias_pad = static_cast<float*>(B.wf3);
@@ -2258,9 +2259,8 @@ int embed_fwd_t(const fgnn_embed_params& p, bool det, const float* x, const uint
       {
         MlpGroup<T> M{};
         M.nmlp = 1;
-        M.mp[0] = &bp.mlp3;
-        M.src[0] = mult; M.c_src[0] = C; M.cr_src[0] = co; M.src_coef[0] = nullptr;
-        M.src[1] = cur; M.c_src[1] = cur_c; M.cr_src[1] = cur_real; M.src_coef[1] = cur_coef; M.nsrc = 2;
+        M.mlp[0] = chain(bp.mlp3);
+        M.src[0] = Src<T>{mult, C, co, nullptr}; M.src[1] = cur; M.nsrc = 2;
         M.wf = reinterpret_cast<T*>(B.wf3); M.bf = B.bf3; M.bt = reinterpret_cast<T*>(B.bt3);
         M.wh = whb + (size_t)2 * dm1 * C * Kh;
         M.bias_pad = static_cast<float*>(B.wf12);
@@ -2274,16 +2274,13 @@ int embed_fwd_t(const fgnn_embed_params& p, bool det, const float* x, const uint
         }
         if (int e = run_mlp_group<T>(M, C, gc, geo, n_c, st)) return e;
       }
-      cur = nxt;
-      cur_c = C;
-      cur_real = co;
-      cur_coef = nxt_coef;
+      cur = Src<T>{nxt, C, co, nxt_coef};
       nxt = (nxt == reinterpret_cast<T*>(B.xa)) ? reinterpret_cast<T*>(B.xb) : reinterpret_cast<T*>(B.xa);
       nxt_coef = (nxt_coef == B.coef3a) ? B.coef3b : B.coef3a;
     }
     const long rows = (long)gc * C * N;
-    pool_finalize_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(B.rowenc, cur_coef, emb + (size_t)g0 * cur_real * N, C,
-                                                                       cur_real, N, rows, n_c);
+    pool_finalize_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(B.rowenc, cur.coef, emb + (size_t)g0 * cur.c_real * N, C,
+                                                                       cur.c_real, N, rows, n_c);
     FGNN_LAUNCHED();
   }
   return FGNN_OK;
@@ -2497,8 +2494,8 @@ int debug_mlp_t(const fgnn_mlp_params& mp, const float* x, float* y, int G, int 
   }
   MlpGroup<T> M{};
   M.nmlp = 1;
-  M.mp[0] = &mp;
-  M.src[0] = xin; M.c_src[0] = M.cr_src[0] = mp.c_in; M.src_coef[0] = nullptr; M.nsrc = 1;
+  M.mlp[0] = chain(mp);
+  M.src[0] = Src<T>{xin, mp.c_in, mp.c_in, nullptr}; M.nsrc = 1;
   M.wf = wf; M.bf = bf; M.bt = bt; M.wh = wh;
   M.out[0] = out; M.out_mode[0] = kLayoutC; M.ones[0] = 0; M.coef[0] = coef;
   M.stat_acc = acc;

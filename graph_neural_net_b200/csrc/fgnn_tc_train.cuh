@@ -1169,79 +1169,30 @@ int zero_pass(const TrainPlan& tp, const TrainBuf& B, void* ws, bool ragged, cud
   return FGNN_OK;
 }
 
-// one 1x1-conv layer (or two sharing their input) as a depth-1 launch of the conv-chain kernel.  The weights have their
-// real shape (co_real, cr_src0 + cr_src1); co_real = 0 and cr_src = 0 mean the stored C and c_src (weights padded here).
+// a depth-1 launch of the conv-chain kernel on the training scratch, as every 1x1 conv of training is: one MLP, one
+// source, outputs in layout C until the caller sets otherwise
 template <typename T>
-struct ConvCall {
-  int nmlp = 1;
-  const float* w[2] = {nullptr, nullptr};     // (co_real, cr_src0 + cr_src1) fp32
-  const float* b[2] = {nullptr, nullptr};     // (co_real) or null
-  const T* src[2] = {nullptr, nullptr};
-  int c_src[2] = {0, 0};
-  int cr_src[2] = {0, 0};
-  int co_real = 0;
-  const float* src_coef[2] = {nullptr, nullptr};
-  int nsrc = 1;
-  T* out[2] = {nullptr, nullptr};
-  Layout out_mode[2] = {kLayoutC, kLayoutC};
-  int ones[2] = {0, 0};
-  int relu = 0;
-  const fgnn_mlp_params* gn[2] = {nullptr, nullptr};   // GraphNorm of the output (last layer): coefficients + statistics
-  float* coef[2] = {nullptr, nullptr};
-  float* gnstat[2] = {nullptr, nullptr};
-};
-
-template <typename T>
-int run_conv(const ConvCall<T>& cc, const TrainPlan& tp, const TrainBuf& B, const int32_t* npg, cudaStream_t st) {
-  fgnn_mlp_params tmp[2];
+MlpGroup<T> conv_group(const TrainBuf& B) {
   MlpGroup<T> M{};
-  M.nmlp = cc.nmlp;
-  M.nsrc = cc.nsrc;
-  for (int s = 0; s < 2; ++s) {
-    M.src[s] = cc.src[s];
-    M.c_src[s] = cc.c_src[s];
-    M.cr_src[s] = cc.cr_src[s] ? cc.cr_src[s] : cc.c_src[s];
-    M.src_coef[s] = cc.src_coef[s];
-  }
-  for (int m = 0; m < cc.nmlp; ++m) {
-    memset(&tmp[m], 0, sizeof(tmp[m]));
-    tmp[m].c_in = M.cr_src[0] + (cc.nsrc > 1 ? M.cr_src[1] : 0);
-    tmp[m].c_out = cc.co_real ? cc.co_real : tp.C;
-    tmp[m].depth = 1;
-    tmp[m].w[0] = cc.w[m];
-    tmp[m].b[0] = cc.b[m] ? cc.b[m] : B.zeros;
-    if (cc.gn[m]) {
-      tmp[m].gn_w = cc.gn[m]->gn_w;
-      tmp[m].gn_b = cc.gn[m]->gn_b;
-      tmp[m].eps = cc.gn[m]->eps;
-      tmp[m].constant_n = cc.gn[m]->constant_n;
-    }
-    M.mp[m] = &tmp[m];
-    M.out[m] = cc.out[m];
-    M.out_mode[m] = cc.out_mode[m];
-    M.ones[m] = cc.ones[m];
-    M.coef[m] = cc.coef[m];
-    M.gnstat[m] = cc.gnstat[m];
-  }
+  M.nmlp = M.nsrc = 1;
   M.wf = reinterpret_cast<T*>(B.wf);
   M.bf = B.bf;
-  M.wh = nullptr;
   M.stat_acc = B.stat_acc;
   M.stat_rec = B.stat_rec;
-  M.relu_out = cc.relu;
-  M.no_coef = cc.gn[0] == nullptr;
-  return run_mlp_group<T>(M, tp.C, tp.G, tp.geo, npg, st);
+  return M;
 }
+
+// layer l of mp as a depth-1 launch (a missing bias reads as zeros); its last layer finalises mp's GraphNorm
+MlpLayers layer(const fgnn_mlp_params& mp, int l, const float* zeros) {
+  return {mp.w[l], {mp.b[l] ? mp.b[l] : zeros}, 1, mp.c_out, l == mp.depth - 1 ? &mp : nullptr};
+}
+
+// a data-gradient conv: wt is a transposed weight zero-padded by transpose_slice_kernel to (C, C per source); no bias, no GraphNorm
+MlpLayers transposed(const float* wt, const TrainBuf& B, int C) { return {wt, {B.zeros}, 1, C, nullptr}; }
 
 // input of block b: the input planes xin for b = 0, else the previous block's pre-norm output and its GraphNorm fold
 template <typename T>
-struct BlockIn {
-  const T* x;
-  int c, c_real;
-  const float* coef;
-};
-template <typename T>
-BlockIn<T> block_in(const fgnn_embed_params& p, const TrainPlan& tp, const TrainBuf& B, int b) {
+Src<T> block_in(const fgnn_embed_params& p, const TrainPlan& tp, const TrainBuf& B, int b) {
   if (b == 0) return {reinterpret_cast<const T*>(B.xin), tp.cin0, tp.cin0, nullptr};
   return {reinterpret_cast<const T*>(B.Z3[b - 1]), tp.C, p.block[b - 1].mlp3.c_out, B.coef[b - 1][2]};
 }
@@ -1254,63 +1205,43 @@ int train_fwd_block(const fgnn_embed_params& p, const TrainPlan& tp, const Train
                     const int32_t* npg, cudaStream_t st) {
   const Geo& geo = tp.geo;
   const int G = tp.G, C = tp.C, D = tp.D;
-  const BlockIn<T> in = block_in<T>(p, tp, B, b);
-  const T* cur = in.x;
-  const int cur_c = in.c, cur_real = in.c_real;
-  const float* cur_coef = in.coef;
+  const Src<T> in = block_in<T>(p, tp, B, b);
   const fgnn_block_params& bp = p.block[b];
   const int co = bp.mlp1.c_out;
-  const fgnn_mlp_params* mlps[3] = {&bp.mlp1, &bp.mlp2, &bp.mlp3};
+  const fgnn_mlp_params* mlps[2] = {&bp.mlp1, &bp.mlp2};
   T* y12[2] = {reinterpret_cast<T*>(B.Y1[b]), reinterpret_cast<T*>(B.Y2[b])};
   const Layout mode12[2] = {kLayoutA, kLayoutB};
   for (int l = 0; l < D; ++l) {
     const bool last = l == D - 1;
-    if (l == 0) {   // mlp1 and mlp2 share the block input: one launch
-      ConvCall<T> cc;
-      cc.nmlp = 2;
-      cc.src[0] = cur; cc.c_src[0] = cur_c; cc.cr_src[0] = cur_real; cc.src_coef[0] = cur_coef; cc.nsrc = 1;
-      cc.co_real = co;
-      for (int m = 0; m < 2; ++m) {
-        cc.w[m] = mlps[m]->w[0]; cc.b[m] = mlps[m]->b[0];
-        cc.out[m] = last ? y12[m] : reinterpret_cast<T*>(B.H[b][m][0]);
-        cc.out_mode[m] = last ? mode12[m] : kLayoutC;
-        cc.ones[m] = last ? 1 : 0;
-        if (last) { cc.gn[m] = mlps[m]; cc.coef[m] = B.coef[b][m]; cc.gnstat[m] = B.gnstat[b][m]; }
+    const int nmlp = l == 0 ? 2 : 1;   // mlp1 and mlp2 share the block input: one launch of their first layers
+    for (int m0 = 0; m0 < 2; m0 += nmlp) {
+      MlpGroup<T> M = conv_group<T>(B);
+      M.nmlp = nmlp;
+      M.src[0] = l == 0 ? in : Src<T>{reinterpret_cast<const T*>(B.H[b][m0][l - 1]), C, co, nullptr};
+      for (int j = 0; j < nmlp; ++j) {
+        const int m = m0 + j;
+        M.mlp[j] = layer(*mlps[m], l, B.zeros);
+        M.out[j] = last ? y12[m] : reinterpret_cast<T*>(B.H[b][m][l]);
+        M.out_mode[j] = last ? mode12[m] : kLayoutC;
+        M.ones[j] = last ? 1 : 0;
+        if (last) { M.coef[j] = B.coef[b][m]; M.gnstat[j] = B.gnstat[b][m]; }
       }
-      cc.relu = last ? 0 : 1;
-      if (int e = run_conv<T>(cc, tp, B, npg, st)) return e;
-    } else {
-      for (int m = 0; m < 2; ++m) {
-        ConvCall<T> cc;
-        cc.src[0] = reinterpret_cast<const T*>(B.H[b][m][l - 1]); cc.c_src[0] = C; cc.cr_src[0] = co;
-        cc.co_real = co;
-        cc.w[0] = mlps[m]->w[l]; cc.b[0] = mlps[m]->b[l];
-        cc.out[0] = last ? y12[m] : reinterpret_cast<T*>(B.H[b][m][l]);
-        cc.out_mode[0] = last ? mode12[m] : kLayoutC;
-        cc.ones[0] = last ? 1 : 0;
-        if (last) { cc.gn[0] = mlps[m]; cc.coef[0] = B.coef[b][m]; cc.gnstat[0] = B.gnstat[b][m]; }
-        cc.relu = last ? 0 : 1;
-        if (int e = run_conv<T>(cc, tp, B, npg, st)) return e;
-      }
+      M.relu_out = !last;
+      if (int e = run_mlp_group<T>(M, C, G, geo, npg, st)) return e;
     }
   }
   T* mult = reinterpret_cast<T*>(B.MULT[b]);
   if (int e = launch_matmul<T>(y12[0], y12[1], mult, B.coef[b][0], B.coef[b][1], G, C, geo, npg, st)) return e;
   for (int l = 0; l < (z3 ? D : D - 1); ++l) {
     const bool last = l == D - 1;
-    ConvCall<T> cc;
-    if (l == 0) {
-      cc.src[0] = mult; cc.c_src[0] = C; cc.cr_src[0] = co; cc.src_coef[0] = nullptr;
-      cc.src[1] = cur; cc.c_src[1] = cur_c; cc.cr_src[1] = cur_real; cc.src_coef[1] = cur_coef; cc.nsrc = 2;
-    } else {
-      cc.src[0] = reinterpret_cast<const T*>(B.H[b][2][l - 1]); cc.c_src[0] = C; cc.cr_src[0] = co;
-    }
-    cc.co_real = co;
-    cc.w[0] = mlps[2]->w[l]; cc.b[0] = mlps[2]->b[l];
-    cc.out[0] = last ? reinterpret_cast<T*>(B.Z3[b]) : reinterpret_cast<T*>(B.H[b][2][l]);
-    if (last) { cc.gn[0] = mlps[2]; cc.coef[0] = B.coef[b][2]; cc.gnstat[0] = B.gnstat[b][2]; }
-    cc.relu = last ? 0 : 1;
-    if (int e = run_conv<T>(cc, tp, B, npg, st)) return e;
+    MlpGroup<T> M = conv_group<T>(B);
+    M.src[0] = Src<T>{l == 0 ? mult : reinterpret_cast<const T*>(B.H[b][2][l - 1]), C, co, nullptr};
+    if (l == 0) { M.src[1] = in; M.nsrc = 2; }
+    M.mlp[0] = layer(bp.mlp3, l, B.zeros);
+    M.out[0] = reinterpret_cast<T*>(last ? B.Z3[b] : B.H[b][2][l]);
+    if (last) { M.coef[0] = B.coef[b][2]; M.gnstat[0] = B.gnstat[b][2]; }
+    M.relu_out = !last;
+    if (int e = run_mlp_group<T>(M, C, G, geo, npg, st)) return e;
   }
   return FGNN_OK;
 }
@@ -1324,7 +1255,7 @@ int train_fwd_pass(const fgnn_embed_params& p, const TrainPlan& tp, const TrainB
   for (int b = 0; b < tp.nb; ++b)
     if (int e = train_fwd_block<T>(p, tp, B, b, true, npg, st)) return e;
   {
-    const BlockIn<T> out = block_in<T>(p, tp, B, tp.nb);
+    const Src<T> out = block_in<T>(p, tp, B, tp.nb);
     dim3 grid((unsigned)((geo.N + 7) / 8), tp.G * tp.C);
     colmax16_kernel<T><<<grid, 256, 0, st>>>(out.x, out.coef, emb, B.arg, tp.C, out.c_real, geo, npg);
     FGNN_LAUNCHED();
@@ -1374,10 +1305,7 @@ struct MlpBwd {
   const float* gnstat;
   void* const* H;               // hidden activations h_0 .. h_{D-2} (layout C)
   int co_real;                  // real output channels (mp's c_out)
-  const T* src[2];
-  int c_src[2];                 // channels of the source planes as stored
-  int cr_src[2];                // of which real
-  const float* src_coef[2];
+  Src<T> src[2];
   int nsrc;
   T* bufs[2];
 };
@@ -1429,11 +1357,11 @@ int mlp_bwd(const MlpBwd<T>& a, const TrainPlan& tp, const TrainBuf& B, const in
     transpose_slice_kernel<<<ceil_div(C * C, 256), 256, 0, st>>>(a.mp->w[l], B.wt[0], C, a.co_real, a.co_real, 0, C, a.co_real, C, 0);
     FGNN_LAUNCHED();
     T* nxt = (curg == a.bufs[0]) ? a.bufs[1] : a.bufs[0];
-    ConvCall<T> cc;
-    cc.src[0] = curg; cc.c_src[0] = C;
-    cc.w[0] = B.wt[0];
-    cc.out[0] = nxt;
-    if (int e = run_conv<T>(cc, tp, B, npg, st)) return e;
+    MlpGroup<T> M = conv_group<T>(B);
+    M.src[0] = Src<T>{curg, C, C, nullptr};
+    M.mlp[0] = transposed(B.wt[0], B, C);
+    M.out[0] = nxt;
+    if (int e = run_mlp_group<T>(M, C, G, geo, npg, st)) return e;
     bi ^= 1;
     if (int e = bsum_begin(bi)) return e;
     prof::begin(prof::kStats, st);
@@ -1446,20 +1374,15 @@ int mlp_bwd(const MlpBwd<T>& a, const TrainPlan& tp, const TrainBuf& B, const in
   }
   // first layer: per-graph pixel GEMM, combined through the per-graph GraphNorm fold of the sources
   {
-    const int k0 = round_up(a.c_src[0], 16), k1 = a.nsrc > 1 ? round_up(a.c_src[1], 16) : 0;
+    const int k0 = round_up(a.src[0].c, 16), k1 = a.nsrc > 1 ? round_up(a.src[1].c, 16) : 0;
     const int Nw = k0 + k1;
     if (!det) FGNN_CUDA(cudaMemsetAsync(B.P, 0, (size_t)G * C * Nw * sizeof(float), st));
-    if (int e = launch_wgrad<T>(curg, C, a.src[0], a.c_src[0], a.nsrc > 1 ? a.src[1] : nullptr, a.c_src[1], B.P, (long)C * Nw, G, geo,
-                                npg, B.wg_rec, st)) return e;
+    if (int e = launch_wgrad<T>(curg, C, a.src[0].x, a.src[0].c, a.nsrc > 1 ? a.src[1].x : nullptr, a.src[1].c, B.P, (long)C * Nw, G,
+                                geo, npg, B.wg_rec, st)) return e;
     CombineFirstArgs ca{};
     ca.P = B.P;
     ca.bsum = B.bsum[bi];
-    ca.coef[0] = a.src_coef[0];
-    ca.coef[1] = a.nsrc > 1 ? a.src_coef[1] : nullptr;
-    ca.c[0] = a.c_src[0];
-    ca.c[1] = a.nsrc > 1 ? a.c_src[1] : 0;
-    ca.cr[0] = a.cr_src[0];
-    ca.cr[1] = a.nsrc > 1 ? a.cr_src[1] : 0;
+    for (int s = 0; s < a.nsrc; ++s) { ca.coef[s] = a.src[s].coef; ca.c[s] = a.src[s].c; ca.cr[s] = a.src[s].c_real; }
     ca.koff[0] = 0;
     ca.koff[1] = k0;
     ca.nsrc = a.nsrc;
@@ -1501,11 +1424,8 @@ int train_bwd_pass(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const
       if (int e = train_fwd_block<T>(p, tp, B, b, false, npg, st)) return e;
     const fgnn_block_params& bp = p.block[b];
     const fgnn_block_grads& bg = gr.block[b];
-    const BlockIn<T> in = block_in<T>(p, tp, B, b);
-    const T* cur = in.x;
-    const int cur_c = in.c, cur_real = in.c_real;
+    const Src<T> in = block_in<T>(p, tp, B, b);
     const int co = bp.mlp1.c_out;
-    const float* cur_coef = in.coef;
     T* A[2] = {reinterpret_cast<T*>(B.A0), reinterpret_cast<T*>(B.A1)};
     T* Bb[2] = {reinterpret_cast<T*>(B.B0), reinterpret_cast<T*>(B.B1)};
     T* DM = reinterpret_cast<T*>(B.DM);
@@ -1521,26 +1441,25 @@ int train_bwd_pass(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const
       a.coef = B.coef[b][2]; a.gnstat = B.gnstat[b][2];
       a.H = B.H[b][2];
       a.co_real = co;
-      a.src[0] = reinterpret_cast<const T*>(B.MULT[b]); a.c_src[0] = C; a.cr_src[0] = co; a.src_coef[0] = nullptr;
-      a.src[1] = cur; a.c_src[1] = cur_c; a.cr_src[1] = cur_real; a.src_coef[1] = cur_coef; a.nsrc = 2;
+      a.src[0] = Src<T>{reinterpret_cast<const T*>(B.MULT[b]), C, co, nullptr}; a.src[1] = in; a.nsrc = 2;
       a.bufs[0] = A[0]; a.bufs[1] = A[1];
       if (int e = mlp_bwd<T>(a, tp, B, npg, st, &g3)) return e;
       // data gradients of the two sources: d mult = W0[:, :co]^T g, d cur = W0[:, co:]^T g (not needed for the raw input)
-      const int cin = co + cur_real;
+      const int cin = co + in.c_real;
       transpose_slice_kernel<<<ceil_div(C * C, 256), 256, 0, st>>>(bp.mlp3.w[0], B.wt[0], C, co, cin, 0, C, co, C, 0);
       FGNN_LAUNCHED();
-      ConvCall<T> cc;
-      cc.src[0] = g3; cc.c_src[0] = C;
-      cc.w[0] = B.wt[0];
-      cc.out[0] = DM;
+      MlpGroup<T> M = conv_group<T>(B);
+      M.src[0] = Src<T>{g3, C, C, nullptr};
+      M.mlp[0] = transposed(B.wt[0], B, C);
+      M.out[0] = DM;
       if (b > 0) {
-        transpose_slice_kernel<<<ceil_div(C * C, 256), 256, 0, st>>>(bp.mlp3.w[0], B.wt[1], C, co, cin, co, C, cur_real, C, 0);
+        transpose_slice_kernel<<<ceil_div(C * C, 256), 256, 0, st>>>(bp.mlp3.w[0], B.wt[1], C, co, cin, co, C, in.c_real, C, 0);
         FGNN_LAUNCHED();
-        cc.nmlp = 2;
-        cc.w[1] = B.wt[1];
-        cc.out[1] = dx3;
+        M.nmlp = 2;
+        M.mlp[1] = transposed(B.wt[1], B, C);
+        M.out[1] = dx3;
       }
-      if (int e = run_conv<T>(cc, tp, B, npg, st)) return e;
+      if (int e = run_mlp_group<T>(M, C, G, geo, npg, st)) return e;
     }
     // ---- matmul ----
     {
@@ -1568,24 +1487,24 @@ int train_bwd_pass(const fgnn_embed_params& p, const fgnn_embed_grads& gr, const
       a.coef = B.coef[b][m]; a.gnstat = B.gnstat[b][m];
       a.H = B.H[b][m];
       a.co_real = co;
-      a.src[0] = cur; a.c_src[0] = cur_c; a.cr_src[0] = cur_real; a.src_coef[0] = cur_coef; a.nsrc = 1;
+      a.src[0] = in; a.nsrc = 1;
       a.bufs[0] = m == 0 ? A[0] : Bb[0];
       a.bufs[1] = m == 0 ? A[1] : Bb[1];
       if (int e = mlp_bwd<T>(a, tp, B, npg, st, &g12[m])) return e;
     }
     if (b > 0) {
       // d cur (through mlp1 and mlp2) = [W0_1^T | W0_2^T] [g1; g2]: one two-source conv
-      transpose_slice_kernel<<<ceil_div(C * C, 256), 256, 0, st>>>(bp.mlp1.w[0], B.wt[0], C, co, cur_real, 0, C, cur_real, 2 * C, 0);
+      transpose_slice_kernel<<<ceil_div(C * C, 256), 256, 0, st>>>(bp.mlp1.w[0], B.wt[0], C, co, in.c_real, 0, C, in.c_real, 2 * C, 0);
       FGNN_LAUNCHED();
-      transpose_slice_kernel<<<ceil_div(C * C, 256), 256, 0, st>>>(bp.mlp2.w[0], B.wt[0], C, co, cur_real, 0, C, cur_real, 2 * C, C);
+      transpose_slice_kernel<<<ceil_div(C * C, 256), 256, 0, st>>>(bp.mlp2.w[0], B.wt[0], C, co, in.c_real, 0, C, in.c_real, 2 * C, C);
       FGNN_LAUNCHED();
-      ConvCall<T> cc;
-      cc.src[0] = g12[0]; cc.c_src[0] = C;
-      cc.src[1] = g12[1]; cc.c_src[1] = C;
-      cc.nsrc = 2;
-      cc.w[0] = B.wt[0];
-      cc.out[0] = dx12;
-      if (int e = run_conv<T>(cc, tp, B, npg, st)) return e;
+      MlpGroup<T> M = conv_group<T>(B);
+      M.src[0] = Src<T>{g12[0], C, C, nullptr};
+      M.src[1] = Src<T>{g12[1], C, C, nullptr};
+      M.nsrc = 2;
+      M.mlp[0] = transposed(B.wt[0], B, C);
+      M.out[0] = dx12;
+      if (int e = run_mlp_group<T>(M, C, G, geo, npg, st)) return e;
       dOutA = dx3;
       dOutB = dx12;
     }
